@@ -271,6 +271,31 @@ def timed_e2e(H, ctx, spec, steps, shard, n_windows, dist, local, total_steps):
             "ms_per_step": 1e3 * e2e_s / steps, "estimate_ms": 1e3 * t_est / steps, "gather_ms": 1e3 * t_gat / steps, "device_ms": o.gpu_ms}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, shard, n_windows, dist=None, device=None, limit=DUMP_LIMIT_BYTES):
+    """Writes what the timed path returned in its last step (hmcgpu_plan_fetch: per-window posterior means and variances,
+    per-chain status) as <out_dir>/<name>.npy in float64, windows in caller order, so that two builds can be compared output
+    for output.  window_index.npy holds the windows written: all of them, or, when that would exceed `limit` bytes, a fixed
+    seeded sample.  Every rank calls it (the windows are gathered to rank 0, which writes)."""
+    import hmc_jl_b200 as H
+    F = res.summary_mean.shape[1]
+    rows = np.concatenate([res.summary_mean, res.summary_var, res.status.astype(np.float64)], axis=1)
+    full = H.gather_window_summaries(rows, shard, n_windows, dist, device=device)
+    if full is None:
+        return None
+    row_bytes = (full.shape[1] + 1) * 8                      # + the window index
+    idx = np.arange(n_windows)
+    if n_windows * row_bytes > limit:
+        idx = np.sort(np.random.default_rng(1234).choice(n_windows, limit // row_bytes, replace=False))
+    arrays = {"summary_mean": full[idx, :F], "summary_var": full[idx, F:2 * F], "status": full[idx, 2 * F:], "window_index": idx}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+    return sorted(arrays)
+
+
 def wide_series(n_ser, length, Kw=3, n_gen=2048):
     """C4 / C5 inputs (SURVEY section 8d): independent series from the truth parameters, numpy default_rng(1234); n_gen distinct
     series tiled to n_ser (device work does not depend on the values being distinct)."""
@@ -335,10 +360,19 @@ def workload_config(args, world):
 
 
 def main():
+    def count(least):
+        def parse(s):
+            v = int(s)
+            if v < least:
+                raise argparse.ArgumentTypeError(f"must be at least {least}")
+            return v
+        return parse
+
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=count(1), default=5, help="timed steps")
+    ap.add_argument("--warmup", type=count(0), default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what their last step computed as DIR/<name>.npy")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--chains", type=int, default=256, help="chains per window per GPU")
     ap.add_argument("--states", type=int, default=3, help="K for --workload c5 (K=3: SURVEY truth; otherwise mu_k=2k, sigma2=0.5)")
@@ -352,6 +386,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-records", action="store_true", help="skip the mid-width / fp64 / C4 sub-records of the N=1 line")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     capture_stdout()
     if args.impl == "reference":
         return run_reference(args)
@@ -417,6 +453,10 @@ def main():
     plan = m.pop("plan")
     res = plan.fetch()
     plan.close()
+    if args.dump_outputs:
+        names = dump_outputs(args.dump_outputs, res, shard, len(we_all), dist, device=f"cuda:{local}" if dist is not None else None)
+        if names:
+            print(f"[bench] wrote {', '.join(names)} to {args.dump_outputs}", file=sys.stderr, flush=True)
     value, dev_s, total_steps, steps_per_run = m["value"], m["dev_s"], m["total_steps"], m["steps_per_run"]
     sweep_ms, dev_ms, sweep_launches = m["sweep_ms"], m["dev_ms"], m["sweep_launches"]
     kernel_name = H.binding.KERNEL_NAMES.get(m["kernel"], str(m["kernel"]))

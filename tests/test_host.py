@@ -427,6 +427,38 @@ def test_bench_issue_roofline_arithmetic():
     assert abs(r["measured_mixed_peak"] - want) < 1e-6 * want and r["frac_of_measured_mixed_peak"] > r["frac"]
 
 
+def test_bench_dump_outputs_layout_and_sampling(H, tmp_path):
+    """bench.dump_outputs writes the fetched per-window outputs in caller window order as float64 .npy files, and a fixed
+    seeded sample of the windows when the whole set would exceed the size limit."""
+    import importlib.util
+    from types import SimpleNamespace
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    nw, F, chains = 50, 7, 3
+    shard = np.random.default_rng(0).permutation(nw)
+    res = SimpleNamespace(summary_mean=shard[:, None] + np.arange(F) / 10.0, summary_var=-shard[:, None] - np.arange(F) / 10.0,
+                          status=np.tile(shard[:, None] % 2, (1, chains)).astype(np.int32))
+    names = b.dump_outputs(str(tmp_path / "all"), res, shard, nw)
+    assert names == ["status", "summary_mean", "summary_var", "window_index"]
+    got = {n: np.load(tmp_path / "all" / f"{n}.npy") for n in names}
+    assert all(a.dtype == np.float64 for a in got.values())
+    np.testing.assert_array_equal(got["window_index"], np.arange(nw))
+    np.testing.assert_array_equal(got["summary_mean"], np.arange(nw)[:, None] + np.arange(F) / 10.0)
+    np.testing.assert_array_equal(got["summary_var"], -np.arange(nw)[:, None] - np.arange(F) / 10.0)
+    np.testing.assert_array_equal(got["status"], np.tile(np.arange(nw)[:, None] % 2, (1, chains)))
+    limit = 20 * (2 * F + chains + 1) * 8
+    for d in ("s1", "s2"):
+        b.dump_outputs(str(tmp_path / d), res, shard, nw, limit=limit)
+    s1 = {n: np.load(tmp_path / "s1" / f"{n}.npy") for n in names}
+    assert sum(a.nbytes for a in s1.values()) <= limit and len(s1["window_index"]) == 20
+    idx = s1["window_index"].astype(np.int64)
+    assert np.all(np.diff(idx) > 0) and idx.max() < nw
+    np.testing.assert_array_equal(s1["summary_mean"], got["summary_mean"][idx])
+    for n in names:                                                                      # the same sample every time
+        np.testing.assert_array_equal(np.load(tmp_path / "s2" / f"{n}.npy"), s1[n])
+
+
 def test_bench_reference_arm_prints_one_contract_line():
     """`bench.py --impl reference` (the CPU port on the host cores; no GPU involved): exactly one JSON line on stdout with
     the contract's keys, whatever the libraries print."""
