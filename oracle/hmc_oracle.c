@@ -50,9 +50,14 @@ void orc_normal_pair(const uint32_t w[4], double* z0, double* z1) {
     if (z1) *z1 = r * sin(th);
 }
 
+/* *m = min(*m, d): the margin outputs of orc_result (NULL: not tracked) */
+static void shrink(double* m, double d) { if (m && d < *m) *m = d; }
+
 /* Marsaglia & Tsang (2000) for shape >= 1; shape < 1 boosted by U^(1/shape).  Attempt k uses block k:
- * words 0,1 -> normal (cos branch), word 2 -> acceptance uniform, word 3 -> boost uniform. */
-double orc_gamma(double shape, uint64_t seed, uint32_t chain, uint32_t sweep, uint32_t purpose) {
+ * words 0,1 -> normal (cos branch), word 2 -> acceptance uniform, word 3 -> boost uniform.
+ * margin (may be NULL): lowered to the distance of every comparison made from its threshold — |v| for v <= 0, |u - s| for the
+ * squeeze u < s, and |log u - r| / max(1, d) for the log test (its rounding error in a lower precision grows with d). */
+static double gamma_m(double shape, uint64_t seed, uint32_t chain, uint32_t sweep, uint32_t purpose, double* margin) {
     double a = shape < 1.0 ? shape + 1.0 : shape;
     double d = a - 1.0 / 3.0, c = 1.0 / sqrt(9.0 * d);
     for (uint32_t k = 0;; ++k) {
@@ -60,17 +65,30 @@ double orc_gamma(double shape, uint64_t seed, uint32_t chain, uint32_t sweep, ui
         orc_block(seed, chain, sweep, purpose, k, w);
         double z; orc_normal_pair(w, &z, NULL);
         double v = 1.0 + c * z;
+        shrink(margin, fabs(v));
         if (v <= 0.0) continue;
         v = v * v * v;
         double u = orc_u01(w[2]);
         double z2 = z * z;
-        if (u < 1.0 - 0.0331 * z2 * z2 || log(u) < 0.5 * z2 + d * (1.0 - v + log(v))) {
+        double sq = 1.0 - 0.0331 * z2 * z2;
+        shrink(margin, fabs(u - sq));
+        int accept = u < sq;
+        if (!accept) {
+            double lu = log(u), r = 0.5 * z2 + d * (1.0 - v + log(v));
+            shrink(margin, fabs(lu - r) / (d > 1.0 ? d : 1.0));
+            accept = lu < r;
+        }
+        if (accept) {
             double g = d * v;
             if (shape < 1.0) g *= pow(orc_u01(w[3]), 1.0 / shape);
             return g;
         }
         if (k > 1000000u) return d; /* unreachable in practice */
     }
+}
+
+double orc_gamma(double shape, uint64_t seed, uint32_t chain, uint32_t sweep, uint32_t purpose) {
+    return gamma_m(shape, seed, chain, sweep, purpose, NULL);
 }
 
 /* ---------------------------------------------------------------- initial state and priors */
@@ -209,11 +227,20 @@ static int64_t categorical(const double* p, int K, double u) {
     return i + 1;
 }
 
+/* distance of u from the nearest of the K - 1 cumulative boundaries categorical() may compare it with */
+static double categorical_margin(const double* p, int K, double u) {
+    double c = 0.0, m = INFINITY;
+    for (int j = 0; j < K - 1; ++j) { c += p[j]; if (fabs(u - c) < m) m = fabs(u - c); }
+    return m;
+}
+
 /* src/Hmc.jl:459-484 */
-void orc_sample_states(int N, int K, const double* Pf, const double* pif, const double* A,
-                       const double* piN, const double* u, int form, int64_t* X) {
+/* margin (may be NULL): lowered to the categorical_margin of every draw */
+static void sample_states_m(int N, int K, const double* Pf, const double* pif, const double* A,
+                            const double* piN, const double* u, int form, int64_t* X, double* margin) {
     double p[MAXK];
     X[N - 1] = categorical(piN, K, u[N - 1]);                   /* :464 */
+    if (margin) shrink(margin, categorical_margin(piN, K, u[N - 1]));
     for (int k = N - 2; k >= 0; --k) {
         int x = (int)X[k + 1] - 1;
         double total = 0.0;
@@ -227,7 +254,13 @@ void orc_sample_states(int N, int K, const double* Pf, const double* pif, const 
         if (gate > EPS64 && total > 0.0) for (int j = 0; j < K; ++j) p[j] /= total;
         else for (int j = 0; j < K; ++j) p[j] = 1.0 / K;
         X[k] = categorical(p, K, u[k]);
+        if (margin) shrink(margin, categorical_margin(p, K, u[k]));
     }
+}
+
+void orc_sample_states(int N, int K, const double* Pf, const double* pif, const double* A,
+                       const double* piN, const double* u, int form, int64_t* X) {
+    sample_states_m(N, K, Pf, pif, A, piN, u, form, X, NULL);
 }
 
 static void matmul(int K, const double* a, const double* b, double* c) {
@@ -265,11 +298,12 @@ void orc_forecast(int K, const double* mu, const double* A, const double* pib, i
 }
 
 /* src/Hmc.jl:302-335 (sigma2, mu), :350-356 (rho), :358-369 (A) given the sufficient statistics */
-void orc_draw_params(int K, const int64_t* Ni, const int64_t* Mi, const double* S, const double* Sm,
-                     const double* S2, const double* Sm2, const int64_t* trans,
-                     const double* xi, const double* alpha, const double* nu, const double* beta, double kappa,
-                     uint64_t seed, uint32_t chain, uint32_t sweep,
-                     double* sigma2, double* mu, double* rho, double* A) {
+/* margin (may be NULL): lowered by every gamma draw (gamma_m) */
+static void draw_params_m(int K, const int64_t* Ni, const int64_t* Mi, const double* S, const double* Sm,
+                          const double* S2, const double* Sm2, const int64_t* trans,
+                          const double* xi, const double* alpha, const double* nu, const double* beta, double kappa,
+                          uint64_t seed, uint32_t chain, uint32_t sweep,
+                          double* sigma2, double* mu, double* rho, double* A, double* margin) {
     double Neff[MAXK], g[MAXK];
     for (int i = 0; i < K; ++i) {
         double mi = Mi ? (double)Mi[i] : 0.0, sm = Sm ? Sm[i] : 0.0, sm2 = Sm2 ? Sm2[i] : 0.0;
@@ -282,7 +316,7 @@ void orc_draw_params(int K, const int64_t* Ni, const int64_t* Mi, const double* 
         double b = beta[i] + 0.5 * S2[i] + (0.5 / (1.0 + kappa)) * sm2
                  + 0.5 * Neff[i] * nu[i] / (Neff[i] + nu[i]) * (dev * dev);       /* :314 */
         if (a > 0.0 && b > 0.0) {
-            double gm = orc_gamma(a, seed, chain, sweep, (ORC_KIND_SIGMA << 16) | (uint32_t)i);
+            double gm = gamma_m(a, seed, chain, sweep, (ORC_KIND_SIGMA << 16) | (uint32_t)i, margin);
             sigma2[i] = b / gm;                                                   /* :320 InverseGamma(a,b) */
         } /* else: reference's catch keeps the old value (:321-329) */
     }
@@ -299,16 +333,24 @@ void orc_draw_params(int K, const int64_t* Ni, const int64_t* Mi, const double* 
         mu[i] = m + s * z0;                                                       /* :334 */
     }
     double tot = 0.0;                                                              /* :354-355 Dirichlet(1..1) */
-    for (int i = 0; i < K; ++i) { g[i] = orc_gamma(1.0, seed, chain, sweep, (ORC_KIND_RHO << 16) | (uint32_t)i); tot += g[i]; }
+    for (int i = 0; i < K; ++i) { g[i] = gamma_m(1.0, seed, chain, sweep, (ORC_KIND_RHO << 16) | (uint32_t)i, margin); tot += g[i]; }
     for (int i = 0; i < K; ++i) rho[i] = g[i] / tot;
     for (int i = 0; i < K; ++i) {                                                  /* :366-368 */
         tot = 0.0;
         for (int j = 0; j < K; ++j) {
-            g[j] = orc_gamma((double)trans[i * K + j], seed, chain, sweep, (ORC_KIND_A << 16) | (uint32_t)(i * K + j));
+            g[j] = gamma_m((double)trans[i * K + j], seed, chain, sweep, (ORC_KIND_A << 16) | (uint32_t)(i * K + j), margin);
             tot += g[j];
         }
         for (int j = 0; j < K; ++j) A[i * K + j] = g[j] / tot;
     }
+}
+
+void orc_draw_params(int K, const int64_t* Ni, const int64_t* Mi, const double* S, const double* Sm,
+                     const double* S2, const double* Sm2, const int64_t* trans,
+                     const double* xi, const double* alpha, const double* nu, const double* beta, double kappa,
+                     uint64_t seed, uint32_t chain, uint32_t sweep,
+                     double* sigma2, double* mu, double* rho, double* A) {
+    draw_params_m(K, Ni, Mi, S, Sm, S2, Sm2, trans, xi, alpha, nu, beta, kappa, seed, chain, sweep, sigma2, mu, rho, A, NULL);
 }
 
 /* ---------------------------------------------------------------- the sampler */
@@ -364,8 +406,10 @@ int orc_gibbs(const orc_problem* p, orc_result* res) {
         for (size_t j = 0; j < KK; ++j) trans[j] = 1;
         for (int t = 0; t + 1 < N; ++t) trans[((int)X[t] - 1) * K + ((int)X[t + 1] - 1)] += 1;
         /* --- draws: σ², μ (β of this sweep), then β .= 2 (:347), ρ, A */
-        orc_draw_params(K, Ni, Mi, S, Sm, S2, Sm2, trans, xi, alpha, nu, beta, p->kappa,
-                        p->seed, p->chain, sweep, sigma2, mu, rho, A);
+        double* gmargin = res->gamma_margin ? res->gamma_margin + sw : NULL;
+        if (gmargin) *gmargin = INFINITY;
+        draw_params_m(K, Ni, Mi, S, Sm, S2, Sm2, trans, xi, alpha, nu, beta, p->kappa,
+                      p->seed, p->chain, sweep, sigma2, mu, rho, A, gmargin);
         memcpy(beta, beta_after, sizeof(double) * (size_t)K);
         /* --- forward / backward (:498-499) */
         double ll;
@@ -413,7 +457,9 @@ int orc_gibbs(const orc_problem* p, orc_result* res) {
             for (int j = 0; j < 4 && i + j < N; ++j) u[N - 1 - (i + j)] = orc_u01(w[j]);
         }
         /* chain-label A for the pif form (Atmp is the un-permuted matrix) */
-        orc_sample_states(N, K, Pf, pif, Atmp, piN, u, (p->flags & ORC_FLAG_PIF_FORM) ? 1 : 0, X);
+        double* smargin = res->state_margin ? res->state_margin + sw : NULL;
+        if (smargin) *smargin = INFINITY;
+        sample_states_m(N, K, Pf, pif, Atmp, piN, u, (p->flags & ORC_FLAG_PIF_FORM) ? 1 : 0, X, smargin);
         /* --- save (:554-560) + forecasts (:858-862) */
         if (sw >= p->burnin) {
             size_t d = (size_t)(sw - p->burnin);

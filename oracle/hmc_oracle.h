@@ -105,6 +105,12 @@ typedef struct {              /* any pointer may be NULL; all [draw]-major row-m
     double* pib_full;  /* nrun*N*K */
     int64_t* X_final;  /* N */
     int64_t n_events;  /* zero-normaliser / non-finite events */
+    /* Per sweep (burnin + nrun entries, indexed by sweep): how far the sweep's discrete decisions were from flipping.  A chain
+     * run in lower precision on the same streams can leave this chain only through such a decision.
+     * state_margin: min over t (X[N] included) of |u_t - nearest cumulative boundary| of the normalised p it was compared with.
+     * gamma_margin: min over the sweep's gamma draws of the distance of each comparison from its threshold (see gamma_m). */
+    double* state_margin;
+    double* gamma_margin;
 } orc_result;
 
 /* src/Hmc.jl:517-562 gibbssample! + :850-865 estimatemodel glue, one chain */

@@ -36,7 +36,7 @@ class _Problem(C.Structure):
 class _Result(C.Structure):
     _fields_ = [("mu", _dp), ("sigma2", _dp), ("A", _dp), ("pi_end", _dp), ("forecasts", _dp),
                 ("loglik", _dp), ("pib_mean", _dp), ("pib_full", _dp), ("X_final", _ip),
-                ("n_events", C.c_int64)]
+                ("n_events", C.c_int64), ("state_margin", _dp), ("gamma_margin", _dp)]
 
 
 def build(force: bool = False) -> str:
@@ -161,7 +161,7 @@ class _Job:
 
     def __init__(self, y, K, burnin, nrun, seed=1234, chain=0, flags=FLAG_REF_Q1, horizons=(12,), y_future=None,
                  X0=None, is_signal=None, xi=None, alpha=None, nu=None, beta0=None, beta=None, kappa=1.0,
-                 want_pib_mean=False, want_pib_full=False):
+                 want_pib_mean=False, want_pib_full=False, want_margins=False):
         self.y = _f64(y)
         N = len(self.y)
         self.N, self.K, self.nrun = N, K, nrun
@@ -176,18 +176,23 @@ class _Job:
             pi_end=np.zeros((nrun, K)), forecasts=np.zeros((nrun, 2 * nh)), loglik=np.zeros(nrun),
             pib_mean=np.zeros((N, K)) if want_pib_mean else None,
             pib_full=np.zeros((nrun, N, K)) if want_pib_full else None,
-            X_final=np.zeros(N, dtype=np.int64), n_events=0)
+            X_final=np.zeros(N, dtype=np.int64), n_events=0,
+            state_margin=np.zeros(burnin + nrun) if want_margins else None,
+            gamma_margin=np.zeros(burnin + nrun) if want_margins else None)
         o = self.out
         self.problem = _Problem(_d(self.y), N, K, None if self.sig is None else self.sig.ctypes.data_as(_u8p),
                                 *[_d(v) for v in self.hp], kappa,
                                 None if self.X0 is None else self.X0.ctypes.data_as(_ip),
                                 burnin, nrun, seed, chain, flags, self.h.ctypes.data_as(_i32p), nh, _d(self.yf))
         self.result = _Result(_d(o.mu), _d(o.sigma2), _d(o.A), _d(o.pi_end), _d(o.forecasts), _d(o.loglik),
-                              _d(o.pib_mean), _d(o.pib_full), o.X_final.ctypes.data_as(_ip), 0)
+                              _d(o.pib_mean), _d(o.pib_full), o.X_final.ctypes.data_as(_ip), 0,
+                              _d(o.state_margin), _d(o.gamma_margin))
 
 
 def gibbs(y, K, burnin, nrun, **kw):
-    """One chain of the reference sampler (src/Hmc.jl:517-562 + :850-865). Returns draw-major arrays."""
+    """One chain of the reference sampler (src/Hmc.jl:517-562 + :850-865). Returns draw-major arrays.
+    want_margins=True adds state_margin / gamma_margin, one entry per sweep (burnin included): how close that sweep's
+    categorical draws and gamma accept/reject tests came to the other outcome (hmc_oracle.h, orc_result)."""
     job = _Job(y, K, burnin, nrun, **kw)
     rc = lib().orc_gibbs(C.byref(job.problem), C.byref(job.result))
     if rc != 0:

@@ -2,16 +2,29 @@
 signal masks, kappa, pi_row_back, user X0) are estimated in fp64 with two kernels that must produce the same chains (same
 Philox streams): K = 2..4 time-parallel warp-per-chain vs thread-per-chain; K = 5..8 thread-per-chain vs lane-per-state; K = 2..4 plain sweeps also on the segment kernel
 (2 / 4 / 8 lanes per chain, or mixed 8 + 4) vs thread-per-chain.
-python scripts/fuzz_kernels.py [n] [seed]"""
+With --precision 32 the same shapes run in fp32 (burnin 0, 3 draws, one series), and each kernel is checked on its own against
+the fp64 oracle chain with the certification of tests/test_fp32_chain_parity.py (fp32 kernels legitimately differ from each
+other in the last bits).
+python scripts/fuzz_kernels.py [n] [seed] [--precision 32]"""
 import os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import hmc_jl_b200 as H
 
-n_cases = int(sys.argv[1]) if len(sys.argv) > 1 else 100
-rng = np.random.default_rng(int(sys.argv[2]) if len(sys.argv) > 2 else 0)
+args = [a for a in sys.argv[1:]]
+fp32 = "--precision" in args and args[args.index("--precision") + 1] == "32"
+if "--precision" in args:
+    i = args.index("--precision")
+    if args[i + 1] not in ("32", "64"):
+        sys.exit("--precision must be 32 or 64")
+    del args[i:i + 2]
+n_cases = int(args[0]) if len(args) > 0 else 100
+rng = np.random.default_rng(int(args[1]) if len(args) > 1 else 0)
 ctx = H.Context(0)
+if fp32:
+    from oracle import oracle as O
+    from test_fp32_chain_parity import KERNELS, check_chains
 bad = 0
 for case in range(n_cases):
     K = int(rng.integers(2, 9))
@@ -36,9 +49,28 @@ for case in range(n_cases):
                   alpha=np.full(K, 2.0), nu=np.full(K, 2.0))
     if rng.random() < 0.3:
         kw.update(X0=[rng.integers(1, K + 1, int(e - s + 1)) for s, e in zip(ws, we)])
-    outs = {}
     for v in ("HMCGPU_SEG_LANES", "HMCGPU_SEG_LONG", "HMCGPU_SCAN_MAX_CHAINS", "HMCGPU_LANE_KERNEL"):
         os.environ.pop(v, None)
+    if fp32:
+        kernels = ["scan", "thread"] if K <= 4 else ["thread", "lane"]
+        if K <= 4 and "is_signal" not in kw:
+            lanes = int(rng.choice([2, 4, 8]))
+            if (we - ws + 1).max() <= lanes * (((1 << (32 // K)) - 1) // 4 * 4):       # seg_max_T
+                kernels.append(f"seg{lanes}")
+        sig = kw.get("is_signal")
+        for name in kernels:
+            for v in ("HMCGPU_SEG_LANES", "HMCGPU_SEG_LONG", "HMCGPU_SCAN_MAX_CHAINS", "HMCGPU_LANE_KERNEL"):
+                os.environ.pop(v, None)
+            os.environ.update(KERNELS[name][0])
+            try:
+                check_chains(H, ctx, O, y[0], ws, we, K, kw["n_chains"], KERNELS[name][1], seed=kw["seed"], hs=kw["horizons"],
+                             alpha=kw.get("alpha"), nu=kw.get("nu"), is_signal=None if sig is None else (sig[0] if sig.ndim == 2 else sig),
+                             kappa=kw.get("kappa", 1.0), X0=kw.get("X0"), pi_row_back=kw.get("pi_row_back", 0), min_certified=0.0)
+            except AssertionError as e:
+                bad += 1
+                print("MISMATCH case", case, name, dict(K=K, ws=ws.tolist(), we=we.tolist()), str(e)[:500], flush=True)
+        continue
+    outs = {}
     run = lambda: H.estimate(ctx, H.ProblemSpec(y, ws, we, **kw))
     if K <= 4:
         os.environ["HMCGPU_SCAN_MAX_CHAINS"] = "1000000"

@@ -668,8 +668,9 @@ def test_wide_gibbs_first_sweeps_follow_the_oracle_chain(H, ctx, oracle, K, T, l
 
 
 def test_wide_gibbs_fp32_posterior_matches_oracle(H, ctx, oracle):
-    """fp32 lane-per-state kernel: pooled posterior means vs the oracle's under identical settings (K=8 mixes slowly from
-    the makeParams start, so both are compared to each other, not to the generating truth)."""
+    """fp32 thread-per-chain kernel at K = 8 (the default for K <= 8; the lane kernel's fp32 chains at K = 5..32 are checked
+    draw by draw in test_fp32_chain_parity.py): pooled posterior means vs the oracle's under identical settings (K=8 mixes
+    slowly from the makeParams start, so both are compared to each other, not to the generating truth)."""
     K = 8
     tr = _truth(K)
     y, _ = synth_hmm(612, seed=3, **tr)

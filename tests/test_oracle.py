@@ -240,6 +240,61 @@ def test_gibbs_deterministic_and_batch(oracle):
     np.testing.assert_allclose(d.mu, a.mu, rtol=1e-9)
 
 
+def test_state_margins_recomputed_from_the_first_sweep(oracle):
+    """want_margins: state_margin[0] is the distance of the sweep-0 STATES uniforms from the nearest cumulative boundary of the
+    categoricals they were compared with.  Recomputed here from the chain's own sweep-0 parameters (makeParams statistics ->
+    draw_params in chain labels -> forward), the uniforms of the Philox-7 stream and the sampled path; moving every u by half
+    the margin keeps the path, moving the closest one 1.5 margins towards its boundary changes it."""
+    K, seed, chain = 3, 17, 5
+    y, _ = synth_hmm(150, seed=2, **K3_TRUTH)
+    N = len(y)
+    flags = oracle.FLAG_REF_Q1 | oracle.FLAG_PIF_FORM
+    r = oracle.gibbs(y, K, 0, 1, seed=seed, chain=chain, flags=flags, want_margins=True)
+    assert oracle.gibbs(y, K, 0, 1, seed=seed, chain=chain, flags=flags).state_margin is None
+    assert r.state_margin.shape == (1,) and r.gamma_margin.shape == (1,)
+    assert 0 < r.gamma_margin[0] < np.inf
+    # sweep 0 in chain labels, as the oracle computes it
+    X0, _, _ = oracle.make_params(y, K)
+    st = X0 - 1
+    Ni = np.bincount(st, minlength=K)
+    S = np.array([sum(y[st == k]) for k in range(K)])       # (sequential sums, as the oracle adds)
+    ybar = np.where(Ni > 0, S / np.maximum(Ni, 1), 0.0)
+    S2 = np.array([sum((y[st == k] - ybar[k]) ** 2) for k in range(K)])
+    trans = np.ones((K, K), dtype=np.int64)
+    np.add.at(trans, (st[:-1], st[1:]), 1)
+    one = np.ones(K)
+    s2, mu, rho, A = oracle.draw_params(Ni, S, S2, trans, np.full(K, sum(y) / N), one, one, one, seed, chain, 0)
+    order = np.argsort(mu, kind="stable")
+    np.testing.assert_array_equal(r.mu[0], mu[order])
+    pif = oracle.forward(y, A, mu, s2, rho, want_Pf=False).pif
+    piN = pif[-1][order]                                    # quirk Q1: X[N] drawn from the relabelled row
+    u = np.zeros(N)
+    for i in range(0, N, 4):
+        w = oracle.philox([i >> 2, oracle.KIND_STATES << 16, 0, chain], [seed & 0xFFFFFFFF, seed >> 32], rounds=7)
+        for j in range(min(4, N - i)):
+            u[N - 1 - (i + j)] = (w[j] + 0.5) * 2.0 ** -32
+    X = oracle.sample_states(pif, A, u, piN=piN, form=1)
+    np.testing.assert_array_equal(X, r.X_final)
+    m, side = np.zeros(N), np.zeros(N)                     # per-step margin and the direction of the nearest boundary
+    for t in range(N - 1, -1, -1):
+        if t == N - 1:
+            p = piN
+        else:
+            x = X[t + 1] - 1
+            p = pif[t] * A[:, x]
+            p = p / p.sum() if pif[t + 1, x] > np.finfo(float).eps and p.sum() > 0 else np.full(K, 1.0 / K)
+        d = u[t] - np.cumsum(p)[:K - 1]
+        j = np.argmin(np.abs(d))
+        m[t], side[t] = abs(d[j]), np.sign(d[j])
+    np.testing.assert_allclose(m.min(), r.state_margin[0], rtol=1e-12)
+    for s in (-0.5, 0.5):
+        np.testing.assert_array_equal(oracle.sample_states(pif, A, u + s * m.min(), piN=piN, form=1), X)
+    t = int(np.argmin(m))
+    v = u.copy()
+    v[t] -= side[t] * 1.5 * m[t]
+    assert oracle.sample_states(pif, A, v, piN=piN, form=1)[t] != X[t]
+
+
 @pytest.mark.parametrize("which", [0, 9, 18])
 def test_golden_posterior_summaries(oracle, which):
     """The oracle reproduces the reference's own posterior means (data/output/official/*_summary.csv, 250k draws
