@@ -229,10 +229,12 @@ def shard_windows(T: Sequence[int], n_shards: int):
 
 def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                      precision=32, draws=False, summary=True, smoothed=False, loglik=False, win_id=None,
-                     win_series=None, ctx: Optional[B.Context] = None, device: int = 0):
-    """Many end-date windows in one call (what the SLURM job array does one process at a time)."""
+                     win_series=None, diagnostics=False, ctx: Optional[B.Context] = None, device: int = 0):
+    """Many end-date windows in one call (what the SLURM job array does one process at a time).  `diagnostics=True` adds
+    `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics)."""
     flags = B.FLAG_REF_Q1 | (B.FLAG_DRAWS if draws else 0) | (B.FLAG_SUMMARY if summary else 0) \
-        | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0)
+        | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0) \
+        | (B.FLAG_DIAGNOSTICS if diagnostics else 0)
     spec = B.ProblemSpec(y, win_start, win_end, K=K, n_chains=n_chains, burnin=burnin, nrun=nrun, seed=seed,
                          horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series)
     own = ctx is None
@@ -329,31 +331,54 @@ def saveresults(samples, opt: EstOpt, directory: str, precision: int = 5, hassig
     return paths
 
 
-def write_summaries(out, K: int, horizons: Sequence[int], dates: Sequence, directory: str):
-    """Per-date posterior means in the layout of the reference's `<var>_summary.csv` (Hmc.runaggregate,
-    src/Hmc.jl:1025-1051: group by date, mean -> columns `<col>_mean`), computed on the device
-    (HMCGPU_FLAG_SUMMARY) instead of from 250 000-row draw files.  One row per window, in caller order."""
-    import os
-    os.makedirs(directory, exist_ok=True)
-    m = np.asarray(out.summary_mean)
+def _summary_tables(table, K: int, horizons: Sequence[int], suffix: str):
+    """Splits an [n_windows, F] table in the summary field order (include/hmcgpu.h) into the reference's per-variable CSV
+    tables: {name: (column names, [n_windows, n_cols] block)}; every column name ends in `suffix`."""
+    m = np.asarray(table)
     nh = len(horizons)
-    cols = {
-        "filtered_means": ([f"state_{i}_mean" for i in range(1, K + 1)], m[:, 0:K]),
-        "filtered_variances": ([f"state_{i}_mean" for i in range(1, K + 1)], m[:, K:2 * K]),
+    states = [f"state_{i}_{suffix}" for i in range(1, K + 1)]
+    return {
+        "filtered_means": (states, m[:, 0:K]),
+        "filtered_variances": (states, m[:, K:2 * K]),
         # summary A index s*K + r = A[r, s]  ->  column-major (i, j) order with trans_i_j = A[i, j]
-        "filtered_trans_probs": ([f"trans_{i}_{j}_mean" for j in range(1, K + 1) for i in range(1, K + 1)], m[:, 2 * K:2 * K + K * K]),
-        "filtered_state_probs": ([f"state_{i}_mean" for i in range(1, K + 1)], m[:, 2 * K + K * K:3 * K + K * K]),
-        "forecasts": (sum([[f"forecast_{h}_mean", f"forecast_error_{h}_mean"] for h in horizons], []),
+        "filtered_trans_probs": ([f"trans_{i}_{j}_{suffix}" for j in range(1, K + 1) for i in range(1, K + 1)], m[:, 2 * K:2 * K + K * K]),
+        "filtered_state_probs": (states, m[:, 2 * K + K * K:3 * K + K * K]),
+        "forecasts": (sum([[f"forecast_{h}_{suffix}", f"forecast_error_{h}_{suffix}"] for h in horizons], []),
                       m[:, 3 * K + K * K:3 * K + K * K + 2 * nh]),
     }
+
+
+def _write_tables(tables, dates: Sequence, directory: str, file_suffix: str):
+    import os
+    os.makedirs(directory, exist_ok=True)
     paths = {}
-    for name, (hdr, data) in cols.items():
-        path = os.path.join(directory, f"{name}_summary.csv")
+    for name, (hdr, data) in tables.items():
+        path = os.path.join(directory, f"{name}_{file_suffix}.csv")
         with open(path, "w") as f:
             f.write(",".join(["date"] + hdr) + "\n")
             for d, row in zip(dates, data):
                 f.write(",".join([str(d)] + [repr(float(v)) for v in row]) + "\n")
         paths[name] = path
+    return paths
+
+
+def write_summaries(out, K: int, horizons: Sequence[int], dates: Sequence, directory: str):
+    """Per-date posterior means in the layout of the reference's `<var>_summary.csv` (Hmc.runaggregate,
+    src/Hmc.jl:1025-1051: group by date, mean -> columns `<col>_mean`), computed on the device
+    (HMCGPU_FLAG_SUMMARY) instead of from 250 000-row draw files.  One row per window, in caller order."""
+    return _write_tables(_summary_tables(out.summary_mean, K, horizons, "mean"), dates, directory, "summary")
+
+
+def write_diagnostics(out, K: int, horizons: Sequence[int], dates: Sequence, directory: str):
+    """Convergence diagnostics next to the summaries: `<var>_rhat.csv` (split-R̂, columns `<col>_rhat`) and `<var>_ess.csv`
+    (effective sample size, columns `<col>_ess`), one row per window in the column layout of write_summaries; computed on the
+    device (HMCGPU_FLAG_DIAGNOSTICS, estimate_windows(diagnostics=True)).  NaN marks a field with a non-finite draw (a forecast
+    horizon past the end of the series) or no within-chain variation.  An ESS whose autocorrelation sum reached the lag cap
+    (out.ess_lag, include/hmcgpu.h) over-estimates the effective sample size.  Returns {"<var>_rhat": path, "<var>_ess": path}."""
+    paths = {}
+    for kind, table in (("rhat", out.rhat), ("ess", out.ess)):
+        for name, path in _write_tables(_summary_tables(table, K, horizons, kind), dates, directory, kind).items():
+            paths[f"{name}_{kind}"] = path
     return paths
 
 

@@ -18,6 +18,7 @@ FLAG_SUMMARY = 4
 FLAG_SMOOTHED_MEAN = 8
 FLAG_LOGLIK = 16
 FLAG_FILTERED_MEAN = 64   # pib_mean / insample_forecast_mean carry the FILTERED means (the reference's published in-sample table)
+FLAG_DIAGNOSTICS = 128    # rhat / ess / ess_lag per window and summary field (split-R̂ and ESS, include/hmcgpu.h)
 
 ERR_ARG, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED, ERR_NODEVICE = -1, -2, -3, -4, -5
 
@@ -55,7 +56,8 @@ class Result(C.Structure):
                 ("summary_mean", _dp), ("summary_var", _dp), ("pib_mean", _dp), ("insample_forecast_mean", _dp), ("status", _i32p),
                 ("gpu_ms", C.c_double), ("sweep_kernel_ms", C.c_double), ("n_launches", C.c_int64),
                 ("n_sweep_launches", C.c_int64), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64),
-                ("state_steps", C.c_int64), ("sweep_launch_ms_sum", C.c_double), ("sweep_kernel", C.c_int32), ("n_tasks", C.c_int32)]
+                ("state_steps", C.c_int64), ("sweep_launch_ms_sum", C.c_double), ("sweep_kernel", C.c_int32), ("n_tasks", C.c_int32),
+                ("rhat", _dp), ("ess", _dp), ("ess_lag", _i32p)]
 
 
 class HmcGpuError(RuntimeError):
@@ -272,12 +274,20 @@ class ProblemSpec:
                        _p(self.horizons, _i32p), self.n_h, _p(self.X0, _i64p), self.precision, self.flags,
                        _p(self.win_init_series, _i32p), self.pi_row_back, self.sig_per_series)
 
-    def alloc_result(self):
+    def alloc_result(self, diagnostics=None):
+        """Output arrays for the flags of this problem.  `diagnostics=True` asks for rhat / ess / ess_lag, which the library
+        fills only with FLAG_DIAGNOSTICS (it cannot tell whether a caller's struct has these fields, so it never checks them);
+        default: whenever the flag is set."""
+        if diagnostics is None:
+            diagnostics = bool(self.flags & FLAG_DIAGNOSTICS)
+        if diagnostics and not self.flags & FLAG_DIAGNOSTICS:
+            raise ValueError("rhat / ess / ess_lag requested without FLAG_DIAGNOSTICS")
         K, nw, nh = self.K, self.n_windows, self.n_h
         R = self.n_chains * self.nrun
         F = 3 * K + K * K + 2 * nh + 1
         o = SimpleNamespace(mu=None, sigma2=None, A=None, pi_end=None, forecasts=None, loglik=None, summary_mean=None,
-                            summary_var=None, pib_mean=None, insample_forecast_mean=None, status=np.zeros((nw, self.n_chains), dtype=np.int32))
+                            summary_var=None, pib_mean=None, insample_forecast_mean=None, status=np.zeros((nw, self.n_chains), dtype=np.int32),
+                            rhat=None, ess=None, ess_lag=None)
         if self.flags & FLAG_DRAWS:
             # Julia column-major (R x K) per window == C arrays [window][k][draw]
             o.mu = np.empty((nw, K, R)); o.sigma2 = np.empty((nw, K, R)); o.A = np.empty((nw, K, K, R))
@@ -289,8 +299,11 @@ class ProblemSpec:
         if self.flags & (FLAG_SMOOTHED_MEAN | FLAG_FILTERED_MEAN):
             o.pib_mean = np.empty(int(self.T.sum()) * K)
             o.insample_forecast_mean = np.empty(int(self.T.sum()) * nh) if nh else None
+        if diagnostics:   # [n_windows, F] in the field order of summary_mean
+            o.rhat = np.empty((nw, F)); o.ess = np.empty((nw, F)); o.ess_lag = np.empty((nw, F), dtype=np.int32)
         res = Result(_p(o.mu), _p(o.sigma2), _p(o.A), _p(o.pi_end), _p(o.forecasts), _p(o.loglik), _p(o.summary_mean),
-                     _p(o.summary_var), _p(o.pib_mean), _p(o.insample_forecast_mean), _p(o.status, _i32p), 0, 0, 0, 0, 0, 0, 0, 0, 0, 0)
+                     _p(o.summary_var), _p(o.pib_mean), _p(o.insample_forecast_mean), _p(o.status, _i32p), 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,
+                     _p(o.rhat), _p(o.ess), _p(o.ess_lag, _i32p))
         return o, res
 
     def finish(self, o, res, rc):

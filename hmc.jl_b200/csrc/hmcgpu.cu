@@ -4,6 +4,7 @@
 #include "gibbs_wide_kernel.cuh"
 #include "gibbs_scan_kernel.cuh"
 #include "gibbs_seg_kernel.cuh"
+#include "diagnostics.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -1317,6 +1318,9 @@ struct hmcgpu_plan {
     std::vector<cudaEvent_t> timing_events;   // pairs around every sweep launch + one end-of-sweeps event per group (timing enabled)
     double launch_ms_sum = 0.0;
     DevBuf d_mu, d_sig2, d_A, d_pie, d_fc, d_ll, d_sum, d_sumsq, d_pibsum, d_fcsum;
+    // HMCGPU_FLAG_DIAGNOSTICS (diagnostics.cuh): streaming state per (slot, field), per-sequence means / variances and lag sums
+    // per (window, field)
+    DevBuf dg_P, dg_S1, dg_head, dg_ring, dg_mean, dg_var, dg_gsum;
     DevBuf d_diag;       // segment kernel: chain-sweeps that fell back to the exact entering vectors
     unsigned long long seg_fallbacks[2] = {0, 0};   // [0] chain-sweeps on the exact path, [1] speculative groups (sum over chain-sweeps)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
@@ -1360,6 +1364,7 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p) {
         return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "n_windows * n_chains = %lld exceeds 2^31 - 65 chains per call", (long long)p->n_windows * p->n_chains);
     if (p->burnin < 0 || p->nrun < 1) return fail(ctx, HMCGPU_ERR_ARG, "burnin < 0 or nrun < 1");
     if (p->burnin + p->nrun > 0xffffffffLL) return fail(ctx, HMCGPU_ERR_ARG, "more than 2^32 sweeps");
+    if ((p->flags & HMCGPU_FLAG_DIAGNOSTICS) && p->nrun < 4) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_DIAGNOSTICS needs nrun >= 4 (two sequences of >= 2 draws per chain)");
     if (p->precision != 32 && p->precision != 64) return fail(ctx, HMCGPU_ERR_ARG, "precision must be 32 or 64");
     if (p->n_h < 0 || p->n_h > kMaxH || (p->n_h > 0 && !p->horizons)) return fail(ctx, HMCGPU_ERR_ARG, "0 <= n_h <= %d", kMaxH);
     if (p->is_signal || p->pi_row_back != 0) {
@@ -1706,6 +1711,16 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer)
         CU(ctx, pl->d_sum.alloc((size_t)nw * pl->F * sizeof(double)));
         CU(ctx, pl->d_sumsq.alloc((size_t)nw * pl->F * sizeof(double)));
     }
+    if (p->flags & HMCGPU_FLAG_DIAGNOSTICS) {
+        const size_t n_sf = (size_t)pl->F * n_slots, nwf = (size_t)nw * pl->F;
+        CU(ctx, pl->dg_P.alloc(n_sf * kDiagLags * sizeof(double)));
+        CU(ctx, pl->dg_S1.alloc(n_sf * sizeof(double)));
+        CU(ctx, pl->dg_head.alloc(n_sf * kDiagLags * sizeof(R)));
+        CU(ctx, pl->dg_ring.alloc(n_sf * kDiagLags * sizeof(R)));
+        CU(ctx, pl->dg_mean.alloc(nwf * 2 * nc * sizeof(double)));
+        CU(ctx, pl->dg_var.alloc(nwf * 2 * nc * sizeof(double)));
+        CU(ctx, pl->dg_gsum.alloc(nwf * kDiagLags * sizeof(double)));
+    }
     if (p->flags & kAccMean) {
         CU(ctx, pl->pacc.alloc((size_t)pi_elems * sizeof(R)));
         if (p->n_h > 0) {
@@ -1877,6 +1892,28 @@ static int plan_run_t(hmcgpu_plan* pl) {
                                                          pl->d_sum.as<double>(), pl->d_sumsq.as<double>());
             CU(ctx, cudaGetLastError());
             ++pl->n_launches;
+        }
+        if (pl->flags & HMCGPU_FLAG_DIAGNOSTICS) {
+            // split-R̂ / ESS: draws [0, nh) form a chain's first sequence, [nrun - nh, nrun) its second; each sequence is reduced
+            // per window right after the chunk holding its last draw, and the state is then reused by the next sequence
+            const long long nh = pl->nrun / 2, h2 = pl->nrun - nh;
+            const int Fd = (pl->flags & HMCGPU_FLAG_LOGLIK) ? pl->F : pl->F - 1;     // (no log-likelihood draws to look at)
+            const DiagState<R> ds{pl->dg_P.as<double>(), pl->dg_S1.as<double>(), pl->dg_head.as<R>(), pl->dg_ring.as<R>(), (long long)pl->F * ns};
+            auto sequence = [&](long long lo, long long hi, long long seq0, long long seq_end, int half) -> int {
+                if (lo >= hi) return 0;
+                diag_accum_kernel<R><<<dim3(ns / 32, Fd), dim3(32, 32), 0, st>>>(ns, pl->chunk, (int)(lo - d0), (int)(hi - lo), lo - seq0, buf, ds);
+                CU(ctx, cudaGetLastError());
+                ++pl->n_launches;
+                if (hi == seq_end) {
+                    diag_half_kernel<R><<<dim3(pl->n_windows, Fd), kDiagLags, 0, st>>>(pl->F, ns, pl->n_chains, nh, half, pl->win_slot0.as<int>(), ds,
+                                                                                       pl->dg_mean.as<double>(), pl->dg_var.as<double>(), pl->dg_gsum.as<double>());
+                    CU(ctx, cudaGetLastError());
+                    ++pl->n_launches;
+                }
+                return 0;
+            };
+            TRY(sequence(d0, std::min<long long>(d0 + n, nh), 0, nh, 0));
+            TRY(sequence(std::max(d0, h2), d0 + n, h2, pl->nrun, 1));
         }
         if (pl->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)) {
             tile_reduce_kernel<R><<<pl->n_windows, 256, 0, st>>>(Kr, Kr, pl->n_chains, pl->win_slot0.as<int>(), pl->wTd.as<int>(),
@@ -2132,6 +2169,8 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     if ((r->pib_mean || r->insample_forecast_mean) && !(pl->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)))
         return fail(ctx, HMCGPU_ERR_ARG, "pib_mean / insample_forecast_mean requested without HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN");
     if (r->loglik && !(pl->flags & HMCGPU_FLAG_LOGLIK)) return fail(ctx, HMCGPU_ERR_ARG, "loglik requested without HMCGPU_FLAG_LOGLIK");
+    // (rhat / ess / ess_lag were appended in ABI version 300: they are read only when the flag says the caller has them)
+    const bool diag = (pl->flags & HMCGPU_FLAG_DIAGNOSTICS) && (r->rhat || r->ess || r->ess_lag);
     CU(ctx, down(r->mu, pl->d_mu, nw * Rr * K * sizeof(double)));
     CU(ctx, down(r->sigma2, pl->d_sig2, nw * Rr * K * sizeof(double)));
     CU(ctx, down(r->A, pl->d_A, nw * Rr * K * K * sizeof(double)));
@@ -2151,6 +2190,20 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
         CU(ctx, cudaGetLastError());
         CU(ctx, down(r->summary_mean, d_mean, (size_t)ne * sizeof(double)));
         CU(ctx, down(r->summary_var, d_var, (size_t)ne * sizeof(double)));
+    }
+    DevBuf d_rhat, d_ess, d_lag;
+    if (diag) {
+        const long long ne = (long long)nw * pl->F;
+        CU(ctx, d_rhat.alloc((size_t)ne * sizeof(double)));
+        CU(ctx, d_ess.alloc((size_t)ne * sizeof(double)));
+        CU(ctx, d_lag.alloc((size_t)ne * sizeof(int)));
+        diag_finish_kernel<<<grid_for(ne, 128), 128, 0, st>>>(ne, pl->F, pl->n_chains, pl->nrun / 2, (pl->flags & HMCGPU_FLAG_LOGLIK) ? 1 : 0,
+                                                              pl->dg_mean.as<double>(), pl->dg_var.as<double>(), pl->dg_gsum.as<double>(),
+                                                              d_rhat.as<double>(), d_ess.as<double>(), d_lag.as<int>());
+        CU(ctx, cudaGetLastError());
+        CU(ctx, down(r->rhat, d_rhat, (size_t)ne * sizeof(double)));
+        CU(ctx, down(r->ess, d_ess, (size_t)ne * sizeof(double)));
+        CU(ctx, down(r->ess_lag, d_lag, (size_t)ne * sizeof(int)));
     }
     if (r->pib_mean) { pibsum.resize((size_t)pl->pib_total); CU(ctx, down(pibsum.data(), pl->d_pibsum, pibsum.size() * sizeof(double))); }
     if (r->insample_forecast_mean && pl->d_fcsum.p) {
@@ -2259,8 +2312,9 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             q.n_windows = n; q.win_series = ser.data(); q.win_start = st.data(); q.win_end = en.data(); q.win_id = id.data();
             if (p->win_init_series) q.win_init_series = iser.data();
             if (p->X0) q.X0 = x0.data();
-            std::vector<double> mu, s2, A, pe, fc, ll, sm, sv, pb, ifc;
-            std::vector<int32_t> status;
+            std::vector<double> mu, s2, A, pe, fc, ll, sm, sv, pb, ifc, rh, es;
+            std::vector<int32_t> status, el;
+            const bool diag = (p->flags & HMCGPU_FLAG_DIAGNOSTICS) != 0;   // (the diagnostics pointers exist only then)
             hmcgpu_result& o = parts[d];
             if (r->mu) { mu.resize(n * Rr * K); o.mu = mu.data(); }
             if (r->sigma2) { s2.resize(n * Rr * K); o.sigma2 = s2.data(); }
@@ -2273,6 +2327,9 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             if (r->pib_mean) { pb.resize(pibn); o.pib_mean = pb.data(); }
             if (r->insample_forecast_mean) { ifc.resize(pibn / K * std::max(1, nh)); o.insample_forecast_mean = ifc.data(); }
             if (r->status) { status.resize((size_t)n * p->n_chains); o.status = status.data(); }
+            if (diag && r->rhat) { rh.resize((size_t)n * F); o.rhat = rh.data(); }
+            if (diag && r->ess) { es.resize((size_t)n * F); o.ess = es.data(); }
+            if (diag && r->ess_lag) { el.resize((size_t)n * F); o.ess_lag = el.data(); }
             rc = hmcgpu_estimate(ctx, &q, &o);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
@@ -2288,6 +2345,9 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
                     if (r->loglik) memcpy(r->loglik + w * Rr, ll.data() + j * Rr, Rr * sizeof(double));
                     if (r->summary_mean) memcpy(r->summary_mean + w * F, sm.data() + (size_t)j * F, F * sizeof(double));
                     if (r->summary_var) memcpy(r->summary_var + w * F, sv.data() + (size_t)j * F, F * sizeof(double));
+                    if (o.rhat) memcpy(r->rhat + w * F, rh.data() + (size_t)j * F, F * sizeof(double));
+                    if (o.ess) memcpy(r->ess + w * F, es.data() + (size_t)j * F, F * sizeof(double));
+                    if (o.ess_lag) memcpy(r->ess_lag + w * F, el.data() + (size_t)j * F, F * sizeof(int32_t));
                     if (r->insample_forecast_mean) memcpy(r->insample_forecast_mean + pib_off[w] / K * nh, ifc.data() + po / K * nh, (size_t)Tw((int)w) * nh * sizeof(double));
                     if (r->pib_mean) memcpy(r->pib_mean + pib_off[w], pb.data() + po, (size_t)Tw((int)w) * K * sizeof(double));
                     po += (size_t)Tw((int)w) * K;

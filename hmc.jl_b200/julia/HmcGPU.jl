@@ -26,6 +26,7 @@ const FLAG_SUMMARY = UInt32(4)
 const FLAG_SMOOTHED_MEAN = UInt32(8)
 const FLAG_FILTERED_MEAN = UInt32(64)
 const FLAG_LOGLIK = UInt32(16)
+const FLAG_DIAGNOSTICS = UInt32(128)
 
 # struct hmcgpu_problem (include/hmcgpu.h)
 struct Problem
@@ -45,6 +46,7 @@ mutable struct Result
     gpu_ms::Float64; sweep_kernel_ms::Float64; n_launches::Int64; n_sweep_launches::Int64
     h2d_bytes::Int64; d2h_bytes::Int64; state_steps::Int64
     sweep_launch_ms_sum::Float64; sweep_kernel::Int32; n_tasks::Int32
+    rhat::Ptr{Float64}; ess::Ptr{Float64}; ess_lag::Ptr{Int32}
 end
 
 struct HmcGpuError <: Exception
@@ -107,7 +109,8 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
     fc = Array{Float64}(undef, R, 2nh, nw)
     status = zeros(Int32, n_chains, nw)
     res = Result(pointer(mu), pointer(sig), pointer(A), pointer(pie), nh > 0 ? pointer(fc) : C_NULL, C_NULL,
-                 C_NULL, C_NULL, C_NULL, C_NULL, pointer(status), 0.0, 0.0, 0, 0, 0, 0, 0, 0.0, 0, 0)
+                 C_NULL, C_NULL, C_NULL, C_NULL, pointer(status), 0.0, 0.0, 0, 0, 0, 0, 0, 0.0, 0, 0,
+                 C_NULL, C_NULL, C_NULL)
     rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu begin
         prob = Problem(pointer(rawdata), y_len, n_series, nw, ptr_or_null(win_series), pointer(win_start), pointer(win_end), C_NULL,
                        D, n_chains, burnin, Nrun, UInt64(seed), ptr_or_null(xi), ptr_or_null(alpha), ptr_or_null(nu), C_NULL, C_NULL,

@@ -56,6 +56,8 @@ extern "C" {
 #define HMCGPU_FLAG_FILTERED_MEAN 64u /* fill pib_mean / insample_forecast_mean with the posterior means of the FILTERED state
                                         probabilities pif[t,:] and of pif[t,:]' A^h mu (what the reference's published in-sample table
                                         data/output/official_insample/forecats_insample.csv holds); K <= 8, not with SMOOTHED_MEAN or signals */
+#define HMCGPU_FLAG_DIAGNOSTICS  128u /* fill rhat / ess / ess_lag: split-R̂ and effective sample size per window and summary field,
+                                        computed on the device from every saved draw; needs nrun >= 4 (see hmcgpu_result) */
 
 typedef struct hmcgpu_ctx hmcgpu_ctx;
 typedef struct hmcgpu_plan hmcgpu_plan;
@@ -116,7 +118,21 @@ typedef struct hmcgpu_problem {
  * insample_forecast_mean: per window N_w x n_h column-major, concatenated (offset_w = n_h * sum_{v<w} N_v): the posterior
  *   mean of pib[t,:]' A^h mu for every date t of the window and every horizon (forecastinsample, src/Hmc.jl:683-699);
  *   the forecast error of date t is this minus y[t+h].  Needs HMCGPU_FLAG_SMOOTHED_MEAN (K <= 4).
- * status[w*n_chains + c]: event count of that chain. */
+ * status[w*n_chains + c]: event count of that chain.
+ * rhat, ess, ess_lag [w*F + f] (HMCGPU_FLAG_DIAGNOSTICS; same fields and order as summary_mean): convergence diagnostics of each
+ *   summary field over the window's chains.  Each chain's nrun saved draws are split into two sequences of n = floor(nrun/2)
+ *   draws (the middle draw of an odd nrun is dropped), M = 2*n_chains sequences in all.  With W the mean of the sequences'
+ *   variances (denominator n-1) and B/n the variance of their means (denominator M-1), var+ = (n-1)/n W + B/n and
+ *   rhat = sqrt(var+ / W): the classic split-R̂ of BDA3, NOT rank-normalised.  ess = M n / tau with
+ *   tau = max(-1 + 2 sum_k P_k, 1/log10(M n)), P_k = rho_2k + rho_2k+1 summed while positive and made non-increasing
+ *   (Geyer's initial monotone sequence), rho_l = 1 - (W - mean_m gamma_m,l) / var+ from the sequences' autocovariances
+ *   gamma_m,l (denominator n).  Lags are capped at 63 (32 pairs): ess_lag is the last lag summed, and ess_lag equal to the
+ *   largest odd lag <= min(63, n-1) means the sum was cut at the cap and ess over-estimates the effective sample size.
+ *   A field with a non-finite draw (e.g. the forecast error of a horizon past the end of the series) or W = 0 (a constant
+ *   field), and the loglik field without HMCGPU_FLAG_LOGLIK, give rhat = ess = NaN and ess_lag = -1.  Bit-identical for a
+ *   window however the windows are batched or sharded (given the same draws).
+ *   These three pointers were appended in ABI version 300 and are read only when HMCGPU_FLAG_DIAGNOSTICS is set, so a caller
+ *   built against the shorter struct is never read past its end. */
 typedef struct hmcgpu_result {
     double* mu;
     double* sigma2;
@@ -144,6 +160,10 @@ typedef struct hmcgpu_result {
                              launch on its stream); divided by n_sweep_launches = the average launch duration */
     int32_t sweep_kernel; /* which sweep kernel the plan chose: HMCGPU_KERNEL_* */
     int32_t n_tasks;      /* warp tasks of that kernel (32 lanes each) */
+    /* ---- appended in ABI version 300 (read only with HMCGPU_FLAG_DIAGNOSTICS) */
+    double* rhat;         /* [n_windows x F] split-R̂ */
+    double* ess;          /* [n_windows x F] effective sample size */
+    int32_t* ess_lag;     /* [n_windows x F] last autocorrelation lag in the ESS sum */
 } hmcgpu_result;
 
 #define HMCGPU_KERNEL_THREAD 0  /* one thread per chain (gibbs_sweeps_kernel), wide batches, K <= 8 */
