@@ -53,11 +53,6 @@ template <typename R> __host__ __device__ constexpr size_t wide_group_bytes(int 
     return (sizeof(R) * ((size_t)K * wide_row_stride(K) + 2 * (size_t)W) + sizeof(int) * (size_t)K * K + 15) / 16 * 16;
 }
 
-#ifndef HMC_WIDE_PACKED
-#define HMC_WIDE_PACKED 0   // 1: the fp32 matrix-vector step of the forward recursion as W/2 FFMA2 in two accumulation chains instead of W FFMA in
-                            // four.  Measured a wash (K = 32: 2.73 vs 2.76e9 state-steps/s, K = 16: 5.51 vs 5.46e9, same box, back to back): the
-                            // step is latency-bound, the 16 saved issue slots buy nothing.  Kept as an A/B knob, off.
-#endif
 #ifndef HMC_WIDE_MINBLOCKS32
 #define HMC_WIDE_MINBLOCKS32 5
 #endif
@@ -133,16 +128,11 @@ __global__ void __launch_bounds__(kWideThreads, sizeof(R) == 8 ? 3 : (W == 32 ? 
         rho = rho / WC::gsum(rho, gm);
         __syncwarp(gm);
         // column s of A in registers (zero outside K x K): pred_s = sum_r pf_r A[r][s]
-        // (fp32: kept as W/2 packed pairs, so the matrix-vector step below is W/2 FFMA2 instead of W FFMA — same products, same
-        //  four accumulation chains, bit-identical sums)
-        constexpr bool kPacked = HMC_WIDE_PACKED && sizeof(R) == 4;
-        R Ac[kPacked ? 1 : W];
-        f2 Ac2[kPacked ? W / 2 : 1];
+        R Ac[W];
 #pragma unroll
         for (int r = 0; r < W; r += 2) {
             const R a0 = (act && r < K) ? Asm[r * KP + s] : R(0), a1 = (act && r + 1 < K) ? Asm[(r + 1) * KP + s] : R(0);
-            if constexpr (kPacked) Ac2[r / 2] = mk2((float)a0, (float)a1);
-            else { Ac[r] = a0; Ac[r + 1] = a1; }
+            Ac[r] = a0; Ac[r + 1] = a1;
         }
 
         // ---- 2. forward filter
@@ -203,26 +193,15 @@ __global__ void __launch_bounds__(kWideThreads, sizeof(R) == 8 ? 3 : (W == 32 ? 
             R acc[4] = {R(0), R(0), R(0), R(0)};
             constexpr int kVec = 16 / (int)sizeof(R);                  // elements per 16-byte shared-memory load
             using V = typename std::conditional<sizeof(R) == 4, float4, double2>::type;
-            if constexpr (kPacked) {
-                f2 a01 = splat2(0.f), a23 = splat2(0.f);
 #pragma unroll
-                for (int r0 = 0; r0 < W; r0 += 4) {
-                    const float4 v = *reinterpret_cast<const float4*>(line + r0);
-                    a01 = fma2(mk2(v.x, v.y), Ac2[r0 / 2], a01);
-                    a23 = fma2(mk2(v.z, v.w), Ac2[r0 / 2 + 1], a23);
-                }
-                acc[0] = (R)a01.v.x; acc[1] = (R)a01.v.y; acc[2] = (R)a23.v.x; acc[3] = (R)a23.v.y;
-            } else {
-#pragma unroll
-                for (int r0 = 0; r0 < W; r0 += kVec) {
-                    const V v = *reinterpret_cast<const V*>(line + r0);
-                    if constexpr (sizeof(R) == 4) {
-                        acc[0] = fma((R)v.x, Ac[r0], acc[0]); acc[1] = fma((R)v.y, Ac[r0 + 1], acc[1]);
-                        acc[2] = fma((R)v.z, Ac[r0 + 2], acc[2]); acc[3] = fma((R)v.w, Ac[r0 + 3], acc[3]);
-                    } else {
-                        acc[(r0 / 2) & 3] = fma((R)v.x, Ac[r0], acc[(r0 / 2) & 3]);
-                        acc[(r0 / 2 + 1) & 3] = fma((R)v.y, Ac[r0 + 1], acc[(r0 / 2 + 1) & 3]);
-                    }
+            for (int r0 = 0; r0 < W; r0 += kVec) {
+                const V v = *reinterpret_cast<const V*>(line + r0);
+                if constexpr (sizeof(R) == 4) {
+                    acc[0] = fma((R)v.x, Ac[r0], acc[0]); acc[1] = fma((R)v.y, Ac[r0 + 1], acc[1]);
+                    acc[2] = fma((R)v.z, Ac[r0 + 2], acc[2]); acc[3] = fma((R)v.w, Ac[r0 + 3], acc[3]);
+                } else {
+                    acc[(r0 / 2) & 3] = fma((R)v.x, Ac[r0], acc[(r0 / 2) & 3]);
+                    acc[(r0 / 2 + 1) & 3] = fma((R)v.y, Ac[r0 + 1], acc[(r0 / 2 + 1) & 3]);
                 }
             }
             const R pred = (acc[0] + acc[1]) + (acc[2] + acc[3]);

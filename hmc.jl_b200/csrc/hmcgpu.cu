@@ -1031,12 +1031,12 @@ __global__ void __launch_bounds__(256) window_init_kernel(int K, const double* _
                                                           const int* __restrict__ wT, const unsigned char* __restrict__ sig,
                                                           const long long* __restrict__ wsbase, int sld,
                                                           const long long* __restrict__ X0u, const long long* __restrict__ x0_off,
-                                                          WinInit* __restrict__ out, const int* __restrict__ win_list, int list_off) {
+                                                          WinInit* __restrict__ out) {
     extern __shared__ unsigned char x0[];                 // X0, one byte per time step
     __shared__ double shd[256];
     __shared__ unsigned long long shu[256];
     __shared__ double mu0[32];
-    const int w = win_list ? win_list[list_off + blockIdx.x] : (int)blockIdx.x;   // (a group's windows, in slot order, when the upload is overlapped)
+    const int w = blockIdx.x;
     const int N = wT[w];
     const double* y = y64 + wbase[w];
     const double* yi = wbase_init ? y64 + wbase_init[w] : y;
@@ -1118,10 +1118,9 @@ __global__ void __launch_bounds__(256) window_init_kernel(int K, const double* _
 template <typename R>
 __global__ void chain_init_kernel(int K, int n_slots, const int* __restrict__ slot_win, const WinInit* __restrict__ wi,
                                   const double* __restrict__ xi_user, int* cnt, int* trans, R* Sd, R* Qd, R* cshift, R* xi,
-                                  R* totS, R* totQ, int* events, int* cntM, R* Sm, R* Qm, R* totSm, R* totQm, int* totM,
-                                  int slot_begin, int slot_end) {
-    const int slot = slot_begin + blockIdx.x * blockDim.x + threadIdx.x;   // slots [slot_begin, slot_end)
-    if (slot >= slot_end) return;
+                                  R* totS, R* totQ, int* events, int* cntM, R* Sm, R* Qm, R* totSm, R* totQm, int* totM) {
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot >= n_slots) return;
     const int w = slot_win[slot];
     events[slot] = 0;
     for (int i = 0; i < K; ++i) {
@@ -1163,11 +1162,9 @@ __global__ void sigw_kernel(long long y_len, int S, const unsigned char* __restr
 // y (fp64, series-major as the host gives it) -> time-major copy in the sweep precision (yr[t * n_series + s]); 32 x 32 tiles
 // through shared memory so that both the reads (along time) and the writes (along the series) are coalesced
 template <typename R>
-__global__ void __launch_bounds__(256) y_layout_kernel(long long y_len, int n_series, int s_begin, int s_end, const double* __restrict__ in, R* __restrict__ yr) {
+__global__ void __launch_bounds__(256) y_layout_kernel(long long y_len, int n_series, const double* __restrict__ in, R* __restrict__ yr) {
     __shared__ double tile[32][33];
-    const long long s0 = s_begin + (long long)blockIdx.x * 32, t0 = (long long)blockIdx.y * 32;   // series [s_begin, s_end) only
-    const int ld = n_series;                                        // stride of the time-major copy
-    n_series = n_series < s_end ? n_series : s_end;
+    const long long s0 = (long long)blockIdx.x * 32, t0 = (long long)blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;          // 32 x 8 threads
 #pragma unroll
     for (int j = ty; j < 32; j += 8) {
@@ -1178,7 +1175,7 @@ __global__ void __launch_bounds__(256) y_layout_kernel(long long y_len, int n_se
 #pragma unroll
     for (int j = ty; j < 32; j += 8) {
         const long long t = t0 + j, sidx = s0 + tx;
-        if (sidx < n_series && t < y_len) yr[t * ld + sidx] = (R)tile[tx][j];
+        if (sidx < n_series && t < y_len) yr[t * n_series + sidx] = (R)tile[tx][j];
     }
 }
 
@@ -1295,15 +1292,9 @@ struct hmcgpu_plan {
     bool scan = false;   // narrow batch: one warp per chain, time-parallel (gibbs_scan_kernel.cuh)
     bool wide = false;
     bool seg = false;    // mid-width batch: L lanes per chain, each lane one contiguous time segment (gibbs_seg_kernel.cuh)
-    // Overlapped first run (hmcgpu_estimate on a wide batch of distinct series): the series are uploaded by plan_run, one
-    // contiguous task group at a time, and a group starts sweeping as soon as ITS series have landed and its windows are initialised
-    bool defer = false;
-    const double* host_y = nullptr;
-    long long y_len = 0;
-    int nser = 0, sld = 1;
-    bool has_sig = false;
-    DevBuf yin, order_d;                      // fp64 series-major upload; window ids in slot order
-    std::vector<int> grp_ser_hi, grp_j1, grp_slot1;   // per group: series uploaded so far (exclusive), windows initialised so far, last slot + 1
+    // fp64 series-major upload, read by the window statistics.  A plan member so that it outlives a failed plan_build until
+    // plan_create_impl has drained the stream; released once the stream has drained at the end of plan_build.
+    DevBuf yin;
     int seg_lanes = 0;   // L (a warp task holds 32 / L chains)
     // Mixed segment counts (mid-width batches with spare thread slots): the n_long longest windows run with 8 lanes per chain,
     // in their own slot range [0, long_slots) with their own warp-task tables (task id = slot / 4)
@@ -1406,7 +1397,7 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p) {
 }
 
 template <typename R>
-static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer) {
+static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     hmcgpu_ctx* ctx = pl->ctx;
     cudaStream_t st = ctx->stream;
     const int K = p->K, nw = p->n_windows, nc = p->n_chains, nser = p->n_series;
@@ -1561,40 +1552,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer)
         }
 
     // task groups: interleaved subsets of the (longest-first) warp tasks, each driven through its own stream
-    // Overlapped upload (see hmcgpu_plan::defer): only from hmcgpu_estimate, for a large upload of distinct series whose index
-    // does not decrease in slot order (then contiguous task groups need contiguous, growing series ranges), thread-per-chain plan.
-    // OPT-IN (HMCGPU_OVERLAP=1): measured on C4 (65 536 series x 2000, 110 sweeps) it barely pays — a warp task's own serial time
-    // for the whole job (94 ms) is nearly the device time of the whole batch (109 ms), so a group that starts when its series
-    // have landed still ends 94 ms later: 152 ms per call with 4 groups (175 with 8) against 160 ms for upload-then-run.
     {
-        const char* e = getenv("HMCGPU_OVERLAP");
-        const char* m = getenv("HMCGPU_OVERLAP_MIN_MB");
-        const size_t min_bytes = (size_t)(m ? atoll(m) : 64) << 20;
-        bool ok = want_defer && (e && atoi(e) != 0) && nser > 1 && (size_t)p->y_len * nser * sizeof(double) >= min_bytes &&
-                  !pl->wide && !pl->scan && !pl->seg && !pl->sig && !p->win_init_series && p->win_series && n_warps >= 64;
-        for (int j = 1; ok && j < nw; ++j) ok = p->win_series[pl->order[j]] >= p->win_series[pl->order[j - 1]];
-        pl->defer = ok;
-    }
-    if (pl->defer) {
-        // contiguous groups of warp tasks; per group: the series its windows need (exclusive upper bound, growing), the windows
-        // to initialise (every window exactly once, by the first group that holds one of its chains) and its last slot
-        int G = 4;
-        if (const char* e = getenv("HMCGPU_GROUPS")) G = std::max(1, std::min(8, atoi(e)));
-        G = std::min(G, n_warps);
-        int ser_hi = 0, j_done = 0;
-        for (int g = 0; g < G; ++g) {
-            const int w0 = (int)((long long)n_warps * g / G), w1 = (int)((long long)n_warps * (g + 1) / G);
-            pl->groups.push_back({w0, 1, w1 - w0, 0, false});
-            const long long slot1 = std::min<long long>((long long)w1 * ts, n_real);
-            const int j1 = (int)std::min<long long>(nw, (slot1 + nc - 1) / nc);      // windows with a chain below slot1
-            for (int j = j_done; j < j1; ++j) ser_hi = std::max(ser_hi, p->win_series[pl->order[j]] + 1);
-            j_done = std::max(j_done, j1);
-            pl->grp_ser_hi.push_back(ser_hi);
-            pl->grp_j1.push_back(j_done);
-            pl->grp_slot1.push_back(w1 * ts);
-        }
-        pl->n_groups = G;
-    } else {
         auto n_groups_for = [&](int tasks) {
             int g = (pl->wide || pl->scan) ? 1 : (tasks >= 1024 ? 4 : (tasks >= 256 ? 2 : 1));
             if (const char* e = getenv("HMCGPU_GROUPS")) g = std::max(1, std::min(8, atoi(e)));
@@ -1629,19 +1587,13 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer)
     DevBuf& yin = pl->yin;
     const size_t ny = (size_t)p->y_len * nser;
     PhaseTrace tr;
-    pl->host_y = p->y; pl->y_len = p->y_len; pl->nser = nser;
     if ((p->y_len + 31) / 32 > 65535) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "series longer than %d observations", 65535 * 32);
     CU(ctx, pl->yr.alloc(ny * sizeof(R)));
-    if (pl->defer) {
-        CU(ctx, yin.alloc(ny * sizeof(double)));             // filled group by group in plan_run
-        CU(ctx, up(pl->order_d, pl->order.data(), nw * sizeof(int)));
-    } else {
-        CU(ctx, up(yin, p->y, ny * sizeof(double)));
-        tr.mark("  series upload enqueued");
-        y_layout_kernel<R><<<dim3((unsigned)((nser + 31) / 32), (unsigned)((p->y_len + 31) / 32)), 256, 0, st>>>(p->y_len, nser, 0, nser, yin.as<double>(), pl->yr.as<R>());
-        CU(ctx, cudaGetLastError());
-        tr.sync_mark(st, "  series layout kernel");
-    }
+    CU(ctx, up(yin, p->y, ny * sizeof(double)));
+    tr.mark("  series upload enqueued");
+    y_layout_kernel<R><<<dim3((unsigned)((nser + 31) / 32), (unsigned)((p->y_len + 31) / 32)), 256, 0, st>>>(p->y_len, nser, yin.as<double>(), pl->yr.as<R>());
+    CU(ctx, cudaGetLastError());
+    tr.sync_mark(st, "  series layout kernel");
     CU(ctx, up(pl->wbase, wbase.data(), nw * sizeof(long long)));
     CU(ctx, up(pl->wTd, pl->wT.data(), nw * sizeof(int)));
     CU(ctx, up(pl->slot_win, slot_win.data(), n_slots * sizeof(int)));
@@ -1733,14 +1685,11 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer)
     const size_t smem = (size_t)pl->max_T;
     if (smem > 200 * 1024) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window longer than %d observations", 200 * 1024);
     if (smem > 48 * 1024) CU(ctx, cudaFuncSetAttribute(window_init_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    pl->sld = sld; pl->has_sig = p->is_signal != nullptr;
-    if (!pl->defer) {
-        window_init_kernel<<<nw, 256, smem, st>>>(K, yin.as<double>(), 1, pl->wbase.as<long long>(), pl->wbase_init.as<long long>(),
-                                                  pl->wTd.as<int>(), p->is_signal ? pl->sigmask_tm.as<unsigned char>() : nullptr,
-                                                  pl->wsbase.as<long long>(), sld, pl->X0.as<long long>(),
-                                                  pl->x0_off.as<long long>(), pl->wi.as<WinInit>(), nullptr, 0);
-        CU(ctx, cudaGetLastError());
-    }
+    window_init_kernel<<<nw, 256, smem, st>>>(K, yin.as<double>(), 1, pl->wbase.as<long long>(), pl->wbase_init.as<long long>(),
+                                              pl->wTd.as<int>(), p->is_signal ? pl->sigmask_tm.as<unsigned char>() : nullptr,
+                                              pl->wsbase.as<long long>(), sld, pl->X0.as<long long>(),
+                                              pl->x0_off.as<long long>(), pl->wi.as<WinInit>());
+    CU(ctx, cudaGetLastError());
     tr.sync_mark(st, "  tables, allocations, window statistics");
     yfut_kernel<R><<<grid_for(n_slots, 128), 128, 0, st>>>(n_slots, p->n_h, pl->slot_win.as<int>(), pl->yfut_w.as<double>(), pl->yfut.as<R>());
     CU(ctx, cudaGetLastError());
@@ -1795,7 +1744,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p, bool want_defer)
     tr.mark("  tables, allocations, init");
     CU(ctx, cudaStreamSynchronize(st));
     tr.mark("  stream drained");
-    if (!pl->defer) pl->yin.release();                       // only the window statistics read the fp64 upload
+    pl->yin.release();                                       // only the window statistics read the fp64 upload
     return HMCGPU_OK;
 }
 
@@ -1826,19 +1775,14 @@ static int plan_run_t(hmcgpu_plan* pl) {
         return cudaSuccess;
     };
     CU(ctx, cudaEventRecord(pl->ev0, st));
-    // (first run of a deferred plan: the series are uploaded group by group below, and every group initialises its own chains)
-    const bool overlap = pl->defer && !pl->ran;
-    auto chain_init = [&](int slot_lo, int slot_hi, cudaStream_t cs) -> cudaError_t {
-        chain_init_kernel<R><<<grid_for(slot_hi - slot_lo, 128), 128, 0, cs>>>(Kr, ns, pl->slot_win.as<int>(), pl->wi.as<WinInit>(),
-                                                                pl->xi_user.as<double>(), pl->cnt.as<int>(), pl->trans.as<int>(),
-                                                                pl->Sd.as<R>(), pl->Qd.as<R>(), pl->cshift.as<R>(), pl->xi.as<R>(),
-                                                                pl->totS.as<R>(), pl->totQ.as<R>(), pl->events.as<int>(),
-                                                                pl->cntM.as<int>(), pl->Sm.as<R>(), pl->Qm.as<R>(), pl->totSm.as<R>(),
-                                                                pl->totQm.as<R>(), pl->totM.as<int>(), slot_lo, slot_hi);
-        ++pl->n_launches;
-        return cudaGetLastError();
-    };
-    if (!overlap) CU(ctx, chain_init(0, ns, st));
+    chain_init_kernel<R><<<grid_for(ns, 128), 128, 0, st>>>(Kr, ns, pl->slot_win.as<int>(), pl->wi.as<WinInit>(),
+                                                             pl->xi_user.as<double>(), pl->cnt.as<int>(), pl->trans.as<int>(),
+                                                             pl->Sd.as<R>(), pl->Qd.as<R>(), pl->cshift.as<R>(), pl->xi.as<R>(),
+                                                             pl->totS.as<R>(), pl->totQ.as<R>(), pl->events.as<int>(),
+                                                             pl->cntM.as<int>(), pl->Sm.as<R>(), pl->Qm.as<R>(), pl->totSm.as<R>(),
+                                                             pl->totQm.as<R>(), pl->totM.as<int>());
+    CU(ctx, cudaGetLastError());
+    ++pl->n_launches;
     if (pl->d_diag.p) CU(ctx, cudaMemsetAsync(pl->d_diag.p, 0, 2 * sizeof(unsigned long long), st));
     if (pl->d_sum.p) { CU(ctx, cudaMemsetAsync(pl->d_sum.p, 0, pl->d_sum.bytes, st)); CU(ctx, cudaMemsetAsync(pl->d_sumsq.p, 0, pl->d_sumsq.bytes, st)); }
     if (pl->pacc.p) { CU(ctx, cudaMemsetAsync(pl->pacc.p, 0, pl->pacc.bytes, st)); CU(ctx, cudaMemsetAsync(pl->d_pibsum.p, 0, pl->d_pibsum.bytes, st)); }
@@ -1994,50 +1938,6 @@ static int plan_run_t(hmcgpu_plan* pl) {
             }
             return 0;
     };
-    if (overlap) {
-        // Series upload overlapped with the sweeps: group g's series go up (pinned staging, the host thread drives it), are laid out
-        // and its windows initialised on the context stream; its own stream then initialises its chains and runs every launch up to
-        // the end of the first draw chunk (none of them waits for another group) while the host uploads the next group's series.
-        const long long first_limit = std::min<long long>(S, pl->burnin + std::min<long long>(pl->nrun, pl->chunk));
-        const size_t smem = (size_t)pl->max_T;
-        int ser_lo = 0, j_lo = 0, slot_lo = 0;
-        PhaseTrace trg;
-        for (int g = 0; g < G; ++g) {
-            const int ser_hi = pl->grp_ser_hi[g], j_hi = pl->grp_j1[g], slot_hi = std::min(ns, pl->grp_slot1[g]);
-            if (ser_hi > ser_lo) {
-                const size_t off = (size_t)ser_lo * pl->y_len, cnt = (size_t)(ser_hi - ser_lo) * pl->y_len;
-                CU(ctx, staged_upload(ctx, pl->yin.as<double>() + off, pl->host_y + off, cnt * sizeof(double), st));
-                pl->h2d += (long long)(cnt * sizeof(double));
-                trg.mark("    group upload");
-                y_layout_kernel<R><<<dim3((unsigned)((ser_hi - ser_lo + 31) / 32), (unsigned)((pl->y_len + 31) / 32)), 256, 0, st>>>(
-                    pl->y_len, pl->nser, ser_lo, ser_hi, pl->yin.as<double>(), pl->yr.as<R>());
-                CU(ctx, cudaGetLastError());
-                ++pl->n_launches;
-                ser_lo = ser_hi;
-            }
-            if (j_hi > j_lo) {
-                window_init_kernel<<<j_hi - j_lo, 256, smem, st>>>(Kr, pl->yin.as<double>(), 1, pl->wbase.as<long long>(), pl->wbase_init.as<long long>(),
-                                                                   pl->wTd.as<int>(), pl->has_sig ? pl->sigmask_tm.as<unsigned char>() : nullptr,
-                                                                   pl->wsbase.as<long long>(), pl->sld, pl->X0.as<long long>(),
-                                                                   pl->x0_off.as<long long>(), pl->wi.as<WinInit>(), pl->order_d.as<int>(), j_lo);
-                CU(ctx, cudaGetLastError());
-                ++pl->n_launches;
-                j_lo = j_hi;
-            }
-            cudaEvent_t ready;
-            CU(ctx, new_event(&ready));
-            CU(ctx, cudaEventRecord(ready, st));
-            CU(ctx, cudaStreamWaitEvent(pl->gstreams[g], ready, 0));
-            if (slot_hi > slot_lo) CU(ctx, chain_init(slot_lo, slot_hi, pl->gstreams[g]));
-            slot_lo = slot_hi;
-            while (next[g] < first_limit) {
-                const int rc = enqueue_one(g, 1);
-                if (rc < 0) return rc;
-                if (rc > 0) break;
-            }
-            trg.mark("    group launches enqueued");
-        }
-    }
     PhaseTrace trr;
     // launches are enqueued round-robin over the groups; a launch never crosses the end of burn-in or of a draw chunk
     bool more = true;
@@ -2049,12 +1949,12 @@ static int plan_run_t(hmcgpu_plan* pl) {
         for (int g : gorder) {
             if (next[g] >= S) continue;
             more = true;
-            const int rc = enqueue_one(g, overlap ? round + 1 : round);
+            const int rc = enqueue_one(g, round);
             if (rc < 0) return rc;
         }
     }
     CU(ctx, cudaEventRecord(pl->ev1, st));                   // st has waited for every group through the last chunk's post
-    trr.mark("    remaining launches enqueued");
+    trr.mark("    launches enqueued");
     CU(ctx, cudaEventSynchronize(pl->ev1));
     trr.mark("    device drained");
     for (int g = 0; g < G; ++g) CU(ctx, cudaStreamSynchronize(pl->gstreams[g]));
@@ -2068,20 +1968,6 @@ static int plan_run_t(hmcgpu_plan* pl) {
         float t = 0.f;
         CU(ctx, cudaEventElapsedTime(&t, pl->evk0, gend[g]));
         pl->sweep_ms = std::max(pl->sweep_ms, (double)t);
-    }
-    if (overlap && getenv("HMCGPU_VERBOSE") && launch_timing) {      // when did every group start and end (ms after the start of the run)?
-        std::vector<float> first(G, -1.f);
-        size_t q = 0;
-        for (auto& pr : launch_pairs) {                              // (the prologue enqueued the groups one after the other; 7 launches per group on the C4 shape this trace was written for)
-            float t = 0.f;
-            if (cudaEventElapsedTime(&t, pl->ev0, pr.first) == cudaSuccess) { const int g = (int)std::min<size_t>(G - 1, q / 7); if (first[g] < 0.f) first[g] = t; }
-            ++q;
-        }
-        for (int g = 0; g < G; ++g) {
-            float t1 = 0.f;
-            cudaEventElapsedTime(&t1, pl->ev0, gend[g]);
-            fprintf(stderr, "[hmcgpu]     group %d: first launch starts %.2f ms, last ends %.2f ms\n", g, first[g], t1);
-        }
     }
     pl->launch_ms_sum = 0.0;
     for (auto& pr : launch_pairs) {
@@ -2103,13 +1989,13 @@ static int plan_run_t(hmcgpu_plan* pl) {
     return HMCGPU_OK;
 }
 
-static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out, bool want_defer = false) {
+static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out) {
     TRY(validate_problem(ctx, p));
     CU(ctx, cudaSetDevice(ctx->device));
     tl_pool = ctx->pool;
     std::unique_ptr<hmcgpu_plan> pl(new hmcgpu_plan());
     pl->ctx = ctx;
-    int rc = (p->precision == 32) ? plan_build<float>(pl.get(), p, want_defer) : plan_build<double>(pl.get(), p, want_defer);
+    int rc = (p->precision == 32) ? plan_build<float>(pl.get(), p) : plan_build<double>(pl.get(), p);
     if (rc != 0) {
         cudaStreamSynchronize(ctx->stream);    // uploads / init kernels may still be queued on buffers the plan is about to release
         cudaGetLastError();
@@ -2117,11 +2003,6 @@ static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_pla
     }
     *out = pl.release();
     return HMCGPU_OK;
-}
-
-static int plan_create_for_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out) {
-    *out = nullptr;
-    GUARD(ctx, plan_create_impl(ctx, p, out, true));
 }
 
 extern "C" int hmcgpu_plan_create(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out) {
@@ -2246,7 +2127,7 @@ extern "C" int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_
     if (!r) return fail(ctx, HMCGPU_ERR_ARG, "result is NULL");
     hmcgpu_plan* pl = nullptr;
     PhaseTrace tr;
-    TRY(plan_create_for_estimate(ctx, p, &pl));            // (may defer the series upload into plan_run, overlapped with the sweeps)
+    TRY(hmcgpu_plan_create(ctx, p, &pl));
     tr.mark("plan_create (upload, init)");
     int rc = hmcgpu_plan_run(pl);
     tr.mark("plan_run (all sweeps)");

@@ -454,38 +454,6 @@ def test_staged_upload_of_large_series_is_bit_identical(H, ctx, monkeypatch):
     assert outs[0].h2d_bytes == outs[1].h2d_bytes
 
 
-def test_overlapped_series_upload_is_bit_identical(H, ctx, monkeypatch):
-    """hmcgpu_estimate on a wide batch of distinct series defers the series upload into the run: contiguous task groups, each
-    starting as soon as ITS series have landed and its windows are initialised, while the host uploads the next group's series
-    (hmcgpu.cu, plan_run_t `overlap`).  Same results as the plain path, bit for bit: ragged windows, several windows per series
-    (a window's chains straddling two groups), 3 chains per window, staged and plain copies."""
-    monkeypatch.setenv("HMCGPU_SCAN_MAX_CHAINS", "0")
-    monkeypatch.setenv("HMCGPU_SEG_LANES", "0")
-    rng = np.random.default_rng(5)
-    base = np.stack([synth_hmm(400, seed=s, **K3_TRUTH)[0] for s in range(6)])
-    nser = 2400
-    ys = np.ascontiguousarray(np.tile(base, (nser // 6, 1)) + 1e-3 * rng.standard_normal((nser, 400)))     # 7.7 MB
-    ser = np.sort(np.concatenate([np.arange(nser), rng.integers(0, nser, 300)])).astype(np.int32)          # 2700 windows, some series twice
-    starts = rng.integers(1, 40, len(ser)).astype(np.int32)
-    ends = (starts + rng.integers(60, 340, len(ser))).astype(np.int32)
-    kw = dict(K=3, n_chains=3, burnin=3, nrun=5, seed=9, horizons=(1, 6), precision=32, flags=H.FLAG_REF_Q1 | H.FLAG_SUMMARY | H.FLAG_DRAWS,
-              win_series=ser)
-    monkeypatch.setenv("HMCGPU_OVERLAP", "0")
-    plain = _run(H, ctx, ys, starts, ends, **kw)
-    assert plain.sweep_kernel == 0 and plain.events == 0
-    for stage_mb in ("0", "1"):
-        monkeypatch.setenv("HMCGPU_OVERLAP", "1")
-        monkeypatch.setenv("HMCGPU_OVERLAP_MIN_MB", "0")
-        monkeypatch.setenv("HMCGPU_STAGE_MB", stage_mb)
-        o = _run(H, ctx, ys, starts, ends, **kw)
-        np.testing.assert_array_equal(o.summary_mean, plain.summary_mean)
-        np.testing.assert_array_equal(o.summary_var, plain.summary_var)
-        for w in (0, 1, 1350, len(ser) - 1):
-            np.testing.assert_array_equal(o.mu[w], plain.mu[w])
-            np.testing.assert_array_equal(o.forecasts[w], plain.forecasts[w])
-        assert o.h2d_bytes == plain.h2d_bytes and o.events == 0
-
-
 def test_plan_run_is_repeatable_and_device_resident(H, ctx):
     y, _ = synth_hmm(220, **K3_TRUTH)
     spec = H.ProblemSpec(y, [1, 1], [200, 150], K=3, n_chains=40, burnin=20, nrun=30, seed=3, horizons=(12,), precision=32,
