@@ -55,20 +55,7 @@ template <typename R, int K> cudaError_t launch_gibbs(const GibbsLaunch& cfg, co
     return with_rows<R, K>(cfg, [&](auto kern) { return go(kern, smem); });
 }
 
-template <typename R, int K> int gibbs_capacity_warps(const GibbsLaunch& cfg) {
-    auto q = [&](auto kern, size_t smem) {
-        int per_sm = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kGibbsThreads, smem) != cudaSuccess) { cudaGetLastError(); per_sm = 1; }
-        return per_sm * cfg.sm_count * (kGibbsThreads / 32);
-    };
-    const bool wr = K > 4 || wide_rows<K>(cfg);
-    const size_t smem = wr ? gibbs_smem_bytes<R, K, true>(cfg.flags & (8u | 64u), cfg.n_h) : gibbs_smem_bytes<R, K, false>(cfg.flags & (8u | 64u), cfg.n_h);
-    return with_rows<R, K>(cfg, [&](auto kern) { return q(kern, smem); });
-}
-
 template cudaError_t launch_gibbs<HMC_R, HMC_K>(const GibbsLaunch&, const GibbsArgs&, cudaStream_t);
-
-template int gibbs_capacity_warps<HMC_R, HMC_K>(const GibbsLaunch&);
 
 #if HMC_K <= 4
 // narrow batches: one warp per chain, time-parallel (gibbs_scan_kernel.cuh); covers every slot in one launch

@@ -20,6 +20,7 @@
 #include <mutex>
 #include <new>
 #include <numeric>
+#include <optional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -207,12 +208,37 @@ extern "C" int hmcgpu_ctx_sync(hmcgpu_ctx* ctx) {
 
 static bool k_supported(int K) { return K >= 2 && K <= 32; }
 static bool k_thread(int K) { return K >= 2 && K <= 4; }       // every feature (smoothed means, signals, K-templated entry points)
-// sweeps: thread-per-chain kernels for K = 2..8, lane-per-state kernel for K = 9..32 (HMCGPU_LANE_KERNEL=1: also for 5..8)
-static bool k_thread_sweep(int K) {
-    if (K >= 2 && K <= 4) return true;
-    const char* e = getenv("HMCGPU_LANE_KERNEL");
-    return K >= 5 && K <= 8 && !(e && atoi(e) != 0);
+// The HMCGPU_* tuning variables (INTEGRATION.md), read once per plan at hmcgpu_plan_create.  An unset optional leaves the
+// choice to the plan; the bools are "value != 0".
+struct Tuning {
+    bool lane_kernel = false, seg_mixed = true, y_smem = true, launch_timing = true, verbose = false;
+    int seg_warm = 32, seg_barriers = 2;
+    std::optional<long long> scan_max_chains, seg_long;
+    std::optional<int> seg_lanes, groups, seg_threads, sweeps_per_launch;
+};
+static Tuning read_tuning() {
+    Tuning t;
+    const char* e;
+    if ((e = getenv("HMCGPU_LANE_KERNEL"))) t.lane_kernel = atoi(e) != 0;
+    if ((e = getenv("HMCGPU_SCAN_MAX_CHAINS"))) t.scan_max_chains = atoll(e);
+    if ((e = getenv("HMCGPU_SEG_LANES"))) t.seg_lanes = atoi(e);
+    if ((e = getenv("HMCGPU_SEG_MIXED"))) t.seg_mixed = atoi(e) != 0;
+    if ((e = getenv("HMCGPU_SEG_LONG"))) t.seg_long = atoll(e);
+    if ((e = getenv("HMCGPU_GROUPS"))) t.groups = std::max(1, std::min(8, atoi(e)));
+    if ((e = getenv("HMCGPU_Y_SMEM"))) t.y_smem = atoi(e) != 0;
+    if ((e = getenv("HMCGPU_SEG_WARMUP"))) t.seg_warm = std::max(0, atoi(e));
+    if ((e = getenv("HMCGPU_SEG_BARRIERS"))) t.seg_barriers = atoi(e);
+    if ((e = getenv("HMCGPU_SEG_THREADS"))) t.seg_threads = atoi(e);
+    if ((e = getenv("HMCGPU_SWEEPS_PER_LAUNCH"))) t.sweeps_per_launch = std::max(1, atoi(e));
+    if ((e = getenv("HMCGPU_LAUNCH_TIMING"))) t.launch_timing = atoi(e) != 0;
+    if ((e = getenv("HMCGPU_VERBOSE"))) t.verbose = atoi(e) != 0;
+    return t;
 }
+
+// sweeps: thread-per-chain kernels for K = 2..8, lane-per-state kernel for K = 9..32 (HMCGPU_LANE_KERNEL=1: also for 5..8)
+static bool k_thread_sweep(int K, const Tuning& t) { return (K >= 2 && K <= 4) || (K >= 5 && K <= 8 && !t.lane_kernel); }
+
+enum class SweepKernel : int32_t { thread = HMCGPU_KERNEL_THREAD, scan = HMCGPU_KERNEL_SCAN, lane = HMCGPU_KERNEL_LANE, seg = HMCGPU_KERNEL_SEG };
 
 #define DISPATCH_K(K, ...)                          \
     switch (K) {                                    \
@@ -222,9 +248,9 @@ static bool k_thread_sweep(int K) {
         default: break;                             \
     }
 #ifdef HMC_DEV_F3   /* experiment builds: only the fp32 K=3 sweep kernels are linked */
-#define DISPATCH_RUN(pl, rc) do { if ((pl)->precision == 32) { if ((pl)->wide) rc = plan_run_t<float, 0>(pl); else if ((pl)->K == 3) rc = plan_run_t<float, 3>(pl); } } while (0)
+#define DISPATCH_RUN(pl, rc) do { if ((pl)->precision == 32) { if ((pl)->sw.kernel == SweepKernel::lane) rc = plan_run_t<float, 0>(pl); else if ((pl)->K == 3) rc = plan_run_t<float, 3>(pl); } } while (0)
 #elif defined(HMC_DEV_D3)   /* ... or only the fp64 K=3 ones */
-#define DISPATCH_RUN(pl, rc) do { if ((pl)->precision == 64) { if ((pl)->wide) rc = plan_run_t<double, 0>(pl); else if ((pl)->K == 3) rc = plan_run_t<double, 3>(pl); } } while (0)
+#define DISPATCH_RUN(pl, rc) do { if ((pl)->precision == 64) { if ((pl)->sw.kernel == SweepKernel::lane) rc = plan_run_t<double, 0>(pl); else if ((pl)->K == 3) rc = plan_run_t<double, 3>(pl); } } while (0)
 #else
 #define DISPATCH_K8(K, ...)                         \
     switch (K) {                                    \
@@ -239,7 +265,7 @@ static bool k_thread_sweep(int K) {
     }
 #define DISPATCH_RUN(pl, rc)                                                                                          \
     do {                                                                                                            \
-        if ((pl)->wide) rc = ((pl)->precision == 32) ? plan_run_t<float, 0>(pl) : plan_run_t<double, 0>(pl);       \
+        if ((pl)->sw.kernel == SweepKernel::lane) rc = ((pl)->precision == 32) ? plan_run_t<float, 0>(pl) : plan_run_t<double, 0>(pl);       \
         else DISPATCH_K8((pl)->K, { rc = ((pl)->precision == 32) ? plan_run_t<float, KK>(pl) : plan_run_t<double, KK>(pl); }) \
     } while (0)
 #endif
@@ -1269,6 +1295,17 @@ __global__ void tile_reduce_kernel(int K, int ncols, int n_chains, const int* __
     }
 }
 
+// Which sweep kernel a plan runs, and how (choose_sweep)
+struct SweepChoice {
+    SweepKernel kernel = SweepKernel::thread;
+    int seg_lanes = 0;           // segment kernel: L lanes per chain (a warp task holds 32 / L chains)
+    // Mixed segment counts (mid-width batches with spare thread slots): the n_long longest windows run with 8 lanes per chain,
+    // in their own slot range with their own warp-task tables (task id = slot / 4)
+    int n_long = 0;
+    int sweeps_per_launch = 16;
+    int seg_threads = 128;       // threads per block of the segment kernel
+};
+
 struct hmcgpu_plan {
     hmcgpu_ctx* ctx = nullptr;
     // problem (host copies)
@@ -1282,27 +1319,21 @@ struct hmcgpu_plan {
     std::vector<long long> pib_off;      // per window (caller order) offset in pib_mean
     long long pib_total = 0;
     long long state_steps = 0;
-    int n_slots = 0, n_warps = 0, chunk = 0, max_T = 0;
+    int n_slots = 0, n_warps = 0, n_tasks = 0, chunk = 0, max_T = 0;   // (n_tasks: warp tasks of both classes)
     GibbsArgs args{};
     // device buffers
     DevBuf yr, wbase, wTd, wi, slot_win, slot_chain, T, ybase, warp_T, warp_pi_off, pi, pacc, facc, cnt, trans, Sd, Qd,
         events, cshift, xi, xi_user, chain_id, out, yfut_w, yfut, win_slot0, win_pib_off, totS, totQ, slot_pi_off;
     DevBuf sigmask, sigmask_tm, sigw, sbase, wsbase, wbase_init, X0, x0_off, cntM, Sm, Qm, totSm, totQm, totM;    // signals tier / user initial states
     bool sig = false;    // SIG kernels: signal mask and / or pi_row_back
-    bool scan = false;   // narrow batch: one warp per chain, time-parallel (gibbs_scan_kernel.cuh)
-    bool wide = false;
-    bool seg = false;    // mid-width batch: L lanes per chain, each lane one contiguous time segment (gibbs_seg_kernel.cuh)
+    Tuning tuning;
+    SweepChoice sw;
     // fp64 series-major upload, read by the window statistics.  A plan member so that it outlives a failed plan_build until
     // plan_create_impl has drained the stream; released once the stream has drained at the end of plan_build.
     DevBuf yin;
-    int seg_lanes = 0;   // L (a warp task holds 32 / L chains)
-    // Mixed segment counts (mid-width batches with spare thread slots): the n_long longest windows run with 8 lanes per chain,
-    // in their own slot range [0, long_slots) with their own warp-task tables (task id = slot / 4)
-    int n_long = 0, long_slots = 0;
-    DevBuf warp_T_long, warp_pi_off_long;
+    DevBuf warp_T_long, warp_pi_off_long;     // warp-task tables of the long class (SweepChoice::n_long)
     struct Group { int task0, stride, n_tasks, lanes; bool long_class; };
     std::vector<Group> groups;                // one stream each (plan_run)
-    int seg_threads = 128; // threads per block of the segment kernel
     int n_groups = 1, n_bufs = 1;
     std::vector<cudaStream_t> gstreams;
     std::vector<cudaEvent_t> pool_events;
@@ -1329,13 +1360,13 @@ struct hmcgpu_plan {
     }
 };
 
-static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p) {
+static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuning& t) {
     if (!ctx) return HMCGPU_ERR_ARG;
     if (!p) return fail(ctx, HMCGPU_ERR_ARG, "problem is NULL");
     if (!p->y || p->y_len < 2 || p->n_series < 1) return fail(ctx, HMCGPU_ERR_ARG, "empty series");
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(ctx, HMCGPU_ERR_ARG, "no windows");
     if (!k_supported(p->K)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "K=%d not supported (2..32)", p->K);
-    if (!k_thread_sweep(p->K) && (p->flags & HMCGPU_FLAG_SMOOTHED_MEAN))
+    if (!k_thread_sweep(p->K, t) && (p->flags & HMCGPU_FLAG_SMOOTHED_MEAN))
         return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "smoothed means are only implemented for K <= 8 (thread-per-chain kernels)");
     if (p->K > 4 && (p->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)) && p->n_h > 0) {
         // the A^h mu vectors of the in-sample forecasts live in shared memory next to the selection tables and the rings
@@ -1345,7 +1376,7 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p) {
             return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "K=%d with %d in-sample forecast horizons needs %zu KB of shared memory per block: use fewer horizons", p->K, p->n_h, need / 1024);
     }
     if (p->flags & HMCGPU_FLAG_FILTERED_MEAN) {
-        if (!k_thread_sweep(p->K)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "filtered means are only implemented for K <= 8");
+        if (!k_thread_sweep(p->K, t)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "filtered means are only implemented for K <= 8");
         if (p->flags & HMCGPU_FLAG_SMOOTHED_MEAN) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_FILTERED_MEAN and HMCGPU_FLAG_SMOOTHED_MEAN share their output arrays: one per call");
         if (p->is_signal || p->pi_row_back != 0) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "is_signal / pi_row_back cannot be combined with HMCGPU_FLAG_FILTERED_MEAN");
     }
@@ -1396,6 +1427,154 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p) {
     return 0;
 }
 
+static int scan_max_T_of(int precision, int K) { DISPATCH_K(K, return precision == 32 ? scan_max_T<float, KK>() : scan_max_T<double, KK>()); return 0; }
+static long long seg_max_T_of(int K, int lanes) { DISPATCH_K(K, return seg_max_T<KK>(lanes)); return 0; }
+
+// The sweep-kernel policy (SweepChoice).  wT / order: the window lengths and the windows by decreasing length.  No device
+// work; ctx gives the SM count and takes the error text.
+static int choose_sweep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const std::vector<int>& wT, const std::vector<int>& order,
+                        const Tuning& t, SweepChoice& c) {
+    const int K = p->K, nw = p->n_windows, nc = p->n_chains, max_T = wT[order[0]];
+    const bool sig = p->is_signal != nullptr || p->pi_row_back != 0;
+    const bool acc_mean = p->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN);   // per-date means: thread-per-chain kernels only
+    const long long n_real = (long long)nw * nc;
+    const long long full = (long long)ctx->sm_count * 16 * 32;     // one wave of thread slots (16 warps per SM)
+    c = SweepChoice{};
+    if (!k_thread_sweep(K, t)) c.kernel = SweepKernel::lane;
+    if (K <= 4 && !acc_mean) {
+        // Narrow batches (the reference's own regime: one chain per end date) cannot fill the GPU with a thread per chain:
+        // below kScanMaxChains chains the time-parallel warp-per-chain kernel is used (K <= 4, plain sweep, window in smem).
+        // (the signals tier has no segment kernel: there the warp-per-chain kernel serves up to 12 288 chains; for the plain
+        //  sweep the segment kernel takes over from ~4000 chains — measured crossover on C2, DESIGN.md section 7)
+        const bool seg_ok = !sig && !(t.seg_lanes && *t.seg_lanes == 0);
+        long long lim = t.scan_max_chains.value_or(seg_ok ? 4096 : 12288);
+        // long windows leave room for fewer resident warps (the window lives in shared memory): scale the bound with them
+        const size_t wb = (size_t)(p->precision / 8) * ((size_t)max_T * (K + 1) + 4 * K);
+        const long long blocks = std::max<long long>(1, std::min<long long>(5, (long long)((227 * 1024) / (4 * wb + 1024))));
+        lim = lim * blocks / 5;
+        if (n_real <= lim && max_T <= scan_max_T_of(p->precision, K)) c.kernel = SweepKernel::scan;
+    }
+    // Mid-width batches (too many chains for a warp each, too few to fill the schedulers with a thread each): L lanes per
+    // chain, one time segment per lane (gibbs_seg_kernel.cuh).  L is chosen so that the batch yields about one full wave of
+    // warps; HMCGPU_SEG_LANES forces it (0 = never).  K <= 4, plain sweep.
+    if (K <= 4 && !acc_mean && !sig && c.kernel != SweepKernel::scan) {
+        int lanes = 0;
+        // measured on C2 (500 windows x c chains, B200): 4 lanes per chain are best up to ~38 000 chains, 2 lanes up to ~90 000,
+        // the thread-per-chain kernel beyond (DESIGN.md section 7); in units of one wave of thread slots:
+        if (n_real * 2 <= full) lanes = 4;
+        // (2 lanes only when the chains share one series: a batch of distinct series streams every observation from HBM in each
+        //  of the segment kernel's passes — C4, 65 536 series: 143 ms with 2 lanes, 139 ms with 4, 109 ms with a thread per chain)
+        else if (n_real * 4 <= 5 * full && p->n_series == 1) lanes = 2;
+        if (t.seg_lanes) lanes = *t.seg_lanes;
+        if (lanes != 0 && lanes != 2 && lanes != 4 && lanes != 8) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_SEG_LANES must be 0, 2, 4 or 8");
+        if (lanes && max_T > seg_max_T_of(K, lanes)) lanes = 0;
+        if (lanes) c.kernel = SweepKernel::seg;
+        c.seg_lanes = lanes;
+        // With 4 lanes per chain and thread slots to spare, the sweep time is the serial time of the LONGEST windows (every warp is
+        // resident from the start; a 16 000-chain batch leaves a fifth of the slots empty).  The longest tenth of the windows (in
+        // `order`) then gets 8 lanes per chain — half the dependent steps per sweep — as far as the slots last.  Measured on C2
+        // (HMCGPU_SEG_LONG sweep, scripts/r2_call_j.sh): 50 of 500 windows +7 % at 16 chains per window, +2 % at 24, +4 % at 32;
+        // 100 windows +7 % at 32 but -5 % at 24; 300 or all of them lose everywhere (8 lanes pay more per-sweep work per chain).
+        // HMCGPU_SEG_MIXED=0 disables it; a forced HMCGPU_SEG_LANES is uniform.
+        if (lanes == 4 && !t.seg_lanes && t.seg_mixed) {
+            const long long spare = full * 115 / 100 - n_real * 4;
+            long long n8 = spare > 0 ? std::min<long long>(nw / 10, spare / ((long long)nc * 4)) : 0;
+            while (n8 > 0 && wT[order[n8 - 1]] < 128) --n8;          // (segments of fewer than 16 steps are all warm-up)
+            if (t.seg_long) n8 = std::max(0ll, std::min<long long>(nw, *t.seg_long));
+            if (n8 * nc >= 32 && max_T <= seg_max_T_of(K, 8)) c.n_long = (int)n8;
+        }
+    }
+    if (c.kernel == SweepKernel::seg) {
+        // 256-thread blocks (8 warps stepping through the phases of a sweep together) when that still gives every SM a block
+        // and a half; otherwise 128.  Warp tasks: 4 chains each in the long class, 32 / L in the rest, each class padded to 32.
+        const long long n8c = (long long)c.n_long * nc, tasks = (n8c + 31) / 32 * 8 + (n_real - n8c + 31) / 32 * c.seg_lanes;
+        c.seg_threads = t.seg_threads.value_or(tasks / (kSegThreads / 32) >= ctx->sm_count * 3 / 2 ? kSegThreads : 128);
+    }
+    // Sweeps per launch.  Short launches bound the damage of the priority-based warp arbiter (a starved warp can only fall
+    // behind by one launch) and give the block scheduler a steady supply of pending blocks from the other groups.  A scan
+    // sweep is a few µs.
+    c.sweeps_per_launch = t.sweeps_per_launch.value_or(c.kernel == SweepKernel::scan ? 64 : 16);
+    return HMCGPU_OK;
+}
+
+// Host tables of the chain slots and warp tasks (uploaded by plan_build)
+struct SlotLayout {
+    std::vector<int> slot_win, slot_chain, Ts, win_slot0, warp_T, warp_T_long;
+    std::vector<long long> ybase, warp_off, warp_off_long, slot_off;   // slot_off: the lane kernel's pi row of each slot
+    std::vector<unsigned> chain_id;
+    long long pi_elems = 0;
+};
+
+// Lays out the plan's chain slots, warp tasks, pi offsets and task groups for its SweepChoice; sets n_slots, n_warps,
+// n_tasks and the groups.
+static SlotLayout layout_slots(hmcgpu_plan* pl, const hmcgpu_problem* p) {
+    const int K = p->K, nw = p->n_windows, nc = p->n_chains, nser = p->n_series;
+    const SweepChoice& c = pl->sw;
+    const bool seg = c.kernel == SweepKernel::seg;
+    const int ts = 32;
+    // slots: windows by decreasing T, chains consecutive; [long class (8 lanes), padded to 32][the rest, padded to 32]
+    const int long_slots = (int)(((long long)c.n_long * nc + ts - 1) / ts * ts);
+    const int n_slots = long_slots + (int)(((long long)nw * nc - (long long)c.n_long * nc + ts - 1) / ts * ts);
+    const int cpt = seg ? 32 / c.seg_lanes : ts;            // chains per warp task
+    const int n_warps = n_slots / cpt;                      // number of warp tasks (task id = slot / cpt; ids below long_slots / cpt are unused when there is a long class)
+    pl->n_slots = n_slots; pl->n_warps = n_warps;
+    SlotLayout s;
+    s.slot_win.assign(n_slots, -1); s.slot_chain.assign(n_slots, 0); s.Ts.assign(n_slots, 0); s.ybase.assign(n_slots, 0);
+    s.chain_id.assign(n_slots, 0); s.slot_off.assign(n_slots, 0); s.win_slot0.assign(nw, 0);
+    s.warp_T.assign(n_warps, 0); s.warp_off.assign(n_warps, 0);
+    for (int j = 0; j < nw; ++j) {
+        const int w = pl->order[j];
+        const int s0w = j < c.n_long ? j * nc : long_slots + (j - c.n_long) * nc;
+        s.win_slot0[w] = s0w;
+        const unsigned long long wid = p->win_id ? (unsigned long long)p->win_id[w] : (unsigned long long)w;
+        for (int cidx = 0; cidx < nc; ++cidx) {
+            const int slot = s0w + cidx;
+            s.slot_win[slot] = w; s.slot_chain[slot] = cidx; s.Ts[slot] = pl->wT[w];
+            s.ybase[slot] = (long long)(p->win_start[w] - 1) * nser + (p->win_series ? p->win_series[w] : 0);   // time-major [y_len][n_series] (the sweeps)
+            s.chain_id[slot] = (unsigned)(wid * (unsigned long long)nc + (unsigned long long)cidx);
+        }
+    }
+    // the long class first (8 lanes per chain: 4 chains per task, task id = slot / 4)
+    s.warp_T_long.assign(long_slots / 4, 0);
+    s.warp_off_long.assign(long_slots / 4, 0);
+    for (int wp = 0; wp < long_slots / 4; ++wp) {
+        int m = 0;
+        for (int l = 0; l < 4; ++l) m = std::max(m, s.Ts[wp * 4 + l]);
+        const int Cs = std::max(4, (m + 31) / 32 * 4);
+        s.warp_T_long[wp] = Cs;
+        s.warp_off_long[wp] = s.pi_elems;
+        s.pi_elems += (long long)Cs * K * 32;
+    }
+    for (int wp = long_slots / cpt; wp < n_warps; ++wp) {
+        int m = 0;
+        for (int l = 0; l < cpt; ++l) m = std::max(m, s.Ts[wp * cpt + l]);
+        s.warp_T[wp] = m;
+        s.warp_off[wp] = s.pi_elems;
+        if (seg) {
+            // segment kernel: every lane owns a frame of C = 4 ceil(T / 4L) rows (warp_T holds C), tiled like the thread kernel's
+            const int Cs = std::max(4, (m + 4 * c.seg_lanes - 1) / (4 * c.seg_lanes) * 4);
+            s.warp_T[wp] = Cs;
+            s.pi_elems += (long long)Cs * K * 32;
+        }
+        // thread-per-chain kernels: rows right-aligned to tiles of 4 time steps (gibbs_kernel.cuh, st_quad)
+        else if (c.kernel != SweepKernel::lane) s.pi_elems += (long long)((m + 3) / 4 * 4) * K * ts;
+        else for (int l = 0; l < ts; ++l) { s.slot_off[wp * ts + l] = s.pi_elems; s.pi_elems += (long long)s.Ts[wp * ts + l] * K; }
+    }
+    // task groups: interleaved subsets of the (longest-first) warp tasks of a class, each driven through its own stream
+    auto add_groups = [&](int task0, int tasks, int lanes, bool long_class) {
+        if (tasks <= 0) return;
+        int g = pl->tuning.groups.value_or((c.kernel == SweepKernel::lane || c.kernel == SweepKernel::scan) ? 1 : (tasks >= 1024 ? 4 : (tasks >= 256 ? 2 : 1)));
+        g = std::max(1, std::min(g, tasks));
+        for (int q = 0; q < g; ++q) pl->groups.push_back({task0 + q, g, (tasks - q + g - 1) / g, lanes, long_class});
+    };
+    const int t_long = long_slots / 4, t_first = long_slots / cpt, t_rest = n_warps - t_first;
+    add_groups(0, t_long, 8, true);
+    add_groups(t_first, t_rest, c.seg_lanes, false);
+    pl->n_groups = (int)pl->groups.size();
+    pl->n_tasks = t_long + t_rest;
+    return s;
+}
+
 template <typename R>
 static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     hmcgpu_ctx* ctx = pl->ctx;
@@ -1407,13 +1586,25 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     pl->wT.resize(nw);
     pl->order.resize(nw);
     pl->pib_off.resize(nw);
+    // per-window tables; forecasts: realised y at end+h per window (NaN outside the series)
+    std::vector<long long> wbase(nw), wbase_init(nw), x0_off(nw);
+    std::vector<double> yfut_w((size_t)nw * std::max(1, p->n_h), NAN);
     long long sumT = 0, pib_total = 0;
     for (int w = 0; w < nw; ++w) {
         pl->wT[w] = p->win_end[w] - p->win_start[w] + 1;
         pl->pib_off[w] = pib_total;
         pib_total += (long long)pl->wT[w] * K;
+        x0_off[w] = sumT;
         sumT += pl->wT[w];
         pl->max_T = std::max(pl->max_T, pl->wT[w]);
+        const int ser = p->win_series ? p->win_series[w] : 0;
+        // the window statistics read the fp64 series as uploaded (series-major: a window is contiguous)
+        wbase[w] = (long long)ser * p->y_len + (p->win_start[w] - 1);
+        wbase_init[w] = (long long)(p->win_init_series ? p->win_init_series[w] : ser) * p->y_len + (p->win_start[w] - 1);
+        for (int j = 0; j < p->n_h; ++j) {
+            const long long idx = (long long)p->win_end[w] + p->horizons[j];   // 1-based
+            if (idx <= p->y_len) yfut_w[(size_t)w * p->n_h + j] = p->y[(size_t)ser * p->y_len + idx - 1];
+        }
     }
     pl->pib_total = pib_total;
     if (k_thread(K) && (long long)pl->max_T - 1 > ((1ll << (64 / K)) - 1)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window too long for K=%d", K);
@@ -1421,155 +1612,15 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     std::iota(pl->order.begin(), pl->order.end(), 0);
     std::stable_sort(pl->order.begin(), pl->order.end(), [&](int a, int b) { return pl->wT[a] > pl->wT[b]; });
 
-    // slots: windows by decreasing T, chains consecutive; padded to a multiple of the task size (32 chains per warp task)
-    pl->wide = !k_thread_sweep(K);
     pl->sig = p->is_signal != nullptr || p->pi_row_back != 0;
-    const unsigned kAccMean = HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN;   // per-date means: thread-per-chain kernels only
-    // Narrow batches (the reference's own regime: one chain per end date) cannot fill the GPU with a thread per chain:
-    // below kScanMaxChains chains the time-parallel warp-per-chain kernel is used (K <= 4, plain sweep, window in smem).
-    {
-        // (the signals tier has no segment kernel: there the warp-per-chain kernel serves up to 12 288 chains; for the plain
-        //  sweep the segment kernel takes over from ~4000 chains — measured crossover on C2, DESIGN.md section 7)
-        const bool seg_ok = !(p->is_signal != nullptr || p->pi_row_back != 0) && !(getenv("HMCGPU_SEG_LANES") && atoi(getenv("HMCGPU_SEG_LANES")) == 0);
-        long long lim = seg_ok ? 4096 : 12288;
-        if (const char* e = getenv("HMCGPU_SCAN_MAX_CHAINS")) lim = atoll(e);
-        const int tmax = p->precision == 32 ? (K == 2 ? scan_max_T<float, 2>() : K == 3 ? scan_max_T<float, 3>() : scan_max_T<float, 4>())
-                                            : (K == 2 ? scan_max_T<double, 2>() : K == 3 ? scan_max_T<double, 3>() : scan_max_T<double, 4>());
-        // long windows leave room for fewer resident warps (the window lives in shared memory): scale the bound with them
-        const size_t wb = (size_t)(p->precision / 8) * ((size_t)pl->max_T * (K + 1) + 4 * K);
-        const long long blocks = std::max<long long>(1, std::min<long long>(5, (long long)((227 * 1024) / (4 * wb + 1024))));
-        lim = lim * blocks / 5;
-        pl->scan = !pl->wide && K <= 4 && !(p->flags & kAccMean) &&
-                   (long long)nw * nc <= lim && pl->max_T <= tmax;
-    }
-    const long long n_real = (long long)nw * nc;
-    // Mid-width batches (too many chains for a warp each, too few to fill the schedulers with a thread each): L lanes per
-    // chain, one time segment per lane (gibbs_seg_kernel.cuh).  L is chosen so that the batch yields about one full wave of
-    // warps; HMCGPU_SEG_LANES forces it (0 = never).  K <= 4, plain sweep.
-    {
-        int lanes = 0;
-        if (!pl->wide && K <= 4 && !pl->sig && !pl->scan && !(p->flags & kAccMean)) {
-            // measured on C2 (500 windows x c chains, B200): 4 lanes per chain are best up to ~38 000 chains, 2 lanes up to ~90 000,
-            // the thread-per-chain kernel beyond (DESIGN.md section 7); in units of one wave of thread slots (16 warps per SM):
-            const long long full = (long long)ctx->sm_count * 16 * 32;
-            if (n_real * 2 <= full) lanes = 4;
-            // (2 lanes only when the chains share one series: a batch of distinct series streams every observation from HBM in each
-            //  of the segment kernel's passes — C4, 65 536 series: 143 ms with 2 lanes, 139 ms with 4, 109 ms with a thread per chain)
-            else if (n_real * 4 <= 5 * full && nser == 1) lanes = 2;
-            if (const char* e = getenv("HMCGPU_SEG_LANES")) lanes = atoi(e);
-            if (lanes != 0 && lanes != 2 && lanes != 4 && lanes != 8) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_SEG_LANES must be 0, 2, 4 or 8");
-            const long long tmax = K == 2 ? seg_max_T<2>(lanes) : K == 3 ? seg_max_T<3>(lanes) : seg_max_T<4>(lanes);
-            if (lanes && pl->max_T > tmax) lanes = 0;
-        }
-        pl->seg = lanes != 0;
-        pl->seg_lanes = lanes;
-        // With 4 lanes per chain and thread slots to spare, the sweep time is the serial time of the LONGEST windows (every warp is
-        // resident from the start; a 16 000-chain batch leaves a fifth of the slots empty).  The longest tenth of the windows (in
-        // `order`) then gets 8 lanes per chain — half the dependent steps per sweep — as far as the slots last.  Measured on C2
-        // (HMCGPU_SEG_LONG sweep, scripts/r2_call_j.sh): 50 of 500 windows +7 % at 16 chains per window, +2 % at 24, +4 % at 32;
-        // 100 windows +7 % at 32 but -5 % at 24; 300 or all of them lose everywhere (8 lanes pay more per-sweep work per chain).
-        // HMCGPU_SEG_MIXED=0 disables it; a forced HMCGPU_SEG_LANES is uniform.
-        if (lanes == 4 && !getenv("HMCGPU_SEG_LANES") && !(getenv("HMCGPU_SEG_MIXED") && atoi(getenv("HMCGPU_SEG_MIXED")) == 0)) {
-            const long long full = (long long)ctx->sm_count * 16 * 32;
-            const long long spare = full * 115 / 100 - n_real * 4;
-            long long n8 = spare > 0 ? std::min<long long>(nw / 10, spare / ((long long)nc * 4)) : 0;
-            while (n8 > 0 && pl->wT[pl->order[n8 - 1]] < 128) --n8;          // (segments of fewer than 16 steps are all warm-up)
-            if (const char* e = getenv("HMCGPU_SEG_LONG")) n8 = std::max(0ll, std::min<long long>(nw, atoll(e)));
-            const long long tmax8 = K == 2 ? seg_max_T<2>(8) : K == 3 ? seg_max_T<3>(8) : seg_max_T<4>(8);
-            if (n8 * nc >= 32 && pl->max_T <= tmax8) pl->n_long = (int)n8;
-        }
-    }
-    const int ts = 32;
-    // slots: [long class (8 lanes), padded to 32][the rest, padded to 32]
-    const int long_slots = (int)(((long long)pl->n_long * nc + ts - 1) / ts * ts);
-    pl->long_slots = long_slots;
-    const int n_slots = long_slots + (int)((n_real - (long long)pl->n_long * nc + ts - 1) / ts * ts);
-    const int cpt = pl->seg ? 32 / pl->seg_lanes : ts;      // chains per warp task
-    const int n_warps = n_slots / cpt;                      // number of warp tasks (task id = slot / cpt; ids below long_slots / cpt are unused when there is a long class)
-    pl->n_slots = n_slots; pl->n_warps = n_warps;
-    std::vector<int> slot_win(n_slots, -1), slot_chain(n_slots, 0), Ts(n_slots, 0), win_slot0(nw), warp_T(n_warps, 0);
-    std::vector<long long> ybase(n_slots, 0), warp_off(n_warps, 0), wbase(nw), wbase_init(nw), x0_off(nw);
-    std::vector<unsigned> chain_id(n_slots, 0);
-    long long x0_total = 0;
-    for (int w = 0; w < nw; ++w) {
-        const int ser = p->win_series ? p->win_series[w] : 0;
-        // the window statistics read the fp64 series as uploaded (series-major: a window is contiguous)
-        wbase[w] = (long long)ser * p->y_len + (p->win_start[w] - 1);
-        wbase_init[w] = (long long)(p->win_init_series ? p->win_init_series[w] : ser) * p->y_len + (p->win_start[w] - 1);
-        x0_off[w] = x0_total;
-        x0_total += pl->wT[w];
-    }
-    for (int j = 0; j < nw; ++j) {
-        const int w = pl->order[j];
-        const int s0w = j < pl->n_long ? j * nc : long_slots + (j - pl->n_long) * nc;
-        win_slot0[w] = s0w;
-        const unsigned long long wid = p->win_id ? (unsigned long long)p->win_id[w] : (unsigned long long)w;
-        for (int cidx = 0; cidx < nc; ++cidx) {
-            const int slot = s0w + cidx;
-            slot_win[slot] = w; slot_chain[slot] = cidx; Ts[slot] = pl->wT[w];
-            ybase[slot] = (long long)(p->win_start[w] - 1) * nser + (p->win_series ? p->win_series[w] : 0);   // time-major [y_len][n_series] (the sweeps)
-            chain_id[slot] = (unsigned)(wid * (unsigned long long)nc + (unsigned long long)cidx);
-        }
-    }
-    long long pi_elems = 0;
-    std::vector<long long> slot_off(n_slots, 0);
-    // the long class first (8 lanes per chain: 4 chains per task, task id = slot / 4)
-    std::vector<int> warp_T_long(long_slots / 4, 0);
-    std::vector<long long> warp_off_long(long_slots / 4, 0);
-    for (int wp = 0; wp < long_slots / 4; ++wp) {
-        int m = 0;
-        for (int l = 0; l < 4; ++l) m = std::max(m, Ts[wp * 4 + l]);
-        const int Cs = std::max(4, (m + 31) / 32 * 4);
-        warp_T_long[wp] = Cs;
-        warp_off_long[wp] = pi_elems;
-        pi_elems += (long long)Cs * K * 32;
-    }
-    for (int wp = long_slots / cpt; wp < n_warps; ++wp) {
-        int m = 0;
-        for (int l = 0; l < cpt; ++l) m = std::max(m, Ts[wp * cpt + l]);
-        warp_T[wp] = m;
-        warp_off[wp] = pi_elems;
-        if (pl->seg) {
-            // segment kernel: every lane owns a frame of C = 4 ceil(T / 4L) rows (warp_T holds C), tiled like the thread kernel's
-            const int Cs = std::max(4, (m + 4 * pl->seg_lanes - 1) / (4 * pl->seg_lanes) * 4);
-            warp_T[wp] = Cs;
-            pi_elems += (long long)Cs * K * 32;
-        }
-        // thread-per-chain kernels: rows right-aligned to tiles of 4 time steps (gibbs_kernel.cuh, st_quad)
-        else if (!pl->wide) pi_elems += (long long)((m + 3) / 4 * 4) * K * ts;
-        else for (int l = 0; l < ts; ++l) { slot_off[wp * ts + l] = pi_elems; pi_elems += (long long)Ts[wp * ts + l] * K; }
-    }
-    // forecasts: realised y at end+h per window (NaN outside the series), horizons sorted ascending
-    std::vector<double> yfut_w((size_t)nw * std::max(1, p->n_h), NAN);
-    std::vector<int> hs(p->n_h);
+    TRY(choose_sweep(ctx, p, pl->wT, pl->order, pl->tuning, pl->sw));
+    const SlotLayout lay = layout_slots(pl, p);
+    const int n_slots = pl->n_slots, n_warps = pl->n_warps;
+    std::vector<int> hs(p->n_h);                            // horizons sorted ascending
     std::iota(hs.begin(), hs.end(), 0);
     std::stable_sort(hs.begin(), hs.end(), [&](int a, int b) { return p->horizons[a] < p->horizons[b]; });
-    for (int w = 0; w < nw; ++w)
-        for (int j = 0; j < p->n_h; ++j) {
-            const long long idx = (long long)p->win_end[w] + p->horizons[j];   // 1-based
-            const int ser = p->win_series ? p->win_series[w] : 0;
-            if (idx <= p->y_len) yfut_w[(size_t)w * p->n_h + j] = p->y[(size_t)ser * p->y_len + idx - 1];
-        }
-
-    // task groups: interleaved subsets of the (longest-first) warp tasks, each driven through its own stream
-    {
-        auto n_groups_for = [&](int tasks) {
-            int g = (pl->wide || pl->scan) ? 1 : (tasks >= 1024 ? 4 : (tasks >= 256 ? 2 : 1));
-            if (const char* e = getenv("HMCGPU_GROUPS")) g = std::max(1, std::min(8, atoi(e)));
-            return std::max(1, std::min(g, tasks));
-        };
-        const int t_long = long_slots / 4, t_first = long_slots / cpt, t_rest = n_warps - t_first;
-        if (t_long > 0) {
-            const int g = n_groups_for(t_long);
-            for (int q = 0; q < g; ++q) pl->groups.push_back({q, g, (t_long - q + g - 1) / g, 8, true});
-        }
-        if (t_rest > 0) {
-            const int g = n_groups_for(t_rest);
-            for (int q = 0; q < g; ++q) pl->groups.push_back({t_first + q, g, (t_rest - q + g - 1) / g, pl->seg_lanes, false});
-        }
-        pl->n_groups = (int)pl->groups.size();
-    }
     // double-buffered draw chunks let the groups drift apart (not with the smoothing accumulators, which are shared)
+    const unsigned kAccMean = HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN;
     pl->n_bufs = (pl->n_groups > 1 && !(p->flags & kAccMean)) ? 2 : 1;
     // chunk of draws per buffer: bound the chunk buffers to ~2 GiB in total
     const size_t per_draw = (size_t)pl->F * n_slots * sizeof(R);
@@ -1596,25 +1647,25 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     tr.sync_mark(st, "  series layout kernel");
     CU(ctx, up(pl->wbase, wbase.data(), nw * sizeof(long long)));
     CU(ctx, up(pl->wTd, pl->wT.data(), nw * sizeof(int)));
-    CU(ctx, up(pl->slot_win, slot_win.data(), n_slots * sizeof(int)));
-    CU(ctx, up(pl->slot_chain, slot_chain.data(), n_slots * sizeof(int)));
-    CU(ctx, up(pl->T, Ts.data(), n_slots * sizeof(int)));
-    CU(ctx, up(pl->ybase, ybase.data(), n_slots * sizeof(long long)));
-    CU(ctx, up(pl->warp_T, warp_T.data(), n_warps * sizeof(int)));
-    CU(ctx, up(pl->warp_pi_off, warp_off.data(), n_warps * sizeof(long long)));
-    if (long_slots > 0) {
-        CU(ctx, up(pl->warp_T_long, warp_T_long.data(), warp_T_long.size() * sizeof(int)));
-        CU(ctx, up(pl->warp_pi_off_long, warp_off_long.data(), warp_off_long.size() * sizeof(long long)));
+    CU(ctx, up(pl->slot_win, lay.slot_win.data(), n_slots * sizeof(int)));
+    CU(ctx, up(pl->slot_chain, lay.slot_chain.data(), n_slots * sizeof(int)));
+    CU(ctx, up(pl->T, lay.Ts.data(), n_slots * sizeof(int)));
+    CU(ctx, up(pl->ybase, lay.ybase.data(), n_slots * sizeof(long long)));
+    CU(ctx, up(pl->warp_T, lay.warp_T.data(), n_warps * sizeof(int)));
+    CU(ctx, up(pl->warp_pi_off, lay.warp_off.data(), n_warps * sizeof(long long)));
+    if (!lay.warp_T_long.empty()) {
+        CU(ctx, up(pl->warp_T_long, lay.warp_T_long.data(), lay.warp_T_long.size() * sizeof(int)));
+        CU(ctx, up(pl->warp_pi_off_long, lay.warp_off_long.data(), lay.warp_off_long.size() * sizeof(long long)));
     }
-    if (pl->wide) CU(ctx, up(pl->slot_pi_off, slot_off.data(), n_slots * sizeof(long long)));
-    CU(ctx, up(pl->chain_id, chain_id.data(), n_slots * sizeof(unsigned)));
-    CU(ctx, up(pl->win_slot0, win_slot0.data(), nw * sizeof(int)));
+    if (pl->sw.kernel == SweepKernel::lane) CU(ctx, up(pl->slot_pi_off, lay.slot_off.data(), n_slots * sizeof(long long)));
+    CU(ctx, up(pl->chain_id, lay.chain_id.data(), n_slots * sizeof(unsigned)));
+    CU(ctx, up(pl->win_slot0, lay.win_slot0.data(), nw * sizeof(int)));
     CU(ctx, up(pl->win_pib_off, pl->pib_off.data(), nw * sizeof(long long)));
     CU(ctx, up(pl->yfut_w, yfut_w.data(), yfut_w.size() * sizeof(double)));
     if (p->xi) CU(ctx, up(pl->xi_user, p->xi, K * sizeof(double)));
     if (p->win_init_series) CU(ctx, up(pl->wbase_init, wbase_init.data(), nw * sizeof(long long)));
     if (p->X0) {
-        CU(ctx, up(pl->X0, p->X0, (size_t)x0_total * sizeof(long long)));
+        CU(ctx, up(pl->X0, p->X0, (size_t)sumT * sizeof(long long)));
         CU(ctx, up(pl->x0_off, x0_off.data(), nw * sizeof(long long)));
     }
     const int sld = (p->is_signal && p->is_signal_per_series) ? nser : 1;
@@ -1622,7 +1673,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     if (pl->sig) {
         std::vector<long long> sbase(n_slots, 0), wsbase(nw, 0);
         for (int w = 0; w < nw; ++w) wsbase[w] = (long long)(p->win_start[w] - 1) * sld + (sld > 1 ? (p->win_series ? p->win_series[w] : 0) : 0);
-        for (int slot = 0; slot < n_slots; ++slot) if (slot_win[slot] >= 0) sbase[slot] = wsbase[slot_win[slot]];
+        for (int slot = 0; slot < n_slots; ++slot) if (lay.slot_win[slot] >= 0) sbase[slot] = wsbase[lay.slot_win[slot]];
         CU(ctx, up(pl->sbase, sbase.data(), n_slots * sizeof(long long)));
         CU(ctx, up(pl->wsbase, wsbase.data(), nw * sizeof(long long)));
         CU(ctx, pl->sigw.alloc((size_t)p->y_len * sld * sizeof(R)));
@@ -1638,7 +1689,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         CU(ctx, pl->totM.alloc((size_t)n_slots * sizeof(int)));
     }
     CU(ctx, pl->wi.alloc(nw * sizeof(WinInit)));
-    CU(ctx, pl->pi.alloc((size_t)pi_elems * sizeof(R)));
+    CU(ctx, pl->pi.alloc((size_t)lay.pi_elems * sizeof(R)));
     CU(ctx, pl->cnt.alloc((size_t)K * n_slots * sizeof(int)));
     CU(ctx, pl->trans.alloc((size_t)K * K * n_slots * sizeof(int)));
     CU(ctx, pl->Sd.alloc((size_t)K * n_slots * sizeof(R)));
@@ -1674,9 +1725,9 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         CU(ctx, pl->dg_gsum.alloc(nwf * kDiagLags * sizeof(double)));
     }
     if (p->flags & kAccMean) {
-        CU(ctx, pl->pacc.alloc((size_t)pi_elems * sizeof(R)));
+        CU(ctx, pl->pacc.alloc((size_t)lay.pi_elems * sizeof(R)));
         if (p->n_h > 0) {
-            CU(ctx, pl->facc.alloc((size_t)pi_elems / K * p->n_h * sizeof(R)));
+            CU(ctx, pl->facc.alloc((size_t)lay.pi_elems / K * p->n_h * sizeof(R)));
             CU(ctx, pl->d_fcsum.alloc((size_t)pib_total / K * p->n_h * sizeof(double)));
         }
         CU(ctx, pl->d_pibsum.alloc((size_t)pib_total * sizeof(double)));
@@ -1712,8 +1763,8 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     a.sigw = pl->sigw.p; a.sbase = pl->sbase.as<long long>(); a.sld = sld; a.cntM = pl->cntM.as<int>(); a.Sm = pl->Sm.p; a.Qm = pl->Qm.p; a.totSm = pl->totSm.p; a.totQm = pl->totQm.p;
     a.totM = pl->totM.as<int>(); a.kappa = p->kappa; a.pi_back = p->pi_row_back;
     // one short series shared by every window (the rolling job), fp64: the thread-per-chain kernel keeps a copy in shared memory
-    a.y_sm_elems = (y_in_smem<R>() && nser == 1 && K <= 4 && !pl->wide && !pl->scan && !pl->seg && (size_t)p->y_len * sizeof(R) <= (size_t)kYSmemMaxBytes &&
-                    !(getenv("HMCGPU_Y_SMEM") && atoi(getenv("HMCGPU_Y_SMEM")) == 0)) ? (int)p->y_len : 0;
+    a.y_sm_elems = (y_in_smem<R>() && nser == 1 && K <= 4 && pl->sw.kernel == SweepKernel::thread && (size_t)p->y_len * sizeof(R) <= (size_t)kYSmemMaxBytes &&
+                    pl->tuning.y_smem) ? (int)p->y_len : 0;
     a.all_signal = 0;
     if (p->is_signal) {
         const size_t nm = (size_t)p->y_len * sld;
@@ -1721,19 +1772,9 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         for (size_t q = 0; q < nm; ++q) ones += p->is_signal[q] != 0;
         a.all_signal = ones == nm;
     }
-    a.seg_warm = 32;
-    if (const char* e = getenv("HMCGPU_SEG_WARMUP")) a.seg_warm = std::max(0, atoi(e));
-    a.seg_barriers = 2;
-    if (const char* e = getenv("HMCGPU_SEG_BARRIERS")) a.seg_barriers = atoi(e);
-    a.diag = nullptr;
-    if (pl->seg) {
-        // 256-thread blocks (8 warps stepping through the phases of a sweep together) when that still gives every SM a block
-        // and a half; otherwise 128
-        pl->seg_threads = ((n_warps - long_slots / cpt + long_slots / 4) / (kSegThreads / 32) >= ctx->sm_count * 3 / 2) ? kSegThreads : 128;
-        if (const char* e = getenv("HMCGPU_SEG_THREADS")) pl->seg_threads = atoi(e);
-        CU(ctx, pl->d_diag.alloc(2 * sizeof(unsigned long long)));
-        a.diag = pl->d_diag.as<unsigned long long>();
-    }
+    a.seg_warm = pl->tuning.seg_warm; a.seg_barriers = pl->tuning.seg_barriers;
+    if (pl->sw.kernel == SweepKernel::seg) CU(ctx, pl->d_diag.alloc(2 * sizeof(unsigned long long)));
+    a.diag = pl->d_diag.as<unsigned long long>();
     for (int g = 0; g < pl->n_groups; ++g) {
         cudaStream_t s2;
         CU(ctx, cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
@@ -1748,19 +1789,12 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     return HMCGPU_OK;
 }
 
-// Sweeps per launch.  Short launches bound the damage of the priority-based warp arbiter (a starved warp can only fall
-// behind by one launch) and give the block scheduler a steady supply of pending blocks from the other groups.
-static int sweeps_per_launch() {
-    if (const char* e = getenv("HMCGPU_SWEEPS_PER_LAUNCH")) return std::max(1, atoi(e));
-    return 16;
-}
-
 template <typename R, int K>
 static int plan_run_t(hmcgpu_plan* pl) {
     hmcgpu_ctx* ctx = pl->ctx;
     cudaStream_t st = ctx->stream;
     const int ns = pl->n_slots, G = pl->n_groups;
-    const int L = (pl->scan && !getenv("HMCGPU_SWEEPS_PER_LAUNCH")) ? 64 : sweeps_per_launch();   // a scan sweep is a few µs
+    const int L = pl->sw.sweeps_per_launch;
     const int Kr = pl->K;                                    // runtime K (the template K is 0 for the lane-per-state kernel)
     pl->n_launches = 0; pl->n_sweep_launches = 0; pl->sweep_ms = 0.0;
     size_t ev_used = 0;
@@ -1793,7 +1827,6 @@ static int plan_run_t(hmcgpu_plan* pl) {
     CU(ctx, cudaEventRecord(pl->evk0, st));                  // start of the sweeps (sweep_kernel_ms)
     for (int g = 0; g < G; ++g) CU(ctx, cudaStreamWaitEvent(pl->gstreams[g], ev_init, 0));
     // an event pair around every sweep launch (its own duration, on its own stream) and one event per group after its last launch
-    static const bool launch_timing = !(getenv("HMCGPU_LAUNCH_TIMING") && atoi(getenv("HMCGPU_LAUNCH_TIMING")) == 0);
     size_t tev_used = 0;
     auto timing_event = [&](cudaEvent_t* e) -> cudaError_t {
         if (tev_used == pl->timing_events.size()) {
@@ -1910,17 +1943,19 @@ static int plan_run_t(hmcgpu_plan* pl) {
             a.warp_T = grp.long_class ? pl->warp_T_long.as<int>() : pl->warp_T.as<int>();
             a.warp_pi_off = grp.long_class ? pl->warp_pi_off_long.as<long long>() : pl->warp_pi_off.as<long long>();
             cudaEvent_t lt0 = nullptr, lt1 = nullptr;
-            if (launch_timing) { CU(ctx, timing_event(&lt0)); CU(ctx, timing_event(&lt1)); CU(ctx, cudaEventRecord(lt0, gs)); }
+            if (pl->tuning.launch_timing) { CU(ctx, timing_event(&lt0)); CU(ctx, timing_event(&lt1)); CU(ctx, cudaEventRecord(lt0, gs)); }
             if constexpr (K == 0) {
                 CU(ctx, (launch_gibbs_wide<R>(cfg, a, pl->K, pl->slot_pi_off.as<long long>(), gs)));
             } else if constexpr (K <= 4) {
-                if (pl->scan) CU(ctx, (launch_gibbs_scan<R, K>(cfg, a, gs)));
-                else if (pl->seg) CU(ctx, (launch_gibbs_seg<R, K>(cfg, a, grp.lanes, pl->seg_threads, gs)));
-                else CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
+                switch (pl->sw.kernel) {
+                    case SweepKernel::scan: CU(ctx, (launch_gibbs_scan<R, K>(cfg, a, gs))); break;
+                    case SweepKernel::seg: CU(ctx, (launch_gibbs_seg<R, K>(cfg, a, grp.lanes, pl->sw.seg_threads, gs))); break;
+                    default: CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
+                }
             } else {
                 CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
             }
-            if (launch_timing) { CU(ctx, cudaEventRecord(lt1, gs)); launch_pairs.emplace_back(lt0, lt1); }
+            if (pl->tuning.launch_timing) { CU(ctx, cudaEventRecord(lt1, gs)); launch_pairs.emplace_back(lt0, lt1); }
             ++pl->n_launches; ++pl->n_sweep_launches;
             next[g] = s0 + n;
             if (next[g] >= S) CU(ctx, cudaEventRecord(gend[g], gs));
@@ -1977,12 +2012,12 @@ static int plan_run_t(hmcgpu_plan* pl) {
     }
     if (pl->d_diag.p) {
         CU(ctx, cudaMemcpy(pl->seg_fallbacks, pl->d_diag.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        if (getenv("HMCGPU_VERBOSE")) {
+        if (pl->tuning.verbose) {
             const double cs = (double)pl->n_windows * pl->n_chains * (double)S;
-            if (pl->n_long) fprintf(stderr, "[hmcgpu] segment kernel: the %d longest of %d windows with 8 lanes per chain\n", pl->n_long, pl->n_windows);
+            if (pl->sw.n_long) fprintf(stderr, "[hmcgpu] segment kernel: the %d longest of %d windows with 8 lanes per chain\n", pl->sw.n_long, pl->n_windows);
             fprintf(stderr, "[hmcgpu] segment kernel (%d lanes per chain, warm-up %d): %llu of %.0f chain-sweeps used the exact entering vectors; "
                             "%.2f speculative groups of 4 steps per chain-sweep\n",
-                    pl->seg_lanes, pl->args.seg_warm, pl->seg_fallbacks[0], cs, (double)pl->seg_fallbacks[1] / cs);
+                    pl->sw.seg_lanes, pl->args.seg_warm, pl->seg_fallbacks[0], cs, (double)pl->seg_fallbacks[1] / cs);
         }
     }
     pl->ran = true;
@@ -1990,11 +2025,13 @@ static int plan_run_t(hmcgpu_plan* pl) {
 }
 
 static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out) {
-    TRY(validate_problem(ctx, p));
+    const Tuning t = read_tuning();
+    TRY(validate_problem(ctx, p, t));
     CU(ctx, cudaSetDevice(ctx->device));
     tl_pool = ctx->pool;
     std::unique_ptr<hmcgpu_plan> pl(new hmcgpu_plan());
     pl->ctx = ctx;
+    pl->tuning = t;
     int rc = (p->precision == 32) ? plan_build<float>(pl.get(), p) : plan_build<double>(pl.get(), p);
     if (rc != 0) {
         cudaStreamSynchronize(ctx->stream);    // uploads / init kernels may still be queued on buffers the plan is about to release
@@ -2110,8 +2147,8 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     r->gpu_ms = pl->gpu_ms; r->sweep_kernel_ms = pl->sweep_ms; r->n_launches = pl->n_launches;
     r->n_sweep_launches = pl->n_sweep_launches; r->h2d_bytes = pl->h2d; r->d2h_bytes = d2h; r->state_steps = pl->state_steps;
     r->sweep_launch_ms_sum = pl->launch_ms_sum;
-    r->sweep_kernel = pl->wide ? HMCGPU_KERNEL_LANE : pl->scan ? HMCGPU_KERNEL_SCAN : pl->seg ? HMCGPU_KERNEL_SEG : HMCGPU_KERNEL_THREAD;
-    r->n_tasks = pl->n_warps - pl->long_slots / (pl->seg ? 32 / pl->seg_lanes : 32) + pl->long_slots / 4;
+    r->sweep_kernel = (int32_t)pl->sw.kernel;
+    r->n_tasks = pl->n_tasks;
     return bad;
 }
 
