@@ -229,14 +229,18 @@ def shard_windows(T: Sequence[int], n_shards: int):
 
 def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                      precision=32, draws=False, summary=True, smoothed=False, loglik=False, win_id=None,
-                     win_series=None, diagnostics=False, ctx: Optional[B.Context] = None, device: int = 0):
+                     win_series=None, diagnostics=False, predictive_grid=None, ctx: Optional[B.Context] = None, device: int = 0):
     """Many end-date windows in one call (what the SLURM job array does one process at a time).  `diagnostics=True` adds
-    `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics)."""
+    `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics).
+    `predictive_grid` (increasing points, shared by every window and horizon) adds the posterior predictive distribution of
+    every forecast: `pred_cdf` [n_windows, n_h, n_grid], `pit` and `log_score` [n_windows, n_h] and `pred_moments`
+    [n_windows, n_h, 3] (mean, variance, skewness); see write_predictive and include/hmcgpu.h."""
     flags = B.FLAG_REF_Q1 | (B.FLAG_DRAWS if draws else 0) | (B.FLAG_SUMMARY if summary else 0) \
         | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0) \
-        | (B.FLAG_DIAGNOSTICS if diagnostics else 0)
+        | (B.FLAG_DIAGNOSTICS if diagnostics else 0) | (B.FLAG_PREDICTIVE if predictive_grid is not None else 0)
     spec = B.ProblemSpec(y, win_start, win_end, K=K, n_chains=n_chains, burnin=burnin, nrun=nrun, seed=seed,
-                         horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series)
+                         horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series,
+                         pred_grid=predictive_grid)
     own = ctx is None
     ctx = ctx or B.Context(device)
     try:
@@ -380,6 +384,50 @@ def write_diagnostics(out, K: int, horizons: Sequence[int], dates: Sequence, dir
         for name, path in _write_tables(_summary_tables(table, K, horizons, kind), dates, directory, kind).items():
             paths[f"{name}_{kind}"] = path
     return paths
+
+
+def write_predictive(out, horizons: Sequence[int], grid: Sequence[float], dates: Sequence, directory: str):
+    """The posterior predictive distributions of estimate_windows(predictive_grid=grid), one row per window in caller order:
+    `predictive_cdf_h<h>.csv` per horizon (date, then the CDF at every grid point; columns named by the point) and
+    `predictive_scores.csv` (date, then pit_<h>, log_score_<h>, mean_<h>, variance_<h>, skewness_<h> per horizon).  PIT and
+    log score are NaN for a horizon past the end of the series.  Returns {"cdf_h<h>": path, ..., "scores": path}."""
+    import os
+    os.makedirs(directory, exist_ok=True)
+    cdf, m = np.asarray(out.pred_cdf), np.asarray(out.pred_moments)
+    grid = [float(g) for g in grid]
+    tables = {f"cdf_h{h}": (f"predictive_cdf_h{h}.csv", [repr(g) for g in grid], cdf[:, j, :]) for j, h in enumerate(horizons)}
+    hdr, cols = [], []
+    for j, h in enumerate(horizons):
+        hdr += [f"pit_{h}", f"log_score_{h}", f"mean_{h}", f"variance_{h}", f"skewness_{h}"]
+        cols += [np.asarray(out.pit)[:, j], np.asarray(out.log_score)[:, j], m[:, j, 0], m[:, j, 1], m[:, j, 2]]
+    tables["scores"] = ("predictive_scores.csv", hdr, np.stack(cols, axis=1))
+    paths = {}
+    for key, (fname, cols_hdr, data) in tables.items():
+        path = os.path.join(directory, fname)
+        with open(path, "w") as f:
+            f.write(",".join(["date"] + cols_hdr) + "\n")
+            for d, row in zip(dates, data):
+                f.write(",".join([str(d)] + [repr(float(v)) for v in row]) + "\n")
+        paths[key] = path
+    return paths
+
+
+def predictive_quantiles(cdf, grid, probs):
+    """Quantiles of a predictive distribution from its CDF on a grid (out.pred_cdf[..., :] over `grid`), by linear
+    interpolation between grid points: accurate to the grid spacing, not better.  `cdf` [..., n_grid] (non-decreasing along the
+    last axis), `probs` [n_p]; returns [..., n_p], NaN where a probability lies outside [cdf[0], cdf[-1]] (the grid does not
+    cover that quantile) or the CDF is NaN."""
+    cdf = np.asarray(cdf, dtype=np.float64)
+    grid = np.asarray(grid, dtype=np.float64)
+    probs = np.atleast_1d(np.asarray(probs, dtype=np.float64))
+    flat = cdf.reshape(-1, cdf.shape[-1])
+    res = np.full((flat.shape[0], len(probs)), np.nan)
+    for i, c in enumerate(flat):
+        if not np.all(np.isfinite(c)):
+            continue
+        inside = (probs >= c[0]) & (probs <= c[-1])
+        res[i, inside] = np.interp(probs[inside], c, grid)
+    return res.reshape(cdf.shape[:-1] + (len(probs),))
 
 
 def forecastinsample(opt: EstOpt, horizon_index: int = -1, ctx: Optional[B.Context] = None, probabilities: str = "smoothed"):

@@ -19,6 +19,7 @@ FLAG_SMOOTHED_MEAN = 8
 FLAG_LOGLIK = 16
 FLAG_FILTERED_MEAN = 64   # pib_mean / insample_forecast_mean carry the FILTERED means (the reference's published in-sample table)
 FLAG_DIAGNOSTICS = 128    # rhat / ess / ess_lag per window and summary field (split-R̂ and ESS, include/hmcgpu.h)
+FLAG_PREDICTIVE = 256     # posterior predictive CDF on a grid, PIT, log score and moments per window and horizon (hmcgpu_predictive)
 
 ERR_ARG, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED, ERR_NODEVICE = -1, -2, -3, -4, -5
 
@@ -28,7 +29,8 @@ SYMBOLS = [
     "hmcgpu_ctx_sync", "hmcgpu_estimate", "hmcgpu_estimate_multi", "hmcgpu_plan_create", "hmcgpu_plan_run",
     "hmcgpu_plan_fetch", "hmcgpu_plan_destroy", "hmcgpu_filter", "hmcgpu_filter_masked", "hmcgpu_smooth", "hmcgpu_sample_states",
     "hmcgpu_draw_params", "hmcgpu_draw_params_signals", "hmcgpu_forecast", "hmcgpu_philox", "hmcgpu_philox_rounds",
-    "hmcgpu_build_info", "hmcgpu_ctx_trim",
+    "hmcgpu_build_info", "hmcgpu_ctx_trim", "hmcgpu_estimate_predictive", "hmcgpu_estimate_multi_predictive",
+    "hmcgpu_plan_fetch_predictive",
 ]
 KERNEL_NAMES = {0: "gibbs_sweeps_kernel (thread per chain)", 1: "gibbs_scan_kernel (warp per chain, time-parallel)",
                 2: "gibbs_wide_kernel (lane per state)", 3: "(reserved)",
@@ -48,7 +50,8 @@ class Problem(C.Structure):
                 ("seed", C.c_uint64), ("xi", _dp), ("alpha", _dp), ("nu", _dp), ("beta0", _dp), ("beta", _dp),
                 ("kappa", C.c_double), ("is_signal", _u8p), ("horizons", _i32p), ("n_h", C.c_int32),
                 ("X0", _i64p), ("precision", C.c_int32), ("flags", C.c_uint32),
-                ("win_init_series", _i32p), ("pi_row_back", C.c_int32), ("is_signal_per_series", C.c_int32)]
+                ("win_init_series", _i32p), ("pi_row_back", C.c_int32), ("is_signal_per_series", C.c_int32),
+                ("pred_grid", _dp), ("n_grid", C.c_int32)]
 
 
 class Result(C.Structure):
@@ -58,6 +61,10 @@ class Result(C.Structure):
                 ("n_sweep_launches", C.c_int64), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64),
                 ("state_steps", C.c_int64), ("sweep_launch_ms_sum", C.c_double), ("sweep_kernel", C.c_int32), ("n_tasks", C.c_int32),
                 ("rhat", _dp), ("ess", _dp), ("ess_lag", _i32p)]
+
+
+class Predictive(C.Structure):
+    _fields_ = [("cdf", _dp), ("pit", _dp), ("log_score", _dp), ("moments", _dp)]
 
 
 class HmcGpuError(RuntimeError):
@@ -101,6 +108,10 @@ def load(build_if_missing: bool = True):
     L.hmcgpu_plan_create.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(C.c_void_p)]
     L.hmcgpu_plan_run.argtypes = [C.c_void_p]
     L.hmcgpu_plan_fetch.argtypes = [C.c_void_p, C.POINTER(Result)]
+    L.hmcgpu_estimate_predictive.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Result), C.POINTER(Predictive)]
+    L.hmcgpu_estimate_multi_predictive.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
+                                                   C.POINTER(Predictive)]
+    L.hmcgpu_plan_fetch_predictive.argtypes = [C.c_void_p, C.POINTER(Predictive)]
     L.hmcgpu_plan_destroy.argtypes = [C.c_void_p]
     L.hmcgpu_plan_destroy.restype = None
     L.hmcgpu_filter.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _dp, C.c_int64,
@@ -238,7 +249,8 @@ class ProblemSpec:
     def __init__(self, y, win_start, win_end, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                  precision=32, flags=FLAG_REF_Q1 | FLAG_DRAWS, win_series=None, win_id=None,
                  xi=None, alpha=None, nu=None, beta0=None, beta=None, kappa=1.0, is_signal=None, X0=None,
-                 win_init_series=None, pi_row_back=0):
+                 win_init_series=None, pi_row_back=0, pred_grid=None):
+        """`pred_grid`: the points of the posterior predictive CDF (FLAG_PREDICTIVE; one grid for every window and horizon)."""
         y = np.asarray(y, dtype=np.float64)
         if y.ndim == 1:
             y = y[None, :]
@@ -266,13 +278,20 @@ class ProblemSpec:
             raise ValueError("X0 must hold sum_w T_w states")
         self.win_init_series = None if win_init_series is None else np.ascontiguousarray(win_init_series, dtype=np.int32)
         self.pi_row_back = int(pi_row_back)
+        # the library reads the grid only with the flag, so a grid without it (or the flag without one) is refused here
+        self.pred_grid = None if pred_grid is None else np.ascontiguousarray(np.ravel(pred_grid), dtype=np.float64)
+        if self.pred_grid is not None and not flags & FLAG_PREDICTIVE:
+            raise ValueError("pred_grid given without FLAG_PREDICTIVE")
+        if flags & FLAG_PREDICTIVE and self.pred_grid is None:
+            raise ValueError("FLAG_PREDICTIVE needs pred_grid")
+        self.n_grid = 0 if self.pred_grid is None else len(self.pred_grid)
 
     def struct(self) -> Problem:
         return Problem(_p(self.y), self.y_len, self.n_series, self.n_windows, _p(self.win_series, _i32p),
                        _p(self.win_start, _i32p), _p(self.win_end, _i32p), _p(self.win_id, _i64p), self.K, self.n_chains,
                        self.burnin, self.nrun, self.seed, *[_p(v) for v in self.hp], self.kappa, _p(self.is_signal, _u8p),
                        _p(self.horizons, _i32p), self.n_h, _p(self.X0, _i64p), self.precision, self.flags,
-                       _p(self.win_init_series, _i32p), self.pi_row_back, self.sig_per_series)
+                       _p(self.win_init_series, _i32p), self.pi_row_back, self.sig_per_series, _p(self.pred_grid), self.n_grid)
 
     def alloc_result(self, diagnostics=None):
         """Output arrays for the flags of this problem.  `diagnostics=True` asks for rhat / ess / ess_lag, which the library
@@ -306,6 +325,16 @@ class ProblemSpec:
                      _p(o.rhat), _p(o.ess), _p(o.ess_lag, _i32p))
         return o, res
 
+    def alloc_predictive(self, o):
+        """Adds the predictive outputs to `o` (pred_cdf [nw, n_h, n_grid], pit / log_score [nw, n_h], pred_moments [nw, n_h, 3]:
+        mean, variance, skewness) and returns the hmcgpu_predictive struct over them; None without FLAG_PREDICTIVE."""
+        if not self.flags & FLAG_PREDICTIVE:
+            return None
+        nw, nh = self.n_windows, self.n_h
+        o.pred_cdf = np.empty((nw, nh, self.n_grid)); o.pit = np.empty((nw, nh)); o.log_score = np.empty((nw, nh))
+        o.pred_moments = np.empty((nw, nh, 3))
+        return Predictive(_p(o.pred_cdf), _p(o.pit), _p(o.log_score), _p(o.pred_moments))
+
     def finish(self, o, res, rc):
         o.events = rc
         o.gpu_ms, o.sweep_kernel_ms = res.gpu_ms, res.sweep_kernel_ms
@@ -330,17 +359,25 @@ class ProblemSpec:
 def estimate(ctx: Context, spec: ProblemSpec):
     """hmcgpu_estimate: host buffers in, all sweeps, host buffers out."""
     o, res = spec.alloc_result()
+    pr = spec.alloc_predictive(o)
     prob = spec.struct()
-    rc = ctx._check(ctx.L.hmcgpu_estimate(ctx.h, C.byref(prob), C.byref(res)))
+    if pr is None:
+        rc = ctx._check(ctx.L.hmcgpu_estimate(ctx.h, C.byref(prob), C.byref(res)))
+    else:
+        rc = ctx._check(ctx.L.hmcgpu_estimate_predictive(ctx.h, C.byref(prob), C.byref(res), C.byref(pr)))
     return spec.finish(o, res, rc)
 
 
 def estimate_multi(devices, spec: ProblemSpec):
     L = load()
     o, res = spec.alloc_result()
+    pr = spec.alloc_predictive(o)
     prob = spec.struct()
     dev = (C.c_int * len(devices))(*devices)
-    rc = L.hmcgpu_estimate_multi(dev, len(devices), C.byref(prob), C.byref(res))
+    if pr is None:
+        rc = L.hmcgpu_estimate_multi(dev, len(devices), C.byref(prob), C.byref(res))
+    else:
+        rc = L.hmcgpu_estimate_multi_predictive(dev, len(devices), C.byref(prob), C.byref(res), C.byref(pr))
     if rc < 0:
         raise HmcGpuError(rc, L.hmcgpu_last_error(None).decode())
     return spec.finish(o, res, rc)
@@ -362,6 +399,9 @@ class Plan:
     def fetch(self):
         o, res = self.spec.alloc_result()
         rc = self.ctx._check(self.ctx.L.hmcgpu_plan_fetch(self.h, C.byref(res)))
+        pr = self.spec.alloc_predictive(o)
+        if pr is not None:
+            self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_predictive(self.h, C.byref(pr)))
         return self.spec.finish(o, res, rc)
 
     def close(self):

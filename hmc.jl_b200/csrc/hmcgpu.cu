@@ -5,6 +5,7 @@
 #include "gibbs_scan_kernel.cuh"
 #include "gibbs_seg_kernel.cuh"
 #include "diagnostics.cuh"
+#include "predictive.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -1343,6 +1344,10 @@ struct hmcgpu_plan {
     // HMCGPU_FLAG_DIAGNOSTICS (diagnostics.cuh): streaming state per (slot, field), per-sequence means / variances and lag sums
     // per (window, field)
     DevBuf dg_P, dg_S1, dg_head, dg_ring, dg_mean, dg_var, dg_gsum;
+    // HMCGPU_FLAG_PREDICTIVE (predictive.cuh): the grid, the shift c_w per window, running sums per (slot, horizon)
+    DevBuf pr_grid, pr_cshift, pr_cdf, pr_score;
+    int n_grid = 0, pr_tg = 32, pr_td = 1;    // threads per slot and draws per tile of pred_accum_kernel
+    PredHorizons pr_h{};
     DevBuf d_diag;       // segment kernel: chain-sweeps that fell back to the exact entering vectors
     unsigned long long seg_fallbacks[2] = {0, 0};   // [0] chain-sweeps on the exact path, [1] speculative groups (sum over chain-sweeps)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
@@ -1389,6 +1394,16 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuni
     if ((p->flags & HMCGPU_FLAG_DIAGNOSTICS) && p->nrun < 4) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_DIAGNOSTICS needs nrun >= 4 (two sequences of >= 2 draws per chain)");
     if (p->precision != 32 && p->precision != 64) return fail(ctx, HMCGPU_ERR_ARG, "precision must be 32 or 64");
     if (p->n_h < 0 || p->n_h > kMaxH || (p->n_h > 0 && !p->horizons)) return fail(ctx, HMCGPU_ERR_ARG, "0 <= n_h <= %d", kMaxH);
+    if (p->flags & HMCGPU_FLAG_PREDICTIVE) {
+        if (p->n_h == 0) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE needs at least one forecast horizon");
+        if (p->n_grid < 1 || p->n_grid > 512 || !p->pred_grid) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE needs 1 <= n_grid <= 512 grid points");
+        for (int g = 0; g < p->n_grid; ++g) {
+            if (!std::isfinite(p->pred_grid[g])) return fail(ctx, HMCGPU_ERR_ARG, "pred_grid[%d] is not finite", g);
+            if (g > 0 && !(p->pred_grid[g] > p->pred_grid[g - 1])) return fail(ctx, HMCGPU_ERR_ARG, "pred_grid is not strictly increasing at %d", g);
+        }
+        if (p->pi_row_back != 0)
+            return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_PREDICTIVE with pi_row_back != 0 (pi_end is then a smoothed row, not the forecasts' vector)");
+    }
     if (p->is_signal || p->pi_row_back != 0) {
         if (!k_thread(p->K)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "is_signal / pi_row_back are only implemented for K <= 4");
         if (p->flags & HMCGPU_FLAG_SMOOTHED_MEAN) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "is_signal / pi_row_back cannot be combined with HMCGPU_FLAG_SMOOTHED_MEAN");
@@ -1724,6 +1739,23 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         CU(ctx, pl->dg_var.alloc(nwf * 2 * nc * sizeof(double)));
         CU(ctx, pl->dg_gsum.alloc(nwf * kDiagLags * sizeof(double)));
     }
+    if (p->flags & HMCGPU_FLAG_PREDICTIVE) {
+        std::vector<double> cw(nw);
+        for (int w = 0; w < nw; ++w) cw[w] = p->y[(size_t)(p->win_series ? p->win_series[w] : 0) * p->y_len + p->win_end[w] - 1];
+        pl->n_grid = p->n_grid;
+        CU(ctx, up(pl->pr_grid, p->pred_grid, (size_t)p->n_grid * sizeof(double)));
+        CU(ctx, up(pl->pr_cshift, cw.data(), nw * sizeof(double)));
+        CU(ctx, pl->pr_cdf.alloc((size_t)n_slots * p->n_h * p->n_grid * sizeof(double)));
+        CU(ctx, pl->pr_score.alloc((size_t)n_slots * p->n_h * kPredScores * sizeof(double)));
+        // threads per slot: the grid rounded up to a power of two >= 32 (two points per thread above 256); then as many draws per
+        // tile as ~45 KB of shared memory hold
+        int tg = 32;
+        while (tg < std::min(p->n_grid, kPredThreads)) tg *= 2;
+        const int sb = kPredThreads / tg;
+        pl->pr_tg = tg;
+        pl->pr_td = (int)std::max<size_t>(1, std::min<size_t>(32, (45u << 10) / pred_smem_bytes(K, p->n_h, sb)));
+        for (int j = 0; j < p->n_h; ++j) { pl->pr_h.h_sorted[j] = p->horizons[hs[j]]; pl->pr_h.h_slot[j] = hs[j]; }
+    }
     if (p->flags & kAccMean) {
         CU(ctx, pl->pacc.alloc((size_t)lay.pi_elems * sizeof(R)));
         if (p->n_h > 0) {
@@ -1891,6 +1923,16 @@ static int plan_run_t(hmcgpu_plan* pl) {
             };
             TRY(sequence(d0, std::min<long long>(d0 + n, nh), 0, nh, 0));
             TRY(sequence(std::max(d0, h2), d0 + n, h2, pl->nrun, 1));
+        }
+        if (pl->flags & HMCGPU_FLAG_PREDICTIVE) {
+            const int sb = kPredThreads / pl->pr_tg;
+            const size_t smem = pred_smem_bytes(Kr, pl->n_h, sb * pl->pr_td);
+            auto accum = pl->n_grid > kPredThreads ? pred_accum_kernel<R, 2> : pred_accum_kernel<R, 1>;
+            accum<<<ns / sb, kPredThreads, smem, st>>>(Kr, pl->n_h, pl->n_grid, ns, pl->chunk, n, k == 0, pl->pr_tg, pl->pr_td, pl->pr_h,
+                                                       pl->slot_win.as<int>(), pl->pr_cshift.as<double>(), pl->yfut_w.as<double>(),
+                                                       pl->pr_grid.as<double>(), buf, pl->pr_cdf.as<double>(), pl->pr_score.as<double>());
+            CU(ctx, cudaGetLastError());
+            ++pl->n_launches;
         }
         if (pl->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)) {
             tile_reduce_kernel<R><<<pl->n_windows, 256, 0, st>>>(Kr, Kr, pl->n_chains, pl->win_slot0.as<int>(), pl->wTd.as<int>(),
@@ -2152,6 +2194,40 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     return bad;
 }
 
+static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    if (!(pl->flags & HMCGPU_FLAG_PREDICTIVE)) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_predictive on a plan without HMCGPU_FLAG_PREDICTIVE");
+    if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_predictive before plan_run");
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const long long nwh = (long long)pl->n_windows * pl->n_h;
+    DevBuf d_cdf, d_pit, d_ls, d_mom;
+    CU(ctx, d_cdf.alloc((size_t)nwh * pl->n_grid * sizeof(double)));
+    CU(ctx, d_pit.alloc((size_t)nwh * sizeof(double)));
+    CU(ctx, d_ls.alloc((size_t)nwh * sizeof(double)));
+    CU(ctx, d_mom.alloc((size_t)nwh * 3 * sizeof(double)));
+    pred_finish_kernel<<<grid_for(nwh * (pl->n_grid + 1), 128), 128, 0, st>>>(pl->n_windows, pl->n_h, pl->n_grid, pl->n_chains,
+                                                                              (double)pl->n_chains * (double)pl->nrun, pl->win_slot0.as<int>(),
+                                                                              pl->pr_cshift.as<double>(), pl->pr_cdf.as<double>(),
+                                                                              pl->pr_score.as<double>(), d_cdf.as<double>(), d_pit.as<double>(),
+                                                                              d_ls.as<double>(), d_mom.as<double>());
+    CU(ctx, cudaGetLastError());
+    auto down = [&](void* host, const DevBuf& b) -> cudaError_t {
+        return host ? cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    };
+    CU(ctx, down(pr->cdf, d_cdf));
+    CU(ctx, down(pr->pit, d_pit));
+    CU(ctx, down(pr->log_score, d_ls));
+    CU(ctx, down(pr->moments, d_mom));
+    CU(ctx, cudaStreamSynchronize(st));
+    return HMCGPU_OK;
+}
+
+extern "C" int hmcgpu_plan_fetch_predictive(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
+    if (!pl || !pr) return HMCGPU_ERR_ARG;
+    GUARD(pl->ctx, plan_fetch_predictive_impl(pl, pr));
+}
+
 extern "C" void hmcgpu_plan_destroy(hmcgpu_plan* pl) {
     if (!pl) return;
     cudaSetDevice(pl->ctx->device);
@@ -2161,7 +2237,13 @@ extern "C" void hmcgpu_plan_destroy(hmcgpu_plan* pl) {
 }
 
 extern "C" int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r) {
+    return hmcgpu_estimate_predictive(ctx, p, r, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr) {
     if (!r) return fail(ctx, HMCGPU_ERR_ARG, "result is NULL");
+    if (p && (p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
+        return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_predictive)");
     hmcgpu_plan* pl = nullptr;
     PhaseTrace tr;
     TRY(hmcgpu_plan_create(ctx, p, &pl));
@@ -2169,6 +2251,10 @@ extern "C" int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_
     int rc = hmcgpu_plan_run(pl);
     tr.mark("plan_run (all sweeps)");
     if (rc == 0) rc = hmcgpu_plan_fetch(pl, r);
+    if (rc >= 0 && (p->flags & HMCGPU_FLAG_PREDICTIVE)) {
+        const int rp = hmcgpu_plan_fetch_predictive(pl, pr);
+        if (rp < 0) rc = rp;
+    }
     tr.mark("plan_fetch (download)");
     hmcgpu_plan_destroy(pl);
     tr.mark("plan_destroy");
@@ -2176,13 +2262,20 @@ extern "C" int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_
 }
 
 // Windows sharded over devices by longest-processing-time-first on T_w; one host thread per device, no collectives.
-static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r);
+static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr);
 extern "C" int hmcgpu_estimate_multi(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r) {
-    if (!devices || n_dev < 1 || !p || !r) return fail(nullptr, HMCGPU_ERR_ARG, "bad arguments");
-    GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r));
+    return hmcgpu_estimate_multi_predictive(devices, n_dev, p, r, nullptr);
 }
 
-static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r) {
+extern "C" int hmcgpu_estimate_multi_predictive(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
+                                                hmcgpu_predictive* pr) {
+    if (!devices || n_dev < 1 || !p || !r) return fail(nullptr, HMCGPU_ERR_ARG, "bad arguments");
+    if ((p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
+        return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_multi_predictive)");
+    GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r, (p->flags & HMCGPU_FLAG_PREDICTIVE) ? pr : nullptr));
+}
+
+static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr) {
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(nullptr, HMCGPU_ERR_ARG, "no windows");
     const int nw = p->n_windows, K = p->K, nh = p->n_h;
     std::vector<int> ord(nw);
@@ -2230,7 +2323,7 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             q.n_windows = n; q.win_series = ser.data(); q.win_start = st.data(); q.win_end = en.data(); q.win_id = id.data();
             if (p->win_init_series) q.win_init_series = iser.data();
             if (p->X0) q.X0 = x0.data();
-            std::vector<double> mu, s2, A, pe, fc, ll, sm, sv, pb, ifc, rh, es;
+            std::vector<double> mu, s2, A, pe, fc, ll, sm, sv, pb, ifc, rh, es, pcdf, ppit, pls, pmom;
             std::vector<int32_t> status, el;
             const bool diag = (p->flags & HMCGPU_FLAG_DIAGNOSTICS) != 0;   // (the diagnostics pointers exist only then)
             hmcgpu_result& o = parts[d];
@@ -2248,7 +2341,13 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             if (diag && r->rhat) { rh.resize((size_t)n * F); o.rhat = rh.data(); }
             if (diag && r->ess) { es.resize((size_t)n * F); o.ess = es.data(); }
             if (diag && r->ess_lag) { el.resize((size_t)n * F); o.ess_lag = el.data(); }
-            rc = hmcgpu_estimate(ctx, &q, &o);
+            hmcgpu_predictive pq{};
+            const size_t ng = pr ? (size_t)nh * p->n_grid : 0;
+            if (pr && pr->cdf) { pcdf.resize(n * ng); pq.cdf = pcdf.data(); }
+            if (pr && pr->pit) { ppit.resize((size_t)n * nh); pq.pit = ppit.data(); }
+            if (pr && pr->log_score) { pls.resize((size_t)n * nh); pq.log_score = pls.data(); }
+            if (pr && pr->moments) { pmom.resize((size_t)n * nh * 3); pq.moments = pmom.data(); }
+            rc = hmcgpu_estimate_predictive(ctx, &q, &o, pr ? &pq : nullptr);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
             if (rc >= 0) {   // scatter this shard's windows into the caller's arrays (host gather)
@@ -2266,6 +2365,10 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
                     if (o.rhat) memcpy(r->rhat + w * F, rh.data() + (size_t)j * F, F * sizeof(double));
                     if (o.ess) memcpy(r->ess + w * F, es.data() + (size_t)j * F, F * sizeof(double));
                     if (o.ess_lag) memcpy(r->ess_lag + w * F, el.data() + (size_t)j * F, F * sizeof(int32_t));
+                    if (pq.cdf) memcpy(pr->cdf + w * ng, pcdf.data() + j * ng, ng * sizeof(double));
+                    if (pq.pit) memcpy(pr->pit + w * nh, ppit.data() + (size_t)j * nh, nh * sizeof(double));
+                    if (pq.log_score) memcpy(pr->log_score + w * nh, pls.data() + (size_t)j * nh, nh * sizeof(double));
+                    if (pq.moments) memcpy(pr->moments + w * nh * 3, pmom.data() + (size_t)j * nh * 3, nh * 3 * sizeof(double));
                     if (r->insample_forecast_mean) memcpy(r->insample_forecast_mean + pib_off[w] / K * nh, ifc.data() + po / K * nh, (size_t)Tw((int)w) * nh * sizeof(double));
                     if (r->pib_mean) memcpy(r->pib_mean + pib_off[w], pb.data() + po, (size_t)Tw((int)w) * K * sizeof(double));
                     po += (size_t)Tw((int)w) * K;

@@ -27,6 +27,7 @@ const FLAG_SMOOTHED_MEAN = UInt32(8)
 const FLAG_FILTERED_MEAN = UInt32(64)
 const FLAG_LOGLIK = UInt32(16)
 const FLAG_DIAGNOSTICS = UInt32(128)
+const FLAG_PREDICTIVE = UInt32(256)
 
 # struct hmcgpu_problem (include/hmcgpu.h)
 struct Problem
@@ -37,6 +38,7 @@ struct Problem
     kappa::Float64; is_signal::Ptr{UInt8}; horizons::Ptr{Int32}; n_h::Int32
     X0::Ptr{Int64}; precision::Int32; flags::UInt32
     win_init_series::Ptr{Int32}; pi_row_back::Int32; is_signal_per_series::Int32
+    pred_grid::Ptr{Float64}; n_grid::Int32
 end
 
 # struct hmcgpu_result
@@ -47,6 +49,11 @@ mutable struct Result
     h2d_bytes::Int64; d2h_bytes::Int64; state_steps::Int64
     sweep_launch_ms_sum::Float64; sweep_kernel::Int32; n_tasks::Int32
     rhat::Ptr{Float64}; ess::Ptr{Float64}; ess_lag::Ptr{Int32}
+end
+
+# struct hmcgpu_predictive (FLAG_PREDICTIVE)
+mutable struct Predictive
+    cdf::Ptr{Float64}; pit::Ptr{Float64}; log_score::Ptr{Float64}; moments::Ptr{Float64}
 end
 
 struct HmcGpuError <: Exception
@@ -99,7 +106,8 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
                   horizons::Vector{Int32} = Int32[12], precision::Int = 64,
                   win_series::Vector{Int32} = Int32[], win_init_series::Vector{Int32} = Int32[],
                   is_signal::Vector{UInt8} = UInt8[], kappa::Float64 = 1.0, pi_row_back::Int = 0,
-                  xi::Vector{Float64} = Float64[], alpha::Vector{Float64} = Float64[], nu::Vector{Float64} = Float64[])
+                  xi::Vector{Float64} = Float64[], alpha::Vector{Float64} = Float64[], nu::Vector{Float64} = Float64[],
+                  pred_grid::Vector{Float64} = Float64[])
     # rawdata: one series (Vector) or y_len × n_series (Matrix, column = series): exactly the library's column-major layout
     y_len, n_series = size(rawdata, 1), size(rawdata, 2)
     ptr_or_null(v) = isempty(v) ? Ptr{eltype(v)}(C_NULL) : pointer(v)
@@ -108,18 +116,25 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
     A = Array{Float64}(undef, R, D, D, nw)
     fc = Array{Float64}(undef, R, 2nh, nw)
     status = zeros(Int32, n_chains, nw)
+    # posterior predictive (non-empty pred_grid): C [w][j][g] row-major = Julia n_grid × n_h × nw
+    ng = length(pred_grid)
+    pcdf = Array{Float64}(undef, ng, nh, nw); pit = Array{Float64}(undef, nh, nw); pls = similar(pit)
+    pmom = Array{Float64}(undef, 3, nh, nw)
+    pred = Predictive(pointer(pcdf), pointer(pit), pointer(pls), pointer(pmom))
     res = Result(pointer(mu), pointer(sig), pointer(A), pointer(pie), nh > 0 ? pointer(fc) : C_NULL, C_NULL,
                  C_NULL, C_NULL, C_NULL, C_NULL, pointer(status), 0.0, 0.0, 0, 0, 0, 0, 0, 0.0, 0, 0,
                  C_NULL, C_NULL, C_NULL)
-    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu begin
+    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu pred_grid pcdf pit pls pmom begin
         prob = Problem(pointer(rawdata), y_len, n_series, nw, ptr_or_null(win_series), pointer(win_start), pointer(win_end), C_NULL,
                        D, n_chains, burnin, Nrun, UInt64(seed), ptr_or_null(xi), ptr_or_null(alpha), ptr_or_null(nu), C_NULL, C_NULL,
-                       kappa, ptr_or_null(is_signal), pointer(horizons), nh, C_NULL, precision, FLAG_REF_Q1 | FLAG_DRAWS,
-                       ptr_or_null(win_init_series), pi_row_back, 0)
-        ccall((:hmcgpu_estimate, LIB), Cint, (Ptr{Cvoid}, Ref{Problem}, Ref{Result}), ctx.h, prob, res)
+                       kappa, ptr_or_null(is_signal), pointer(horizons), nh, C_NULL, precision,
+                       FLAG_REF_Q1 | FLAG_DRAWS | (ng > 0 ? FLAG_PREDICTIVE : UInt32(0)),
+                       ptr_or_null(win_init_series), pi_row_back, 0, ptr_or_null(pred_grid), ng)
+        ccall((:hmcgpu_estimate_predictive, LIB), Cint, (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}), ctx.h, prob, res, pred)
     end
     rc < 0 && throw(HmcGpuError(rc, lasterror(ctx)))
-    return (μ = mu, σ = sig, A = A, πbend = pie, forecasts = fc, status = status, events = rc, gpu_ms = res.gpu_ms)
+    return (μ = mu, σ = sig, A = A, πbend = pie, forecasts = fc, status = status, events = rc, gpu_ms = res.gpu_ms,
+            pred_cdf = pcdf, pit = pit, log_score = pls, pred_moments = pmom)
 end
 
 # 0/1 flags over rawdata: 1 = the index belongs to opt.signalRange (hmcgpu_problem.is_signal)

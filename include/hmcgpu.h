@@ -58,6 +58,8 @@ extern "C" {
                                         data/output/official_insample/forecats_insample.csv holds); K <= 8, not with SMOOTHED_MEAN or signals */
 #define HMCGPU_FLAG_DIAGNOSTICS  128u /* fill rhat / ess / ess_lag: split-R̂ and effective sample size per window and summary field,
                                         computed on the device from every saved draw; needs nrun >= 4 (see hmcgpu_result) */
+#define HMCGPU_FLAG_PREDICTIVE  256u /* fill hmcgpu_predictive: posterior predictive CDF on pred_grid, PIT, log score and moments per
+                                        window and horizon, computed on the device from every saved draw (see hmcgpu_predictive) */
 
 typedef struct hmcgpu_ctx hmcgpu_ctx;
 typedef struct hmcgpu_plan hmcgpu_plan;
@@ -101,6 +103,10 @@ typedef struct hmcgpu_problem {
                                  samples.πb[:, opt.endIndex, :] with signalLen rows after endIndex (:893).  K <= 4. */
     int32_t is_signal_per_series; /* 0: is_signal holds y_len flags; 1: y_len flags per series (many end dates, each with its
                                  own signalRange, in one call) */
+    /* ---- appended in ABI version 400: read only with HMCGPU_FLAG_PREDICTIVE (older callers are never read past their end) */
+    const double* pred_grid;  /* [n_grid] finite, strictly increasing points at which the predictive CDF is evaluated; shared by
+                                 every window and horizon */
+    int32_t n_grid;           /* 1..512 */
 } hmcgpu_problem;
 
 /* Caller-allocated outputs; any pointer may be NULL.  R = n_chains*nrun draws per window, draw index
@@ -166,6 +172,31 @@ typedef struct hmcgpu_result {
     int32_t* ess_lag;     /* [n_windows x F] last autocorrelation lag in the ESS sum */
 } hmcgpu_result;
 
+/* Posterior predictive distribution (HMCGPU_FLAG_PREDICTIVE); caller-allocated, any pointer may be NULL.
+ * Draw d of window w (emitted fields: mu_s, sigma2_s, A[r][s], pi = pi_end) gives for horizon h_j = horizons[j] the mixture
+ *   weights v = pi' A^h_j (v_s = sum_r pi_r (A^h_j)[r][s], so sum_s v_s mu_s is the draw's forecast field),
+ *   F_d(x) = sum_s v_s Phi((x - mu_s) / sqrt(sigma2_s)),   p_d(x) = sum_s v_s phi((x - mu_s) / sqrt(sigma2_s)) / sqrt(sigma2_s).
+ * Pooled over the R = n_chains*nrun draws, with y+ = y[end_w + h_j] of the window's series (the value the forecast error uses,
+ * fp64; NaN past the end of the series) and c_w = y[end_w]:
+ *   cdf[(w*n_h + j)*n_grid + g] = (1/R) sum_d F_d(pred_grid[g])
+ *   pit[w*n_h + j]              = (1/R) sum_d F_d(y+)            (NaN when y+ is NaN)
+ *   log_score[w*n_h + j]        = log((1/R) sum_d p_d(y+))       (NaN when y+ is NaN)
+ *   moments[(w*n_h + j)*3 + k]  = mean, variance, skewness of the pooled mixture, from the raw moments about c_w
+ *                                 M1 = sum_s v_s (mu_s - c_w), M2 = sum_s v_s ((mu_s - c_w)^2 + sigma2_s),
+ *                                 M3 = sum_s v_s ((mu_s - c_w)^3 + 3 (mu_s - c_w) sigma2_s) averaged over the draws
+ * All predictive arithmetic is fp64 on the draws as the plan produced them, converted to double, whatever the precision.  A window
+ * with a non-finite mu / sigma2 / A / pi_end draw gets NaN in every output.  Every sum runs in draw order, then chain order, with
+ * no atomics: a window's outputs are bit-identical however the windows are batched, chunked or sharded.
+ * Needs n_h >= 1, 1 <= n_grid <= 512 and pi_row_back == 0 (with pi_row_back the emitted pi_end is a smoothed row, not the vector
+ * the forecasts are built from).  Device state: 8 * n_slots * n_h * (n_grid + 5) bytes (n_slots ~ n_windows * n_chains, e.g.
+ * 0.85 GB for 128 000 chains, n_h = 12, n_grid = 64), allocated only with the flag. */
+typedef struct hmcgpu_predictive {
+    double* cdf;          /* [n_windows][n_h][n_grid] */
+    double* pit;          /* [n_windows][n_h] */
+    double* log_score;    /* [n_windows][n_h] */
+    double* moments;      /* [n_windows][n_h][3] */
+} hmcgpu_predictive;
+
 #define HMCGPU_KERNEL_THREAD 0  /* one thread per chain (gibbs_sweeps_kernel), wide batches, K <= 8 */
 #define HMCGPU_KERNEL_SCAN 1    /* one warp per chain, time-parallel scans (gibbs_scan_kernel), narrow batches */
 #define HMCGPU_KERNEL_LANE 2    /* one lane per state (gibbs_wide_kernel), K = 9..32 */
@@ -188,10 +219,17 @@ int hmcgpu_ctx_sync(hmcgpu_ctx* ctx);
  * they are also released when an allocation on this context fails and at hmcgpu_ctx_destroy). */
 int hmcgpu_ctx_trim(hmcgpu_ctx* ctx);
 
-/* Whole estimation, host buffers in and out (H2D, all sweeps, D2H inside the call). */
+/* Whole estimation, host buffers in and out (H2D, all sweeps, D2H inside the call).  = hmcgpu_estimate_predictive(.., NULL) */
 int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r);
-/* Same, windows sharded over several GPUs by sum of T_w (one host thread per device, no collectives). */
+/* Same, windows sharded over several GPUs by sum of T_w (one host thread per device, no collectives).
+ * = hmcgpu_estimate_multi_predictive(.., NULL) */
 int hmcgpu_estimate_multi(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r);
+/* The same two calls filling the posterior predictive outputs too.  With HMCGPU_FLAG_PREDICTIVE, pr must not be NULL
+ * (HMCGPU_ERR_ARG: the library does not compute what it would discard); without it pr is ignored.  The multi-GPU form
+ * scatters each shard's rows into the caller's window order. */
+int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr);
+int hmcgpu_estimate_multi_predictive(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
+                                     hmcgpu_predictive* pr);
 
 /* Split form: create uploads inputs and allocates device state; run executes every sweep (inputs resident
  * in HBM, no host transfers); fetch copies the requested outputs back.  run may be repeated (it restarts
@@ -199,6 +237,8 @@ int hmcgpu_estimate_multi(const int* devices, int n_devices, const hmcgpu_proble
 int hmcgpu_plan_create(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_plan** out);
 int hmcgpu_plan_run(hmcgpu_plan* plan);
 int hmcgpu_plan_fetch(hmcgpu_plan* plan, hmcgpu_result* r);
+/* Posterior predictive outputs of the last run; HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_PREDICTIVE or before a run. */
+int hmcgpu_plan_fetch_predictive(hmcgpu_plan* plan, hmcgpu_predictive* pr);
 void hmcgpu_plan_destroy(hmcgpu_plan* plan);
 
 /* Forward filter for fixed parameters.  y: [T] shared by the batch (y_batch_stride = 0) or [B][T]
