@@ -1218,6 +1218,12 @@ __global__ void summary_finish_kernel(long long n_elems, int F, double n, int ha
     var[i] = zero ? 0.0 : fmax(0.0, __dsub_rn(sumsq[i] / n, __dmul_rn(m, m)));      // rounded operation by operation, as the host did
 }
 
+// per-date posterior means (pib_mean, insample_forecast_mean) from the sums over the n saved draws of a window
+__global__ void mean_finish_kernel(long long n_elems, double n, const double* __restrict__ sum, double* __restrict__ mean) {
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i < n_elems) mean[i] = sum[i] / n;
+}
+
 template <typename R>
 __global__ void yfut_kernel(int n_slots, int n_h, const int* __restrict__ slot_win, const double* __restrict__ yfut_w, R* __restrict__ out) {
     const int slot = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1318,7 +1324,7 @@ struct hmcgpu_plan {
     std::vector<int> wT;                 // per window (caller order)
     std::vector<int> order;              // windows sorted by T descending: order[j] = caller index
     std::vector<long long> pib_off;      // per window (caller order) offset in pib_mean
-    long long pib_total = 0;
+    std::vector<int> slot0;              // per window (caller order) its first chain slot (SlotLayout::win_slot0)
     long long state_steps = 0;
     int n_slots = 0, n_warps = 0, n_tasks = 0, chunk = 0, max_T = 0;   // (n_tasks: warp tasks of both classes)
     GibbsArgs args{};
@@ -1340,7 +1346,10 @@ struct hmcgpu_plan {
     std::vector<cudaEvent_t> pool_events;
     std::vector<cudaEvent_t> timing_events;   // pairs around every sweep launch + one end-of-sweeps event per group (timing enabled)
     double launch_ms_sum = 0.0;
-    DevBuf d_mu, d_sig2, d_A, d_pie, d_fc, d_ll, d_sum, d_sumsq, d_pibsum, d_fcsum;
+    DevBuf d_sum, d_sumsq, d_pibsum, d_fcsum;
+    // the per-window outputs (window_outputs), laid out like the caller's arrays: the draws gathered per chunk, the rest
+    // finished at fetch
+    DevBuf d_mu, d_sig2, d_A, d_pie, d_fc, d_ll, d_mean, d_var, d_pib, d_ifc, d_rhat, d_ess, d_lag, d_cdf, d_pit, d_ls, d_mom;
     // HMCGPU_FLAG_DIAGNOSTICS (diagnostics.cuh): streaming state per (slot, field), per-sequence means / variances and lag sums
     // per (window, field)
     DevBuf dg_P, dg_S1, dg_head, dg_ring, dg_mean, dg_var, dg_gsum;
@@ -1364,6 +1373,68 @@ struct hmcgpu_plan {
         if (evk1) cudaEventDestroy(evk1);
     }
 };
+
+// F: fields per window of the summaries and diagnostics (mu[K], sigma2[K], A[K*K], pi_end[K], forecasts[2*n_h], loglik)
+static int summary_fields(int K, int n_h) { return 3 * K + K * K + 2 * n_h + 1; }
+
+// One per-window output of hmcgpu_result / hmcgpu_predictive.  Window w holds per_window + per_step * T_w elements; the windows
+// are concatenated in caller order, in the caller's array and in the plan's device buffer `dev` alike.
+struct WinOut {
+    const char* name;
+    bool pred;                 // a field of hmcgpu_predictive (else of hmcgpu_result)
+    size_t field;              // offset of the caller's pointer in that struct
+    size_t elem;               // bytes per element
+    long long per_window, per_step;
+    bool on;                   // the flags produce it
+    bool gated;                // the caller's pointer is read only when `on` (fields appended to the ABI: older structs end before them)
+    const char* need;          // the flag that is missing when it is not on
+    DevBuf hmcgpu_plan::*dev;  // NULL for status, which is read from the chain slots
+    // elements of n windows of sum_T steps in all; elems(w, T_0 + ... + T_{w-1}) is the offset of window w
+    long long elems(long long n, long long sum_T) const { return per_window * n + per_step * sum_T; }
+    void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr) const {     // NULL: not requested, or not readable
+        const void* s = pred ? (const void*)pr : (const void*)r;
+        void* p = nullptr;
+        if (s && (on || !gated)) memcpy(&p, (const char*)s + field, sizeof p);
+        return p;
+    }
+    void set(hmcgpu_result* r, hmcgpu_predictive* pr, void* p) const { memcpy((char*)(pred ? (void*)pr : (void*)r) + field, &p, sizeof p); }
+};
+
+static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long long nrun, int n_grid, unsigned flags) {
+    const long long R = (long long)n_chains * nrun, F = summary_fields(K, n_h);
+    const bool draws = flags & HMCGPU_FLAG_DRAWS, summary = flags & HMCGPU_FLAG_SUMMARY, diag = flags & HMCGPU_FLAG_DIAGNOSTICS,
+               pred = flags & HMCGPU_FLAG_PREDICTIVE, mean = flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN);
+    const bool ll = draws && (flags & HMCGPU_FLAG_LOGLIK);
+    const char* D = "HMCGPU_FLAG_DRAWS";
+    const char* M = "HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN";
+    const size_t f8 = sizeof(double), i4 = sizeof(int32_t);
+    using P = hmcgpu_plan;
+#define RES(f) #f, false, offsetof(hmcgpu_result, f)
+#define PRED(f) #f, true, offsetof(hmcgpu_predictive, f)
+    std::vector<WinOut> o = {
+        {RES(mu), f8, R * K, 0, draws, false, D, &P::d_mu},
+        {RES(sigma2), f8, R * K, 0, draws, false, D, &P::d_sig2},
+        {RES(A), f8, R * K * K, 0, draws, false, D, &P::d_A},
+        {RES(pi_end), f8, R * K, 0, draws, false, D, &P::d_pie},
+        {RES(forecasts), f8, R * 2 * n_h, 0, draws, false, D, &P::d_fc},
+        {RES(loglik), f8, R, 0, ll, false, draws ? "HMCGPU_FLAG_LOGLIK" : D, &P::d_ll},
+        {RES(summary_mean), f8, F, 0, summary, false, "HMCGPU_FLAG_SUMMARY", &P::d_mean},
+        {RES(summary_var), f8, F, 0, summary, false, "HMCGPU_FLAG_SUMMARY", &P::d_var},
+        {RES(pib_mean), f8, 0, K, mean, false, M, &P::d_pib},
+        {RES(insample_forecast_mean), f8, 0, n_h, mean, false, M, &P::d_ifc},
+        {RES(status), i4, n_chains, 0, true, false, "", nullptr},
+        {RES(rhat), f8, F, 0, diag, true, "", &P::d_rhat},
+        {RES(ess), f8, F, 0, diag, true, "", &P::d_ess},
+        {RES(ess_lag), i4, F, 0, diag, true, "", &P::d_lag},
+        {PRED(cdf), f8, (long long)n_h * n_grid, 0, pred, true, "", &P::d_cdf},
+        {PRED(pit), f8, n_h, 0, pred, true, "", &P::d_pit},
+        {PRED(log_score), f8, n_h, 0, pred, true, "", &P::d_ls},
+        {PRED(moments), f8, 3ll * n_h, 0, pred, true, "", &P::d_mom},
+    };
+#undef RES
+#undef PRED
+    return o;
+}
 
 static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuning& t) {
     if (!ctx) return HMCGPU_ERR_ARG;
@@ -1597,7 +1668,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     const int K = p->K, nw = p->n_windows, nc = p->n_chains, nser = p->n_series;
     pl->K = K; pl->n_chains = nc; pl->n_windows = nw; pl->n_h = p->n_h; pl->precision = p->precision;
     pl->burnin = p->burnin; pl->nrun = p->nrun; pl->flags = p->flags; pl->seed = p->seed;
-    pl->F = 3 * K + K * K + 2 * p->n_h + 1;
+    pl->F = summary_fields(K, p->n_h);
     pl->wT.resize(nw);
     pl->order.resize(nw);
     pl->pib_off.resize(nw);
@@ -1621,7 +1692,6 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
             if (idx <= p->y_len) yfut_w[(size_t)w * p->n_h + j] = p->y[(size_t)ser * p->y_len + idx - 1];
         }
     }
-    pl->pib_total = pib_total;
     if (k_thread(K) && (long long)pl->max_T - 1 > ((1ll << (64 / K)) - 1)) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window too long for K=%d", K);
     pl->state_steps = sumT * nc * (p->burnin + p->nrun);
     std::iota(pl->order.begin(), pl->order.end(), 0);
@@ -1675,6 +1745,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     if (pl->sw.kernel == SweepKernel::lane) CU(ctx, up(pl->slot_pi_off, lay.slot_off.data(), n_slots * sizeof(long long)));
     CU(ctx, up(pl->chain_id, lay.chain_id.data(), n_slots * sizeof(unsigned)));
     CU(ctx, up(pl->win_slot0, lay.win_slot0.data(), nw * sizeof(int)));
+    pl->slot0 = lay.win_slot0;
     CU(ctx, up(pl->win_pib_off, pl->pib_off.data(), nw * sizeof(long long)));
     CU(ctx, up(pl->yfut_w, yfut_w.data(), yfut_w.size() * sizeof(double)));
     if (p->xi) CU(ctx, up(pl->xi_user, p->xi, K * sizeof(double)));
@@ -1716,15 +1787,6 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     CU(ctx, pl->totQ.alloc((size_t)n_slots * sizeof(R)));
     CU(ctx, pl->out.alloc(per_draw * (size_t)chunk * pl->n_bufs));
     CU(ctx, pl->yfut.alloc((size_t)std::max(1, p->n_h) * n_slots * sizeof(R)));
-    const size_t Rr = (size_t)nc * p->nrun;
-    if (p->flags & HMCGPU_FLAG_DRAWS) {
-        CU(ctx, pl->d_mu.alloc((size_t)nw * Rr * K * sizeof(double)));
-        CU(ctx, pl->d_sig2.alloc((size_t)nw * Rr * K * sizeof(double)));
-        CU(ctx, pl->d_A.alloc((size_t)nw * Rr * K * K * sizeof(double)));
-        CU(ctx, pl->d_pie.alloc((size_t)nw * Rr * K * sizeof(double)));
-        if (p->n_h > 0) CU(ctx, pl->d_fc.alloc((size_t)nw * Rr * 2 * p->n_h * sizeof(double)));
-        if (p->flags & HMCGPU_FLAG_LOGLIK) CU(ctx, pl->d_ll.alloc((size_t)nw * Rr * sizeof(double)));
-    }
     if (p->flags & HMCGPU_FLAG_SUMMARY) {
         CU(ctx, pl->d_sum.alloc((size_t)nw * pl->F * sizeof(double)));
         CU(ctx, pl->d_sumsq.alloc((size_t)nw * pl->F * sizeof(double)));
@@ -1764,6 +1826,8 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         }
         CU(ctx, pl->d_pibsum.alloc((size_t)pib_total * sizeof(double)));
     }
+    for (const WinOut& o : window_outputs(K, p->n_h, nc, p->nrun, pl->n_grid, p->flags))
+        if (o.on && o.dev) CU(ctx, (pl->*o.dev).alloc((size_t)o.elems(nw, sumT) * o.elem));
     // window statistics (once per plan)
     const size_t smem = (size_t)pl->max_T;
     if (smem > 200 * 1024) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window longer than %d observations", 200 * 1024);
@@ -2109,80 +2173,54 @@ extern "C" int hmcgpu_plan_fetch(hmcgpu_plan* pl, hmcgpu_result* r) {
     GUARD(pl->ctx, plan_fetch_impl(pl, r));
 }
 
+// Enqueues the copy of every requested output the plan holds (of r, or of pr) into the caller's arrays; adds the bytes to *bytes
+// (NULL: the predictive outputs, which hmcgpu_result's d2h_bytes does not count)
+static int download(hmcgpu_plan* pl, const std::vector<WinOut>& outs, const hmcgpu_result* r, const hmcgpu_predictive* pr,
+                    long long* bytes) {
+    for (const WinOut& o : outs) {
+        void* host = o.get(r, pr);
+        if (!host || !o.dev || !(pl->*o.dev).p) continue;         // (an output of no elements has no buffer)
+        const DevBuf& b = pl->*o.dev;
+        CU(pl->ctx, cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, pl->ctx->stream));
+        if (bytes) *bytes += (long long)b.bytes;
+    }
+    return HMCGPU_OK;
+}
+
 static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     hmcgpu_ctx* ctx = pl->ctx;
     if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch before plan_run");
+    const std::vector<WinOut> outs = window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, pl->flags);
+    for (const WinOut& o : outs)
+        if (!o.on && o.get(r, nullptr)) return fail(ctx, HMCGPU_ERR_ARG, "%s requested without %s", o.name, o.need);
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const int K = pl->K, nw = pl->n_windows;
-    const size_t Rr = (size_t)pl->n_chains * pl->nrun;
+    const int nc = pl->n_chains, has_ll = (pl->flags & HMCGPU_FLAG_LOGLIK) ? 1 : 0;
+    const double n = (double)nc * (double)pl->nrun;
+    // finished on the device from the run's sums (these launches are not plan_run's: n_launches leaves them out)
+    const long long ne = (long long)pl->n_windows * pl->F, npib = (long long)(pl->d_pib.bytes / sizeof(double)),
+                    nifc = (long long)(pl->d_ifc.bytes / sizeof(double));
+    if (pl->d_mean.p)
+        summary_finish_kernel<<<grid_for(ne, 256), 256, 0, st>>>(ne, pl->F, n, has_ll, pl->d_sum.as<double>(), pl->d_sumsq.as<double>(),
+                                                                 pl->d_mean.as<double>(), pl->d_var.as<double>());
+    if (pl->d_rhat.p)
+        diag_finish_kernel<<<grid_for(ne, 128), 128, 0, st>>>(ne, pl->F, nc, pl->nrun / 2, has_ll, pl->dg_mean.as<double>(),
+                                                              pl->dg_var.as<double>(), pl->dg_gsum.as<double>(), pl->d_rhat.as<double>(),
+                                                              pl->d_ess.as<double>(), pl->d_lag.as<int>());
+    if (pl->d_pib.p) mean_finish_kernel<<<grid_for(npib, 256), 256, 0, st>>>(npib, n, pl->d_pibsum.as<double>(), pl->d_pib.as<double>());
+    if (pl->d_ifc.p) mean_finish_kernel<<<grid_for(nifc, 256), 256, 0, st>>>(nifc, n, pl->d_fcsum.as<double>(), pl->d_ifc.as<double>());
+    CU(ctx, cudaGetLastError());
     long long d2h = 0;
-    auto down = [&](void* host, const DevBuf& b, size_t bytes) -> cudaError_t {
-        if (!host || !b.p) return cudaSuccess;
-        d2h += (long long)bytes;
-        return cudaMemcpyAsync(host, b.p, bytes, cudaMemcpyDeviceToHost, st);
-    };
-    if ((r->mu || r->sigma2 || r->A || r->pi_end || r->forecasts || r->loglik) && !(pl->flags & HMCGPU_FLAG_DRAWS))
-        return fail(ctx, HMCGPU_ERR_ARG, "per-draw outputs requested without HMCGPU_FLAG_DRAWS");
-    if ((r->summary_mean || r->summary_var) && !(pl->flags & HMCGPU_FLAG_SUMMARY))
-        return fail(ctx, HMCGPU_ERR_ARG, "summary requested without HMCGPU_FLAG_SUMMARY");
-    if ((r->pib_mean || r->insample_forecast_mean) && !(pl->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)))
-        return fail(ctx, HMCGPU_ERR_ARG, "pib_mean / insample_forecast_mean requested without HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN");
-    if (r->loglik && !(pl->flags & HMCGPU_FLAG_LOGLIK)) return fail(ctx, HMCGPU_ERR_ARG, "loglik requested without HMCGPU_FLAG_LOGLIK");
-    // (rhat / ess / ess_lag were appended in ABI version 300: they are read only when the flag says the caller has them)
-    const bool diag = (pl->flags & HMCGPU_FLAG_DIAGNOSTICS) && (r->rhat || r->ess || r->ess_lag);
-    CU(ctx, down(r->mu, pl->d_mu, nw * Rr * K * sizeof(double)));
-    CU(ctx, down(r->sigma2, pl->d_sig2, nw * Rr * K * sizeof(double)));
-    CU(ctx, down(r->A, pl->d_A, nw * Rr * K * K * sizeof(double)));
-    CU(ctx, down(r->pi_end, pl->d_pie, nw * Rr * K * sizeof(double)));
-    CU(ctx, down(r->forecasts, pl->d_fc, nw * Rr * 2 * pl->n_h * sizeof(double)));
-    CU(ctx, down(r->loglik, pl->d_ll, nw * Rr * sizeof(double)));
-    std::vector<double> pibsum, fcsum;
+    TRY(download(pl, outs, r, nullptr, &d2h));
     std::vector<int> ev(pl->n_slots);
-    DevBuf d_mean, d_var;                                     // (released after the stream has drained, below)
-    if (r->summary_mean || r->summary_var) {
-        // finished on the device and copied straight into the caller's arrays (no host-side pass over n_windows x F values)
-        const long long ne = (long long)nw * pl->F;
-        CU(ctx, d_mean.alloc((size_t)ne * sizeof(double)));
-        CU(ctx, d_var.alloc((size_t)ne * sizeof(double)));
-        summary_finish_kernel<<<grid_for(ne, 256), 256, 0, st>>>(ne, pl->F, (double)Rr, (pl->flags & HMCGPU_FLAG_LOGLIK) ? 1 : 0,
-                                                                 pl->d_sum.as<double>(), pl->d_sumsq.as<double>(), d_mean.as<double>(), d_var.as<double>());
-        CU(ctx, cudaGetLastError());
-        CU(ctx, down(r->summary_mean, d_mean, (size_t)ne * sizeof(double)));
-        CU(ctx, down(r->summary_var, d_var, (size_t)ne * sizeof(double)));
-    }
-    DevBuf d_rhat, d_ess, d_lag;
-    if (diag) {
-        const long long ne = (long long)nw * pl->F;
-        CU(ctx, d_rhat.alloc((size_t)ne * sizeof(double)));
-        CU(ctx, d_ess.alloc((size_t)ne * sizeof(double)));
-        CU(ctx, d_lag.alloc((size_t)ne * sizeof(int)));
-        diag_finish_kernel<<<grid_for(ne, 128), 128, 0, st>>>(ne, pl->F, pl->n_chains, pl->nrun / 2, (pl->flags & HMCGPU_FLAG_LOGLIK) ? 1 : 0,
-                                                              pl->dg_mean.as<double>(), pl->dg_var.as<double>(), pl->dg_gsum.as<double>(),
-                                                              d_rhat.as<double>(), d_ess.as<double>(), d_lag.as<int>());
-        CU(ctx, cudaGetLastError());
-        CU(ctx, down(r->rhat, d_rhat, (size_t)ne * sizeof(double)));
-        CU(ctx, down(r->ess, d_ess, (size_t)ne * sizeof(double)));
-        CU(ctx, down(r->ess_lag, d_lag, (size_t)ne * sizeof(int)));
-    }
-    if (r->pib_mean) { pibsum.resize((size_t)pl->pib_total); CU(ctx, down(pibsum.data(), pl->d_pibsum, pibsum.size() * sizeof(double))); }
-    if (r->insample_forecast_mean && pl->d_fcsum.p) {
-        fcsum.resize((size_t)pl->pib_total / K * pl->n_h);
-        CU(ctx, down(fcsum.data(), pl->d_fcsum, fcsum.size() * sizeof(double)));
-    }
-    CU(ctx, down(ev.data(), pl->events, ev.size() * sizeof(int)));
+    CU(ctx, cudaMemcpyAsync(ev.data(), pl->events.p, ev.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+    d2h += (long long)(ev.size() * sizeof(int));
     CU(ctx, cudaStreamSynchronize(st));
-    const double n = (double)Rr;
-    for (size_t i = 0; i < pibsum.size(); ++i) r->pib_mean[i] = pibsum[i] / n;
-    for (size_t i = 0; i < fcsum.size(); ++i) r->insample_forecast_mean[i] = fcsum[i] / n;
-    // slot order -> caller order
-    std::vector<int> slot_win(pl->n_slots), slot_chain(pl->n_slots);
     int bad = 0;
-    for (int j = 0; j < nw; ++j) {
-        const int w = pl->order[j];
-        for (int c = 0; c < pl->n_chains; ++c) {
-            const int e = ev[(size_t)j * pl->n_chains + c];
-            if (r->status) r->status[(size_t)w * pl->n_chains + c] = e;
+    for (int w = 0; w < pl->n_windows; ++w) {
+        for (int c = 0; c < nc; ++c) {
+            const int e = ev[(size_t)pl->slot0[w] + c];
+            if (r->status) r->status[(size_t)w * nc + c] = e;
             bad += e != 0;
         }
     }
@@ -2201,24 +2239,13 @@ static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const long long nwh = (long long)pl->n_windows * pl->n_h;
-    DevBuf d_cdf, d_pit, d_ls, d_mom;
-    CU(ctx, d_cdf.alloc((size_t)nwh * pl->n_grid * sizeof(double)));
-    CU(ctx, d_pit.alloc((size_t)nwh * sizeof(double)));
-    CU(ctx, d_ls.alloc((size_t)nwh * sizeof(double)));
-    CU(ctx, d_mom.alloc((size_t)nwh * 3 * sizeof(double)));
     pred_finish_kernel<<<grid_for(nwh * (pl->n_grid + 1), 128), 128, 0, st>>>(pl->n_windows, pl->n_h, pl->n_grid, pl->n_chains,
                                                                               (double)pl->n_chains * (double)pl->nrun, pl->win_slot0.as<int>(),
                                                                               pl->pr_cshift.as<double>(), pl->pr_cdf.as<double>(),
-                                                                              pl->pr_score.as<double>(), d_cdf.as<double>(), d_pit.as<double>(),
-                                                                              d_ls.as<double>(), d_mom.as<double>());
+                                                                              pl->pr_score.as<double>(), pl->d_cdf.as<double>(), pl->d_pit.as<double>(),
+                                                                              pl->d_ls.as<double>(), pl->d_mom.as<double>());
     CU(ctx, cudaGetLastError());
-    auto down = [&](void* host, const DevBuf& b) -> cudaError_t {
-        return host ? cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess;
-    };
-    CU(ctx, down(pr->cdf, d_cdf));
-    CU(ctx, down(pr->pit, d_pit));
-    CU(ctx, down(pr->log_score, d_ls));
-    CU(ctx, down(pr->moments, d_mom));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, pl->flags), nullptr, pr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));
     return HMCGPU_OK;
 }
@@ -2277,7 +2304,7 @@ extern "C" int hmcgpu_estimate_multi_predictive(const int* devices, int n_dev, c
 
 static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr) {
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(nullptr, HMCGPU_ERR_ARG, "no windows");
-    const int nw = p->n_windows, K = p->K, nh = p->n_h;
+    const int nw = p->n_windows;
     std::vector<int> ord(nw);
     std::iota(ord.begin(), ord.end(), 0);
     auto Tw = [&](int w) { return p->win_end[w] - p->win_start[w] + 1; };
@@ -2289,11 +2316,10 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
         shard[d].push_back(w);
         load[d] += Tw(w);
     }
-    const size_t Rr = (size_t)p->n_chains * p->nrun;
-    const int F = 3 * K + K * K + 2 * nh + 1;
-    std::vector<long long> pib_off(nw);
-    long long acc = 0;
-    for (int w = 0; w < nw; ++w) { pib_off[w] = acc; acc += (long long)Tw(w) * K; }
+    std::vector<long long> T0(nw + 1, 0);                   // T_0 + ... + T_{w-1}: window w's offset in X0 and the ragged outputs
+    for (int w = 0; w < nw; ++w) T0[w + 1] = T0[w] + Tw(w);
+    // (pr is given only with HMCGPU_FLAG_PREDICTIVE, the only case in which n_grid may be read)
+    const std::vector<WinOut> outs = window_outputs(p->K, p->n_h, p->n_chains, p->nrun, pr ? p->n_grid : 0, p->flags);
     std::vector<int> rcs(n_dev, 0);
     std::vector<std::string> errs(n_dev);
     std::vector<hmcgpu_result> parts(n_dev);
@@ -2310,69 +2336,40 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             if (rc != 0) { rcs[d] = rc; errs[d] = hmcgpu_last_error(nullptr); return; }
             std::vector<int32_t> ser(n), iser(n), st(n), en(n);
             std::vector<int64_t> id(n), x0;
-            size_t pibn = 0;
+            long long sum_T = 0;
             for (int j = 0; j < n; ++j) {
                 const int w = ws[j];
                 ser[j] = p->win_series ? p->win_series[w] : 0; st[j] = p->win_start[w]; en[j] = p->win_end[w];
                 iser[j] = p->win_init_series ? p->win_init_series[w] : ser[j];
                 id[j] = p->win_id ? p->win_id[w] : w;
-                pibn += (size_t)Tw(w) * K;
-                if (p->X0) x0.insert(x0.end(), p->X0 + pib_off[w] / K, p->X0 + pib_off[w] / K + Tw(w));
+                sum_T += Tw(w);
+                if (p->X0) x0.insert(x0.end(), p->X0 + T0[w], p->X0 + T0[w + 1]);
             }
             hmcgpu_problem q = *p;
             q.n_windows = n; q.win_series = ser.data(); q.win_start = st.data(); q.win_end = en.data(); q.win_id = id.data();
             if (p->win_init_series) q.win_init_series = iser.data();
             if (p->X0) q.X0 = x0.data();
-            std::vector<double> mu, s2, A, pe, fc, ll, sm, sv, pb, ifc, rh, es, pcdf, ppit, pls, pmom;
-            std::vector<int32_t> status, el;
-            const bool diag = (p->flags & HMCGPU_FLAG_DIAGNOSTICS) != 0;   // (the diagnostics pointers exist only then)
+            // the shard's outputs in host staging arrays (of at least one byte: a requested output stays a non-NULL pointer)
             hmcgpu_result& o = parts[d];
-            if (r->mu) { mu.resize(n * Rr * K); o.mu = mu.data(); }
-            if (r->sigma2) { s2.resize(n * Rr * K); o.sigma2 = s2.data(); }
-            if (r->A) { A.resize(n * Rr * K * K); o.A = A.data(); }
-            if (r->pi_end) { pe.resize(n * Rr * K); o.pi_end = pe.data(); }
-            if (r->forecasts) { fc.resize(n * Rr * 2 * nh); o.forecasts = fc.data(); }
-            if (r->loglik) { ll.resize(n * Rr); o.loglik = ll.data(); }
-            if (r->summary_mean) { sm.resize((size_t)n * F); o.summary_mean = sm.data(); }
-            if (r->summary_var) { sv.resize((size_t)n * F); o.summary_var = sv.data(); }
-            if (r->pib_mean) { pb.resize(pibn); o.pib_mean = pb.data(); }
-            if (r->insample_forecast_mean) { ifc.resize(pibn / K * std::max(1, nh)); o.insample_forecast_mean = ifc.data(); }
-            if (r->status) { status.resize((size_t)n * p->n_chains); o.status = status.data(); }
-            if (diag && r->rhat) { rh.resize((size_t)n * F); o.rhat = rh.data(); }
-            if (diag && r->ess) { es.resize((size_t)n * F); o.ess = es.data(); }
-            if (diag && r->ess_lag) { el.resize((size_t)n * F); o.ess_lag = el.data(); }
             hmcgpu_predictive pq{};
-            const size_t ng = pr ? (size_t)nh * p->n_grid : 0;
-            if (pr && pr->cdf) { pcdf.resize(n * ng); pq.cdf = pcdf.data(); }
-            if (pr && pr->pit) { ppit.resize((size_t)n * nh); pq.pit = ppit.data(); }
-            if (pr && pr->log_score) { pls.resize((size_t)n * nh); pq.log_score = pls.data(); }
-            if (pr && pr->moments) { pmom.resize((size_t)n * nh * 3); pq.moments = pmom.data(); }
+            std::vector<std::vector<char>> stage(outs.size());
+            for (size_t i = 0; i < outs.size(); ++i) {
+                if (!outs[i].get(r, pr)) continue;
+                stage[i].resize(std::max<size_t>(1, (size_t)outs[i].elems(n, sum_T) * outs[i].elem));
+                outs[i].set(&o, &pq, stage[i].data());
+            }
             rc = hmcgpu_estimate_predictive(ctx, &q, &o, pr ? &pq : nullptr);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
-            if (rc >= 0) {   // scatter this shard's windows into the caller's arrays (host gather)
-                size_t po = 0;
+            for (size_t i = 0; rc >= 0 && i < outs.size(); ++i) {   // scatter this shard's windows into the caller's arrays
+                const WinOut& x = outs[i];
+                char* dst = (char*)x.get(r, pr);
+                if (!dst) continue;
+                long long t = 0;                                 // steps of the shard's windows before window j
                 for (int j = 0; j < n; ++j) {
-                    const size_t w = (size_t)ws[j];
-                    if (r->mu) memcpy(r->mu + w * Rr * K, mu.data() + j * Rr * K, Rr * K * sizeof(double));
-                    if (r->sigma2) memcpy(r->sigma2 + w * Rr * K, s2.data() + j * Rr * K, Rr * K * sizeof(double));
-                    if (r->A) memcpy(r->A + w * Rr * K * K, A.data() + j * Rr * K * K, Rr * K * K * sizeof(double));
-                    if (r->pi_end) memcpy(r->pi_end + w * Rr * K, pe.data() + j * Rr * K, Rr * K * sizeof(double));
-                    if (r->forecasts) memcpy(r->forecasts + w * Rr * 2 * nh, fc.data() + j * Rr * 2 * nh, Rr * 2 * nh * sizeof(double));
-                    if (r->loglik) memcpy(r->loglik + w * Rr, ll.data() + j * Rr, Rr * sizeof(double));
-                    if (r->summary_mean) memcpy(r->summary_mean + w * F, sm.data() + (size_t)j * F, F * sizeof(double));
-                    if (r->summary_var) memcpy(r->summary_var + w * F, sv.data() + (size_t)j * F, F * sizeof(double));
-                    if (o.rhat) memcpy(r->rhat + w * F, rh.data() + (size_t)j * F, F * sizeof(double));
-                    if (o.ess) memcpy(r->ess + w * F, es.data() + (size_t)j * F, F * sizeof(double));
-                    if (o.ess_lag) memcpy(r->ess_lag + w * F, el.data() + (size_t)j * F, F * sizeof(int32_t));
-                    if (pq.cdf) memcpy(pr->cdf + w * ng, pcdf.data() + j * ng, ng * sizeof(double));
-                    if (pq.pit) memcpy(pr->pit + w * nh, ppit.data() + (size_t)j * nh, nh * sizeof(double));
-                    if (pq.log_score) memcpy(pr->log_score + w * nh, pls.data() + (size_t)j * nh, nh * sizeof(double));
-                    if (pq.moments) memcpy(pr->moments + w * nh * 3, pmom.data() + (size_t)j * nh * 3, nh * 3 * sizeof(double));
-                    if (r->insample_forecast_mean) memcpy(r->insample_forecast_mean + pib_off[w] / K * nh, ifc.data() + po / K * nh, (size_t)Tw((int)w) * nh * sizeof(double));
-                    if (r->pib_mean) memcpy(r->pib_mean + pib_off[w], pb.data() + po, (size_t)Tw((int)w) * K * sizeof(double));
-                    po += (size_t)Tw((int)w) * K;
-                    if (r->status) memcpy(r->status + w * p->n_chains, status.data() + (size_t)j * p->n_chains, p->n_chains * sizeof(int32_t));
+                    const int w = ws[j];
+                    memcpy(dst + x.elems(w, T0[w]) * x.elem, stage[i].data() + x.elems(j, t) * x.elem, x.elems(1, Tw(w)) * x.elem);
+                    t += Tw(w);
                 }
             }
             hmcgpu_ctx_destroy(ctx);
