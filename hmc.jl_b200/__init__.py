@@ -6,11 +6,11 @@ api.py (mirror of Hmc.estopt / Hmc.estimatemodel / Hmc.estimatesignals!), julia/
 """
 from . import build  # noqa: F401
 from .api import (EstOpt, estimatemodel, estimatesignals, estimate_windows, shard_windows, expanding_windows,  # noqa: F401
-                  gather_window_summaries, saveresults, write_summaries, write_diagnostics, write_predictive,
+                  gather_window_summaries, saveresults, write_summaries, write_diagnostics, write_predictive, write_ranked,
                   predictive_quantiles, forecastinsample,
                   signal_summaries, calcdispersion, calccorr, write_signal_summaries, write_dispersion,
                   makeparams_states, sample_and_forecast_all, saveinsampleforecasts, smoothStates, savesmoothresults)
 from .binding import (Context, HmcGpuError, Plan, ProblemSpec, estimate, estimate_multi, load, lib_path,  # noqa: F401
                       FLAG_REF_Q1, FLAG_DRAWS, FLAG_SUMMARY, FLAG_SMOOTHED_MEAN, FLAG_LOGLIK, FLAG_FILTERED_MEAN, FLAG_DIAGNOSTICS,
-                      FLAG_PREDICTIVE, Predictive,
+                      FLAG_PREDICTIVE, FLAG_RANKED, Predictive, Ranked,
                       SYMBOLS)

@@ -229,18 +229,24 @@ def shard_windows(T: Sequence[int], n_shards: int):
 
 def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                      precision=32, draws=False, summary=True, smoothed=False, loglik=False, win_id=None,
-                     win_series=None, diagnostics=False, predictive_grid=None, ctx: Optional[B.Context] = None, device: int = 0):
+                     win_series=None, diagnostics=False, predictive_grid=None, quantiles=None, rank_diagnostics=False,
+                     ctx: Optional[B.Context] = None, device: int = 0):
     """Many end-date windows in one call (what the SLURM job array does one process at a time).  `diagnostics=True` adds
     `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics).
     `predictive_grid` (increasing points, shared by every window and horizon) adds the posterior predictive distribution of
     every forecast: `pred_cdf` [n_windows, n_h, n_grid], `pit` and `log_score` [n_windows, n_h] and `pred_moments`
-    [n_windows, n_h, 3] (mean, variance, skewness); see write_predictive and include/hmcgpu.h."""
+    [n_windows, n_h, 3] (mean, variance, skewness); see write_predictive and include/hmcgpu.h.  `quantiles` (probabilities
+    in [0, 1]) and / or `rank_diagnostics=True` keep every saved draw on the device (HMCGPU_FLAG_RANKED) and add the exact
+    posterior `quantiles` [n_windows, F, n_probs], the rank-normalised split-R̂ `rhat_rank` and the bulk / tail effective
+    sample sizes `ess_bulk` / `ess_tail` [n_windows, F]; see write_ranked."""
+    ranked = quantiles is not None or rank_diagnostics
     flags = B.FLAG_REF_Q1 | (B.FLAG_DRAWS if draws else 0) | (B.FLAG_SUMMARY if summary else 0) \
         | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0) \
-        | (B.FLAG_DIAGNOSTICS if diagnostics else 0) | (B.FLAG_PREDICTIVE if predictive_grid is not None else 0)
+        | (B.FLAG_DIAGNOSTICS if diagnostics else 0) | (B.FLAG_PREDICTIVE if predictive_grid is not None else 0) \
+        | (B.FLAG_RANKED if ranked else 0)
     spec = B.ProblemSpec(y, win_start, win_end, K=K, n_chains=n_chains, burnin=burnin, nrun=nrun, seed=seed,
                          horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series,
-                         pred_grid=predictive_grid)
+                         pred_grid=predictive_grid, quantile_probs=quantiles)
     own = ctx is None
     ctx = ctx or B.Context(device)
     try:
@@ -381,6 +387,21 @@ def write_diagnostics(out, K: int, horizons: Sequence[int], dates: Sequence, dir
     (out.ess_lag, include/hmcgpu.h) over-estimates the effective sample size.  Returns {"<var>_rhat": path, "<var>_ess": path}."""
     paths = {}
     for kind, table in (("rhat", out.rhat), ("ess", out.ess)):
+        for name, path in _write_tables(_summary_tables(table, K, horizons, kind), dates, directory, kind).items():
+            paths[f"{name}_{kind}"] = path
+    return paths
+
+
+def write_ranked(out, K: int, horizons: Sequence[int], dates: Sequence, directory: str):
+    """The ranked outputs of estimate_windows(quantiles=..., rank_diagnostics=True) in the column layout of write_summaries,
+    one row per window in caller order: `<var>_q<pct>.csv` per quantile probability (columns `<col>_q<pct>`, e.g. `_q5` for
+    0.05), `<var>_rhat_rank.csv` (rank-normalised split-R̂), `<var>_ess_bulk.csv` and `<var>_ess_tail.csv`.  NaN marks a field
+    with a non-finite draw; R̂ / ESS are also NaN for a field (or a tail indicator) without within-chain variation.
+    Returns {"<var>_<kind>": path}."""
+    tables = [(f"q{100 * float(p):g}", np.asarray(out.quantiles)[:, :, j]) for j, p in enumerate(out.quantile_probs)]
+    tables += [("rhat_rank", out.rhat_rank), ("ess_bulk", out.ess_bulk), ("ess_tail", out.ess_tail)]
+    paths = {}
+    for kind, table in tables:
         for name, path in _write_tables(_summary_tables(table, K, horizons, kind), dates, directory, kind).items():
             paths[f"{name}_{kind}"] = path
     return paths

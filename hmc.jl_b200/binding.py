@@ -20,6 +20,7 @@ FLAG_LOGLIK = 16
 FLAG_FILTERED_MEAN = 64   # pib_mean / insample_forecast_mean carry the FILTERED means (the reference's published in-sample table)
 FLAG_DIAGNOSTICS = 128    # rhat / ess / ess_lag per window and summary field (split-R̂ and ESS, include/hmcgpu.h)
 FLAG_PREDICTIVE = 256     # posterior predictive CDF on a grid, PIT, log score and moments per window and horizon (hmcgpu_predictive)
+FLAG_RANKED = 512         # keep every saved draw on the device: exact quantiles, rank-normalised R̂, bulk / tail ESS (hmcgpu_ranked)
 
 ERR_ARG, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED, ERR_NODEVICE = -1, -2, -3, -4, -5
 
@@ -30,7 +31,7 @@ SYMBOLS = [
     "hmcgpu_plan_fetch", "hmcgpu_plan_destroy", "hmcgpu_filter", "hmcgpu_filter_masked", "hmcgpu_smooth", "hmcgpu_sample_states",
     "hmcgpu_draw_params", "hmcgpu_draw_params_signals", "hmcgpu_forecast", "hmcgpu_philox", "hmcgpu_philox_rounds",
     "hmcgpu_build_info", "hmcgpu_ctx_trim", "hmcgpu_estimate_predictive", "hmcgpu_estimate_multi_predictive",
-    "hmcgpu_plan_fetch_predictive",
+    "hmcgpu_plan_fetch_predictive", "hmcgpu_estimate_ranked", "hmcgpu_estimate_multi_ranked", "hmcgpu_plan_fetch_ranked",
 ]
 KERNEL_NAMES = {0: "gibbs_sweeps_kernel (thread per chain)", 1: "gibbs_scan_kernel (warp per chain, time-parallel)",
                 2: "gibbs_wide_kernel (lane per state)", 3: "(reserved)",
@@ -65,6 +66,10 @@ class Result(C.Structure):
 
 class Predictive(C.Structure):
     _fields_ = [("cdf", _dp), ("pit", _dp), ("log_score", _dp), ("moments", _dp)]
+
+
+class Ranked(C.Structure):
+    _fields_ = [("probs", _dp), ("n_probs", C.c_int32), ("quantiles", _dp), ("rhat_rank", _dp), ("ess_bulk", _dp), ("ess_tail", _dp)]
 
 
 class HmcGpuError(RuntimeError):
@@ -112,6 +117,10 @@ def load(build_if_missing: bool = True):
     L.hmcgpu_estimate_multi_predictive.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
                                                    C.POINTER(Predictive)]
     L.hmcgpu_plan_fetch_predictive.argtypes = [C.c_void_p, C.POINTER(Predictive)]
+    L.hmcgpu_estimate_ranked.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Result), C.POINTER(Predictive), C.POINTER(Ranked)]
+    L.hmcgpu_estimate_multi_ranked.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
+                                               C.POINTER(Predictive), C.POINTER(Ranked)]
+    L.hmcgpu_plan_fetch_ranked.argtypes = [C.c_void_p, C.POINTER(Ranked)]
     L.hmcgpu_plan_destroy.argtypes = [C.c_void_p]
     L.hmcgpu_plan_destroy.restype = None
     L.hmcgpu_filter.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _dp, C.c_int64,
@@ -137,6 +146,10 @@ def _f64(a):
 
 def _p(a, t=_dp):
     return None if a is None else a.ctypes.data_as(t)
+
+
+def _ref(st):
+    return None if st is None else C.byref(st)
 
 
 class Context:
@@ -249,8 +262,9 @@ class ProblemSpec:
     def __init__(self, y, win_start, win_end, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                  precision=32, flags=FLAG_REF_Q1 | FLAG_DRAWS, win_series=None, win_id=None,
                  xi=None, alpha=None, nu=None, beta0=None, beta=None, kappa=1.0, is_signal=None, X0=None,
-                 win_init_series=None, pi_row_back=0, pred_grid=None):
-        """`pred_grid`: the points of the posterior predictive CDF (FLAG_PREDICTIVE; one grid for every window and horizon)."""
+                 win_init_series=None, pi_row_back=0, pred_grid=None, quantile_probs=None):
+        """`pred_grid`: the points of the posterior predictive CDF (FLAG_PREDICTIVE; one grid for every window and horizon).
+        `quantile_probs`: the probabilities of the exact posterior quantiles of every summary field (FLAG_RANKED; passed at fetch)."""
         y = np.asarray(y, dtype=np.float64)
         if y.ndim == 1:
             y = y[None, :]
@@ -285,6 +299,10 @@ class ProblemSpec:
         if flags & FLAG_PREDICTIVE and self.pred_grid is None:
             raise ValueError("FLAG_PREDICTIVE needs pred_grid")
         self.n_grid = 0 if self.pred_grid is None else len(self.pred_grid)
+        # host-side only (hmcgpu_ranked carries them to the fetch); without the flag nothing would compute them
+        self.quantile_probs = None if quantile_probs is None else np.ascontiguousarray(np.ravel(quantile_probs), dtype=np.float64)
+        if self.quantile_probs is not None and not flags & FLAG_RANKED:
+            raise ValueError("quantile_probs given without FLAG_RANKED")
 
     def struct(self) -> Problem:
         return Problem(_p(self.y), self.y_len, self.n_series, self.n_windows, _p(self.win_series, _i32p),
@@ -335,6 +353,20 @@ class ProblemSpec:
         o.pred_moments = np.empty((nw, nh, 3))
         return Predictive(_p(o.pred_cdf), _p(o.pit), _p(o.log_score), _p(o.pred_moments))
 
+    def alloc_ranked(self, o, probs=None):
+        """Adds the ranked outputs to `o` (quantiles [nw, F, n_probs] at `probs`, default quantile_probs; rhat_rank / ess_bulk /
+        ess_tail [nw, F] in the field order of summary_mean) and returns the hmcgpu_ranked struct over them; None without
+        FLAG_RANKED."""
+        if not self.flags & FLAG_RANKED:
+            return None
+        probs = self.quantile_probs if probs is None else np.ascontiguousarray(np.ravel(probs), dtype=np.float64)
+        probs = np.zeros(0) if probs is None else probs
+        nw, F = self.n_windows, 3 * self.K + self.K * self.K + 2 * self.n_h + 1
+        o.quantile_probs = probs
+        o.quantiles = np.empty((nw, F, len(probs)))
+        o.rhat_rank = np.empty((nw, F)); o.ess_bulk = np.empty((nw, F)); o.ess_tail = np.empty((nw, F))
+        return Ranked(_p(probs), len(probs), _p(o.quantiles), _p(o.rhat_rank), _p(o.ess_bulk), _p(o.ess_tail))
+
     def finish(self, o, res, rc):
         o.events = rc
         o.gpu_ms, o.sweep_kernel_ms = res.gpu_ms, res.sweep_kernel_ms
@@ -360,8 +392,11 @@ def estimate(ctx: Context, spec: ProblemSpec):
     """hmcgpu_estimate: host buffers in, all sweeps, host buffers out."""
     o, res = spec.alloc_result()
     pr = spec.alloc_predictive(o)
+    rk = spec.alloc_ranked(o)
     prob = spec.struct()
-    if pr is None:
+    if rk is not None:
+        rc = ctx._check(ctx.L.hmcgpu_estimate_ranked(ctx.h, C.byref(prob), C.byref(res), _ref(pr), C.byref(rk)))
+    elif pr is None:
         rc = ctx._check(ctx.L.hmcgpu_estimate(ctx.h, C.byref(prob), C.byref(res)))
     else:
         rc = ctx._check(ctx.L.hmcgpu_estimate_predictive(ctx.h, C.byref(prob), C.byref(res), C.byref(pr)))
@@ -372,9 +407,12 @@ def estimate_multi(devices, spec: ProblemSpec):
     L = load()
     o, res = spec.alloc_result()
     pr = spec.alloc_predictive(o)
+    rk = spec.alloc_ranked(o)
     prob = spec.struct()
     dev = (C.c_int * len(devices))(*devices)
-    if pr is None:
+    if rk is not None:
+        rc = L.hmcgpu_estimate_multi_ranked(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), C.byref(rk))
+    elif pr is None:
         rc = L.hmcgpu_estimate_multi(dev, len(devices), C.byref(prob), C.byref(res))
     else:
         rc = L.hmcgpu_estimate_multi_predictive(dev, len(devices), C.byref(prob), C.byref(res), C.byref(pr))
@@ -402,7 +440,19 @@ class Plan:
         pr = self.spec.alloc_predictive(o)
         if pr is not None:
             self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_predictive(self.h, C.byref(pr)))
+        if self.spec.flags & FLAG_RANKED:
+            self.fetch_ranked(out=o)
         return self.spec.finish(o, res, rc)
+
+    def fetch_ranked(self, probs=None, out=None):
+        """hmcgpu_plan_fetch_ranked: the ranked outputs of the last run (quantiles at `probs`, default the spec's
+        quantile_probs), computed now from the retained draws; may be called again with other probabilities."""
+        o = SimpleNamespace() if out is None else out
+        rk = self.spec.alloc_ranked(o, probs)
+        if rk is None:
+            raise ValueError("fetch_ranked on a plan without FLAG_RANKED")
+        self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_ranked(self.h, C.byref(rk)))
+        return o
 
     def close(self):
         if getattr(self, "h", None):

@@ -6,6 +6,7 @@
 #include "gibbs_seg_kernel.cuh"
 #include "diagnostics.cuh"
 #include "predictive.cuh"
+#include "ranked.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -1349,7 +1350,8 @@ struct hmcgpu_plan {
     DevBuf d_sum, d_sumsq, d_pibsum, d_fcsum;
     // the per-window outputs (window_outputs), laid out like the caller's arrays: the draws gathered per chunk, the rest
     // finished at fetch
-    DevBuf d_mu, d_sig2, d_A, d_pie, d_fc, d_ll, d_mean, d_var, d_pib, d_ifc, d_rhat, d_ess, d_lag, d_cdf, d_pit, d_ls, d_mom;
+    DevBuf d_mu, d_sig2, d_A, d_pie, d_fc, d_ll, d_mean, d_var, d_pib, d_ifc, d_rhat, d_ess, d_lag, d_cdf, d_pit, d_ls, d_mom, d_quant,
+        d_rrank, d_essb, d_esst;
     // HMCGPU_FLAG_DIAGNOSTICS (diagnostics.cuh): streaming state per (slot, field), per-sequence means / variances and lag sums
     // per (window, field)
     DevBuf dg_P, dg_S1, dg_head, dg_ring, dg_mean, dg_var, dg_gsum;
@@ -1357,6 +1359,8 @@ struct hmcgpu_plan {
     DevBuf pr_grid, pr_cshift, pr_cdf, pr_score;
     int n_grid = 0, pr_tg = 32, pr_td = 1;    // threads per slot and draws per tile of pred_accum_kernel
     PredHorizons pr_h{};
+    // HMCGPU_FLAG_RANKED (ranked.cuh): every saved draw, keep[((w*F + f)*n_chains + c)*nrun + i]
+    DevBuf rk_keep;
     DevBuf d_diag;       // segment kernel: chain-sweeps that fell back to the exact entering vectors
     unsigned long long seg_fallbacks[2] = {0, 0};   // [0] chain-sweeps on the exact path, [1] speculative groups (sum over chain-sweeps)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
@@ -1377,11 +1381,12 @@ struct hmcgpu_plan {
 // F: fields per window of the summaries and diagnostics (mu[K], sigma2[K], A[K*K], pi_end[K], forecasts[2*n_h], loglik)
 static int summary_fields(int K, int n_h) { return 3 * K + K * K + 2 * n_h + 1; }
 
-// One per-window output of hmcgpu_result / hmcgpu_predictive.  Window w holds per_window + per_step * T_w elements; the windows
-// are concatenated in caller order, in the caller's array and in the plan's device buffer `dev` alike.
+// One per-window output of hmcgpu_result / hmcgpu_predictive / hmcgpu_ranked.  Window w holds per_window + per_step * T_w
+// elements; the windows are concatenated in caller order, in the caller's array and in the plan's device buffer `dev` alike.
+enum class OutStruct { result, predictive, ranked };
 struct WinOut {
     const char* name;
-    bool pred;                 // a field of hmcgpu_predictive (else of hmcgpu_result)
+    OutStruct in;              // the struct that holds the caller's pointer
     size_t field;              // offset of the caller's pointer in that struct
     size_t elem;               // bytes per element
     long long per_window, per_step;
@@ -1391,26 +1396,33 @@ struct WinOut {
     DevBuf hmcgpu_plan::*dev;  // NULL for status, which is read from the chain slots
     // elements of n windows of sum_T steps in all; elems(w, T_0 + ... + T_{w-1}) is the offset of window w
     long long elems(long long n, long long sum_T) const { return per_window * n + per_step * sum_T; }
-    void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr) const {     // NULL: not requested, or not readable
-        const void* s = pred ? (const void*)pr : (const void*)r;
+    void* base(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk) const {
+        return in == OutStruct::result ? (void*)r : in == OutStruct::predictive ? (void*)pr : (void*)rk;
+    }
+    // NULL: not requested, or not readable
+    void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk = nullptr) const {
+        const void* s = base(r, pr, rk);
         void* p = nullptr;
         if (s && (on || !gated)) memcpy(&p, (const char*)s + field, sizeof p);
         return p;
     }
-    void set(hmcgpu_result* r, hmcgpu_predictive* pr, void* p) const { memcpy((char*)(pred ? (void*)pr : (void*)r) + field, &p, sizeof p); }
+    void set(hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk, void* p) const { memcpy((char*)base(r, pr, rk) + field, &p, sizeof p); }
 };
 
-static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long long nrun, int n_grid, unsigned flags) {
+// n_probs: quantiles per field of the ranked outputs (known at hmcgpu_plan_fetch_ranked)
+static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long long nrun, int n_grid, int n_probs, unsigned flags) {
     const long long R = (long long)n_chains * nrun, F = summary_fields(K, n_h);
     const bool draws = flags & HMCGPU_FLAG_DRAWS, summary = flags & HMCGPU_FLAG_SUMMARY, diag = flags & HMCGPU_FLAG_DIAGNOSTICS,
-               pred = flags & HMCGPU_FLAG_PREDICTIVE, mean = flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN);
+               pred = flags & HMCGPU_FLAG_PREDICTIVE, mean = flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN),
+               ranked = flags & HMCGPU_FLAG_RANKED;
     const bool ll = draws && (flags & HMCGPU_FLAG_LOGLIK);
     const char* D = "HMCGPU_FLAG_DRAWS";
     const char* M = "HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN";
     const size_t f8 = sizeof(double), i4 = sizeof(int32_t);
     using P = hmcgpu_plan;
-#define RES(f) #f, false, offsetof(hmcgpu_result, f)
-#define PRED(f) #f, true, offsetof(hmcgpu_predictive, f)
+#define RES(f) #f, OutStruct::result, offsetof(hmcgpu_result, f)
+#define PRED(f) #f, OutStruct::predictive, offsetof(hmcgpu_predictive, f)
+#define RANK(f) #f, OutStruct::ranked, offsetof(hmcgpu_ranked, f)
     std::vector<WinOut> o = {
         {RES(mu), f8, R * K, 0, draws, false, D, &P::d_mu},
         {RES(sigma2), f8, R * K, 0, draws, false, D, &P::d_sig2},
@@ -1430,9 +1442,14 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
         {PRED(pit), f8, n_h, 0, pred, true, "", &P::d_pit},
         {PRED(log_score), f8, n_h, 0, pred, true, "", &P::d_ls},
         {PRED(moments), f8, 3ll * n_h, 0, pred, true, "", &P::d_mom},
+        {RANK(quantiles), f8, F * n_probs, 0, ranked, true, "", &P::d_quant},
+        {RANK(rhat_rank), f8, F, 0, ranked, true, "", &P::d_rrank},
+        {RANK(ess_bulk), f8, F, 0, ranked, true, "", &P::d_essb},
+        {RANK(ess_tail), f8, F, 0, ranked, true, "", &P::d_esst},
     };
 #undef RES
 #undef PRED
+#undef RANK
     return o;
 }
 
@@ -1463,6 +1480,12 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuni
     if (p->burnin < 0 || p->nrun < 1) return fail(ctx, HMCGPU_ERR_ARG, "burnin < 0 or nrun < 1");
     if (p->burnin + p->nrun > 0xffffffffLL) return fail(ctx, HMCGPU_ERR_ARG, "more than 2^32 sweeps");
     if ((p->flags & HMCGPU_FLAG_DIAGNOSTICS) && p->nrun < 4) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_DIAGNOSTICS needs nrun >= 4 (two sequences of >= 2 draws per chain)");
+    if (p->flags & HMCGPU_FLAG_RANKED) {
+        if (p->nrun < 4) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_RANKED needs nrun >= 4 (two sequences of >= 2 draws per chain)");
+        // (positions within a field's draws are 32-bit in the sort)
+        if ((long long)p->n_chains * p->nrun >= 0x80000000LL)
+            return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_RANKED needs n_chains * nrun < 2^31 (got %lld)", (long long)p->n_chains * p->nrun);
+    }
     if (p->precision != 32 && p->precision != 64) return fail(ctx, HMCGPU_ERR_ARG, "precision must be 32 or 64");
     if (p->n_h < 0 || p->n_h > kMaxH || (p->n_h > 0 && !p->horizons)) return fail(ctx, HMCGPU_ERR_ARG, "0 <= n_h <= %d", kMaxH);
     if (p->flags & HMCGPU_FLAG_PREDICTIVE) {
@@ -1826,8 +1849,10 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
         }
         CU(ctx, pl->d_pibsum.alloc((size_t)pib_total * sizeof(double)));
     }
-    for (const WinOut& o : window_outputs(K, p->n_h, nc, p->nrun, pl->n_grid, p->flags))
-        if (o.on && o.dev) CU(ctx, (pl->*o.dev).alloc((size_t)o.elems(nw, sumT) * o.elem));
+    // (the ranked outputs are allocated at hmcgpu_plan_fetch_ranked, which knows n_probs)
+    for (const WinOut& o : window_outputs(K, p->n_h, nc, p->nrun, pl->n_grid, 0, p->flags))
+        if (o.on && o.dev && o.in != OutStruct::ranked) CU(ctx, (pl->*o.dev).alloc((size_t)o.elems(nw, sumT) * o.elem));
+    if (p->flags & HMCGPU_FLAG_RANKED) CU(ctx, pl->rk_keep.alloc((size_t)nw * pl->F * nc * (size_t)p->nrun * sizeof(R)));
     // window statistics (once per plan)
     const size_t smem = (size_t)pl->max_T;
     if (smem > 200 * 1024) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window longer than %d observations", 200 * 1024);
@@ -1988,6 +2013,12 @@ static int plan_run_t(hmcgpu_plan* pl) {
             TRY(sequence(d0, std::min<long long>(d0 + n, nh), 0, nh, 0));
             TRY(sequence(std::max(d0, h2), d0 + n, h2, pl->nrun, 1));
         }
+        if (pl->flags & HMCGPU_FLAG_RANKED) {
+            ranked_keep_kernel<R><<<dim3(pl->n_windows, pl->F), dim3(32, 8), 0, st>>>(pl->F, ns, pl->chunk, n, d0, pl->nrun, pl->n_chains,
+                                                                                     pl->win_slot0.as<int>(), buf, pl->rk_keep.as<R>());
+            CU(ctx, cudaGetLastError());
+            ++pl->n_launches;
+        }
         if (pl->flags & HMCGPU_FLAG_PREDICTIVE) {
             const int sb = kPredThreads / pl->pr_tg;
             const size_t smem = pred_smem_bytes(Kr, pl->n_h, sb * pl->pr_td);
@@ -2134,6 +2165,14 @@ static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_pla
     const Tuning t = read_tuning();
     TRY(validate_problem(ctx, p, t));
     CU(ctx, cudaSetDevice(ctx->device));
+    if (p->flags & HMCGPU_FLAG_RANKED) {
+        // the retained draws are the one allocation that grows with nrun: refuse a shape whose draws cannot fit before allocating
+        size_t free_b = 0, total_b = 0;
+        CU(ctx, cudaMemGetInfo(&free_b, &total_b));
+        const double keep = (double)p->n_windows * summary_fields(p->K, p->n_h) * p->n_chains * (double)p->nrun * (p->precision / 8);
+        if (keep > (double)total_b)
+            return fail(ctx, HMCGPU_ERR_ALLOC, "HMCGPU_FLAG_RANKED retains %.0f bytes of draws, more than the device's %zu bytes", keep, total_b);
+    }
     tl_pool = ctx->pool;
     std::unique_ptr<hmcgpu_plan> pl(new hmcgpu_plan());
     pl->ctx = ctx;
@@ -2173,12 +2212,12 @@ extern "C" int hmcgpu_plan_fetch(hmcgpu_plan* pl, hmcgpu_result* r) {
     GUARD(pl->ctx, plan_fetch_impl(pl, r));
 }
 
-// Enqueues the copy of every requested output the plan holds (of r, or of pr) into the caller's arrays; adds the bytes to *bytes
-// (NULL: the predictive outputs, which hmcgpu_result's d2h_bytes does not count)
+// Enqueues the copy of every requested output the plan holds (of r, pr or rk) into the caller's arrays; adds the bytes to *bytes
+// (NULL: the predictive and ranked outputs, which hmcgpu_result's d2h_bytes does not count)
 static int download(hmcgpu_plan* pl, const std::vector<WinOut>& outs, const hmcgpu_result* r, const hmcgpu_predictive* pr,
-                    long long* bytes) {
+                    const hmcgpu_ranked* rk, long long* bytes) {
     for (const WinOut& o : outs) {
-        void* host = o.get(r, pr);
+        void* host = o.get(r, pr, rk);
         if (!host || !o.dev || !(pl->*o.dev).p) continue;         // (an output of no elements has no buffer)
         const DevBuf& b = pl->*o.dev;
         CU(pl->ctx, cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, pl->ctx->stream));
@@ -2190,7 +2229,7 @@ static int download(hmcgpu_plan* pl, const std::vector<WinOut>& outs, const hmcg
 static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     hmcgpu_ctx* ctx = pl->ctx;
     if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch before plan_run");
-    const std::vector<WinOut> outs = window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, pl->flags);
+    const std::vector<WinOut> outs = window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags);
     for (const WinOut& o : outs)
         if (!o.on && o.get(r, nullptr)) return fail(ctx, HMCGPU_ERR_ARG, "%s requested without %s", o.name, o.need);
     CU(ctx, cudaSetDevice(ctx->device));
@@ -2211,7 +2250,7 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     if (pl->d_ifc.p) mean_finish_kernel<<<grid_for(nifc, 256), 256, 0, st>>>(nifc, n, pl->d_fcsum.as<double>(), pl->d_ifc.as<double>());
     CU(ctx, cudaGetLastError());
     long long d2h = 0;
-    TRY(download(pl, outs, r, nullptr, &d2h));
+    TRY(download(pl, outs, r, nullptr, nullptr, &d2h));
     std::vector<int> ev(pl->n_slots);
     CU(ctx, cudaMemcpyAsync(ev.data(), pl->events.p, ev.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
     d2h += (long long)(ev.size() * sizeof(int));
@@ -2245,7 +2284,7 @@ static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
                                                                               pl->pr_score.as<double>(), pl->d_cdf.as<double>(), pl->d_pit.as<double>(),
                                                                               pl->d_ls.as<double>(), pl->d_mom.as<double>());
     CU(ctx, cudaGetLastError());
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, pl->flags), nullptr, pr, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, pr, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));
     return HMCGPU_OK;
 }
@@ -2253,6 +2292,124 @@ static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
 extern "C" int hmcgpu_plan_fetch_predictive(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
     if (!pl || !pr) return HMCGPU_ERR_ARG;
     GUARD(pl->ctx, plan_fetch_predictive_impl(pl, pr));
+}
+
+static int check_ranked(hmcgpu_ctx* ctx, const hmcgpu_ranked* rk) {
+    if (rk->n_probs < 0 || rk->n_probs > kRankedMaxProbs)
+        return fail(ctx, HMCGPU_ERR_ARG, "hmcgpu_ranked.n_probs = %d is outside 0..%d", rk->n_probs, kRankedMaxProbs);
+    if (rk->n_probs > 0 && !rk->probs) return fail(ctx, HMCGPU_ERR_ARG, "hmcgpu_ranked.probs is NULL with n_probs = %d", rk->n_probs);
+    for (int k = 0; k < rk->n_probs; ++k)
+        if (!std::isfinite(rk->probs[k]) || rk->probs[k] < 0.0 || rk->probs[k] > 1.0)
+            return fail(ctx, HMCGPU_ERR_ARG, "hmcgpu_ranked.probs[%d] = %g is not a finite probability in [0, 1]", k, rk->probs[k]);
+    return HMCGPU_OK;
+}
+
+// The ranked outputs of every (window, field) segment of the retained draws (ranked.cuh), in batches of segments whose scratch
+// stays near 2 GiB (at least one segment).  These launches are not plan_run's: n_launches leaves them out.
+template <typename R>
+static int fetch_ranked_t(hmcgpu_plan* pl, const hmcgpu_ranked* rk) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    cudaStream_t st = ctx->stream;
+    const int nc = pl->n_chains, M = 2 * nc;
+    const long long Rs = (long long)nc * pl->nrun, n_seg = (long long)pl->n_windows * pl->F, nh = pl->nrun / 2;
+    RankedProbs probs{};
+    probs.n = rk->n_probs;
+    for (int k = 0; k < rk->n_probs; ++k) probs.p[k] = rk->probs[k];
+    CU(ctx, pl->d_quant.alloc((size_t)n_seg * rk->n_probs * sizeof(double)));
+    CU(ctx, pl->d_rrank.alloc((size_t)n_seg * sizeof(double)));
+    CU(ctx, pl->d_essb.alloc((size_t)n_seg * sizeof(double)));
+    CU(ctx, pl->d_esst.alloc((size_t)n_seg * sizeof(double)));
+    // per segment: two key and two position buffers for the sort, the normal scores, the per-sequence statistics
+    const size_t seg_bytes = (size_t)Rs * (2 * sizeof(unsigned long long) + 2 * sizeof(int) + sizeof(double)) +
+                             (size_t)M * (kDiagLags + 2) * sizeof(double) + 256;
+    const long long B = std::max<long long>(1, std::min<long long>({n_seg, (long long)((2ull << 30) / seg_bytes), 0x7fffffffLL / Rs}));
+    const size_t nB = (size_t)B * Rs;
+    DevBuf keys0, keys1, pos0, pos1, z, g, smean, svar, gsum, qs, bad, rh, es, lag, offs, temp;
+    CU(ctx, keys0.alloc(nB * sizeof(unsigned long long)));
+    CU(ctx, keys1.alloc(nB * sizeof(unsigned long long)));
+    CU(ctx, pos0.alloc(nB * sizeof(int)));
+    CU(ctx, pos1.alloc(nB * sizeof(int)));
+    CU(ctx, z.alloc(nB * sizeof(double)));
+    CU(ctx, g.alloc((size_t)B * M * kDiagLags * sizeof(double)));
+    CU(ctx, smean.alloc((size_t)B * M * sizeof(double)));
+    CU(ctx, svar.alloc((size_t)B * M * sizeof(double)));
+    CU(ctx, gsum.alloc((size_t)B * kDiagLags * sizeof(double)));
+    CU(ctx, qs.alloc((size_t)B * kRankedQuants * sizeof(double)));
+    CU(ctx, bad.alloc((size_t)B));
+    CU(ctx, rh.alloc((size_t)4 * B * sizeof(double)));
+    CU(ctx, es.alloc((size_t)4 * B * sizeof(double)));
+    CU(ctx, lag.alloc((size_t)4 * B * sizeof(int)));
+    std::vector<int> off(B + 1);
+    for (long long s = 0; s <= B; ++s) off[s] = (int)(s * Rs);
+    CU(ctx, offs.alloc(off.size() * sizeof(int)));
+    CU(ctx, cudaMemcpyAsync(offs.p, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    for (long long s0 = 0; s0 < n_seg; s0 += B) {
+        const int nb = (int)std::min<long long>(B, n_seg - s0);
+        const long long N = (long long)nb * Rs;
+        const R* x = pl->rk_keep.as<R>() + (size_t)s0 * Rs;
+        // keys of x (fold: of |x - q(0.5)|) sorted per segment, then the normal scores of their ranks into z; returns the sorted keys
+        auto scores = [&](const double* fold, const unsigned long long** sorted) -> int {
+            ranked_keys_kernel<R><<<grid_for(N, 256), 256, 0, st>>>(N, Rs, x, fold, keys0.as<unsigned long long>(), pos0.as<int>());
+            CU(ctx, cudaGetLastError());
+            cub::DoubleBuffer<unsigned long long> kb(keys0.as<unsigned long long>(), keys1.as<unsigned long long>());
+            cub::DoubleBuffer<int> pb(pos0.as<int>(), pos1.as<int>());
+            size_t tb = 0;
+            CU(ctx, ranked_sort(nullptr, tb, kb, pb, (int)N, nb, offs.as<int>(), st));
+            if (tb > temp.bytes) CU(ctx, temp.alloc(tb));
+            CU(ctx, ranked_sort(temp.p, tb, kb, pb, (int)N, nb, offs.as<int>(), st));
+            ranked_scores_kernel<<<grid_for(N, 256), 256, 0, st>>>(N, Rs, kb.Current(), pb.Current(), z.as<double>());
+            CU(ctx, cudaGetLastError());
+            *sorted = kb.Current();
+            return HMCGPU_OK;
+        };
+        // split R̂ / ESS of one transformed sequence (normal scores z, or the indicator 1[x <= qs[qi]]) into rh / es row t
+        auto split = [&](bool use_z, int qi, int t) -> int {
+            const long long n_seqs = (long long)nb * M;
+            ranked_stats_kernel<R><<<grid_for(n_seqs, kRankedSeqWarps), 32 * kRankedSeqWarps, 0, st>>>(
+                n_seqs, nc, pl->nrun, nh, Rs, use_z ? z.as<double>() : nullptr, x, qs.as<double>(), qi, smean.as<double>(),
+                svar.as<double>(), g.as<double>());
+            ranked_chain_sum_kernel<<<grid_for((long long)nb * kDiagLags, 256), 256, 0, st>>>((long long)nb * kDiagLags, nc, g.as<double>(),
+                                                                                           gsum.as<double>());
+            // (has_loglik = 1: ranked_quantiles_kernel's `bad` covers the log-likelihood field)
+            diag_finish_kernel<<<grid_for(nb, 128), 128, 0, st>>>(nb, pl->F, nc, nh, 1, smean.as<double>(), svar.as<double>(), gsum.as<double>(),
+                                                                  rh.as<double>() + (size_t)t * nb, es.as<double>() + (size_t)t * nb,
+                                                                  lag.as<int>() + (size_t)t * nb);
+            CU(ctx, cudaGetLastError());
+            return HMCGPU_OK;
+        };
+        const unsigned long long* sorted = nullptr;
+        TRY(scores(nullptr, &sorted));
+        ranked_quantiles_kernel<<<grid_for(nb, 128), 128, 0, st>>>(nb, s0, Rs, pl->F, (pl->flags & HMCGPU_FLAG_LOGLIK) ? 1 : 0, sorted, probs,
+                                                                   pl->d_quant.as<double>(), qs.as<double>(), bad.as<unsigned char>());
+        CU(ctx, cudaGetLastError());
+        TRY(split(true, 0, 0));                 // bulk
+        TRY(split(false, 0, 2));                // tail: 1[x <= q(0.05)]
+        TRY(split(false, 2, 3));                // tail: 1[x <= q(0.95)]
+        TRY(scores(qs.as<double>(), &sorted));  // folded about q(0.5)
+        TRY(split(true, 0, 1));
+        ranked_combine_kernel<<<grid_for(nb, 128), 128, 0, st>>>(nb, s0, bad.as<unsigned char>(), rh.as<double>(), es.as<double>(),
+                                                                 pl->d_rrank.as<double>(), pl->d_essb.as<double>(), pl->d_esst.as<double>());
+        CU(ctx, cudaGetLastError());
+    }
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, nc, pl->nrun, pl->n_grid, rk->n_probs, pl->flags), nullptr, nullptr, rk, nullptr));
+    CU(ctx, cudaStreamSynchronize(st));         // (the scratch goes back to the pool when this returns)
+    return HMCGPU_OK;
+}
+
+static int plan_fetch_ranked_impl(hmcgpu_plan* pl, hmcgpu_ranked* rk) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    if (!(pl->flags & HMCGPU_FLAG_RANKED)) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_ranked on a plan without HMCGPU_FLAG_RANKED");
+    if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_ranked before plan_run");
+    TRY(check_ranked(ctx, rk));
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_pool = ctx->pool;
+    return pl->precision == 32 ? fetch_ranked_t<float>(pl, rk) : fetch_ranked_t<double>(pl, rk);
+}
+
+extern "C" int hmcgpu_plan_fetch_ranked(hmcgpu_plan* pl, hmcgpu_ranked* rk) {
+    if (!pl) return HMCGPU_ERR_ARG;
+    if (!rk) return fail(pl->ctx, HMCGPU_ERR_ARG, "hmcgpu_ranked is NULL");
+    GUARD(pl->ctx, plan_fetch_ranked_impl(pl, rk));
 }
 
 extern "C" void hmcgpu_plan_destroy(hmcgpu_plan* pl) {
@@ -2268,9 +2425,17 @@ extern "C" int hmcgpu_estimate(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_
 }
 
 extern "C" int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr) {
+    return hmcgpu_estimate_ranked(ctx, p, r, pr, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk) {
     if (!r) return fail(ctx, HMCGPU_ERR_ARG, "result is NULL");
     if (p && (p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
         return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_predictive)");
+    if (p && (p->flags & HMCGPU_FLAG_RANKED)) {
+        if (!rk) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_RANKED without hmcgpu_ranked outputs (use hmcgpu_estimate_ranked)");
+        TRY(check_ranked(ctx, rk));             // (before the chains run)
+    }
     hmcgpu_plan* pl = nullptr;
     PhaseTrace tr;
     TRY(hmcgpu_plan_create(ctx, p, &pl));
@@ -2282,6 +2447,10 @@ extern "C" int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem*
         const int rp = hmcgpu_plan_fetch_predictive(pl, pr);
         if (rp < 0) rc = rp;
     }
+    if (rc >= 0 && (p->flags & HMCGPU_FLAG_RANKED)) {
+        const int rp = hmcgpu_plan_fetch_ranked(pl, rk);
+        if (rp < 0) rc = rp;
+    }
     tr.mark("plan_fetch (download)");
     hmcgpu_plan_destroy(pl);
     tr.mark("plan_destroy");
@@ -2289,20 +2458,32 @@ extern "C" int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem*
 }
 
 // Windows sharded over devices by longest-processing-time-first on T_w; one host thread per device, no collectives.
-static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr);
+static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
+                               hmcgpu_ranked* rk);
 extern "C" int hmcgpu_estimate_multi(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r) {
-    return hmcgpu_estimate_multi_predictive(devices, n_dev, p, r, nullptr);
+    return hmcgpu_estimate_multi_ranked(devices, n_dev, p, r, nullptr, nullptr);
 }
 
 extern "C" int hmcgpu_estimate_multi_predictive(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
                                                 hmcgpu_predictive* pr) {
+    return hmcgpu_estimate_multi_ranked(devices, n_dev, p, r, pr, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_multi_ranked(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
+                                            hmcgpu_predictive* pr, hmcgpu_ranked* rk) {
     if (!devices || n_dev < 1 || !p || !r) return fail(nullptr, HMCGPU_ERR_ARG, "bad arguments");
     if ((p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
         return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_multi_predictive)");
-    GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r, (p->flags & HMCGPU_FLAG_PREDICTIVE) ? pr : nullptr));
+    if (p->flags & HMCGPU_FLAG_RANKED) {
+        if (!rk) return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_RANKED without hmcgpu_ranked outputs (use hmcgpu_estimate_multi_ranked)");
+        TRY(check_ranked(nullptr, rk));
+    }
+    GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r, (p->flags & HMCGPU_FLAG_PREDICTIVE) ? pr : nullptr,
+                                       (p->flags & HMCGPU_FLAG_RANKED) ? rk : nullptr));
 }
 
-static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr) {
+static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
+                               hmcgpu_ranked* rk) {
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(nullptr, HMCGPU_ERR_ARG, "no windows");
     const int nw = p->n_windows;
     std::vector<int> ord(nw);
@@ -2318,8 +2499,8 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
     }
     std::vector<long long> T0(nw + 1, 0);                   // T_0 + ... + T_{w-1}: window w's offset in X0 and the ragged outputs
     for (int w = 0; w < nw; ++w) T0[w + 1] = T0[w] + Tw(w);
-    // (pr is given only with HMCGPU_FLAG_PREDICTIVE, the only case in which n_grid may be read)
-    const std::vector<WinOut> outs = window_outputs(p->K, p->n_h, p->n_chains, p->nrun, pr ? p->n_grid : 0, p->flags);
+    // (pr is given only with HMCGPU_FLAG_PREDICTIVE, the only case in which n_grid may be read; rk only with HMCGPU_FLAG_RANKED)
+    const std::vector<WinOut> outs = window_outputs(p->K, p->n_h, p->n_chains, p->nrun, pr ? p->n_grid : 0, rk ? rk->n_probs : 0, p->flags);
     std::vector<int> rcs(n_dev, 0);
     std::vector<std::string> errs(n_dev);
     std::vector<hmcgpu_result> parts(n_dev);
@@ -2352,18 +2533,20 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             // the shard's outputs in host staging arrays (of at least one byte: a requested output stays a non-NULL pointer)
             hmcgpu_result& o = parts[d];
             hmcgpu_predictive pq{};
+            hmcgpu_ranked rq{};
+            if (rk) { rq.probs = rk->probs; rq.n_probs = rk->n_probs; }
             std::vector<std::vector<char>> stage(outs.size());
             for (size_t i = 0; i < outs.size(); ++i) {
-                if (!outs[i].get(r, pr)) continue;
+                if (!outs[i].get(r, pr, rk)) continue;
                 stage[i].resize(std::max<size_t>(1, (size_t)outs[i].elems(n, sum_T) * outs[i].elem));
-                outs[i].set(&o, &pq, stage[i].data());
+                outs[i].set(&o, &pq, &rq, stage[i].data());
             }
-            rc = hmcgpu_estimate_predictive(ctx, &q, &o, pr ? &pq : nullptr);
+            rc = hmcgpu_estimate_ranked(ctx, &q, &o, pr ? &pq : nullptr, rk ? &rq : nullptr);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
             for (size_t i = 0; rc >= 0 && i < outs.size(); ++i) {   // scatter this shard's windows into the caller's arrays
                 const WinOut& x = outs[i];
-                char* dst = (char*)x.get(r, pr);
+                char* dst = (char*)x.get(r, pr, rk);
                 if (!dst) continue;
                 long long t = 0;                                 // steps of the shard's windows before window j
                 for (int j = 0; j < n; ++j) {

@@ -28,6 +28,7 @@ const FLAG_FILTERED_MEAN = UInt32(64)
 const FLAG_LOGLIK = UInt32(16)
 const FLAG_DIAGNOSTICS = UInt32(128)
 const FLAG_PREDICTIVE = UInt32(256)
+const FLAG_RANKED = UInt32(512)
 
 # struct hmcgpu_problem (include/hmcgpu.h)
 struct Problem
@@ -54,6 +55,12 @@ end
 # struct hmcgpu_predictive (FLAG_PREDICTIVE)
 mutable struct Predictive
     cdf::Ptr{Float64}; pit::Ptr{Float64}; log_score::Ptr{Float64}; moments::Ptr{Float64}
+end
+
+# struct hmcgpu_ranked (FLAG_RANKED)
+mutable struct Ranked
+    probs::Ptr{Float64}; n_probs::Int32
+    quantiles::Ptr{Float64}; rhat_rank::Ptr{Float64}; ess_bulk::Ptr{Float64}; ess_tail::Ptr{Float64}
 end
 
 struct HmcGpuError <: Exception
@@ -107,7 +114,8 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
                   win_series::Vector{Int32} = Int32[], win_init_series::Vector{Int32} = Int32[],
                   is_signal::Vector{UInt8} = UInt8[], kappa::Float64 = 1.0, pi_row_back::Int = 0,
                   xi::Vector{Float64} = Float64[], alpha::Vector{Float64} = Float64[], nu::Vector{Float64} = Float64[],
-                  pred_grid::Vector{Float64} = Float64[])
+                  pred_grid::Vector{Float64} = Float64[], quantile_probs::Vector{Float64} = Float64[],
+                  rank_diagnostics::Bool = false)
     # rawdata: one series (Vector) or y_len × n_series (Matrix, column = series): exactly the library's column-major layout
     y_len, n_series = size(rawdata, 1), size(rawdata, 2)
     ptr_or_null(v) = isempty(v) ? Ptr{eltype(v)}(C_NULL) : pointer(v)
@@ -121,20 +129,44 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
     pcdf = Array{Float64}(undef, ng, nh, nw); pit = Array{Float64}(undef, nh, nw); pls = similar(pit)
     pmom = Array{Float64}(undef, 3, nh, nw)
     pred = Predictive(pointer(pcdf), pointer(pit), pointer(pls), pointer(pmom))
+    # ranked outputs (quantile probabilities or rank_diagnostics): C [w][f][k] row-major = Julia n_probs × F × nw, [w][f] = F × nw
+    ranked = !isempty(quantile_probs) || rank_diagnostics
+    F, nq = 3D + D * D + 2nh + 1, length(quantile_probs)
+    rq = Array{Float64}(undef, nq, F, nw); rrh = Array{Float64}(undef, F, nw); reb = similar(rrh); ret = similar(rrh)
+    rk = Ranked(ptr_or_null(quantile_probs), nq, ptr_or_null(rq), pointer(rrh), pointer(reb), pointer(ret))
     res = Result(pointer(mu), pointer(sig), pointer(A), pointer(pie), nh > 0 ? pointer(fc) : C_NULL, C_NULL,
                  C_NULL, C_NULL, C_NULL, C_NULL, pointer(status), 0.0, 0.0, 0, 0, 0, 0, 0, 0.0, 0, 0,
                  C_NULL, C_NULL, C_NULL)
-    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu pred_grid pcdf pit pls pmom begin
+    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu pred_grid pcdf pit pls pmom quantile_probs rq rrh reb ret begin
         prob = Problem(pointer(rawdata), y_len, n_series, nw, ptr_or_null(win_series), pointer(win_start), pointer(win_end), C_NULL,
                        D, n_chains, burnin, Nrun, UInt64(seed), ptr_or_null(xi), ptr_or_null(alpha), ptr_or_null(nu), C_NULL, C_NULL,
                        kappa, ptr_or_null(is_signal), pointer(horizons), nh, C_NULL, precision,
-                       FLAG_REF_Q1 | FLAG_DRAWS | (ng > 0 ? FLAG_PREDICTIVE : UInt32(0)),
+                       FLAG_REF_Q1 | FLAG_DRAWS | (ng > 0 ? FLAG_PREDICTIVE : UInt32(0)) | (ranked ? FLAG_RANKED : UInt32(0)),
                        ptr_or_null(win_init_series), pi_row_back, 0, ptr_or_null(pred_grid), ng)
-        ccall((:hmcgpu_estimate_predictive, LIB), Cint, (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}), ctx.h, prob, res, pred)
+        ccall((:hmcgpu_estimate_ranked, LIB), Cint, (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}),
+              ctx.h, prob, res, pred, rk)
     end
     rc < 0 && throw(HmcGpuError(rc, lasterror(ctx)))
     return (μ = mu, σ = sig, A = A, πbend = pie, forecasts = fc, status = status, events = rc, gpu_ms = res.gpu_ms,
-            pred_cdf = pcdf, pit = pit, log_score = pls, pred_moments = pmom)
+            pred_cdf = pcdf, pit = pit, log_score = pls, pred_moments = pmom,
+            quantiles = rq, rhat_rank = rrh, ess_bulk = reb, ess_tail = ret)
+end
+
+# The multi-GPU form over caller-built structs (hmcgpu_estimate_multi_ranked): windows sharded over `devices`, every output
+# scattered back into the caller's window order.  Returns the event count; throws on an error.
+function estimate_multi_ranked(devices::Vector{Cint}, prob::Problem, res::Result, pred::Predictive, rk::Ranked)
+    rc = ccall((:hmcgpu_estimate_multi_ranked, LIB), Cint, (Ptr{Cint}, Cint, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}),
+               devices, length(devices), prob, res, pred, rk)
+    rc < 0 && throw(HmcGpuError(rc, unsafe_string(ccall((:hmcgpu_last_error, LIB), Cstring, (Ptr{Cvoid},), C_NULL))))
+    return rc
+end
+
+# The ranked outputs of the last run of a plan (hmcgpu_plan_fetch_ranked), computed from the retained draws; may be called again
+# with other rk.probs.  `ctx` is the plan's context (for the error message).
+function plan_fetch_ranked!(ctx::Context, plan::Ptr{Cvoid}, rk::Ranked)
+    rc = ccall((:hmcgpu_plan_fetch_ranked, LIB), Cint, (Ptr{Cvoid}, Ref{Ranked}), plan, rk)
+    rc < 0 && throw(HmcGpuError(rc, lasterror(ctx)))
+    return rk
 end
 
 # 0/1 flags over rawdata: 1 = the index belongs to opt.signalRange (hmcgpu_problem.is_signal)

@@ -60,6 +60,8 @@ extern "C" {
                                         computed on the device from every saved draw; needs nrun >= 4 (see hmcgpu_result) */
 #define HMCGPU_FLAG_PREDICTIVE  256u /* fill hmcgpu_predictive: posterior predictive CDF on pred_grid, PIT, log score and moments per
                                         window and horizon, computed on the device from every saved draw (see hmcgpu_predictive) */
+#define HMCGPU_FLAG_RANKED  512u     /* keep every saved draw on the device so that hmcgpu_plan_fetch_ranked can compute exact quantiles,
+                                        rank-normalised R̂ and bulk / tail ESS; needs nrun >= 4 and n_chains * nrun < 2^31 (see hmcgpu_ranked) */
 
 typedef struct hmcgpu_ctx hmcgpu_ctx;
 typedef struct hmcgpu_plan hmcgpu_plan;
@@ -197,6 +199,34 @@ typedef struct hmcgpu_predictive {
     double* moments;      /* [n_windows][n_h][3] */
 } hmcgpu_predictive;
 
+/* Ranked outputs (HMCGPU_FLAG_RANKED); caller-allocated, any output pointer may be NULL.  Per window w and summary field f (the
+ * fields and order of summary_mean), over the R = n_chains*nrun saved draws x_d converted to double (d = chain*nrun + i):
+ *   quantiles[(w*F + f)*n_probs + k]  type 7 (numpy method="linear"): with h = (R-1) p_k and the sorted draws x_(j) (0-based),
+ *                                     q(p) = x_(floor h) + (h - floor h) (x_(floor h + 1) - x_(floor h))
+ *   ranks r_d                         1-based over the R draws, ties averaged, -0.0 and +0.0 tied; normal scores
+ *                                     z_d = Phi^-1((r_d - 3/8) / (R + 1/4))
+ *   bulk R̂ / ESS                      the split-R̂ and ESS of rhat / ess above: same split, Geyer's initial monotone sequence, lags
+ *                                     capped at 63, applied to z
+ *   folded R̂                          the same applied to the normal scores of |x - q(0.5)| (fold taken in fp64)
+ *   rhat_rank[w*F + f]                max(bulk R̂, folded R̂)
+ *   ess_bulk[w*F + f]                 the bulk ESS
+ *   ess_tail[w*F + f]                 min(ESS of 1[x <= q(0.05)], ESS of 1[x <= q(0.95)])
+ * A field with a non-finite draw, and the loglik field without HMCGPU_FLAG_LOGLIK, get NaN in every output, quantiles included.
+ * R̂ and ESS are NaN where the split-R̂ definition gives NaN (W = 0: a constant field, a constant indicator); rhat_rank and
+ * ess_tail are NaN when either of their parts is.  A constant field's quantiles are the constant.  Every sum runs in a fixed
+ * order with no atomics: a window's outputs are bit-identical however the windows are batched, chunked or sharded.
+ * Device memory: n_windows * F * n_chains * nrun * (precision / 8) bytes of retained draws (C2: 500 windows x 43 fields x 256
+ * chains x 1000 draws in fp32 = 22 GB), checked against the device's total memory at hmcgpu_plan_create (HMCGPU_ERR_ALLOC when
+ * they do not fit), plus about 2 GiB of scratch at fetch. */
+typedef struct hmcgpu_ranked {
+    const double* probs;  /* [n_probs] quantile probabilities, finite, in [0, 1] (input) */
+    int32_t n_probs;      /* 0..64; 0 = no quantiles */
+    double* quantiles;    /* [n_windows][F][n_probs] */
+    double* rhat_rank;    /* [n_windows x F] rank-normalised split-R̂: max(bulk, folded) */
+    double* ess_bulk;     /* [n_windows x F] */
+    double* ess_tail;     /* [n_windows x F] */
+} hmcgpu_ranked;
+
 #define HMCGPU_KERNEL_THREAD 0  /* one thread per chain (gibbs_sweeps_kernel), wide batches, K <= 8 */
 #define HMCGPU_KERNEL_SCAN 1    /* one warp per chain, time-parallel scans (gibbs_scan_kernel), narrow batches */
 #define HMCGPU_KERNEL_LANE 2    /* one lane per state (gibbs_wide_kernel), K = 9..32 */
@@ -230,6 +260,11 @@ int hmcgpu_estimate_multi(const int* devices, int n_devices, const hmcgpu_proble
 int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr);
 int hmcgpu_estimate_multi_predictive(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
                                      hmcgpu_predictive* pr);
+/* The same filling the ranked outputs too (hmcgpu_estimate_predictive and hmcgpu_estimate_multi_predictive are these with
+ * rk = NULL).  With HMCGPU_FLAG_RANKED, rk must not be NULL (HMCGPU_ERR_ARG); without it rk is ignored. */
+int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk);
+int hmcgpu_estimate_multi_ranked(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
+                                 hmcgpu_predictive* pr, hmcgpu_ranked* rk);
 
 /* Split form: create uploads inputs and allocates device state; run executes every sweep (inputs resident
  * in HBM, no host transfers); fetch copies the requested outputs back.  run may be repeated (it restarts
@@ -239,6 +274,10 @@ int hmcgpu_plan_run(hmcgpu_plan* plan);
 int hmcgpu_plan_fetch(hmcgpu_plan* plan, hmcgpu_result* r);
 /* Posterior predictive outputs of the last run; HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_PREDICTIVE or before a run. */
 int hmcgpu_plan_fetch_predictive(hmcgpu_plan* plan, hmcgpu_predictive* pr);
+/* Ranked outputs of the last run, computed now from the retained draws; may be called again with other probs without running
+ * the plan again.  HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_RANKED, before a run, with n_probs outside 0..64 or a
+ * probability that is not finite or outside [0, 1]. */
+int hmcgpu_plan_fetch_ranked(hmcgpu_plan* plan, hmcgpu_ranked* rk);
 void hmcgpu_plan_destroy(hmcgpu_plan* plan);
 
 /* Forward filter for fixed parameters.  y: [T] shared by the batch (y_batch_stride = 0) or [B][T]
