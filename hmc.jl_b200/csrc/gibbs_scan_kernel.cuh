@@ -22,7 +22,7 @@
 // tier (SIG: signal mask, kappa-weighted statistics, pi_row_back — estimatesignals! runs 100 copies x ONE chain); no
 // smoothed-mean accumulators.
 #pragma once
-#include "gibbs_kernel.cuh"
+#include "lane_draws.cuh"
 
 namespace hmc {
 
@@ -87,44 +87,26 @@ struct ScanWarp {
 
     // Conjugate draws with the K*K + 2K gamma variates spread over the lanes (each has its own Philox purpose stream, so
     // they are independent): lane i < K draws the gamma of sigma2_i, lane K+i that of rho_i, lane 2K + i*K + j that of
-    // A[i][j].  Arithmetic, order of operations and streams are those of draw_params (hmm_device.cuh): same results.
+    // A[i][j].  The posterior of each state is state_posterior, the streams those of draw_params (hmm_device.cuh): same
+    // results.  (The segment kernel's draw_params_lanes with L = 32 draws the same bits, but here its variate selection
+    // costs ~20 more instructions per sweep on the critical path of a one-chain run: C1 0.2 % slower, B200 at 1000 W.)
     static __device__ __forceinline__ int draw_params_warp(const int lane, const int (&cnt)[K], const R (&Sd)[K], const R (&Qd)[K],
                                                           const int (&trans)[K][K], R c, const Hyper<R, K>& hp, const RngKey& key,
                                                           uint32_t sweep, R (&sig2)[K], R (&mu)[K], R (&rho)[K], R (&A)[K][K],
                                                           const SigStats<R, K>& sg) {
         int events = 0;
-        R ga[K], gb[K], neff[K], sumd[K], ntot[K];
+        StatePosterior<R> post[K];
         R shape = R(1);
         uint32_t purpose = (KIND_RHO << 16);
         bool mine = false;
 #pragma unroll
         for (int i = 0; i < K; ++i) {
-            const R n = (R)cnt[i];
-            const R dbar = cnt[i] > 0 ? Sd[i] / n : R(0);
-            R s2 = Qd[i] - n * dbar * dbar;
-            s2 = s2 > R(0) ? s2 : R(0);
-            R totalbar = cnt[i] > 0 ? dbar + c : R(0);
-            R ne = n, extra = R(0);
-            ga[i] = hp.alpha[i] + R(0.5) * n;
-            sumd[i] = Sd[i]; ntot[i] = n;
-            if constexpr (SIG) {                                   // signals: same formulas as draw_params<SIG> (:267-314)
-                const R m = (R)sg.m[i];
-                const R sbar = sg.m[i] > 0 ? sg.Sm[i] / m : R(0);
-                R sm2 = sg.Qm[i] - m * sbar * sbar;
-                sm2 = sm2 > R(0) ? sm2 : R(0);
-                sumd[i] = Sd[i] + sg.Sm[i]; ntot[i] = n + m;
-                totalbar = (cnt[i] + sg.m[i]) > 0 ? sumd[i] / ntot[i] + c : R(0);
-                ne = n + m * sg.k1;
-                ga[i] += R(0.5) * m;
-                extra = R(0.5) * sg.k1 * sm2;
-            }
-            const R dev = totalbar - hp.xi[i];
-            R b = hp.beta[i] + R(0.5) * s2;
-            if constexpr (SIG) b += extra;
-            b += R(0.5) * ne * hp.nu[i] / (ne + hp.nu[i]) * (dev * dev);
-            gb[i] = b;
-            neff[i] = ne;
-            if (lane == i) { shape = ga[i]; purpose = (KIND_SIGMA << 16) | (uint32_t)i; mine = ga[i] > R(0) && b > R(0); }
+            if constexpr (SIG)
+                post[i] = state_posterior<R, true>(cnt[i], Sd[i], Qd[i], c, hp.alpha[i], hp.beta[i], hp.nu[i], hp.xi[i],
+                                                   sg.m[i], sg.Sm[i], sg.Qm[i], sg.k1);
+            else
+                post[i] = state_posterior<R>(cnt[i], Sd[i], Qd[i], c, hp.alpha[i], hp.beta[i], hp.nu[i], hp.xi[i]);
+            if (lane == i) { shape = post[i].a; purpose = (KIND_SIGMA << 16) | (uint32_t)i; mine = post[i].a > R(0) && post[i].b > R(0); }
             if (lane == K + i) { shape = R(1); purpose = (KIND_RHO << 16) | (uint32_t)i; mine = true; }
 #pragma unroll
             for (int j = 0; j < K; ++j)
@@ -140,16 +122,10 @@ struct ScanWarp {
 #pragma unroll
         for (int i = 0; i < K; ++i) {
             const R gi = __shfl_sync(kFull, g, i);
-            if (ga[i] > R(0) && gb[i] > R(0)) sig2[i] = gb[i] / gi; else ++events;
+            if (post[i].a > R(0) && post[i].b > R(0)) sig2[i] = post[i].b / gi; else ++events;
         }
 #pragma unroll
-        for (int i = 0; i < K; ++i) {
-            const R n = neff[i];
-            const R sum_y = sumd[i] + ntot[i] * c;
-            const R m = (sum_y + hp.nu[i] * hp.xi[i]) / (n + hp.nu[i]);
-            const R sd = M<R>::sqrt(sig2[i] / (n + hp.nu[i]));
-            mu[i] = m + sd * __shfl_sync(kFull, z, i);
-        }
+        for (int i = 0; i < K; ++i) mu[i] = post[i].mean(c, hp.nu[i], hp.xi[i]) + post[i].sd(sig2[i], hp.nu[i]) * __shfl_sync(kFull, z, i);
         {
             R tot = R(0);
 #pragma unroll
@@ -223,30 +199,14 @@ struct ScanWarp {
         int cnt[K], trans[K][K];
         R Sd[K], Qd[K], sig2[K], mu[K], rho[K], A[K][K];
         Hyper<R, K> hp;
-#pragma unroll
-        for (int i = 0; i < K; ++i) {
-            cnt[i] = a.cnt[i * ns + slot];
-            Sd[i] = reinterpret_cast<const R*>(a.Sd)[i * ns + slot];
-            Qd[i] = reinterpret_cast<const R*>(a.Qd)[i * ns + slot];
-            hp.xi[i] = reinterpret_cast<const R*>(a.xi)[i * ns + slot];
-            hp.alpha[i] = (R)a.alpha[i];
-            hp.nu[i] = (R)a.nu[i];
-            sig2[i] = R(1);
-#pragma unroll
-            for (int j = 0; j < K; ++j) trans[i][j] = a.trans[(i * K + j) * ns + slot];
-        }
-        int events = 0;
         SigStats<R, K> sg;                                          // statistics of the signals (SIG; cnt/Sd/Qd: observations)
+        load_chain_stats<R, K, SIG>(a, ns, slot, cnt, Sd, Qd, trans, hp, &sg);
+#pragma unroll
+        for (int i = 0; i < K; ++i) sig2[i] = R(1);
+        int events = 0;
         const R* s0 = nullptr;                                      // emission z-scale of row t: s0[t*sld], sign = signal flag
         long long sld = 0;
         if constexpr (SIG) {
-#pragma unroll
-            for (int i = 0; i < K; ++i) {
-                sg.m[i] = a.cntM[i * ns + slot];
-                sg.Sm[i] = reinterpret_cast<const R*>(a.Sm)[i * ns + slot];
-                sg.Qm[i] = reinterpret_cast<const R*>(a.Qm)[i * ns + slot];
-            }
-            sg.k1 = (R)(1.0 / (1.0 + a.kappa));
             sld = a.sld;
             s0 = reinterpret_cast<const R*>(a.sigw) + a.sbase[slot];
         }
@@ -568,22 +528,7 @@ struct ScanWarp {
             __syncwarp();
         }
 
-        if (lane == 0) {
-#pragma unroll
-            for (int i = 0; i < K; ++i) {
-                a.cnt[i * ns + slot] = cnt[i];
-                reinterpret_cast<R*>(a.Sd)[i * ns + slot] = Sd[i];
-                reinterpret_cast<R*>(a.Qd)[i * ns + slot] = Qd[i];
-#pragma unroll
-                for (int j = 0; j < K; ++j) a.trans[(i * K + j) * ns + slot] = trans[i][j];
-                if constexpr (SIG) {
-                    a.cntM[i * ns + slot] = sg.m[i];
-                    reinterpret_cast<R*>(a.Sm)[i * ns + slot] = sg.Sm[i];
-                    reinterpret_cast<R*>(a.Qm)[i * ns + slot] = sg.Qm[i];
-                }
-            }
-            a.events[slot] += events;
-        }
+        if (lane == 0) store_chain_stats<R, K, SIG>(a, ns, slot, cnt, Sd, Qd, trans, events, &sg);
     }
 };
 

@@ -30,7 +30,7 @@
 // chain follows the oracle's chain (phase 2 only re-associates the products that carry the filtered vector to a segment
 // boundary).  K <= 4, plain sweep (no smoothed means, no signals), segment length <= 2^(32/K) - 1.
 #pragma once
-#include "gibbs_kernel.cuh"
+#include "lane_draws.cuh"
 
 namespace hmc {
 
@@ -430,7 +430,7 @@ struct SegWarp {
 
     // Conjugate draws with the K*K + 2K gamma variates spread over the L lanes of a chain (each variate has its own Philox
     // purpose stream, so they are independent): variate g is drawn by lane g % L in its round g / L and handed round by shuffles.
-    // Arithmetic, order of operations and streams are those of draw_params (hmm_device.cuh): same results, bit for bit.
+    // The posterior of each state is state_posterior, the streams those of draw_params (hmm_device.cuh): same results, bit for bit.
     static constexpr int kNG = K * K + 2 * K;
     static constexpr int kRounds = (kNG + L - 1) / L;
     static __device__ __forceinline__ int draw_params_lanes(const int q, const int base_lane, const int (&cnt)[K], const R (&Sd)[K],
@@ -438,25 +438,14 @@ struct SegWarp {
                                                             const RngKey& key, uint32_t sweep, R (&sig2)[K], R (&mu)[K], R (&rho)[K],
                                                             R (&A)[K][K]) {
         int events = 0;
-        R gb[K], neff[K], sumd[K], ntot[K];
+        StatePosterior<R> post[K];
         R shape[kNG];
         uint32_t purpose[kNG];
         bool valid[kNG];
 #pragma unroll
         for (int i = 0; i < K; ++i) {
-            const R n = (R)cnt[i];
-            const R dbar = cnt[i] > 0 ? Sd[i] / n : R(0);
-            R s2 = Qd[i] - n * dbar * dbar;
-            s2 = s2 > R(0) ? s2 : R(0);
-            const R totalbar = cnt[i] > 0 ? dbar + c : R(0);
-            const R a = hp.alpha[i] + R(0.5) * n;
-            sumd[i] = Sd[i]; ntot[i] = n;
-            const R dev = totalbar - hp.xi[i];
-            R b = hp.beta[i] + R(0.5) * s2;
-            b += R(0.5) * n * hp.nu[i] / (n + hp.nu[i]) * (dev * dev);
-            gb[i] = b;
-            neff[i] = n;
-            shape[i] = a; purpose[i] = (KIND_SIGMA << 16) | (uint32_t)i; valid[i] = a > R(0) && b > R(0);
+            post[i] = state_posterior<R>(cnt[i], Sd[i], Qd[i], c, hp.alpha[i], hp.beta[i], hp.nu[i], hp.xi[i]);
+            shape[i] = post[i].a; purpose[i] = (KIND_SIGMA << 16) | (uint32_t)i; valid[i] = post[i].a > R(0) && post[i].b > R(0);
             shape[K + i] = R(1); purpose[K + i] = (KIND_RHO << 16) | (uint32_t)i; valid[K + i] = true;
 #pragma unroll
             for (int j = 0; j < K; ++j) {
@@ -473,9 +462,8 @@ struct SegWarp {
             bool mine = false;
 #pragma unroll
             for (int l = 0; l < L; ++l) {
-                if (m * L + l < kNG) {
-                    if (q == l) { sh = shape[(m * L + l) < kNG ? (m * L + l) : 0]; pu = purpose[(m * L + l) < kNG ? (m * L + l) : 0]; mine = valid[(m * L + l) < kNG ? (m * L + l) : 0]; }
-                }
+                const int g = m * L + l;
+                if (g < kNG && q == l) { sh = shape[g]; pu = purpose[g]; mine = valid[g]; }
             }
             gl[m] = R(1);
             if (mine) gl[m] = gamma_mt<R>(sh, key, sweep, pu);
@@ -500,16 +488,10 @@ struct SegWarp {
 #pragma unroll
         for (int i = 0; i < K; ++i) {
             const R gi = G(i);
-            if (valid[i]) sig2[i] = gb[i] / gi; else ++events;     // :320 InverseGamma(a,b); reference: catch + keep old value (:321-329)
+            if (valid[i]) sig2[i] = post[i].b / gi; else ++events;     // :320 InverseGamma(a,b); reference: catch + keep old value (:321-329)
         }
 #pragma unroll
-        for (int i = 0; i < K; ++i) {
-            const R n = neff[i];
-            const R sum_y = sumd[i] + ntot[i] * c;
-            const R m = (sum_y + hp.nu[i] * hp.xi[i]) / (n + hp.nu[i]);   // :331
-            const R sd = M<R>::sqrt(sig2[i] / (n + hp.nu[i]));            // :332
-            mu[i] = m + sd * zs[i];                                       // :334
-        }
+        for (int i = 0; i < K; ++i) mu[i] = post[i].mean(c, hp.nu[i], hp.xi[i]) + post[i].sd(sig2[i], hp.nu[i]) * zs[i];   // :331-334
         {
             R tot = R(0);
 #pragma unroll
@@ -583,18 +565,9 @@ struct SegWarp {
         int cnt[K], trans[K][K];
         R Sd[K], Qd[K], sig2[K], mu[K], rho[K];
         Hyper<R, K> hp;
+        load_chain_stats<R, K>(a, ns, slot, cnt, Sd, Qd, trans, hp);
 #pragma unroll
-        for (int i = 0; i < K; ++i) {
-            cnt[i] = a.cnt[i * ns + slot];
-            Sd[i] = reinterpret_cast<const R*>(a.Sd)[i * ns + slot];
-            Qd[i] = reinterpret_cast<const R*>(a.Qd)[i * ns + slot];
-            hp.xi[i] = reinterpret_cast<const R*>(a.xi)[i * ns + slot];
-            hp.alpha[i] = (R)a.alpha[i];
-            hp.nu[i] = (R)a.nu[i];
-            sig2[i] = R(1);
-#pragma unroll
-            for (int j = 0; j < K; ++j) trans[i][j] = a.trans[(i * K + j) * ns + slot];
-        }
+        for (int i = 0; i < K; ++i) sig2[i] = R(1);
         int events = 0;                                              // this lane's share (summed over the chain's lanes at the end)
         const int warm_steps = a.seg_warm;                           // time steps of warm-up in front of a segment (seg_warmup)
 
@@ -797,17 +770,7 @@ struct SegWarp {
         }
 
         events = gsum(events);
-        if (q == 0) {
-#pragma unroll
-            for (int i = 0; i < K; ++i) {
-                a.cnt[i * ns + slot] = cnt[i];
-                reinterpret_cast<R*>(a.Sd)[i * ns + slot] = Sd[i];
-                reinterpret_cast<R*>(a.Qd)[i * ns + slot] = Qd[i];
-#pragma unroll
-                for (int j = 0; j < K; ++j) a.trans[(i * K + j) * ns + slot] = trans[i][j];
-            }
-            a.events[slot] += events;
-        }
+        if (q == 0) store_chain_stats<R, K>(a, ns, slot, cnt, Sd, Qd, trans, events);
     }
 };
 

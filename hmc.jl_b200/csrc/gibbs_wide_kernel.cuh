@@ -11,7 +11,7 @@
 // are interchangeable behind the plan.
 // Reference lines as in gibbs_kernel.cuh (src/Hmc.jl:231-369 draws, :371-440 forward, :459-484 backward, :501-513 relabel).
 #pragma once
-#include "gibbs_kernel.cuh"
+#include "lane_draws.cuh"
 
 namespace hmc {
 
@@ -100,21 +100,11 @@ __global__ void __launch_bounds__(kWideThreads, sizeof(R) == 8 ? 3 : (W == 32 ? 
         // ---- 1. conjugate draws: lane s draws sigma2_s, mu_s, its share of rho and row s of A
         R rho = R(0);
         if (act) {
-            const R beta = (R)(gs == 0 ? a.beta0[s] : a.beta[s]);
-            const R n = (R)cnt;
-            const R dbar = cnt > 0 ? Sd / n : R(0);
-            R s2 = Qd - n * dbar * dbar;
-            s2 = s2 > R(0) ? s2 : R(0);
-            const R totalbar = cnt > 0 ? dbar + c : R(0);
-            const R dev = totalbar - xi;
-            const R ga = alpha + R(0.5) * n;
-            const R gb = beta + R(0.5) * s2 + R(0.5) * n * nu / (n + nu) * (dev * dev);
-            if (ga > R(0) && gb > R(0)) sig2 = gb / gamma_mt<R>(ga, key, sweep, (KIND_SIGMA << 16) | (uint32_t)s);
+            const StatePosterior<R> p = state_posterior<R>(cnt, Sd, Qd, c, alpha, (R)(gs == 0 ? a.beta0[s] : a.beta[s]), nu, xi);
+            if (p.a > R(0) && p.b > R(0)) sig2 = p.b / gamma_mt<R>(p.a, key, sweep, (KIND_SIGMA << 16) | (uint32_t)s);
             else ++events;
-            const R m = (Sd + n * c + nu * xi) / (n + nu);
-            const R sd = M<R>::sqrt(sig2 / (n + nu));
             const uint4 w = rng_block(key, sweep, (KIND_MU << 16), (uint32_t)(s >> 1));
-            mu = m + sd * ((s & 1) ? normal_from<R>(w.z, w.w) : normal_from<R>(w.x, w.y));
+            mu = p.mean(c, nu, xi) + p.sd(sig2, nu) * ((s & 1) ? normal_from<R>(w.z, w.w) : normal_from<R>(w.x, w.y));
             rho = gamma_mt<R>(R(1), key, sweep, (KIND_RHO << 16) | (uint32_t)s);
             R rowsum = R(0);
             for (int j = 0; j < K; ++j) {
