@@ -23,10 +23,9 @@
 // smoothed-mean accumulators.
 #pragma once
 #include "lane_draws.cuh"
+#include "plan_policy.cuh"    // kScanThreads, scan_max_T
 
 namespace hmc {
-
-constexpr int kScanThreads = 128;     // 4 chains per block
 
 // per-warp shared memory: pif rows [T][K], uniforms [T], A by columns [K][4]
 template <typename R, int K> __host__ __device__ constexpr size_t scan_warp_bytes(int max_T) {
@@ -542,7 +541,5 @@ __global__ void __launch_bounds__(kScanThreads) gibbs_scan_kernel(const GibbsArg
 }
 
 template <typename R, int K> cudaError_t launch_gibbs_scan(const GibbsLaunch& cfg, const GibbsArgs& a, cudaStream_t st);
-// largest window the scan kernel can hold in shared memory (4 chains per block)
-template <typename R, int K> constexpr int scan_max_T() { return (int)((200 * 1024 / (kScanThreads / 32) - 64) / (sizeof(R) * (K + 1))); }
 
 }  // namespace hmc

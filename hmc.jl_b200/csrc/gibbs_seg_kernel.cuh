@@ -31,17 +31,10 @@
 // boundary).  K <= 4, plain sweep (no smoothed means, no signals), segment length <= 2^(32/K) - 1.
 #pragma once
 #include "lane_draws.cuh"
+#include "plan_policy.cuh"    // kSegThreads (threads per block), seg_max_T
 
 namespace hmc {
 
-// Threads per block.  The warps of a block step through the phases of a sweep together (two named barriers per sweep): a
-// scheduler then holds warps that run the SAME loop, which keeps that loop in the ~6 KB L0 instruction cache.  Without the
-// alignment the four warps of a scheduler sit in different loops (filter, sampler, draws, ...), every 128-byte line of every
-// loop misses L0 and the kernel spends 2.5 cycles per issued instruction waiting for instructions (ncu stall_no_instruction).
-#ifndef HMC_SEG_THREADS
-#define HMC_SEG_THREADS 256
-#endif
-constexpr int kSegThreads = HMC_SEG_THREADS;
 static_assert(kSegThreads % kGibbsThreads == 0, "whole selection tables");
 
 // (the selection table of GibbsWarp is laid out for kGibbsThreads threads: one table per kGibbsThreads threads of the block)
@@ -787,7 +780,5 @@ __global__ void __launch_bounds__(kSegThreads, (sizeof(R) == 8 ? 384 : 512) / kS
 
 // lanes per chain; a warp task holds 32 / lanes chains (plan.seg_lanes); threads per block (<= kSegThreads)
 template <typename R, int K> cudaError_t launch_gibbs_seg(const GibbsLaunch& cfg, const GibbsArgs& a, int lanes, int threads, cudaStream_t st);
-// longest window the segment kernel takes with this many lanes per chain (packed 32-bit transition counters per segment)
-template <int K> constexpr long long seg_max_T(int lanes) { return (long long)lanes * (((1ll << (32 / K)) - 1) / 4 * 4); }
 
 }  // namespace hmc

@@ -7,6 +7,7 @@
 #include "diagnostics.cuh"
 #include "predictive.cuh"
 #include "ranked.cuh"
+#include "plan_policy.cuh"
 
 #include <algorithm>
 #include <chrono>
@@ -210,37 +211,6 @@ extern "C" int hmcgpu_ctx_sync(hmcgpu_ctx* ctx) {
 
 static bool k_supported(int K) { return K >= 2 && K <= 32; }
 static bool k_thread(int K) { return K >= 2 && K <= 4; }       // every feature (smoothed means, signals, K-templated entry points)
-// The HMCGPU_* tuning variables (INTEGRATION.md), read once per plan at hmcgpu_plan_create.  An unset optional leaves the
-// choice to the plan; the bools are "value != 0".
-struct Tuning {
-    bool lane_kernel = false, seg_mixed = true, y_smem = true, launch_timing = true, verbose = false;
-    int seg_warm = 32, seg_barriers = 2;
-    std::optional<long long> scan_max_chains, seg_long;
-    std::optional<int> seg_lanes, groups, seg_threads, sweeps_per_launch;
-};
-static Tuning read_tuning() {
-    Tuning t;
-    const char* e;
-    if ((e = getenv("HMCGPU_LANE_KERNEL"))) t.lane_kernel = atoi(e) != 0;
-    if ((e = getenv("HMCGPU_SCAN_MAX_CHAINS"))) t.scan_max_chains = atoll(e);
-    if ((e = getenv("HMCGPU_SEG_LANES"))) t.seg_lanes = atoi(e);
-    if ((e = getenv("HMCGPU_SEG_MIXED"))) t.seg_mixed = atoi(e) != 0;
-    if ((e = getenv("HMCGPU_SEG_LONG"))) t.seg_long = atoll(e);
-    if ((e = getenv("HMCGPU_GROUPS"))) t.groups = std::max(1, std::min(8, atoi(e)));
-    if ((e = getenv("HMCGPU_Y_SMEM"))) t.y_smem = atoi(e) != 0;
-    if ((e = getenv("HMCGPU_SEG_WARMUP"))) t.seg_warm = std::max(0, atoi(e));
-    if ((e = getenv("HMCGPU_SEG_BARRIERS"))) t.seg_barriers = atoi(e);
-    if ((e = getenv("HMCGPU_SEG_THREADS"))) t.seg_threads = atoi(e);
-    if ((e = getenv("HMCGPU_SWEEPS_PER_LAUNCH"))) t.sweeps_per_launch = std::max(1, atoi(e));
-    if ((e = getenv("HMCGPU_LAUNCH_TIMING"))) t.launch_timing = atoi(e) != 0;
-    if ((e = getenv("HMCGPU_VERBOSE"))) t.verbose = atoi(e) != 0;
-    return t;
-}
-
-// sweeps: thread-per-chain kernels for K = 2..8, lane-per-state kernel for K = 9..32 (HMCGPU_LANE_KERNEL=1: also for 5..8)
-static bool k_thread_sweep(int K, const Tuning& t) { return (K >= 2 && K <= 4) || (K >= 5 && K <= 8 && !t.lane_kernel); }
-
-enum class SweepKernel : int32_t { thread = HMCGPU_KERNEL_THREAD, scan = HMCGPU_KERNEL_SCAN, lane = HMCGPU_KERNEL_LANE, seg = HMCGPU_KERNEL_SEG };
 
 #define DISPATCH_K(K, ...)                          \
     switch (K) {                                    \
@@ -1303,17 +1273,6 @@ __global__ void tile_reduce_kernel(int K, int ncols, int n_chains, const int* __
     }
 }
 
-// Which sweep kernel a plan runs, and how (choose_sweep)
-struct SweepChoice {
-    SweepKernel kernel = SweepKernel::thread;
-    int seg_lanes = 0;           // segment kernel: L lanes per chain (a warp task holds 32 / L chains)
-    // Mixed segment counts (mid-width batches with spare thread slots): the n_long longest windows run with 8 lanes per chain,
-    // in their own slot range with their own warp-task tables (task id = slot / 4)
-    int n_long = 0;
-    int sweeps_per_launch = 16;
-    int seg_threads = 128;       // threads per block of the segment kernel
-};
-
 struct hmcgpu_plan {
     hmcgpu_ctx* ctx = nullptr;
     // problem (host copies)
@@ -1340,9 +1299,8 @@ struct hmcgpu_plan {
     // plan_create_impl has drained the stream; released once the stream has drained at the end of plan_build.
     DevBuf yin;
     DevBuf warp_T_long, warp_pi_off_long;     // warp-task tables of the long class (SweepChoice::n_long)
-    struct Group { int task0, stride, n_tasks, lanes; bool long_class; };
-    std::vector<Group> groups;                // one stream each (plan_run)
-    int n_groups = 1, n_bufs = 1;
+    std::vector<TaskGroup> groups;            // one stream each (plan_run)
+    int n_bufs = 1;
     std::vector<cudaStream_t> gstreams;
     std::vector<cudaEvent_t> pool_events;
     std::vector<cudaEvent_t> timing_events;   // pairs around every sweep launch + one end-of-sweeps event per group (timing enabled)
@@ -1536,154 +1494,6 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuni
     return 0;
 }
 
-static int scan_max_T_of(int precision, int K) { DISPATCH_K(K, return precision == 32 ? scan_max_T<float, KK>() : scan_max_T<double, KK>()); return 0; }
-static long long seg_max_T_of(int K, int lanes) { DISPATCH_K(K, return seg_max_T<KK>(lanes)); return 0; }
-
-// The sweep-kernel policy (SweepChoice).  wT / order: the window lengths and the windows by decreasing length.  No device
-// work; ctx gives the SM count and takes the error text.
-static int choose_sweep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const std::vector<int>& wT, const std::vector<int>& order,
-                        const Tuning& t, SweepChoice& c) {
-    const int K = p->K, nw = p->n_windows, nc = p->n_chains, max_T = wT[order[0]];
-    const bool sig = p->is_signal != nullptr || p->pi_row_back != 0;
-    const bool acc_mean = p->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN);   // per-date means: thread-per-chain kernels only
-    const long long n_real = (long long)nw * nc;
-    const long long full = (long long)ctx->sm_count * 16 * 32;     // one wave of thread slots (16 warps per SM)
-    c = SweepChoice{};
-    if (!k_thread_sweep(K, t)) c.kernel = SweepKernel::lane;
-    if (K <= 4 && !acc_mean) {
-        // Narrow batches (the reference's own regime: one chain per end date) cannot fill the GPU with a thread per chain:
-        // below kScanMaxChains chains the time-parallel warp-per-chain kernel is used (K <= 4, plain sweep, window in smem).
-        // (the signals tier has no segment kernel: there the warp-per-chain kernel serves up to 12 288 chains; for the plain
-        //  sweep the segment kernel takes over from ~4000 chains — measured crossover on C2, DESIGN.md section 7)
-        const bool seg_ok = !sig && !(t.seg_lanes && *t.seg_lanes == 0);
-        long long lim = t.scan_max_chains.value_or(seg_ok ? 4096 : 12288);
-        // long windows leave room for fewer resident warps (the window lives in shared memory): scale the bound with them
-        const size_t wb = (size_t)(p->precision / 8) * ((size_t)max_T * (K + 1) + 4 * K);
-        const long long blocks = std::max<long long>(1, std::min<long long>(5, (long long)((227 * 1024) / (4 * wb + 1024))));
-        lim = lim * blocks / 5;
-        if (n_real <= lim && max_T <= scan_max_T_of(p->precision, K)) c.kernel = SweepKernel::scan;
-    }
-    // Mid-width batches (too many chains for a warp each, too few to fill the schedulers with a thread each): L lanes per
-    // chain, one time segment per lane (gibbs_seg_kernel.cuh).  L is chosen so that the batch yields about one full wave of
-    // warps; HMCGPU_SEG_LANES forces it (0 = never).  K <= 4, plain sweep.
-    if (K <= 4 && !acc_mean && !sig && c.kernel != SweepKernel::scan) {
-        int lanes = 0;
-        // measured on C2 (500 windows x c chains, B200): 4 lanes per chain are best up to ~38 000 chains, 2 lanes up to ~90 000,
-        // the thread-per-chain kernel beyond (DESIGN.md section 7); in units of one wave of thread slots:
-        if (n_real * 2 <= full) lanes = 4;
-        // (2 lanes only when the chains share one series: a batch of distinct series streams every observation from HBM in each
-        //  of the segment kernel's passes — C4, 65 536 series: 143 ms with 2 lanes, 139 ms with 4, 109 ms with a thread per chain)
-        else if (n_real * 4 <= 5 * full && p->n_series == 1) lanes = 2;
-        if (t.seg_lanes) lanes = *t.seg_lanes;
-        if (lanes != 0 && lanes != 2 && lanes != 4 && lanes != 8) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_SEG_LANES must be 0, 2, 4 or 8");
-        if (lanes && max_T > seg_max_T_of(K, lanes)) lanes = 0;
-        if (lanes) c.kernel = SweepKernel::seg;
-        c.seg_lanes = lanes;
-        // With 4 lanes per chain and thread slots to spare, the sweep time is the serial time of the LONGEST windows (every warp is
-        // resident from the start; a 16 000-chain batch leaves a fifth of the slots empty).  The longest tenth of the windows (in
-        // `order`) then gets 8 lanes per chain — half the dependent steps per sweep — as far as the slots last.  Measured on C2
-        // (HMCGPU_SEG_LONG sweep, scripts/r2_call_j.sh): 50 of 500 windows +7 % at 16 chains per window, +2 % at 24, +4 % at 32;
-        // 100 windows +7 % at 32 but -5 % at 24; 300 or all of them lose everywhere (8 lanes pay more per-sweep work per chain).
-        // HMCGPU_SEG_MIXED=0 disables it; a forced HMCGPU_SEG_LANES is uniform.
-        if (lanes == 4 && !t.seg_lanes && t.seg_mixed) {
-            const long long spare = full * 115 / 100 - n_real * 4;
-            long long n8 = spare > 0 ? std::min<long long>(nw / 10, spare / ((long long)nc * 4)) : 0;
-            while (n8 > 0 && wT[order[n8 - 1]] < 128) --n8;          // (segments of fewer than 16 steps are all warm-up)
-            if (t.seg_long) n8 = std::max(0ll, std::min<long long>(nw, *t.seg_long));
-            if (n8 * nc >= 32 && max_T <= seg_max_T_of(K, 8)) c.n_long = (int)n8;
-        }
-    }
-    if (c.kernel == SweepKernel::seg) {
-        // 256-thread blocks (8 warps stepping through the phases of a sweep together) when that still gives every SM a block
-        // and a half; otherwise 128.  Warp tasks: 4 chains each in the long class, 32 / L in the rest, each class padded to 32.
-        const long long n8c = (long long)c.n_long * nc, tasks = (n8c + 31) / 32 * 8 + (n_real - n8c + 31) / 32 * c.seg_lanes;
-        c.seg_threads = t.seg_threads.value_or(tasks / (kSegThreads / 32) >= ctx->sm_count * 3 / 2 ? kSegThreads : 128);
-    }
-    // Sweeps per launch.  Short launches bound the damage of the priority-based warp arbiter (a starved warp can only fall
-    // behind by one launch) and give the block scheduler a steady supply of pending blocks from the other groups.  A scan
-    // sweep is a few µs.
-    c.sweeps_per_launch = t.sweeps_per_launch.value_or(c.kernel == SweepKernel::scan ? 64 : 16);
-    return HMCGPU_OK;
-}
-
-// Host tables of the chain slots and warp tasks (uploaded by plan_build)
-struct SlotLayout {
-    std::vector<int> slot_win, slot_chain, Ts, win_slot0, warp_T, warp_T_long;
-    std::vector<long long> ybase, warp_off, warp_off_long, slot_off;   // slot_off: the lane kernel's pi row of each slot
-    std::vector<unsigned> chain_id;
-    long long pi_elems = 0;
-};
-
-// Lays out the plan's chain slots, warp tasks, pi offsets and task groups for its SweepChoice; sets n_slots, n_warps,
-// n_tasks and the groups.
-static SlotLayout layout_slots(hmcgpu_plan* pl, const hmcgpu_problem* p) {
-    const int K = p->K, nw = p->n_windows, nc = p->n_chains, nser = p->n_series;
-    const SweepChoice& c = pl->sw;
-    const bool seg = c.kernel == SweepKernel::seg;
-    const int ts = 32;
-    // slots: windows by decreasing T, chains consecutive; [long class (8 lanes), padded to 32][the rest, padded to 32]
-    const int long_slots = (int)(((long long)c.n_long * nc + ts - 1) / ts * ts);
-    const int n_slots = long_slots + (int)(((long long)nw * nc - (long long)c.n_long * nc + ts - 1) / ts * ts);
-    const int cpt = seg ? 32 / c.seg_lanes : ts;            // chains per warp task
-    const int n_warps = n_slots / cpt;                      // number of warp tasks (task id = slot / cpt; ids below long_slots / cpt are unused when there is a long class)
-    pl->n_slots = n_slots; pl->n_warps = n_warps;
-    SlotLayout s;
-    s.slot_win.assign(n_slots, -1); s.slot_chain.assign(n_slots, 0); s.Ts.assign(n_slots, 0); s.ybase.assign(n_slots, 0);
-    s.chain_id.assign(n_slots, 0); s.slot_off.assign(n_slots, 0); s.win_slot0.assign(nw, 0);
-    s.warp_T.assign(n_warps, 0); s.warp_off.assign(n_warps, 0);
-    for (int j = 0; j < nw; ++j) {
-        const int w = pl->order[j];
-        const int s0w = j < c.n_long ? j * nc : long_slots + (j - c.n_long) * nc;
-        s.win_slot0[w] = s0w;
-        const unsigned long long wid = p->win_id ? (unsigned long long)p->win_id[w] : (unsigned long long)w;
-        for (int cidx = 0; cidx < nc; ++cidx) {
-            const int slot = s0w + cidx;
-            s.slot_win[slot] = w; s.slot_chain[slot] = cidx; s.Ts[slot] = pl->wT[w];
-            s.ybase[slot] = (long long)(p->win_start[w] - 1) * nser + (p->win_series ? p->win_series[w] : 0);   // time-major [y_len][n_series] (the sweeps)
-            s.chain_id[slot] = (unsigned)(wid * (unsigned long long)nc + (unsigned long long)cidx);
-        }
-    }
-    // the long class first (8 lanes per chain: 4 chains per task, task id = slot / 4)
-    s.warp_T_long.assign(long_slots / 4, 0);
-    s.warp_off_long.assign(long_slots / 4, 0);
-    for (int wp = 0; wp < long_slots / 4; ++wp) {
-        int m = 0;
-        for (int l = 0; l < 4; ++l) m = std::max(m, s.Ts[wp * 4 + l]);
-        const int Cs = std::max(4, (m + 31) / 32 * 4);
-        s.warp_T_long[wp] = Cs;
-        s.warp_off_long[wp] = s.pi_elems;
-        s.pi_elems += (long long)Cs * K * 32;
-    }
-    for (int wp = long_slots / cpt; wp < n_warps; ++wp) {
-        int m = 0;
-        for (int l = 0; l < cpt; ++l) m = std::max(m, s.Ts[wp * cpt + l]);
-        s.warp_T[wp] = m;
-        s.warp_off[wp] = s.pi_elems;
-        if (seg) {
-            // segment kernel: every lane owns a frame of C = 4 ceil(T / 4L) rows (warp_T holds C), tiled like the thread kernel's
-            const int Cs = std::max(4, (m + 4 * c.seg_lanes - 1) / (4 * c.seg_lanes) * 4);
-            s.warp_T[wp] = Cs;
-            s.pi_elems += (long long)Cs * K * 32;
-        }
-        // thread-per-chain kernels: rows right-aligned to tiles of 4 time steps (gibbs_kernel.cuh, st_quad)
-        else if (c.kernel != SweepKernel::lane) s.pi_elems += (long long)((m + 3) / 4 * 4) * K * ts;
-        else for (int l = 0; l < ts; ++l) { s.slot_off[wp * ts + l] = s.pi_elems; s.pi_elems += (long long)s.Ts[wp * ts + l] * K; }
-    }
-    // task groups: interleaved subsets of the (longest-first) warp tasks of a class, each driven through its own stream
-    auto add_groups = [&](int task0, int tasks, int lanes, bool long_class) {
-        if (tasks <= 0) return;
-        int g = pl->tuning.groups.value_or((c.kernel == SweepKernel::lane || c.kernel == SweepKernel::scan) ? 1 : (tasks >= 1024 ? 4 : (tasks >= 256 ? 2 : 1)));
-        g = std::max(1, std::min(g, tasks));
-        for (int q = 0; q < g; ++q) pl->groups.push_back({task0 + q, g, (tasks - q + g - 1) / g, lanes, long_class});
-    };
-    const int t_long = long_slots / 4, t_first = long_slots / cpt, t_rest = n_warps - t_first;
-    add_groups(0, t_long, 8, true);
-    add_groups(t_first, t_rest, c.seg_lanes, false);
-    pl->n_groups = (int)pl->groups.size();
-    pl->n_tasks = t_long + t_rest;
-    return s;
-}
-
 template <typename R>
 static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     hmcgpu_ctx* ctx = pl->ctx;
@@ -1721,20 +1531,18 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     std::stable_sort(pl->order.begin(), pl->order.end(), [&](int a, int b) { return pl->wT[a] > pl->wT[b]; });
 
     pl->sig = p->is_signal != nullptr || p->pi_row_back != 0;
-    TRY(choose_sweep(ctx, p, pl->wT, pl->order, pl->tuning, pl->sw));
-    const SlotLayout lay = layout_slots(pl, p);
-    const int n_slots = pl->n_slots, n_warps = pl->n_warps;
+    const char* msg = nullptr;
+    if (const int rc = choose_sweep(ctx->sm_count, p, pl->wT, pl->order, pl->tuning, pl->sw, &msg)) return fail(ctx, rc, "%s", msg);
+    const SlotLayout lay = layout_slots(p, pl->wT, pl->order, pl->sw, pl->tuning);
+    const int n_slots = lay.n_slots, n_warps = lay.n_warps;
+    pl->n_slots = n_slots; pl->n_warps = n_warps; pl->n_tasks = lay.n_tasks; pl->groups = lay.groups;
     std::vector<int> hs(p->n_h);                            // horizons sorted ascending
     std::iota(hs.begin(), hs.end(), 0);
     std::stable_sort(hs.begin(), hs.end(), [&](int a, int b) { return p->horizons[a] < p->horizons[b]; });
-    // double-buffered draw chunks let the groups drift apart (not with the smoothing accumulators, which are shared)
+    const DrawChunks dc = draw_chunks((int)pl->groups.size(), p->flags, pl->F, n_slots, sizeof(R), p->nrun);
+    pl->chunk = dc.chunk; pl->n_bufs = dc.n_bufs;
     const unsigned kAccMean = HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN;
-    pl->n_bufs = (pl->n_groups > 1 && !(p->flags & kAccMean)) ? 2 : 1;
-    // chunk of draws per buffer: bound the chunk buffers to ~2 GiB in total
     const size_t per_draw = (size_t)pl->F * n_slots * sizeof(R);
-    long long chunk = std::max<long long>(1, (long long)((2ull << 30) / pl->n_bufs / per_draw));
-    chunk = std::min<long long>(chunk, std::min<long long>(p->nrun, 1024));
-    pl->chunk = (int)chunk;
 
     // ---- device allocation + upload
     auto up = [&](DevBuf& b, const void* host, size_t bytes) -> cudaError_t {
@@ -1808,7 +1616,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     CU(ctx, pl->xi.alloc((size_t)K * n_slots * sizeof(R)));
     CU(ctx, pl->totS.alloc((size_t)n_slots * sizeof(R)));
     CU(ctx, pl->totQ.alloc((size_t)n_slots * sizeof(R)));
-    CU(ctx, pl->out.alloc(per_draw * (size_t)chunk * pl->n_bufs));
+    CU(ctx, pl->out.alloc(per_draw * (size_t)pl->chunk * pl->n_bufs));
     CU(ctx, pl->yfut.alloc((size_t)std::max(1, p->n_h) * n_slots * sizeof(R)));
     if (p->flags & HMCGPU_FLAG_SUMMARY) {
         CU(ctx, pl->d_sum.alloc((size_t)nw * pl->F * sizeof(double)));
@@ -1896,7 +1704,7 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     a.seg_warm = pl->tuning.seg_warm; a.seg_barriers = pl->tuning.seg_barriers;
     if (pl->sw.kernel == SweepKernel::seg) CU(ctx, pl->d_diag.alloc(2 * sizeof(unsigned long long)));
     a.diag = pl->d_diag.as<unsigned long long>();
-    for (int g = 0; g < pl->n_groups; ++g) {
+    for (size_t g = 0; g < pl->groups.size(); ++g) {
         cudaStream_t s2;
         CU(ctx, cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
         pl->gstreams.push_back(s2);
@@ -1914,8 +1722,7 @@ template <typename R, int K>
 static int plan_run_t(hmcgpu_plan* pl) {
     hmcgpu_ctx* ctx = pl->ctx;
     cudaStream_t st = ctx->stream;
-    const int ns = pl->n_slots, G = pl->n_groups;
-    const int L = pl->sw.sweeps_per_launch;
+    const int ns = pl->n_slots, G = (int)pl->groups.size();
     const int Kr = pl->K;                                    // runtime K (the template K is 0 for the lane-per-state kernel)
     pl->n_launches = 0; pl->n_sweep_launches = 0; pl->sweep_ms = 0.0;
     size_t ev_used = 0;
@@ -1967,10 +1774,8 @@ static int plan_run_t(hmcgpu_plan* pl) {
     const long long S = pl->burnin + pl->nrun;
     const long long n_chunks = (pl->nrun + pl->chunk - 1) / pl->chunk;
     const size_t buf_elems = (size_t)pl->F * pl->chunk * ns;
-    std::vector<long long> next(G, 0);                       // next sweep of each group
     std::vector<cudaEvent_t> post_done(n_chunks, nullptr);   // post-processing of chunk k finished
     std::vector<std::vector<cudaEvent_t>> chunk_done(n_chunks, std::vector<cudaEvent_t>(G, nullptr));
-    long long posted = 0;                                    // chunks whose post-processing has been enqueued
     auto enqueue_post = [&](long long k) -> int {
         for (int g = 0; g < G; ++g) CU(ctx, cudaStreamWaitEvent(st, chunk_done[k][g], 0));
         const long long d0 = k * pl->chunk;
@@ -2047,82 +1852,43 @@ static int plan_run_t(hmcgpu_plan* pl) {
         CU(ctx, cudaEventRecord(post_done[k], st));
         return 0;
     };
-    GibbsArgs a = pl->args;
-    // one launch of group g (0 = enqueued, 1 = nothing to do yet: its next chunk buffer is not released, < 0 = error)
-    auto enqueue_one = [&](const int g, const long long round) -> int {
-            const long long s0 = next[g];
-            if (s0 >= S) return 1;
-            if (s0 >= pl->burnin && (s0 - pl->burnin) % pl->chunk == 0) {
-                const long long k0 = (s0 - pl->burnin) / pl->chunk;
-                if (k0 >= pl->n_bufs && post_done[k0 - pl->n_bufs] == nullptr) return 1;   // buffer not released yet: next round
-            }
-            // stagger: the first launch of group g is (g+1)/G of a normal one, so the groups' launch boundaries interleave
-            long long n = (round == 0 && G > 1) ? std::max<long long>(1, (long long)L * (g + 1) / G) : L;
-            long long limit = S;
-            if (s0 < pl->burnin) limit = pl->burnin;
-            else limit = pl->burnin + std::min<long long>(pl->nrun, ((s0 - pl->burnin) / pl->chunk + 1) * pl->chunk);
-            n = std::min(n, limit - s0);
-            cudaStream_t gs = pl->gstreams[g];
-            long long k = -1;
-            if (s0 >= pl->burnin) {
-                k = (s0 - pl->burnin) / pl->chunk;
-                // the chunk's buffer must have been consumed by the post-processing of chunk k - n_bufs
-                if ((s0 - pl->burnin) % pl->chunk == 0 && k >= pl->n_bufs) CU(ctx, cudaStreamWaitEvent(gs, post_done[k - pl->n_bufs], 0));
-                a.draw0 = k * pl->chunk;
-                a.out = pl->out.as<R>() + (size_t)(k % pl->n_bufs) * buf_elems;
-            } else {
-                a.draw0 = 0;
-                a.out = pl->out.p;
-            }
-            a.sweep0 = s0; a.n_sweeps = (int)n;
-            const hmcgpu_plan::Group& grp = pl->groups[g];
-            a.task0 = grp.task0; a.task_stride = grp.stride; a.n_tasks = grp.n_tasks;
-            a.warp_T = grp.long_class ? pl->warp_T_long.as<int>() : pl->warp_T.as<int>();
-            a.warp_pi_off = grp.long_class ? pl->warp_pi_off_long.as<long long>() : pl->warp_pi_off.as<long long>();
-            cudaEvent_t lt0 = nullptr, lt1 = nullptr;
-            if (pl->tuning.launch_timing) { CU(ctx, timing_event(&lt0)); CU(ctx, timing_event(&lt1)); CU(ctx, cudaEventRecord(lt0, gs)); }
-            if constexpr (K == 0) {
-                CU(ctx, (launch_gibbs_wide<R>(cfg, a, pl->K, pl->slot_pi_off.as<long long>(), gs)));
-            } else if constexpr (K <= 4) {
-                switch (pl->sw.kernel) {
-                    case SweepKernel::scan: CU(ctx, (launch_gibbs_scan<R, K>(cfg, a, gs))); break;
-                    case SweepKernel::seg: CU(ctx, (launch_gibbs_seg<R, K>(cfg, a, grp.lanes, pl->sw.seg_threads, gs))); break;
-                    default: CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
-                }
-            } else {
-                CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
-            }
-            if (pl->tuning.launch_timing) { CU(ctx, cudaEventRecord(lt1, gs)); launch_pairs.emplace_back(lt0, lt1); }
-            ++pl->n_launches; ++pl->n_sweep_launches;
-            next[g] = s0 + n;
-            if (next[g] >= S) CU(ctx, cudaEventRecord(gend[g], gs));
-            if (k >= 0 && next[g] == pl->burnin + std::min<long long>(pl->nrun, (k + 1) * pl->chunk)) {
-                CU(ctx, new_event(&chunk_done[k][g]));
-                CU(ctx, cudaEventRecord(chunk_done[k][g], gs));
-            }
-            // post-process every chunk all groups have finished enqueuing
-            while (posted < n_chunks) {
-                bool ready = true;
-                for (int g2 = 0; g2 < G; ++g2) ready = ready && chunk_done[posted][g2] != nullptr;
-                if (!ready) break;
-                TRY(enqueue_post(posted));
-                ++posted;
-            }
-            return 0;
-    };
     PhaseTrace trr;
-    // launches are enqueued round-robin over the groups; a launch never crosses the end of burn-in or of a draw chunk
-    bool more = true;
-    for (long long round = 0; more; ++round) {
-        more = false;
-        std::vector<int> gorder(G);
-        std::iota(gorder.begin(), gorder.end(), 0);
-        std::stable_sort(gorder.begin(), gorder.end(), [&](int x, int y2) { return next[x] < next[y2]; });   // laggards first
-        for (int g : gorder) {
-            if (next[g] >= S) continue;
-            more = true;
-            const int rc = enqueue_one(g, round);
-            if (rc < 0) return rc;
+    GibbsArgs a = pl->args;
+    // the sweep launches and the per-chunk post-processing, in the order launch_schedule gives
+    for (const RunOp& op : launch_schedule(pl->burnin, pl->nrun, pl->chunk, pl->n_bufs, G, pl->sw.sweeps_per_launch)) {
+        if (op.post) {
+            TRY(enqueue_post(op.chunk));
+            continue;
+        }
+        const int g = op.group;
+        cudaStream_t gs = pl->gstreams[g];
+        if (op.wait >= 0) CU(ctx, cudaStreamWaitEvent(gs, post_done[op.wait], 0));   // the chunk's buffer has been consumed
+        a.draw0 = op.chunk >= 0 ? op.chunk * pl->chunk : 0;
+        a.out = op.chunk >= 0 ? pl->out.as<R>() + (size_t)(op.chunk % pl->n_bufs) * buf_elems : pl->out.as<R>();
+        a.sweep0 = op.sweep0; a.n_sweeps = (int)op.n_sweeps;
+        const TaskGroup& grp = pl->groups[g];
+        a.task0 = grp.task0; a.task_stride = grp.stride; a.n_tasks = grp.n_tasks;
+        a.warp_T = grp.long_class ? pl->warp_T_long.as<int>() : pl->warp_T.as<int>();
+        a.warp_pi_off = grp.long_class ? pl->warp_pi_off_long.as<long long>() : pl->warp_pi_off.as<long long>();
+        cudaEvent_t lt0 = nullptr, lt1 = nullptr;
+        if (pl->tuning.launch_timing) { CU(ctx, timing_event(&lt0)); CU(ctx, timing_event(&lt1)); CU(ctx, cudaEventRecord(lt0, gs)); }
+        if constexpr (K == 0) {
+            CU(ctx, (launch_gibbs_wide<R>(cfg, a, pl->K, pl->slot_pi_off.as<long long>(), gs)));
+        } else if constexpr (K <= 4) {
+            switch (pl->sw.kernel) {
+                case SweepKernel::scan: CU(ctx, (launch_gibbs_scan<R, K>(cfg, a, gs))); break;
+                case SweepKernel::seg: CU(ctx, (launch_gibbs_seg<R, K>(cfg, a, grp.lanes, pl->sw.seg_threads, gs))); break;
+                default: CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
+            }
+        } else {
+            CU(ctx, (launch_gibbs<R, K>(cfg, a, gs)));
+        }
+        if (pl->tuning.launch_timing) { CU(ctx, cudaEventRecord(lt1, gs)); launch_pairs.emplace_back(lt0, lt1); }
+        ++pl->n_launches; ++pl->n_sweep_launches;
+        if (op.last) CU(ctx, cudaEventRecord(gend[g], gs));
+        if (op.closes_chunk) {
+            CU(ctx, new_event(&chunk_done[op.chunk][g]));
+            CU(ctx, cudaEventRecord(chunk_done[op.chunk][g], gs));
         }
     }
     CU(ctx, cudaEventRecord(pl->ev1, st));                   // st has waited for every group through the last chunk's post
