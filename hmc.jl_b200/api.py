@@ -230,7 +230,7 @@ def shard_windows(T: Sequence[int], n_shards: int):
 def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                      precision=32, draws=False, summary=True, smoothed=False, loglik=False, win_id=None,
                      win_series=None, diagnostics=False, predictive_grid=None, quantiles=None, rank_diagnostics=False,
-                     ctx: Optional[B.Context] = None, device: int = 0):
+                     onestep=False, ctx: Optional[B.Context] = None, device: int = 0):
     """Many end-date windows in one call (what the SLURM job array does one process at a time).  `diagnostics=True` adds
     `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics).
     `predictive_grid` (increasing points, shared by every window and horizon) adds the posterior predictive distribution of
@@ -238,12 +238,14 @@ def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nru
     [n_windows, n_h, 3] (mean, variance, skewness); see write_predictive and include/hmcgpu.h.  `quantiles` (probabilities
     in [0, 1]) and / or `rank_diagnostics=True` keep every saved draw on the device (HMCGPU_FLAG_RANKED) and add the exact
     posterior `quantiles` [n_windows, F, n_probs], the rank-normalised split-R̂ `rhat_rank` and the bulk / tail effective
-    sample sizes `ess_bulk` / `ess_tail` [n_windows, F]; see write_ranked."""
+    sample sizes `ess_bulk` / `ess_tail` [n_windows, F]; see write_ranked.  `onestep=True` (HMCGPU_FLAG_ONESTEP, K <= 8) scores
+    every in-sample date by its one-step-ahead posterior predictive: `onestep_pit`, `lpd` and `lpd_var` (lists of [N_w] arrays)
+    and `waic` [n_windows, 4] (lppd, p_waic, elpd_waic, se); see pseudo_residuals, compare_waic and write_onestep."""
     ranked = quantiles is not None or rank_diagnostics
     flags = B.FLAG_REF_Q1 | (B.FLAG_DRAWS if draws else 0) | (B.FLAG_SUMMARY if summary else 0) \
         | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0) \
         | (B.FLAG_DIAGNOSTICS if diagnostics else 0) | (B.FLAG_PREDICTIVE if predictive_grid is not None else 0) \
-        | (B.FLAG_RANKED if ranked else 0)
+        | (B.FLAG_RANKED if ranked else 0) | (B.FLAG_ONESTEP if onestep else 0)
     spec = B.ProblemSpec(y, win_start, win_end, K=K, n_chains=n_chains, burnin=burnin, nrun=nrun, seed=seed,
                          horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series,
                          pred_grid=predictive_grid, quantile_probs=quantiles)
@@ -430,6 +432,51 @@ def write_predictive(out, horizons: Sequence[int], grid: Sequence[float], dates:
             for d, row in zip(dates, data):
                 f.write(",".join([str(d)] + [repr(float(v)) for v in row]) + "\n")
         paths[key] = path
+    return paths
+
+
+def pseudo_residuals(pit):
+    """Normal pseudo-residuals Phi^-1(pit) of one-step-ahead PIT values (Zucchini & MacDonald, HMMs for Time Series, ch. 6): for a
+    well-specified model they are close to iid N(0, 1).  Accepts an array or a list of per-window arrays (out.onestep_pit)."""
+    from scipy.special import ndtri
+    if isinstance(pit, list):
+        return [ndtri(np.asarray(p, dtype=np.float64)) for p in pit]
+    return ndtri(np.asarray(pit, dtype=np.float64))
+
+
+def compare_waic(a, b):
+    """Per-window WAIC comparison of two fits of the same windows (e.g. K = 3 against K = 2), from estimate_windows(onestep=True)
+    outputs.  With e_t = lpd_t - lpd_var_t the pointwise elpd of each date, returns `elpd_diff` [n_windows] = elpd_waic(a) -
+    elpd_waic(b) and `se_diff` [n_windows] = sqrt(N var_t(e_a,t - e_b,t)) (variance over the dates with denominator N - 1, as the
+    loo package does).  A positive difference of several se_diff favours `a`."""
+    if len(a.lpd) != len(b.lpd) or any(len(x) != len(y) for x, y in zip(a.lpd, b.lpd)):
+        raise ValueError("compare_waic needs the same windows (and window lengths) in both fits")
+    diff, se = np.empty(len(a.lpd)), np.empty(len(a.lpd))
+    for w in range(len(a.lpd)):
+        d = (np.asarray(a.lpd[w]) - np.asarray(a.lpd_var[w])) - (np.asarray(b.lpd[w]) - np.asarray(b.lpd_var[w]))
+        diff[w] = np.asarray(a.waic)[w, 2] - np.asarray(b.waic)[w, 2]
+        se[w] = np.sqrt(len(d) * np.var(d, ddof=1))
+    return SimpleNamespace(elpd_diff=diff, se_diff=se)
+
+
+def write_onestep(out, dates: Sequence, directory: str):
+    """The one-step-ahead scores of estimate_windows(onestep=True), windows in caller order: `onestep_scores.csv` with one row per
+    (window, in-sample date): the window's end date, the date's 1-based position in the window, pit, its normal pseudo-residual,
+    lpd and lpd_var; and `waic.csv` with one row per window: end date, lppd, p_waic, elpd_waic, se.  Returns {"scores": path,
+    "waic": path}."""
+    import os
+    os.makedirs(directory, exist_ok=True)
+    paths = {"scores": os.path.join(directory, "onestep_scores.csv"), "waic": os.path.join(directory, "waic.csv")}
+    res = pseudo_residuals(out.onestep_pit)
+    with open(paths["scores"], "w") as f:
+        f.write("date,t,pit,pseudo_residual,lpd,lpd_var\n")
+        for d, pit, z, lpd, var in zip(dates, out.onestep_pit, res, out.lpd, out.lpd_var):
+            for t in range(len(pit)):
+                f.write(",".join([str(d), str(t + 1)] + [repr(float(v[t])) for v in (pit, z, lpd, var)]) + "\n")
+    with open(paths["waic"], "w") as f:
+        f.write("date,lppd,p_waic,elpd_waic,se\n")
+        for d, row in zip(dates, np.asarray(out.waic)):
+            f.write(",".join([str(d)] + [repr(float(v)) for v in row]) + "\n")
     return paths
 
 

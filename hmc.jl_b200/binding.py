@@ -21,6 +21,7 @@ FLAG_FILTERED_MEAN = 64   # pib_mean / insample_forecast_mean carry the FILTERED
 FLAG_DIAGNOSTICS = 128    # rhat / ess / ess_lag per window and summary field (split-R̂ and ESS, include/hmcgpu.h)
 FLAG_PREDICTIVE = 256     # posterior predictive CDF on a grid, PIT, log score and moments per window and horizon (hmcgpu_predictive)
 FLAG_RANKED = 512         # keep every saved draw on the device: exact quantiles, rank-normalised R̂, bulk / tail ESS (hmcgpu_ranked)
+FLAG_ONESTEP = 1024       # one-step-ahead PIT and log predictive density of every in-sample date, WAIC per window (hmcgpu_onestep)
 
 ERR_ARG, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED, ERR_NODEVICE = -1, -2, -3, -4, -5
 
@@ -32,6 +33,7 @@ SYMBOLS = [
     "hmcgpu_draw_params", "hmcgpu_draw_params_signals", "hmcgpu_forecast", "hmcgpu_philox", "hmcgpu_philox_rounds",
     "hmcgpu_build_info", "hmcgpu_ctx_trim", "hmcgpu_estimate_predictive", "hmcgpu_estimate_multi_predictive",
     "hmcgpu_plan_fetch_predictive", "hmcgpu_estimate_ranked", "hmcgpu_estimate_multi_ranked", "hmcgpu_plan_fetch_ranked",
+    "hmcgpu_estimate_onestep", "hmcgpu_estimate_multi_onestep", "hmcgpu_plan_fetch_onestep",
 ]
 KERNEL_NAMES = {0: "gibbs_sweeps_kernel (thread per chain)", 1: "gibbs_scan_kernel (warp per chain, time-parallel)",
                 2: "gibbs_wide_kernel (lane per state)", 3: "(reserved)",
@@ -70,6 +72,10 @@ class Predictive(C.Structure):
 
 class Ranked(C.Structure):
     _fields_ = [("probs", _dp), ("n_probs", C.c_int32), ("quantiles", _dp), ("rhat_rank", _dp), ("ess_bulk", _dp), ("ess_tail", _dp)]
+
+
+class Onestep(C.Structure):
+    _fields_ = [("pit", _dp), ("lpd", _dp), ("lpd_var", _dp), ("waic", _dp)]
 
 
 class HmcGpuError(RuntimeError):
@@ -121,6 +127,11 @@ def load(build_if_missing: bool = True):
     L.hmcgpu_estimate_multi_ranked.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
                                                C.POINTER(Predictive), C.POINTER(Ranked)]
     L.hmcgpu_plan_fetch_ranked.argtypes = [C.c_void_p, C.POINTER(Ranked)]
+    L.hmcgpu_estimate_onestep.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Result), C.POINTER(Predictive), C.POINTER(Ranked),
+                                          C.POINTER(Onestep)]
+    L.hmcgpu_estimate_multi_onestep.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
+                                                C.POINTER(Predictive), C.POINTER(Ranked), C.POINTER(Onestep)]
+    L.hmcgpu_plan_fetch_onestep.argtypes = [C.c_void_p, C.POINTER(Onestep)]
     L.hmcgpu_plan_destroy.argtypes = [C.c_void_p]
     L.hmcgpu_plan_destroy.restype = None
     L.hmcgpu_filter.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _dp, C.c_int64,
@@ -367,6 +378,17 @@ class ProblemSpec:
         o.rhat_rank = np.empty((nw, F)); o.ess_bulk = np.empty((nw, F)); o.ess_tail = np.empty((nw, F))
         return Ranked(_p(probs), len(probs), _p(o.quantiles), _p(o.rhat_rank), _p(o.ess_bulk), _p(o.ess_tail))
 
+    def alloc_onestep(self, o):
+        """Adds the one-step-ahead scores to `o` (onestep_pit, lpd, lpd_var: per date, windows concatenated, split per window by
+        finish; waic [nw, 4]: lppd, p_waic, elpd_waic, se) and returns the hmcgpu_onestep struct over them; None without
+        FLAG_ONESTEP.  (`onestep_pit`: `pit` is the forecast PIT of FLAG_PREDICTIVE.)"""
+        if not self.flags & FLAG_ONESTEP:
+            return None
+        n = int(self.T.sum())
+        o.onestep_pit = np.empty(n); o.lpd = np.empty(n); o.lpd_var = np.empty(n)
+        o.waic = np.empty((self.n_windows, 4))
+        return Onestep(_p(o.onestep_pit), _p(o.lpd), _p(o.lpd_var), _p(o.waic))
+
     def finish(self, o, res, rc):
         o.events = rc
         o.gpu_ms, o.sweep_kernel_ms = res.gpu_ms, res.sweep_kernel_ms
@@ -385,6 +407,9 @@ class ProblemSpec:
                 parts.append(o.insample_forecast_mean[off:off + n * nh].reshape(nh, n).T)
                 off += n * nh
             o.insample_forecast_mean = parts
+        if getattr(o, "lpd", None) is not None and not isinstance(o.lpd, list):   # per-window [N_w]
+            cut = np.cumsum(self.T)[:-1]
+            o.onestep_pit, o.lpd, o.lpd_var = (np.split(a, cut) for a in (o.onestep_pit, o.lpd, o.lpd_var))
         return o
 
 
@@ -393,8 +418,11 @@ def estimate(ctx: Context, spec: ProblemSpec):
     o, res = spec.alloc_result()
     pr = spec.alloc_predictive(o)
     rk = spec.alloc_ranked(o)
+    os_ = spec.alloc_onestep(o)
     prob = spec.struct()
-    if rk is not None:
+    if os_ is not None:
+        rc = ctx._check(ctx.L.hmcgpu_estimate_onestep(ctx.h, C.byref(prob), C.byref(res), _ref(pr), _ref(rk), C.byref(os_)))
+    elif rk is not None:
         rc = ctx._check(ctx.L.hmcgpu_estimate_ranked(ctx.h, C.byref(prob), C.byref(res), _ref(pr), C.byref(rk)))
     elif pr is None:
         rc = ctx._check(ctx.L.hmcgpu_estimate(ctx.h, C.byref(prob), C.byref(res)))
@@ -408,9 +436,12 @@ def estimate_multi(devices, spec: ProblemSpec):
     o, res = spec.alloc_result()
     pr = spec.alloc_predictive(o)
     rk = spec.alloc_ranked(o)
+    os_ = spec.alloc_onestep(o)
     prob = spec.struct()
     dev = (C.c_int * len(devices))(*devices)
-    if rk is not None:
+    if os_ is not None:
+        rc = L.hmcgpu_estimate_multi_onestep(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), _ref(rk), C.byref(os_))
+    elif rk is not None:
         rc = L.hmcgpu_estimate_multi_ranked(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), C.byref(rk))
     elif pr is None:
         rc = L.hmcgpu_estimate_multi(dev, len(devices), C.byref(prob), C.byref(res))
@@ -442,7 +473,19 @@ class Plan:
             self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_predictive(self.h, C.byref(pr)))
         if self.spec.flags & FLAG_RANKED:
             self.fetch_ranked(out=o)
+        if self.spec.flags & FLAG_ONESTEP:
+            self.fetch_onestep(out=o)
         return self.spec.finish(o, res, rc)
+
+    def fetch_onestep(self, out=None):
+        """hmcgpu_plan_fetch_onestep: the one-step-ahead scores of the last run (onestep_pit / lpd / lpd_var concatenated over
+        the windows, waic [nw, 4]; finish splits them per window)."""
+        o = SimpleNamespace() if out is None else out
+        os_ = self.spec.alloc_onestep(o)
+        if os_ is None:
+            raise ValueError("fetch_onestep on a plan without FLAG_ONESTEP")
+        self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_onestep(self.h, C.byref(os_)))
+        return o
 
     def fetch_ranked(self, probs=None, out=None):
         """hmcgpu_plan_fetch_ranked: the ranked outputs of the last run (quantiles at `probs`, default the spec's

@@ -5,5 +5,5 @@
 #ifndef HMC_SRC_HASH
 #define HMC_SRC_HASH "unknown"
 #endif
-extern "C" int hmcgpu_version(void) { return 500; }
-extern "C" const char* hmcgpu_build_info(void) { return "500;" HMC_SRC_HASH; }
+extern "C" int hmcgpu_version(void) { return 600; }
+extern "C" const char* hmcgpu_build_info(void) { return "600;" HMC_SRC_HASH; }

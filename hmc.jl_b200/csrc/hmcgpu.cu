@@ -7,6 +7,7 @@
 #include "diagnostics.cuh"
 #include "predictive.cuh"
 #include "ranked.cuh"
+#include "onestep.cuh"
 #include "plan_policy.cuh"
 
 #include <algorithm>
@@ -1319,6 +1320,9 @@ struct hmcgpu_plan {
     PredHorizons pr_h{};
     // HMCGPU_FLAG_RANKED (ranked.cuh): every saved draw, keep[((w*F + f)*n_chains + c)*nrun + i]
     DevBuf rk_keep;
+    // HMCGPU_FLAG_ONESTEP (onestep.cuh): kOsState running values per (slot, date), os_n = n_chains * sum_w T_w of each
+    DevBuf os_state, d_ospit, d_oslpd, d_osvar, d_waic;
+    long long os_n = 0;
     DevBuf d_diag;       // segment kernel: chain-sweeps that fell back to the exact entering vectors
     unsigned long long seg_fallbacks[2] = {0, 0};   // [0] chain-sweeps on the exact path, [1] speculative groups (sum over chain-sweeps)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
@@ -1339,9 +1343,10 @@ struct hmcgpu_plan {
 // F: fields per window of the summaries and diagnostics (mu[K], sigma2[K], A[K*K], pi_end[K], forecasts[2*n_h], loglik)
 static int summary_fields(int K, int n_h) { return 3 * K + K * K + 2 * n_h + 1; }
 
-// One per-window output of hmcgpu_result / hmcgpu_predictive / hmcgpu_ranked.  Window w holds per_window + per_step * T_w
-// elements; the windows are concatenated in caller order, in the caller's array and in the plan's device buffer `dev` alike.
-enum class OutStruct { result, predictive, ranked };
+// One per-window output of hmcgpu_result / hmcgpu_predictive / hmcgpu_ranked / hmcgpu_onestep.  Window w holds
+// per_window + per_step * T_w elements; the windows are concatenated in caller order, in the caller's array and in the plan's
+// device buffer `dev` alike.
+enum class OutStruct { result, predictive, ranked, onestep };
 struct WinOut {
     const char* name;
     OutStruct in;              // the struct that holds the caller's pointer
@@ -1354,17 +1359,25 @@ struct WinOut {
     DevBuf hmcgpu_plan::*dev;  // NULL for status, which is read from the chain slots
     // elements of n windows of sum_T steps in all; elems(w, T_0 + ... + T_{w-1}) is the offset of window w
     long long elems(long long n, long long sum_T) const { return per_window * n + per_step * sum_T; }
-    void* base(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk) const {
-        return in == OutStruct::result ? (void*)r : in == OutStruct::predictive ? (void*)pr : (void*)rk;
+    void* base(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk, const hmcgpu_onestep* os) const {
+        switch (in) {
+            case OutStruct::result: return (void*)r;
+            case OutStruct::predictive: return (void*)pr;
+            case OutStruct::ranked: return (void*)rk;
+            default: return (void*)os;
+        }
     }
     // NULL: not requested, or not readable
-    void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk = nullptr) const {
-        const void* s = base(r, pr, rk);
+    void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk = nullptr,
+              const hmcgpu_onestep* os = nullptr) const {
+        const void* s = base(r, pr, rk, os);
         void* p = nullptr;
         if (s && (on || !gated)) memcpy(&p, (const char*)s + field, sizeof p);
         return p;
     }
-    void set(hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk, void* p) const { memcpy((char*)base(r, pr, rk) + field, &p, sizeof p); }
+    void set(hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os, void* p) const {
+        memcpy((char*)base(r, pr, rk, os) + field, &p, sizeof p);
+    }
 };
 
 // n_probs: quantiles per field of the ranked outputs (known at hmcgpu_plan_fetch_ranked)
@@ -1372,7 +1385,7 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
     const long long R = (long long)n_chains * nrun, F = summary_fields(K, n_h);
     const bool draws = flags & HMCGPU_FLAG_DRAWS, summary = flags & HMCGPU_FLAG_SUMMARY, diag = flags & HMCGPU_FLAG_DIAGNOSTICS,
                pred = flags & HMCGPU_FLAG_PREDICTIVE, mean = flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN),
-               ranked = flags & HMCGPU_FLAG_RANKED;
+               ranked = flags & HMCGPU_FLAG_RANKED, onestep = flags & HMCGPU_FLAG_ONESTEP;
     const bool ll = draws && (flags & HMCGPU_FLAG_LOGLIK);
     const char* D = "HMCGPU_FLAG_DRAWS";
     const char* M = "HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN";
@@ -1381,6 +1394,7 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
 #define RES(f) #f, OutStruct::result, offsetof(hmcgpu_result, f)
 #define PRED(f) #f, OutStruct::predictive, offsetof(hmcgpu_predictive, f)
 #define RANK(f) #f, OutStruct::ranked, offsetof(hmcgpu_ranked, f)
+#define ONE(f) #f, OutStruct::onestep, offsetof(hmcgpu_onestep, f)
     std::vector<WinOut> o = {
         {RES(mu), f8, R * K, 0, draws, false, D, &P::d_mu},
         {RES(sigma2), f8, R * K, 0, draws, false, D, &P::d_sig2},
@@ -1404,10 +1418,15 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
         {RANK(rhat_rank), f8, F, 0, ranked, true, "", &P::d_rrank},
         {RANK(ess_bulk), f8, F, 0, ranked, true, "", &P::d_essb},
         {RANK(ess_tail), f8, F, 0, ranked, true, "", &P::d_esst},
+        {ONE(pit), f8, 0, 1, onestep, true, "", &P::d_ospit},
+        {ONE(lpd), f8, 0, 1, onestep, true, "", &P::d_oslpd},
+        {ONE(lpd_var), f8, 0, 1, onestep, true, "", &P::d_osvar},
+        {ONE(waic), f8, 4, 0, onestep, true, "", &P::d_waic},
     };
 #undef RES
 #undef PRED
 #undef RANK
+#undef ONE
     return o;
 }
 
@@ -1443,6 +1462,13 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuni
         // (positions within a field's draws are 32-bit in the sort)
         if ((long long)p->n_chains * p->nrun >= 0x80000000LL)
             return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_RANKED needs n_chains * nrun < 2^31 (got %lld)", (long long)p->n_chains * p->nrun);
+    }
+    if (p->flags & HMCGPU_FLAG_ONESTEP) {
+        if ((long long)p->n_chains * p->nrun < 2)
+            return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_ONESTEP needs n_chains * nrun >= 2 draws per window (lpd_var divides by R - 1)");
+        if (p->is_signal)
+            return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_ONESTEP with is_signal (signal rows have another emission; their scores are not one-step-ahead predictions)");
+        if (p->K > kOsMaxK) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_ONESTEP is only implemented for K <= %d (got K=%d)", kOsMaxK, p->K);
     }
     if (p->precision != 32 && p->precision != 64) return fail(ctx, HMCGPU_ERR_ARG, "precision must be 32 or 64");
     if (p->n_h < 0 || p->n_h > kMaxH || (p->n_h > 0 && !p->horizons)) return fail(ctx, HMCGPU_ERR_ARG, "0 <= n_h <= %d", kMaxH);
@@ -1661,6 +1687,10 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     for (const WinOut& o : window_outputs(K, p->n_h, nc, p->nrun, pl->n_grid, 0, p->flags))
         if (o.on && o.dev && o.in != OutStruct::ranked) CU(ctx, (pl->*o.dev).alloc((size_t)o.elems(nw, sumT) * o.elem));
     if (p->flags & HMCGPU_FLAG_RANKED) CU(ctx, pl->rk_keep.alloc((size_t)nw * pl->F * nc * (size_t)p->nrun * sizeof(R)));
+    if (p->flags & HMCGPU_FLAG_ONESTEP) {
+        pl->os_n = (long long)nc * sumT;
+        CU(ctx, pl->os_state.alloc((size_t)kOsState * pl->os_n * sizeof(double)));
+    }
     // window statistics (once per plan)
     const size_t smem = (size_t)pl->max_T;
     if (smem > 200 * 1024) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "window longer than %d observations", 200 * 1024);
@@ -1834,6 +1864,12 @@ static int plan_run_t(hmcgpu_plan* pl) {
             CU(ctx, cudaGetLastError());
             ++pl->n_launches;
         }
+        if (pl->flags & HMCGPU_FLAG_ONESTEP) {
+            CU(ctx, launch_onestep_accum<R>(Kr, ns, pl->chunk, n, d0, pl->n_chains, pl->slot_win.as<int>(), pl->slot_chain.as<int>(),
+                                            pl->wTd.as<int>(), pl->win_pib_off.as<long long>(), pl->ybase.as<long long>(),
+                                            pl->args.yld, pl->yr.as<R>(), buf, pl->os_state.as<double>(), pl->os_n, st));
+            ++pl->n_launches;
+        }
         if (pl->flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN)) {
             tile_reduce_kernel<R><<<pl->n_windows, 256, 0, st>>>(Kr, Kr, pl->n_chains, pl->win_slot0.as<int>(), pl->wTd.as<int>(),
                                                                  pl->warp_pi_off.as<long long>(), pl->warp_T.as<int>(), pl->win_pib_off.as<long long>(),
@@ -1939,6 +1975,16 @@ static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_pla
         if (keep > (double)total_b)
             return fail(ctx, HMCGPU_ERR_ALLOC, "HMCGPU_FLAG_RANKED retains %.0f bytes of draws, more than the device's %zu bytes", keep, total_b);
     }
+    if (p->flags & HMCGPU_FLAG_ONESTEP) {
+        // kOsState fp64 values per (chain, date): checked before anything is allocated, like the retained draws
+        size_t free_b = 0, total_b = 0;
+        CU(ctx, cudaMemGetInfo(&free_b, &total_b));
+        double dates = 0.0;
+        for (int w = 0; w < p->n_windows; ++w) dates += (double)p->win_end[w] - p->win_start[w] + 1;
+        const double need = dates * p->n_chains * kOsState * sizeof(double);
+        if (need > (double)total_b)
+            return fail(ctx, HMCGPU_ERR_ALLOC, "HMCGPU_FLAG_ONESTEP keeps %.0f bytes of running state, more than the device's %zu bytes", need, total_b);
+    }
     tl_pool = ctx->pool;
     std::unique_ptr<hmcgpu_plan> pl(new hmcgpu_plan());
     pl->ctx = ctx;
@@ -1978,12 +2024,12 @@ extern "C" int hmcgpu_plan_fetch(hmcgpu_plan* pl, hmcgpu_result* r) {
     GUARD(pl->ctx, plan_fetch_impl(pl, r));
 }
 
-// Enqueues the copy of every requested output the plan holds (of r, pr or rk) into the caller's arrays; adds the bytes to *bytes
-// (NULL: the predictive and ranked outputs, which hmcgpu_result's d2h_bytes does not count)
+// Enqueues the copy of every requested output the plan holds (of r, pr, rk or os) into the caller's arrays; adds the bytes to
+// *bytes (NULL: the predictive, ranked and one-step outputs, which hmcgpu_result's d2h_bytes does not count)
 static int download(hmcgpu_plan* pl, const std::vector<WinOut>& outs, const hmcgpu_result* r, const hmcgpu_predictive* pr,
-                    const hmcgpu_ranked* rk, long long* bytes) {
+                    const hmcgpu_ranked* rk, const hmcgpu_onestep* os, long long* bytes) {
     for (const WinOut& o : outs) {
-        void* host = o.get(r, pr, rk);
+        void* host = o.get(r, pr, rk, os);
         if (!host || !o.dev || !(pl->*o.dev).p) continue;         // (an output of no elements has no buffer)
         const DevBuf& b = pl->*o.dev;
         CU(pl->ctx, cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, pl->ctx->stream));
@@ -2016,7 +2062,7 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     if (pl->d_ifc.p) mean_finish_kernel<<<grid_for(nifc, 256), 256, 0, st>>>(nifc, n, pl->d_fcsum.as<double>(), pl->d_ifc.as<double>());
     CU(ctx, cudaGetLastError());
     long long d2h = 0;
-    TRY(download(pl, outs, r, nullptr, nullptr, &d2h));
+    TRY(download(pl, outs, r, nullptr, nullptr, nullptr, &d2h));
     std::vector<int> ev(pl->n_slots);
     CU(ctx, cudaMemcpyAsync(ev.data(), pl->events.p, ev.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
     d2h += (long long)(ev.size() * sizeof(int));
@@ -2050,7 +2096,7 @@ static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
                                                                               pl->pr_score.as<double>(), pl->d_cdf.as<double>(), pl->d_pit.as<double>(),
                                                                               pl->d_ls.as<double>(), pl->d_mom.as<double>());
     CU(ctx, cudaGetLastError());
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, pr, nullptr, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, pr, nullptr, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));
     return HMCGPU_OK;
 }
@@ -2157,7 +2203,7 @@ static int fetch_ranked_t(hmcgpu_plan* pl, const hmcgpu_ranked* rk) {
                                                                  pl->d_rrank.as<double>(), pl->d_essb.as<double>(), pl->d_esst.as<double>());
         CU(ctx, cudaGetLastError());
     }
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, nc, pl->nrun, pl->n_grid, rk->n_probs, pl->flags), nullptr, nullptr, rk, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, nc, pl->nrun, pl->n_grid, rk->n_probs, pl->flags), nullptr, nullptr, rk, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));         // (the scratch goes back to the pool when this returns)
     return HMCGPU_OK;
 }
@@ -2178,6 +2224,28 @@ extern "C" int hmcgpu_plan_fetch_ranked(hmcgpu_plan* pl, hmcgpu_ranked* rk) {
     GUARD(pl->ctx, plan_fetch_ranked_impl(pl, rk));
 }
 
+static int plan_fetch_onestep_impl(hmcgpu_plan* pl, hmcgpu_onestep* os) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    if (!(pl->flags & HMCGPU_FLAG_ONESTEP)) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_onestep on a plan without HMCGPU_FLAG_ONESTEP");
+    if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_onestep before plan_run");
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    // (not plan_run's launch: n_launches leaves it out)
+    onestep_finish_kernel<<<pl->n_windows, 128, 0, st>>>(pl->K, pl->n_chains, pl->nrun, pl->wTd.as<int>(), pl->win_pib_off.as<long long>(),
+                                                         pl->os_state.as<double>(), pl->os_n, pl->d_ospit.as<double>(),
+                                                         pl->d_oslpd.as<double>(), pl->d_osvar.as<double>(), pl->d_waic.as<double>());
+    CU(ctx, cudaGetLastError());
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, nullptr, nullptr, os, nullptr));
+    CU(ctx, cudaStreamSynchronize(st));
+    return HMCGPU_OK;
+}
+
+extern "C" int hmcgpu_plan_fetch_onestep(hmcgpu_plan* pl, hmcgpu_onestep* os) {
+    if (!pl) return HMCGPU_ERR_ARG;
+    if (!os) return fail(pl->ctx, HMCGPU_ERR_ARG, "hmcgpu_onestep is NULL");
+    GUARD(pl->ctx, plan_fetch_onestep_impl(pl, os));
+}
+
 extern "C" void hmcgpu_plan_destroy(hmcgpu_plan* pl) {
     if (!pl) return;
     cudaSetDevice(pl->ctx->device);
@@ -2195,7 +2263,14 @@ extern "C" int hmcgpu_estimate_predictive(hmcgpu_ctx* ctx, const hmcgpu_problem*
 }
 
 extern "C" int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk) {
+    return hmcgpu_estimate_onestep(ctx, p, r, pr, rk, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk,
+                                       hmcgpu_onestep* os) {
     if (!r) return fail(ctx, HMCGPU_ERR_ARG, "result is NULL");
+    if (p && (p->flags & HMCGPU_FLAG_ONESTEP) && !os)
+        return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_ONESTEP without hmcgpu_onestep outputs (use hmcgpu_estimate_onestep)");
     if (p && (p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
         return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_predictive)");
     if (p && (p->flags & HMCGPU_FLAG_RANKED)) {
@@ -2217,6 +2292,10 @@ extern "C" int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, 
         const int rp = hmcgpu_plan_fetch_ranked(pl, rk);
         if (rp < 0) rc = rp;
     }
+    if (rc >= 0 && (p->flags & HMCGPU_FLAG_ONESTEP)) {
+        const int rp = hmcgpu_plan_fetch_onestep(pl, os);
+        if (rp < 0) rc = rp;
+    }
     tr.mark("plan_fetch (download)");
     hmcgpu_plan_destroy(pl);
     tr.mark("plan_destroy");
@@ -2225,7 +2304,7 @@ extern "C" int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, 
 
 // Windows sharded over devices by longest-processing-time-first on T_w; one host thread per device, no collectives.
 static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
-                               hmcgpu_ranked* rk);
+                               hmcgpu_ranked* rk, hmcgpu_onestep* os);
 extern "C" int hmcgpu_estimate_multi(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r) {
     return hmcgpu_estimate_multi_ranked(devices, n_dev, p, r, nullptr, nullptr);
 }
@@ -2237,7 +2316,14 @@ extern "C" int hmcgpu_estimate_multi_predictive(const int* devices, int n_dev, c
 
 extern "C" int hmcgpu_estimate_multi_ranked(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
                                             hmcgpu_predictive* pr, hmcgpu_ranked* rk) {
+    return hmcgpu_estimate_multi_onestep(devices, n_dev, p, r, pr, rk, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_multi_onestep(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
+                                             hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os) {
     if (!devices || n_dev < 1 || !p || !r) return fail(nullptr, HMCGPU_ERR_ARG, "bad arguments");
+    if ((p->flags & HMCGPU_FLAG_ONESTEP) && !os)
+        return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_ONESTEP without hmcgpu_onestep outputs (use hmcgpu_estimate_multi_onestep)");
     if ((p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
         return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_PREDICTIVE without hmcgpu_predictive outputs (use hmcgpu_estimate_multi_predictive)");
     if (p->flags & HMCGPU_FLAG_RANKED) {
@@ -2245,11 +2331,11 @@ extern "C" int hmcgpu_estimate_multi_ranked(const int* devices, int n_dev, const
         TRY(check_ranked(nullptr, rk));
     }
     GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r, (p->flags & HMCGPU_FLAG_PREDICTIVE) ? pr : nullptr,
-                                       (p->flags & HMCGPU_FLAG_RANKED) ? rk : nullptr));
+                                       (p->flags & HMCGPU_FLAG_RANKED) ? rk : nullptr, (p->flags & HMCGPU_FLAG_ONESTEP) ? os : nullptr));
 }
 
 static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
-                               hmcgpu_ranked* rk) {
+                               hmcgpu_ranked* rk, hmcgpu_onestep* os) {
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(nullptr, HMCGPU_ERR_ARG, "no windows");
     const int nw = p->n_windows;
     std::vector<int> ord(nw);
@@ -2300,19 +2386,20 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             hmcgpu_result& o = parts[d];
             hmcgpu_predictive pq{};
             hmcgpu_ranked rq{};
+            hmcgpu_onestep oq{};
             if (rk) { rq.probs = rk->probs; rq.n_probs = rk->n_probs; }
             std::vector<std::vector<char>> stage(outs.size());
             for (size_t i = 0; i < outs.size(); ++i) {
-                if (!outs[i].get(r, pr, rk)) continue;
+                if (!outs[i].get(r, pr, rk, os)) continue;
                 stage[i].resize(std::max<size_t>(1, (size_t)outs[i].elems(n, sum_T) * outs[i].elem));
-                outs[i].set(&o, &pq, &rq, stage[i].data());
+                outs[i].set(&o, &pq, &rq, &oq, stage[i].data());
             }
-            rc = hmcgpu_estimate_ranked(ctx, &q, &o, pr ? &pq : nullptr, rk ? &rq : nullptr);
+            rc = hmcgpu_estimate_onestep(ctx, &q, &o, pr ? &pq : nullptr, rk ? &rq : nullptr, os ? &oq : nullptr);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
             for (size_t i = 0; rc >= 0 && i < outs.size(); ++i) {   // scatter this shard's windows into the caller's arrays
                 const WinOut& x = outs[i];
-                char* dst = (char*)x.get(r, pr, rk);
+                char* dst = (char*)x.get(r, pr, rk, os);
                 if (!dst) continue;
                 long long t = 0;                                 // steps of the shard's windows before window j
                 for (int j = 0; j < n; ++j) {

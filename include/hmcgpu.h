@@ -62,6 +62,9 @@ extern "C" {
                                         window and horizon, computed on the device from every saved draw (see hmcgpu_predictive) */
 #define HMCGPU_FLAG_RANKED  512u     /* keep every saved draw on the device so that hmcgpu_plan_fetch_ranked can compute exact quantiles,
                                         rank-normalised R̂ and bulk / tail ESS; needs nrun >= 4 and n_chains * nrun < 2^31 (see hmcgpu_ranked) */
+#define HMCGPU_FLAG_ONESTEP  1024u   /* fill hmcgpu_onestep: the one-step-ahead posterior predictive PIT and log density of every date
+                                        of every window, and WAIC per window, computed on the device from every saved draw; K <= 8,
+                                        no is_signal, n_chains * nrun >= 2 (see hmcgpu_onestep) */
 
 typedef struct hmcgpu_ctx hmcgpu_ctx;
 typedef struct hmcgpu_plan hmcgpu_plan;
@@ -227,6 +230,39 @@ typedef struct hmcgpu_ranked {
     double* ess_tail;     /* [n_windows x F] */
 } hmcgpu_ranked;
 
+/* One-step-ahead scores of the in-sample dates (HMCGPU_FLAG_ONESTEP); caller-allocated, any pointer may be NULL.
+ * For window w with N = N_w dates y_1..y_N (its own series, win_series, from win_start), each saved draw d (emitted mu_s,
+ * sigma2_s and A[r][s] = field 2K + s*K + r, in the increasing-mu labelling) is run through the forward filter from the UNIFORM
+ * initial distribution, in the log domain:
+ *   w_1,s  = 1/K
+ *   l_t,s  = log w_t,s + log phi(y_t; mu_s, sigma2_s)
+ *   ell_t,d = log sum_s exp(l_t,s)                        = log p(y_t | y_1..t-1, theta_d)
+ *   F_t,d  = sum_s w_t,s Phi((y_t - mu_s) / sqrt(sigma2_s))  one-step-ahead predictive CDF at the realised value
+ *   alpha_t,s = exp(l_t,s - ell_t,d),   w_t+1,s = sum_r alpha_t,r A[r][s]
+ * The uniform start is not an approximation: the sampler draws rho from Dirichlet(1,...,1) at every sweep without looking at the
+ * data (src/Hmc.jl:350-356), p(y | theta, rho) is linear in rho and E[rho] = 1/K, so the uniform start gives the likelihood with
+ * rho integrated out.  Sum_t ell_t,d therefore differs from the per-draw loglik field, which uses the sweep's sampled rho.
+ * Pooled over the R = n_chains*nrun draws of the window (per-date arrays: windows concatenated, window w at offset
+ * sum_{v<w} N_v, like pib_mean):
+ *   pit[off_w + t]      = (1/R) sum_d F_t,d
+ *   lpd[off_w + t]      = log((1/R) sum_d exp(ell_t,d))
+ *   lpd_var[off_w + t]  = sample variance over d of ell_t,d (denominator R - 1)
+ *   waic[w*4 + 0..3]    = lppd = sum_t lpd_t, p_waic = sum_t lpd_var_t, elpd_waic = lppd - p_waic,
+ *                         se = sqrt(N var_t(lpd_t - lpd_var_t)) with the variance over t taken with denominator N - 1
+ * A window with a non-finite mu / sigma2 / A draw gets NaN in every output.  The per-draw filter runs in the plan's precision (as
+ * the chain that produced the draw) and stays finite for an observation 50 sd from every state mean; every sum over draws and
+ * chains (PIT sums, the log-sum-exp, the running mean / M2) is fp64 and runs in draw order, then chain order, with no atomics: a
+ * window's outputs are bit-identical however the windows are batched, chunked or sharded.  Needs K <= 8 and no is_signal (signal
+ * rows have another emission); pi_row_back is allowed (pi_end is not read).  Device state: 5 doubles per (chain, date),
+ * 40 * n_chains * sum_w N_w bytes (C2: 500 windows x 256 chains, sum_w N_w = 175 250: 1.8 GB), checked against the device's total
+ * memory at hmcgpu_plan_create (HMCGPU_ERR_ALLOC) and allocated only with the flag. */
+typedef struct hmcgpu_onestep {
+    double* pit;          /* [sum_w N_w] */
+    double* lpd;          /* [sum_w N_w] */
+    double* lpd_var;      /* [sum_w N_w] */
+    double* waic;         /* [n_windows][4]: lppd, p_waic, elpd_waic, se */
+} hmcgpu_onestep;
+
 #define HMCGPU_KERNEL_THREAD 0  /* one thread per chain (gibbs_sweeps_kernel), wide batches, K <= 8 */
 #define HMCGPU_KERNEL_SCAN 1    /* one warp per chain, time-parallel scans (gibbs_scan_kernel), narrow batches */
 #define HMCGPU_KERNEL_LANE 2    /* one lane per state (gibbs_wide_kernel), K = 9..32 */
@@ -265,6 +301,12 @@ int hmcgpu_estimate_multi_predictive(const int* devices, int n_devices, const hm
 int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk);
 int hmcgpu_estimate_multi_ranked(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
                                  hmcgpu_predictive* pr, hmcgpu_ranked* rk);
+/* The same filling the one-step-ahead scores too (hmcgpu_estimate_ranked and hmcgpu_estimate_multi_ranked are these with
+ * os = NULL).  With HMCGPU_FLAG_ONESTEP, os must not be NULL (HMCGPU_ERR_ARG); without it os is ignored. */
+int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk,
+                            hmcgpu_onestep* os);
+int hmcgpu_estimate_multi_onestep(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
+                                  hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os);
 
 /* Split form: create uploads inputs and allocates device state; run executes every sweep (inputs resident
  * in HBM, no host transfers); fetch copies the requested outputs back.  run may be repeated (it restarts
@@ -278,6 +320,8 @@ int hmcgpu_plan_fetch_predictive(hmcgpu_plan* plan, hmcgpu_predictive* pr);
  * the plan again.  HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_RANKED, before a run, with n_probs outside 0..64 or a
  * probability that is not finite or outside [0, 1]. */
 int hmcgpu_plan_fetch_ranked(hmcgpu_plan* plan, hmcgpu_ranked* rk);
+/* One-step-ahead scores of the last run; HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_ONESTEP or before a run. */
+int hmcgpu_plan_fetch_onestep(hmcgpu_plan* plan, hmcgpu_onestep* os);
 void hmcgpu_plan_destroy(hmcgpu_plan* plan);
 
 /* Forward filter for fixed parameters.  y: [T] shared by the batch (y_batch_stride = 0) or [B][T]
