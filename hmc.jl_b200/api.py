@@ -230,7 +230,7 @@ def shard_windows(T: Sequence[int], n_shards: int):
 def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nrun=1000, seed=1234, horizons=(12,),
                      precision=32, draws=False, summary=True, smoothed=False, loglik=False, win_id=None,
                      win_series=None, diagnostics=False, predictive_grid=None, quantiles=None, rank_diagnostics=False,
-                     onestep=False, ctx: Optional[B.Context] = None, device: int = 0):
+                     onestep=False, loo=False, ctx: Optional[B.Context] = None, device: int = 0):
     """Many end-date windows in one call (what the SLURM job array does one process at a time).  `diagnostics=True` adds
     `rhat`, `ess` and `ess_lag` [n_windows, F] (split-R̂ and effective sample size per summary field; see write_diagnostics).
     `predictive_grid` (increasing points, shared by every window and horizon) adds the posterior predictive distribution of
@@ -240,12 +240,15 @@ def estimate_windows(y, win_start, win_end, *, K=3, n_chains=1, burnin=1000, nru
     posterior `quantiles` [n_windows, F, n_probs], the rank-normalised split-R̂ `rhat_rank` and the bulk / tail effective
     sample sizes `ess_bulk` / `ess_tail` [n_windows, F]; see write_ranked.  `onestep=True` (HMCGPU_FLAG_ONESTEP, K <= 8) scores
     every in-sample date by its one-step-ahead posterior predictive: `onestep_pit`, `lpd` and `lpd_var` (lists of [N_w] arrays)
-    and `waic` [n_windows, 4] (lppd, p_waic, elpd_waic, se); see pseudo_residuals, compare_waic and write_onestep."""
+    and `waic` [n_windows, 4] (lppd, p_waic, elpd_waic, se); see pseudo_residuals, compare_waic and write_onestep.  `loo=True`
+    (HMCGPU_FLAG_LOO, K <= 8) adds PSIS-LOO cross-validation of every in-sample date: `loo_elpd`, `loo_lppd`, `pareto_k` and
+    `loo_pit` (lists of [N_w] arrays) and `loo` [n_windows, 6] (elpd_loo, se, p_loo, lppd, max k̂, dates with k̂ above the
+    threshold); see compare_loo and write_loo."""
     ranked = quantiles is not None or rank_diagnostics
     flags = B.FLAG_REF_Q1 | (B.FLAG_DRAWS if draws else 0) | (B.FLAG_SUMMARY if summary else 0) \
         | (B.FLAG_SMOOTHED_MEAN if smoothed else 0) | (B.FLAG_LOGLIK if loglik else 0) \
         | (B.FLAG_DIAGNOSTICS if diagnostics else 0) | (B.FLAG_PREDICTIVE if predictive_grid is not None else 0) \
-        | (B.FLAG_RANKED if ranked else 0) | (B.FLAG_ONESTEP if onestep else 0)
+        | (B.FLAG_RANKED if ranked else 0) | (B.FLAG_ONESTEP if onestep else 0) | (B.FLAG_LOO if loo else 0)
     spec = B.ProblemSpec(y, win_start, win_end, K=K, n_chains=n_chains, burnin=burnin, nrun=nrun, seed=seed,
                          horizons=list(horizons), precision=precision, flags=flags, win_id=win_id, win_series=win_series,
                          pred_grid=predictive_grid, quantile_probs=quantiles)
@@ -457,6 +460,41 @@ def compare_waic(a, b):
         diff[w] = np.asarray(a.waic)[w, 2] - np.asarray(b.waic)[w, 2]
         se[w] = np.sqrt(len(d) * np.var(d, ddof=1))
     return SimpleNamespace(elpd_diff=diff, se_diff=se)
+
+
+def compare_loo(a, b):
+    """Per-window PSIS-LOO comparison of two fits of the same windows (e.g. K = 3 against K = 2), from estimate_windows(loo=True)
+    outputs: `elpd_diff` [n_windows] = sum_t (elpd_a,t - elpd_b,t) and `se_diff` [n_windows] = sqrt(N var_t(elpd_a,t - elpd_b,t))
+    (denominator N - 1, as the loo package's loo_compare).  A positive difference of several se_diff favours `a`; read
+    `pareto_k` of both fits first: a date above the threshold makes its elpd (and so the difference) unreliable."""
+    if len(a.loo_elpd) != len(b.loo_elpd) or any(len(x) != len(y) for x, y in zip(a.loo_elpd, b.loo_elpd)):
+        raise ValueError("compare_loo needs the same windows (and window lengths) in both fits")
+    diff, se = np.empty(len(a.loo_elpd)), np.empty(len(a.loo_elpd))
+    for w in range(len(a.loo_elpd)):
+        d = np.asarray(a.loo_elpd[w]) - np.asarray(b.loo_elpd[w])
+        diff[w] = d.sum()
+        se[w] = np.sqrt(len(d) * np.var(d, ddof=1))
+    return SimpleNamespace(elpd_diff=diff, se_diff=se)
+
+
+def write_loo(out, dates: Sequence, directory: str):
+    """The PSIS-LOO outputs of estimate_windows(loo=True), windows in caller order: `loo_scores.csv` with one row per (window,
+    in-sample date): the window's end date, the date's 1-based position in the window, elpd, lppd, pareto_k and the LOO-PIT; and
+    `loo.csv` with one row per window: end date, elpd_loo, se, p_loo, lppd, max_k, n_high_k.  Returns {"scores": path,
+    "loo": path}."""
+    import os
+    os.makedirs(directory, exist_ok=True)
+    paths = {"scores": os.path.join(directory, "loo_scores.csv"), "loo": os.path.join(directory, "loo.csv")}
+    with open(paths["scores"], "w") as f:
+        f.write("date,t,elpd,lppd,pareto_k,pit\n")
+        for d, e, l, k, p in zip(dates, out.loo_elpd, out.loo_lppd, out.pareto_k, out.loo_pit):
+            for t in range(len(e)):
+                f.write(",".join([str(d), str(t + 1)] + [repr(float(v[t])) for v in (e, l, k, p)]) + "\n")
+    with open(paths["loo"], "w") as f:
+        f.write("date,elpd_loo,se,p_loo,lppd,max_k,n_high_k\n")
+        for d, row in zip(dates, np.asarray(out.loo)):
+            f.write(",".join([str(d)] + [repr(float(v)) for v in row]) + "\n")
+    return paths
 
 
 def write_onestep(out, dates: Sequence, directory: str):

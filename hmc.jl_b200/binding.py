@@ -22,6 +22,7 @@ FLAG_DIAGNOSTICS = 128    # rhat / ess / ess_lag per window and summary field (s
 FLAG_PREDICTIVE = 256     # posterior predictive CDF on a grid, PIT, log score and moments per window and horizon (hmcgpu_predictive)
 FLAG_RANKED = 512         # keep every saved draw on the device: exact quantiles, rank-normalised R̂, bulk / tail ESS (hmcgpu_ranked)
 FLAG_ONESTEP = 1024       # one-step-ahead PIT and log predictive density of every in-sample date, WAIC per window (hmcgpu_onestep)
+FLAG_LOO = 2048           # PSIS-LOO of every in-sample date: leave-one-out density, Pareto k̂, LOO-PIT; per-window elpd_loo (hmcgpu_loo)
 
 ERR_ARG, ERR_CUDA, ERR_ALLOC, ERR_UNSUPPORTED, ERR_NODEVICE = -1, -2, -3, -4, -5
 
@@ -34,6 +35,7 @@ SYMBOLS = [
     "hmcgpu_build_info", "hmcgpu_ctx_trim", "hmcgpu_estimate_predictive", "hmcgpu_estimate_multi_predictive",
     "hmcgpu_plan_fetch_predictive", "hmcgpu_estimate_ranked", "hmcgpu_estimate_multi_ranked", "hmcgpu_plan_fetch_ranked",
     "hmcgpu_estimate_onestep", "hmcgpu_estimate_multi_onestep", "hmcgpu_plan_fetch_onestep",
+    "hmcgpu_estimate_loo", "hmcgpu_estimate_multi_loo", "hmcgpu_plan_fetch_loo",
 ]
 KERNEL_NAMES = {0: "gibbs_sweeps_kernel (thread per chain)", 1: "gibbs_scan_kernel (warp per chain, time-parallel)",
                 2: "gibbs_wide_kernel (lane per state)", 3: "(reserved)",
@@ -76,6 +78,10 @@ class Ranked(C.Structure):
 
 class Onestep(C.Structure):
     _fields_ = [("pit", _dp), ("lpd", _dp), ("lpd_var", _dp), ("waic", _dp)]
+
+
+class Loo(C.Structure):
+    _fields_ = [("elpd", _dp), ("lppd", _dp), ("pareto_k", _dp), ("pit", _dp), ("summary", _dp)]
 
 
 class HmcGpuError(RuntimeError):
@@ -132,6 +138,11 @@ def load(build_if_missing: bool = True):
     L.hmcgpu_estimate_multi_onestep.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
                                                 C.POINTER(Predictive), C.POINTER(Ranked), C.POINTER(Onestep)]
     L.hmcgpu_plan_fetch_onestep.argtypes = [C.c_void_p, C.POINTER(Onestep)]
+    L.hmcgpu_estimate_loo.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Result), C.POINTER(Predictive), C.POINTER(Ranked),
+                                      C.POINTER(Onestep), C.POINTER(Loo)]
+    L.hmcgpu_estimate_multi_loo.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(Problem), C.POINTER(Result),
+                                            C.POINTER(Predictive), C.POINTER(Ranked), C.POINTER(Onestep), C.POINTER(Loo)]
+    L.hmcgpu_plan_fetch_loo.argtypes = [C.c_void_p, C.POINTER(Loo)]
     L.hmcgpu_plan_destroy.argtypes = [C.c_void_p]
     L.hmcgpu_plan_destroy.restype = None
     L.hmcgpu_filter.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _dp, C.c_int64,
@@ -389,6 +400,17 @@ class ProblemSpec:
         o.waic = np.empty((self.n_windows, 4))
         return Onestep(_p(o.onestep_pit), _p(o.lpd), _p(o.lpd_var), _p(o.waic))
 
+    def alloc_loo(self, o):
+        """Adds the PSIS-LOO outputs to `o` (loo_elpd, loo_lppd, pareto_k, loo_pit: per date, windows concatenated, split per
+        window by finish; loo [nw, 6]: elpd_loo, se, p_loo, lppd, max k̂, dates with k̂ above the threshold) and returns the
+        hmcgpu_loo struct over them; None without FLAG_LOO."""
+        if not self.flags & FLAG_LOO:
+            return None
+        n = int(self.T.sum())
+        o.loo_elpd = np.empty(n); o.loo_lppd = np.empty(n); o.pareto_k = np.empty(n); o.loo_pit = np.empty(n)
+        o.loo = np.empty((self.n_windows, 6))
+        return Loo(_p(o.loo_elpd), _p(o.loo_lppd), _p(o.pareto_k), _p(o.loo_pit), _p(o.loo))
+
     def finish(self, o, res, rc):
         o.events = rc
         o.gpu_ms, o.sweep_kernel_ms = res.gpu_ms, res.sweep_kernel_ms
@@ -410,6 +432,9 @@ class ProblemSpec:
         if getattr(o, "lpd", None) is not None and not isinstance(o.lpd, list):   # per-window [N_w]
             cut = np.cumsum(self.T)[:-1]
             o.onestep_pit, o.lpd, o.lpd_var = (np.split(a, cut) for a in (o.onestep_pit, o.lpd, o.lpd_var))
+        if getattr(o, "loo_elpd", None) is not None and not isinstance(o.loo_elpd, list):   # per-window [N_w]
+            cut = np.cumsum(self.T)[:-1]
+            o.loo_elpd, o.loo_lppd, o.pareto_k, o.loo_pit = (np.split(a, cut) for a in (o.loo_elpd, o.loo_lppd, o.pareto_k, o.loo_pit))
         return o
 
 
@@ -419,8 +444,11 @@ def estimate(ctx: Context, spec: ProblemSpec):
     pr = spec.alloc_predictive(o)
     rk = spec.alloc_ranked(o)
     os_ = spec.alloc_onestep(o)
+    lo = spec.alloc_loo(o)
     prob = spec.struct()
-    if os_ is not None:
+    if lo is not None:
+        rc = ctx._check(ctx.L.hmcgpu_estimate_loo(ctx.h, C.byref(prob), C.byref(res), _ref(pr), _ref(rk), _ref(os_), C.byref(lo)))
+    elif os_ is not None:
         rc = ctx._check(ctx.L.hmcgpu_estimate_onestep(ctx.h, C.byref(prob), C.byref(res), _ref(pr), _ref(rk), C.byref(os_)))
     elif rk is not None:
         rc = ctx._check(ctx.L.hmcgpu_estimate_ranked(ctx.h, C.byref(prob), C.byref(res), _ref(pr), C.byref(rk)))
@@ -437,9 +465,12 @@ def estimate_multi(devices, spec: ProblemSpec):
     pr = spec.alloc_predictive(o)
     rk = spec.alloc_ranked(o)
     os_ = spec.alloc_onestep(o)
+    lo = spec.alloc_loo(o)
     prob = spec.struct()
     dev = (C.c_int * len(devices))(*devices)
-    if os_ is not None:
+    if lo is not None:
+        rc = L.hmcgpu_estimate_multi_loo(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), _ref(rk), _ref(os_), C.byref(lo))
+    elif os_ is not None:
         rc = L.hmcgpu_estimate_multi_onestep(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), _ref(rk), C.byref(os_))
     elif rk is not None:
         rc = L.hmcgpu_estimate_multi_ranked(dev, len(devices), C.byref(prob), C.byref(res), _ref(pr), C.byref(rk))
@@ -475,7 +506,19 @@ class Plan:
             self.fetch_ranked(out=o)
         if self.spec.flags & FLAG_ONESTEP:
             self.fetch_onestep(out=o)
+        if self.spec.flags & FLAG_LOO:
+            self.fetch_loo(out=o)
         return self.spec.finish(o, res, rc)
+
+    def fetch_loo(self, out=None):
+        """hmcgpu_plan_fetch_loo: the PSIS-LOO outputs of the last run, computed now from the kept draws (loo_elpd / loo_lppd /
+        pareto_k / loo_pit concatenated over the windows, loo [nw, 6]; finish splits them per window)."""
+        o = SimpleNamespace() if out is None else out
+        lo = self.spec.alloc_loo(o)
+        if lo is None:
+            raise ValueError("fetch_loo on a plan without FLAG_LOO")
+        self.ctx._check(self.ctx.L.hmcgpu_plan_fetch_loo(self.h, C.byref(lo)))
+        return o
 
     def fetch_onestep(self, out=None):
         """hmcgpu_plan_fetch_onestep: the one-step-ahead scores of the last run (onestep_pit / lpd / lpd_var concatenated over

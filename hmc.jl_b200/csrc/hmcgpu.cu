@@ -8,6 +8,7 @@
 #include "predictive.cuh"
 #include "ranked.cuh"
 #include "onestep.cuh"
+#include "loo.cuh"
 #include "plan_policy.cuh"
 
 #include <algorithm>
@@ -1323,6 +1324,9 @@ struct hmcgpu_plan {
     // HMCGPU_FLAG_ONESTEP (onestep.cuh): kOsState running values per (slot, date), os_n = n_chains * sum_w T_w of each
     DevBuf os_state, d_ospit, d_oslpd, d_osvar, d_waic;
     long long os_n = 0;
+    // HMCGPU_FLAG_LOO (loo.cuh): mu, sigma2, A of every saved draw, keep[((w*F' + f)*n_chains + c)*nrun + i], F' = 2K + K^2
+    // (not allocated with HMCGPU_FLAG_RANKED, whose rk_keep holds them); the per-date and per-window outputs
+    DevBuf lo_keep, d_lelpd, d_llppd, d_lpk, d_lpit, d_lsum;
     DevBuf d_diag;       // segment kernel: chain-sweeps that fell back to the exact entering vectors
     unsigned long long seg_fallbacks[2] = {0, 0};   // [0] chain-sweeps on the exact path, [1] speculative groups (sum over chain-sweeps)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
@@ -1343,10 +1347,10 @@ struct hmcgpu_plan {
 // F: fields per window of the summaries and diagnostics (mu[K], sigma2[K], A[K*K], pi_end[K], forecasts[2*n_h], loglik)
 static int summary_fields(int K, int n_h) { return 3 * K + K * K + 2 * n_h + 1; }
 
-// One per-window output of hmcgpu_result / hmcgpu_predictive / hmcgpu_ranked / hmcgpu_onestep.  Window w holds
+// One per-window output of hmcgpu_result / hmcgpu_predictive / hmcgpu_ranked / hmcgpu_onestep / hmcgpu_loo.  Window w holds
 // per_window + per_step * T_w elements; the windows are concatenated in caller order, in the caller's array and in the plan's
 // device buffer `dev` alike.
-enum class OutStruct { result, predictive, ranked, onestep };
+enum class OutStruct { result, predictive, ranked, onestep, loo };
 struct WinOut {
     const char* name;
     OutStruct in;              // the struct that holds the caller's pointer
@@ -1359,24 +1363,26 @@ struct WinOut {
     DevBuf hmcgpu_plan::*dev;  // NULL for status, which is read from the chain slots
     // elements of n windows of sum_T steps in all; elems(w, T_0 + ... + T_{w-1}) is the offset of window w
     long long elems(long long n, long long sum_T) const { return per_window * n + per_step * sum_T; }
-    void* base(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk, const hmcgpu_onestep* os) const {
+    void* base(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk, const hmcgpu_onestep* os,
+               const hmcgpu_loo* lo) const {
         switch (in) {
             case OutStruct::result: return (void*)r;
             case OutStruct::predictive: return (void*)pr;
             case OutStruct::ranked: return (void*)rk;
-            default: return (void*)os;
+            case OutStruct::onestep: return (void*)os;
+            default: return (void*)lo;
         }
     }
     // NULL: not requested, or not readable
     void* get(const hmcgpu_result* r, const hmcgpu_predictive* pr, const hmcgpu_ranked* rk = nullptr,
-              const hmcgpu_onestep* os = nullptr) const {
-        const void* s = base(r, pr, rk, os);
+              const hmcgpu_onestep* os = nullptr, const hmcgpu_loo* lo = nullptr) const {
+        const void* s = base(r, pr, rk, os, lo);
         void* p = nullptr;
         if (s && (on || !gated)) memcpy(&p, (const char*)s + field, sizeof p);
         return p;
     }
-    void set(hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os, void* p) const {
-        memcpy((char*)base(r, pr, rk, os) + field, &p, sizeof p);
+    void set(hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os, hmcgpu_loo* lo, void* p) const {
+        memcpy((char*)base(r, pr, rk, os, lo) + field, &p, sizeof p);
     }
 };
 
@@ -1385,7 +1391,7 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
     const long long R = (long long)n_chains * nrun, F = summary_fields(K, n_h);
     const bool draws = flags & HMCGPU_FLAG_DRAWS, summary = flags & HMCGPU_FLAG_SUMMARY, diag = flags & HMCGPU_FLAG_DIAGNOSTICS,
                pred = flags & HMCGPU_FLAG_PREDICTIVE, mean = flags & (HMCGPU_FLAG_SMOOTHED_MEAN | HMCGPU_FLAG_FILTERED_MEAN),
-               ranked = flags & HMCGPU_FLAG_RANKED, onestep = flags & HMCGPU_FLAG_ONESTEP;
+               ranked = flags & HMCGPU_FLAG_RANKED, onestep = flags & HMCGPU_FLAG_ONESTEP, loo = flags & HMCGPU_FLAG_LOO;
     const bool ll = draws && (flags & HMCGPU_FLAG_LOGLIK);
     const char* D = "HMCGPU_FLAG_DRAWS";
     const char* M = "HMCGPU_FLAG_SMOOTHED_MEAN or HMCGPU_FLAG_FILTERED_MEAN";
@@ -1395,6 +1401,7 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
 #define PRED(f) #f, OutStruct::predictive, offsetof(hmcgpu_predictive, f)
 #define RANK(f) #f, OutStruct::ranked, offsetof(hmcgpu_ranked, f)
 #define ONE(f) #f, OutStruct::onestep, offsetof(hmcgpu_onestep, f)
+#define LOO(f) #f, OutStruct::loo, offsetof(hmcgpu_loo, f)
     std::vector<WinOut> o = {
         {RES(mu), f8, R * K, 0, draws, false, D, &P::d_mu},
         {RES(sigma2), f8, R * K, 0, draws, false, D, &P::d_sig2},
@@ -1422,11 +1429,17 @@ static std::vector<WinOut> window_outputs(int K, int n_h, int n_chains, long lon
         {ONE(lpd), f8, 0, 1, onestep, true, "", &P::d_oslpd},
         {ONE(lpd_var), f8, 0, 1, onestep, true, "", &P::d_osvar},
         {ONE(waic), f8, 4, 0, onestep, true, "", &P::d_waic},
+        {LOO(elpd), f8, 0, 1, loo, true, "", &P::d_lelpd},
+        {LOO(lppd), f8, 0, 1, loo, true, "", &P::d_llppd},
+        {LOO(pareto_k), f8, 0, 1, loo, true, "", &P::d_lpk},
+        {LOO(pit), f8, 0, 1, loo, true, "", &P::d_lpit},
+        {LOO(summary), f8, kLooSummary, 0, loo, true, "", &P::d_lsum},
     };
 #undef RES
 #undef PRED
 #undef RANK
 #undef ONE
+#undef LOO
     return o;
 }
 
@@ -1469,6 +1482,16 @@ static int validate_problem(hmcgpu_ctx* ctx, const hmcgpu_problem* p, const Tuni
         if (p->is_signal)
             return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_ONESTEP with is_signal (signal rows have another emission; their scores are not one-step-ahead predictions)");
         if (p->K > kOsMaxK) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_ONESTEP is only implemented for K <= %d (got K=%d)", kOsMaxK, p->K);
+    }
+    if (p->flags & HMCGPU_FLAG_LOO) {
+        const long long R = (long long)p->n_chains * p->nrun;
+        if (R < 2) return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_LOO needs n_chains * nrun >= 2 draws per window");
+        // (the Pareto tail of up to 3 sqrt(R) values and their draw indices sits in shared memory)
+        if (R > kLooMaxDraws)
+            return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_LOO needs n_chains * nrun <= 2^24 draws per window (got %lld)", R);
+        if (p->is_signal)
+            return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_LOO with is_signal (signal rows have another emission; their scores are not predictions of the data)");
+        if (p->K > kOsMaxK) return fail(ctx, HMCGPU_ERR_UNSUPPORTED, "HMCGPU_FLAG_LOO is only implemented for K <= %d (got K=%d)", kOsMaxK, p->K);
     }
     if (p->precision != 32 && p->precision != 64) return fail(ctx, HMCGPU_ERR_ARG, "precision must be 32 or 64");
     if (p->n_h < 0 || p->n_h > kMaxH || (p->n_h > 0 && !p->horizons)) return fail(ctx, HMCGPU_ERR_ARG, "0 <= n_h <= %d", kMaxH);
@@ -1687,6 +1710,8 @@ static int plan_build(hmcgpu_plan* pl, const hmcgpu_problem* p) {
     for (const WinOut& o : window_outputs(K, p->n_h, nc, p->nrun, pl->n_grid, 0, p->flags))
         if (o.on && o.dev && o.in != OutStruct::ranked) CU(ctx, (pl->*o.dev).alloc((size_t)o.elems(nw, sumT) * o.elem));
     if (p->flags & HMCGPU_FLAG_RANKED) CU(ctx, pl->rk_keep.alloc((size_t)nw * pl->F * nc * (size_t)p->nrun * sizeof(R)));
+    if ((p->flags & HMCGPU_FLAG_LOO) && !(p->flags & HMCGPU_FLAG_RANKED))
+        CU(ctx, pl->lo_keep.alloc((size_t)nw * (2 * K + K * K) * nc * (size_t)p->nrun * sizeof(R)));
     if (p->flags & HMCGPU_FLAG_ONESTEP) {
         pl->os_n = (long long)nc * sumT;
         CU(ctx, pl->os_state.alloc((size_t)kOsState * pl->os_n * sizeof(double)));
@@ -1854,6 +1879,13 @@ static int plan_run_t(hmcgpu_plan* pl) {
             CU(ctx, cudaGetLastError());
             ++pl->n_launches;
         }
+        if ((pl->flags & HMCGPU_FLAG_LOO) && !(pl->flags & HMCGPU_FLAG_RANKED)) {
+            const int Fl = 2 * Kr + Kr * Kr;                 // mu, sigma2, A: the leading summary fields
+            ranked_keep_kernel<R><<<dim3(pl->n_windows, Fl), dim3(32, 8), 0, st>>>(Fl, ns, pl->chunk, n, d0, pl->nrun, pl->n_chains,
+                                                                                 pl->win_slot0.as<int>(), buf, pl->lo_keep.as<R>());
+            CU(ctx, cudaGetLastError());
+            ++pl->n_launches;
+        }
         if (pl->flags & HMCGPU_FLAG_PREDICTIVE) {
             const int sb = kPredThreads / pl->pr_tg;
             const size_t smem = pred_smem_bytes(Kr, pl->n_h, sb * pl->pr_td);
@@ -1985,6 +2017,18 @@ static int plan_create_impl(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_pla
         if (need > (double)total_b)
             return fail(ctx, HMCGPU_ERR_ALLOC, "HMCGPU_FLAG_ONESTEP keeps %.0f bytes of running state, more than the device's %zu bytes", need, total_b);
     }
+    if (p->flags & HMCGPU_FLAG_LOO) {
+        // the kept mu / sigma2 / A draws (none beyond HMCGPU_FLAG_RANKED's) and one batch of fetch scratch
+        size_t free_b = 0, total_b = 0;
+        CU(ctx, cudaMemGetInfo(&free_b, &total_b));
+        double dates = 0.0;
+        for (int w = 0; w < p->n_windows; ++w) dates += (double)p->win_end[w] - p->win_start[w] + 1;
+        const double R = (double)p->n_chains * (double)p->nrun, per_date = (double)loo_date_bytes((long long)R, p->K, p->precision / 8);
+        const double keep = (p->flags & HMCGPU_FLAG_RANKED) ? 0.0 : (double)p->n_windows * (2 * p->K + p->K * p->K) * R * (p->precision / 8);
+        const double need = keep + std::min(dates, std::max(1.0, std::floor((double)t.loo_scratch / per_date))) * per_date;
+        if (need > (double)total_b)
+            return fail(ctx, HMCGPU_ERR_ALLOC, "HMCGPU_FLAG_LOO needs %.0f bytes of kept draws and fetch scratch, more than the device's %zu bytes", need, total_b);
+    }
     tl_pool = ctx->pool;
     std::unique_ptr<hmcgpu_plan> pl(new hmcgpu_plan());
     pl->ctx = ctx;
@@ -2024,12 +2068,12 @@ extern "C" int hmcgpu_plan_fetch(hmcgpu_plan* pl, hmcgpu_result* r) {
     GUARD(pl->ctx, plan_fetch_impl(pl, r));
 }
 
-// Enqueues the copy of every requested output the plan holds (of r, pr, rk or os) into the caller's arrays; adds the bytes to
-// *bytes (NULL: the predictive, ranked and one-step outputs, which hmcgpu_result's d2h_bytes does not count)
+// Enqueues the copy of every requested output the plan holds (of r, pr, rk, os or lo) into the caller's arrays; adds the bytes
+// to *bytes (NULL: the predictive, ranked, one-step and LOO outputs, which hmcgpu_result's d2h_bytes does not count)
 static int download(hmcgpu_plan* pl, const std::vector<WinOut>& outs, const hmcgpu_result* r, const hmcgpu_predictive* pr,
-                    const hmcgpu_ranked* rk, const hmcgpu_onestep* os, long long* bytes) {
+                    const hmcgpu_ranked* rk, const hmcgpu_onestep* os, const hmcgpu_loo* lo, long long* bytes) {
     for (const WinOut& o : outs) {
-        void* host = o.get(r, pr, rk, os);
+        void* host = o.get(r, pr, rk, os, lo);
         if (!host || !o.dev || !(pl->*o.dev).p) continue;         // (an output of no elements has no buffer)
         const DevBuf& b = pl->*o.dev;
         CU(pl->ctx, cudaMemcpyAsync(host, b.p, b.bytes, cudaMemcpyDeviceToHost, pl->ctx->stream));
@@ -2062,7 +2106,7 @@ static int plan_fetch_impl(hmcgpu_plan* pl, hmcgpu_result* r) {
     if (pl->d_ifc.p) mean_finish_kernel<<<grid_for(nifc, 256), 256, 0, st>>>(nifc, n, pl->d_fcsum.as<double>(), pl->d_ifc.as<double>());
     CU(ctx, cudaGetLastError());
     long long d2h = 0;
-    TRY(download(pl, outs, r, nullptr, nullptr, nullptr, &d2h));
+    TRY(download(pl, outs, r, nullptr, nullptr, nullptr, nullptr, &d2h));
     std::vector<int> ev(pl->n_slots);
     CU(ctx, cudaMemcpyAsync(ev.data(), pl->events.p, ev.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
     d2h += (long long)(ev.size() * sizeof(int));
@@ -2096,7 +2140,7 @@ static int plan_fetch_predictive_impl(hmcgpu_plan* pl, hmcgpu_predictive* pr) {
                                                                               pl->pr_score.as<double>(), pl->d_cdf.as<double>(), pl->d_pit.as<double>(),
                                                                               pl->d_ls.as<double>(), pl->d_mom.as<double>());
     CU(ctx, cudaGetLastError());
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, pr, nullptr, nullptr, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, pr, nullptr, nullptr, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));
     return HMCGPU_OK;
 }
@@ -2203,7 +2247,7 @@ static int fetch_ranked_t(hmcgpu_plan* pl, const hmcgpu_ranked* rk) {
                                                                  pl->d_rrank.as<double>(), pl->d_essb.as<double>(), pl->d_esst.as<double>());
         CU(ctx, cudaGetLastError());
     }
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, nc, pl->nrun, pl->n_grid, rk->n_probs, pl->flags), nullptr, nullptr, rk, nullptr, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, nc, pl->nrun, pl->n_grid, rk->n_probs, pl->flags), nullptr, nullptr, rk, nullptr, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));         // (the scratch goes back to the pool when this returns)
     return HMCGPU_OK;
 }
@@ -2235,7 +2279,7 @@ static int plan_fetch_onestep_impl(hmcgpu_plan* pl, hmcgpu_onestep* os) {
                                                          pl->os_state.as<double>(), pl->os_n, pl->d_ospit.as<double>(),
                                                          pl->d_oslpd.as<double>(), pl->d_osvar.as<double>(), pl->d_waic.as<double>());
     CU(ctx, cudaGetLastError());
-    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, nullptr, nullptr, os, nullptr));
+    TRY(download(pl, window_outputs(pl->K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, nullptr, nullptr, os, nullptr, nullptr));
     CU(ctx, cudaStreamSynchronize(st));
     return HMCGPU_OK;
 }
@@ -2244,6 +2288,73 @@ extern "C" int hmcgpu_plan_fetch_onestep(hmcgpu_plan* pl, hmcgpu_onestep* os) {
     if (!pl) return HMCGPU_ERR_ARG;
     if (!os) return fail(pl->ctx, HMCGPU_ERR_ARG, "hmcgpu_onestep is NULL");
     GUARD(pl->ctx, plan_fetch_onestep_impl(pl, os));
+}
+
+// PSIS-LOO of every date (loo.cuh), in batches of dates whose scratch stays under Tuning::loo_scratch (at least one date).  These
+// launches are not plan_run's: n_launches leaves them out.
+template <typename R>
+static int fetch_loo_t(hmcgpu_plan* pl, const hmcgpu_loo* lo) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    cudaStream_t st = ctx->stream;
+    const int K = pl->K, nw = pl->n_windows;
+    const long long Rd = (long long)pl->n_chains * pl->nrun;
+    const bool rk = pl->flags & HMCGPU_FLAG_RANKED;
+    const R* keep = rk ? pl->rk_keep.as<R>() : pl->lo_keep.as<R>();
+    const int Fs = rk ? pl->F : 2 * K + K * K;
+    long long sumT = 0;
+    for (int w = 0; w < nw; ++w) sumT += pl->wT[w];
+    const size_t per_date = loo_date_bytes(Rd, K, sizeof(R));
+    const long long B = std::max<long long>(1, std::min<long long>(sumT, (long long)(pl->tuning.loo_scratch / per_date)));
+    // the pieces of every batch: batch b covers the dates [b*B, (b+1)*B) of the windows concatenated in caller order
+    std::vector<LooPiece> pieces;
+    std::vector<long long> first{0};
+    for (long long g0 = 0; g0 < sumT; g0 += B) {
+        const long long g1 = std::min(sumT, g0 + B);
+        for (int w = 0; w < nw; ++w) {
+            const long long o = pl->pib_off[w] / K, e = o + pl->wT[w];
+            if (e <= g0 || o >= g1) continue;
+            pieces.push_back({w, (int)(std::max(g0, o) - o), (int)(std::min(g1, e) - o), (int)(std::max(g0, o) - g0)});
+        }
+        first.push_back((long long)pieces.size());
+    }
+    DevBuf dp, ell, F, lb;
+    CU(ctx, dp.alloc(pieces.size() * sizeof(LooPiece)));
+    CU(ctx, cudaMemcpyAsync(dp.p, pieces.data(), pieces.size() * sizeof(LooPiece), cudaMemcpyHostToDevice, st));
+    CU(ctx, ell.alloc((size_t)B * Rd * sizeof(double)));
+    CU(ctx, F.alloc((size_t)B * Rd * sizeof(double)));
+    CU(ctx, lb.alloc((size_t)B * K * Rd * sizeof(R)));
+    const size_t smem = loo_psis_smem(Rd);
+    if (smem > 48 * 1024) CU(ctx, cudaFuncSetAttribute(loo_psis_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (size_t b = 0; b + 1 < first.size(); ++b) {
+        const long long g0 = (long long)b * B, nb = std::min(sumT, g0 + B) - g0;
+        CU(ctx, launch_loo_terms<R>(K, Rd, Fs, (int)(first[b + 1] - first[b]), dp.as<LooPiece>() + first[b], keep, pl->wTd.as<int>(),
+                                    pl->win_slot0.as<int>(), pl->ybase.as<long long>(), pl->args.yld, pl->yr.as<R>(), lb.as<R>(),
+                                    ell.as<double>(), F.as<double>(), st));
+        loo_psis_kernel<<<(unsigned)nb, kLooThreads, smem, st>>>(Rd, g0, ell.as<double>(), F.as<double>(), pl->d_lelpd.as<double>(),
+                                                               pl->d_llppd.as<double>(), pl->d_lpk.as<double>(), pl->d_lpit.as<double>());
+        CU(ctx, cudaGetLastError());
+    }
+    loo_finish_kernel<<<grid_for(nw, 128), 128, 0, st>>>(nw, K, Rd, pl->wTd.as<int>(), pl->win_pib_off.as<long long>(), pl->d_lelpd.as<double>(),
+                                                        pl->d_llppd.as<double>(), pl->d_lpk.as<double>(), pl->d_lsum.as<double>());
+    CU(ctx, cudaGetLastError());
+    TRY(download(pl, window_outputs(K, pl->n_h, pl->n_chains, pl->nrun, pl->n_grid, 0, pl->flags), nullptr, nullptr, nullptr, nullptr, lo, nullptr));
+    CU(ctx, cudaStreamSynchronize(st));         // (the scratch goes back to the pool when this returns)
+    return HMCGPU_OK;
+}
+
+static int plan_fetch_loo_impl(hmcgpu_plan* pl, hmcgpu_loo* lo) {
+    hmcgpu_ctx* ctx = pl->ctx;
+    if (!(pl->flags & HMCGPU_FLAG_LOO)) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_loo on a plan without HMCGPU_FLAG_LOO");
+    if (!pl->ran) return fail(ctx, HMCGPU_ERR_ARG, "plan_fetch_loo before plan_run");
+    CU(ctx, cudaSetDevice(ctx->device));
+    tl_pool = ctx->pool;
+    return pl->precision == 32 ? fetch_loo_t<float>(pl, lo) : fetch_loo_t<double>(pl, lo);
+}
+
+extern "C" int hmcgpu_plan_fetch_loo(hmcgpu_plan* pl, hmcgpu_loo* lo) {
+    if (!pl) return HMCGPU_ERR_ARG;
+    if (!lo) return fail(pl->ctx, HMCGPU_ERR_ARG, "hmcgpu_loo is NULL");
+    GUARD(pl->ctx, plan_fetch_loo_impl(pl, lo));
 }
 
 extern "C" void hmcgpu_plan_destroy(hmcgpu_plan* pl) {
@@ -2268,7 +2379,14 @@ extern "C" int hmcgpu_estimate_ranked(hmcgpu_ctx* ctx, const hmcgpu_problem* p, 
 
 extern "C" int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk,
                                        hmcgpu_onestep* os) {
+    return hmcgpu_estimate_loo(ctx, p, r, pr, rk, os, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_loo(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk,
+                                   hmcgpu_onestep* os, hmcgpu_loo* lo) {
     if (!r) return fail(ctx, HMCGPU_ERR_ARG, "result is NULL");
+    if (p && (p->flags & HMCGPU_FLAG_LOO) && !lo)
+        return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_LOO without hmcgpu_loo outputs (use hmcgpu_estimate_loo)");
     if (p && (p->flags & HMCGPU_FLAG_ONESTEP) && !os)
         return fail(ctx, HMCGPU_ERR_ARG, "HMCGPU_FLAG_ONESTEP without hmcgpu_onestep outputs (use hmcgpu_estimate_onestep)");
     if (p && (p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
@@ -2296,6 +2414,10 @@ extern "C" int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p,
         const int rp = hmcgpu_plan_fetch_onestep(pl, os);
         if (rp < 0) rc = rp;
     }
+    if (rc >= 0 && (p->flags & HMCGPU_FLAG_LOO)) {
+        const int rp = hmcgpu_plan_fetch_loo(pl, lo);
+        if (rp < 0) rc = rp;
+    }
     tr.mark("plan_fetch (download)");
     hmcgpu_plan_destroy(pl);
     tr.mark("plan_destroy");
@@ -2304,7 +2426,7 @@ extern "C" int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p,
 
 // Windows sharded over devices by longest-processing-time-first on T_w; one host thread per device, no collectives.
 static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
-                               hmcgpu_ranked* rk, hmcgpu_onestep* os);
+                               hmcgpu_ranked* rk, hmcgpu_onestep* os, hmcgpu_loo* lo);
 extern "C" int hmcgpu_estimate_multi(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r) {
     return hmcgpu_estimate_multi_ranked(devices, n_dev, p, r, nullptr, nullptr);
 }
@@ -2321,7 +2443,14 @@ extern "C" int hmcgpu_estimate_multi_ranked(const int* devices, int n_dev, const
 
 extern "C" int hmcgpu_estimate_multi_onestep(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
                                              hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os) {
+    return hmcgpu_estimate_multi_loo(devices, n_dev, p, r, pr, rk, os, nullptr);
+}
+
+extern "C" int hmcgpu_estimate_multi_loo(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r,
+                                         hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os, hmcgpu_loo* lo) {
     if (!devices || n_dev < 1 || !p || !r) return fail(nullptr, HMCGPU_ERR_ARG, "bad arguments");
+    if ((p->flags & HMCGPU_FLAG_LOO) && !lo)
+        return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_LOO without hmcgpu_loo outputs (use hmcgpu_estimate_multi_loo)");
     if ((p->flags & HMCGPU_FLAG_ONESTEP) && !os)
         return fail(nullptr, HMCGPU_ERR_ARG, "HMCGPU_FLAG_ONESTEP without hmcgpu_onestep outputs (use hmcgpu_estimate_multi_onestep)");
     if ((p->flags & HMCGPU_FLAG_PREDICTIVE) && !pr)
@@ -2331,11 +2460,12 @@ extern "C" int hmcgpu_estimate_multi_onestep(const int* devices, int n_dev, cons
         TRY(check_ranked(nullptr, rk));
     }
     GUARD(nullptr, estimate_multi_impl(devices, n_dev, p, r, (p->flags & HMCGPU_FLAG_PREDICTIVE) ? pr : nullptr,
-                                       (p->flags & HMCGPU_FLAG_RANKED) ? rk : nullptr, (p->flags & HMCGPU_FLAG_ONESTEP) ? os : nullptr));
+                                       (p->flags & HMCGPU_FLAG_RANKED) ? rk : nullptr, (p->flags & HMCGPU_FLAG_ONESTEP) ? os : nullptr,
+                                       (p->flags & HMCGPU_FLAG_LOO) ? lo : nullptr));
 }
 
 static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr,
-                               hmcgpu_ranked* rk, hmcgpu_onestep* os) {
+                               hmcgpu_ranked* rk, hmcgpu_onestep* os, hmcgpu_loo* lo) {
     if (p->n_windows < 1 || !p->win_start || !p->win_end) return fail(nullptr, HMCGPU_ERR_ARG, "no windows");
     const int nw = p->n_windows;
     std::vector<int> ord(nw);
@@ -2387,19 +2517,20 @@ static int estimate_multi_impl(const int* devices, int n_dev, const hmcgpu_probl
             hmcgpu_predictive pq{};
             hmcgpu_ranked rq{};
             hmcgpu_onestep oq{};
+            hmcgpu_loo lq{};
             if (rk) { rq.probs = rk->probs; rq.n_probs = rk->n_probs; }
             std::vector<std::vector<char>> stage(outs.size());
             for (size_t i = 0; i < outs.size(); ++i) {
-                if (!outs[i].get(r, pr, rk, os)) continue;
+                if (!outs[i].get(r, pr, rk, os, lo)) continue;
                 stage[i].resize(std::max<size_t>(1, (size_t)outs[i].elems(n, sum_T) * outs[i].elem));
-                outs[i].set(&o, &pq, &rq, &oq, stage[i].data());
+                outs[i].set(&o, &pq, &rq, &oq, &lq, stage[i].data());
             }
-            rc = hmcgpu_estimate_onestep(ctx, &q, &o, pr ? &pq : nullptr, rk ? &rq : nullptr, os ? &oq : nullptr);
+            rc = hmcgpu_estimate_loo(ctx, &q, &o, pr ? &pq : nullptr, rk ? &rq : nullptr, os ? &oq : nullptr, lo ? &lq : nullptr);
             rcs[d] = rc;
             if (rc < 0) errs[d] = hmcgpu_last_error(ctx);
             for (size_t i = 0; rc >= 0 && i < outs.size(); ++i) {   // scatter this shard's windows into the caller's arrays
                 const WinOut& x = outs[i];
-                char* dst = (char*)x.get(r, pr, rk, os);
+                char* dst = (char*)x.get(r, pr, rk, os, lo);
                 if (!dst) continue;
                 long long t = 0;                                 // steps of the shard's windows before window j
                 for (int j = 0; j < n; ++j) {

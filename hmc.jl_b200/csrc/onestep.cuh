@@ -44,6 +44,73 @@ template <typename R, int K> struct OsTrans<R, K, true> {
     __device__ __forceinline__ R& at(int r, int s) { return p[(r * K + s) * 32 + lane]; }
 };
 
+// log w in the log base of the plan's precision (log2 in fp32, as the fp32 emission; natural in fp64)
+template <typename R> __device__ __forceinline__ R os_log(R x) {
+    if constexpr (sizeof(R) == 4) return Real<float>::lg2(x);
+    else return log(x);
+}
+
+// log phi(y; mu_s, sigma2_s) in that base
+template <typename R, int K>
+__device__ __forceinline__ R os_log_emission(const Emission<R, K>& em, const R (&lnrm)[K], int s, R y) {
+    if constexpr (sizeof(R) == 4) { const float d = y - em.mu[s]; return fmaf(d * d, em.q[s], em.c[s]); }
+    else { const double z = (y - em.mu[s]) * em.isd[s]; return lnrm[s] - 0.5 * (z * z); }
+}
+
+// One step of the forward filter at y_t from the predictive weights wt = w_t (the step of onestep_accum_kernel, shared with
+// loo_terms_kernel): l[s] = log w_t,s + log phi_s(y_t) in the precision's log base, cdf[s] = Phi(z_t,s),
+// ell = log p(y_t | y_1..t-1) (natural log, fp64), F = sum_s w_t,s cdf[s]; then wt <- w_t+1 = alpha_t A.
+template <typename R, int K, typename Trans>
+__device__ __forceinline__ void os_forward_step(const Emission<R, K>& em, const R (&isd)[K], const R (&lnrm)[K], R yt, R (&wt)[K],
+                                                Trans& A, R (&l)[K], R (&cdf)[K], double& ell, R& F) {
+    R a[K], mx;
+    F = R(0);
+    if constexpr (sizeof(R) == 4) {                  // log2 domain, as the fp32 emission
+#pragma unroll
+        for (int s = 0; s < K; ++s) {
+            const float d = yt - em.mu[s];
+            l[s] = Real<float>::lg2(wt[s]) + fmaf(d * d, em.q[s], em.c[s]);
+            cdf[s] = normcdff(d * isd[s]);
+            F = fmaf(wt[s], cdf[s], F);
+        }
+        mx = l[0];
+#pragma unroll
+        for (int s = 1; s < K; ++s) mx = fmaxf(mx, l[s]);
+        float sum = 0.f;
+#pragma unroll
+        for (int s = 0; s < K; ++s) { a[s] = Real<float>::ex2(l[s] - mx); sum += a[s]; }
+        ell = ((double)mx + (double)Real<float>::lg2(sum)) * 0.6931471805599453;
+        const float inv = Real<float>::rcp(sum);
+#pragma unroll
+        for (int s = 0; s < K; ++s) a[s] *= inv;
+    } else {
+#pragma unroll
+        for (int s = 0; s < K; ++s) {
+            const double z = (yt - em.mu[s]) * isd[s];
+            l[s] = log(wt[s]) + lnrm[s] - 0.5 * (z * z);
+            cdf[s] = normcdf(z);
+            F = fma(wt[s], cdf[s], F);
+        }
+        mx = l[0];
+#pragma unroll
+        for (int s = 1; s < K; ++s) mx = fmax(mx, l[s]);
+        double sum = 0.0;
+#pragma unroll
+        for (int s = 0; s < K; ++s) { a[s] = exp(l[s] - mx); sum += a[s]; }
+        ell = mx + log(sum);
+#pragma unroll
+        for (int s = 0; s < K; ++s) a[s] /= sum;
+    }
+    // a holds the filtered probabilities alpha_t; predict the next date's weights
+#pragma unroll
+    for (int s = 0; s < K; ++s) {
+        R v = a[0] * A.at(0, s);
+#pragma unroll
+        for (int r = 1; r < K; ++r) v = fma(a[r], A.at(r, s), v);
+        wt[s] = v;
+    }
+}
+
 // Adds draws [0, n_i) of a chunk (draws d0 .. d0 + n_i - 1 of every chain) to the running state.  d0 == 0 starts from the empty
 // state (first chunk of a run).
 template <typename R, int K>
@@ -114,51 +181,9 @@ __global__ void __launch_bounds__(32 * os_warps<R, K>()) onestep_accum_kernel(in
             const R yl = (t0 + lane < N) ? ys[(long long)(t0 + lane) * yld] : R(0);
             for (int tt = 0; tt < nt; ++tt) {
                 const R yt = __shfl_sync(0xffffffffu, yl, tt);
-                R l[K], mx;
+                R l[K], cdf[K], F;
                 double ell;
-                R F = R(0);
-                if constexpr (sizeof(R) == 4) {                  // log2 domain, as the fp32 emission
-#pragma unroll
-                    for (int s = 0; s < K; ++s) {
-                        const float d = yt - em.mu[s];
-                        l[s] = Real<float>::lg2(wt[s]) + fmaf(d * d, em.q[s], em.c[s]);
-                        F = fmaf(wt[s], normcdff(d * isd[s]), F);
-                    }
-                    mx = l[0];
-#pragma unroll
-                    for (int s = 1; s < K; ++s) mx = fmaxf(mx, l[s]);
-                    float sum = 0.f;
-#pragma unroll
-                    for (int s = 0; s < K; ++s) { l[s] = Real<float>::ex2(l[s] - mx); sum += l[s]; }
-                    ell = ((double)mx + (double)Real<float>::lg2(sum)) * 0.6931471805599453;
-                    const float inv = Real<float>::rcp(sum);
-#pragma unroll
-                    for (int s = 0; s < K; ++s) l[s] *= inv;
-                } else {
-#pragma unroll
-                    for (int s = 0; s < K; ++s) {
-                        const double z = (yt - em.mu[s]) * isd[s];
-                        l[s] = log(wt[s]) + lnrm[s] - 0.5 * (z * z);
-                        F = fma(wt[s], normcdf(z), F);
-                    }
-                    mx = l[0];
-#pragma unroll
-                    for (int s = 1; s < K; ++s) mx = fmax(mx, l[s]);
-                    double sum = 0.0;
-#pragma unroll
-                    for (int s = 0; s < K; ++s) { l[s] = exp(l[s] - mx); sum += l[s]; }
-                    ell = mx + log(sum);
-#pragma unroll
-                    for (int s = 0; s < K; ++s) l[s] /= sum;
-                }
-                // l now holds the filtered probabilities alpha_t; predict the next date's weights
-#pragma unroll
-                for (int s = 0; s < K; ++s) {
-                    R a = l[0] * A.at(0, s);
-#pragma unroll
-                    for (int r = 1; r < K; ++r) a = fma(l[r], A.at(r, s), a);
-                    wt[s] = a;
-                }
+                os_forward_step<R, K>(em, isd, lnrm, yt, wt, A, l, cdf, ell, F);
                 tl[lane][tt] = bad ? (double)NAN : ell;
                 tF[lane][tt] = bad ? (double)NAN : (double)F;
             }

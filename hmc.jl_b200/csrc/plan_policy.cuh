@@ -40,6 +40,9 @@ struct Tuning {
     int seg_warm = 32, seg_barriers = 2;
     std::optional<long long> scan_max_chains, seg_long;
     std::optional<int> seg_lanes, groups, seg_threads, sweeps_per_launch;
+    // HMCGPU_FLAG_LOO: the fetch scratch of one batch of dates (ell, F and the backward vectors), HMCGPU_LOO_SCRATCH_MB; a smaller
+    // bound only cuts the dates into more batches, whose outputs are the same bit for bit
+    size_t loo_scratch = 4ull << 30;
 };
 inline Tuning read_tuning() {
     Tuning t;
@@ -57,6 +60,7 @@ inline Tuning read_tuning() {
     if ((e = getenv("HMCGPU_SWEEPS_PER_LAUNCH"))) t.sweeps_per_launch = std::max(1, atoi(e));
     if ((e = getenv("HMCGPU_LAUNCH_TIMING"))) t.launch_timing = atoi(e) != 0;
     if ((e = getenv("HMCGPU_VERBOSE"))) t.verbose = atoi(e) != 0;
+    if ((e = getenv("HMCGPU_LOO_SCRATCH_MB"))) t.loo_scratch = (size_t)std::max(1LL, atoll(e)) << 20;
     return t;
 }
 

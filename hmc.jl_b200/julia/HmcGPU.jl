@@ -30,6 +30,7 @@ const FLAG_DIAGNOSTICS = UInt32(128)
 const FLAG_PREDICTIVE = UInt32(256)
 const FLAG_RANKED = UInt32(512)
 const FLAG_ONESTEP = UInt32(1024)
+const FLAG_LOO = UInt32(2048)
 
 # struct hmcgpu_problem (include/hmcgpu.h)
 struct Problem
@@ -67,6 +68,11 @@ end
 # struct hmcgpu_onestep (FLAG_ONESTEP)
 mutable struct Onestep
     pit::Ptr{Float64}; lpd::Ptr{Float64}; lpd_var::Ptr{Float64}; waic::Ptr{Float64}
+end
+
+# struct hmcgpu_loo (FLAG_LOO)
+mutable struct Loo
+    elpd::Ptr{Float64}; lppd::Ptr{Float64}; pareto_k::Ptr{Float64}; pit::Ptr{Float64}; summary::Ptr{Float64}
 end
 
 struct HmcGpuError <: Exception
@@ -114,6 +120,8 @@ Returns per-window arrays in the reference's layouts: μ[w] (R×D), σ[w] (R×D)
 forecasts[w] (R×2|H|) with R = n_chains*Nrun (chain-major).  The output buffers are Julia column-major already
 (hmcgpu_result), so they are wrapped without a copy.  `onestep = true` adds the one-step-ahead scores of every in-sample
 date (hmcgpu_onestep): `onestep_pit[w]`, `lpd[w]` and `lpd_var[w]` (N_w each) and `waic` (4 × nw: lppd, p_waic, elpd_waic, se).
+`loo = true` adds PSIS-LOO of every in-sample date (hmcgpu_loo): `loo_elpd[w]`, `loo_lppd[w]`, `pareto_k[w]` and `loo_pit[w]`
+(N_w each) and `loo` (6 × nw: elpd_loo, se, p_loo, lppd, max k̂, dates with k̂ above the threshold).
 """
 function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{Int32}, win_end::Vector{Int32};
                   D::Int = 3, n_chains::Int = 1, burnin::Int = 1_000, Nrun::Int = 1_000, seed::Integer = 1234,
@@ -122,7 +130,7 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
                   is_signal::Vector{UInt8} = UInt8[], kappa::Float64 = 1.0, pi_row_back::Int = 0,
                   xi::Vector{Float64} = Float64[], alpha::Vector{Float64} = Float64[], nu::Vector{Float64} = Float64[],
                   pred_grid::Vector{Float64} = Float64[], quantile_probs::Vector{Float64} = Float64[],
-                  rank_diagnostics::Bool = false, onestep::Bool = false)
+                  rank_diagnostics::Bool = false, onestep::Bool = false, loo::Bool = false)
     # rawdata: one series (Vector) or y_len × n_series (Matrix, column = series): exactly the library's column-major layout
     y_len, n_series = size(rawdata, 1), size(rawdata, 2)
     ptr_or_null(v) = isempty(v) ? Ptr{eltype(v)}(C_NULL) : pointer(v)
@@ -145,16 +153,23 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
     sumT = onestep ? Int(sum(win_end .- win_start .+ 1)) : 0
     opit = Vector{Float64}(undef, sumT); olpd = similar(opit); ovar = similar(opit); owaic = Array{Float64}(undef, 4, onestep ? nw : 0)
     os = Onestep(ptr_or_null(opit), ptr_or_null(olpd), ptr_or_null(ovar), ptr_or_null(owaic))
+    # PSIS-LOO (loo = true): per date, windows concatenated; summary C [w][6] = Julia 6 × nw
+    sumL = loo ? Int(sum(win_end .- win_start .+ 1)) : 0
+    lelpd = Vector{Float64}(undef, sumL); llppd = similar(lelpd); lpk = similar(lelpd); lpit = similar(lelpd)
+    lsum = Array{Float64}(undef, 6, loo ? nw : 0)
+    lo = Loo(ptr_or_null(lelpd), ptr_or_null(llppd), ptr_or_null(lpk), ptr_or_null(lpit), ptr_or_null(lsum))
     res = Result(pointer(mu), pointer(sig), pointer(A), pointer(pie), nh > 0 ? pointer(fc) : C_NULL, C_NULL,
                  C_NULL, C_NULL, C_NULL, C_NULL, pointer(status), 0.0, 0.0, 0, 0, 0, 0, 0, 0.0, 0, 0,
                  C_NULL, C_NULL, C_NULL)
-    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu pred_grid pcdf pit pls pmom quantile_probs rq rrh reb ret opit olpd ovar owaic begin
+    rc = GC.@preserve rawdata win_start win_end horizons mu sig A pie fc status win_series win_init_series is_signal xi alpha nu pred_grid pcdf pit pls pmom quantile_probs rq rrh reb ret opit olpd ovar owaic lelpd llppd lpk lpit lsum begin
         prob = Problem(pointer(rawdata), y_len, n_series, nw, ptr_or_null(win_series), pointer(win_start), pointer(win_end), C_NULL,
                        D, n_chains, burnin, Nrun, UInt64(seed), ptr_or_null(xi), ptr_or_null(alpha), ptr_or_null(nu), C_NULL, C_NULL,
                        kappa, ptr_or_null(is_signal), pointer(horizons), nh, C_NULL, precision,
                        FLAG_REF_Q1 | FLAG_DRAWS | (ng > 0 ? FLAG_PREDICTIVE : UInt32(0)) | (ranked ? FLAG_RANKED : UInt32(0)) |
-                       (onestep ? FLAG_ONESTEP : UInt32(0)),
+                       (onestep ? FLAG_ONESTEP : UInt32(0)) | (loo ? FLAG_LOO : UInt32(0)),
                        ptr_or_null(win_init_series), pi_row_back, 0, ptr_or_null(pred_grid), ng)
+        loo ? ccall((:hmcgpu_estimate_loo, LIB), Cint,
+                    (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}, Ref{Onestep}, Ref{Loo}), ctx.h, prob, res, pred, rk, os, lo) :
         onestep ? ccall((:hmcgpu_estimate_onestep, LIB), Cint,
                         (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}, Ref{Onestep}), ctx.h, prob, res, pred, rk, os) :
                   ccall((:hmcgpu_estimate_ranked, LIB), Cint, (Ptr{Cvoid}, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}),
@@ -162,11 +177,12 @@ function estimate(ctx::Context, rawdata::VecOrMat{Float64}, win_start::Vector{In
     end
     rc < 0 && throw(HmcGpuError(rc, lasterror(ctx)))
     offs = cumsum(vcat(0, Int.(win_end .- win_start .+ 1)))
-    per_window(v) = onestep ? [v[offs[w] + 1:offs[w + 1]] for w in 1:nw] : Vector{Float64}[]
+    per_window(v) = !isempty(v) ? [v[offs[w] + 1:offs[w + 1]] for w in 1:nw] : Vector{Float64}[]
     return (μ = mu, σ = sig, A = A, πbend = pie, forecasts = fc, status = status, events = rc, gpu_ms = res.gpu_ms,
             pred_cdf = pcdf, pit = pit, log_score = pls, pred_moments = pmom,
             quantiles = rq, rhat_rank = rrh, ess_bulk = reb, ess_tail = ret,
-            onestep_pit = per_window(opit), lpd = per_window(olpd), lpd_var = per_window(ovar), waic = owaic)
+            onestep_pit = per_window(opit), lpd = per_window(olpd), lpd_var = per_window(ovar), waic = owaic,
+            loo_elpd = per_window(lelpd), loo_lppd = per_window(llppd), pareto_k = per_window(lpk), loo_pit = per_window(lpit), loo = lsum)
 end
 
 # The multi-GPU form over caller-built structs (hmcgpu_estimate_multi_ranked): windows sharded over `devices`, every output
@@ -185,6 +201,23 @@ function estimate_multi_onestep(devices::Vector{Cint}, prob::Problem, res::Resul
                devices, length(devices), prob, res, pred, rk, os)
     rc < 0 && throw(HmcGpuError(rc, unsafe_string(ccall((:hmcgpu_last_error, LIB), Cstring, (Ptr{Cvoid},), C_NULL))))
     return rc
+end
+
+# The same with the PSIS-LOO outputs (hmcgpu_estimate_multi_loo); estimate_multi_onestep is this with lo = NULL.
+function estimate_multi_loo(devices::Vector{Cint}, prob::Problem, res::Result, pred::Predictive, rk::Ranked, os::Onestep, lo::Loo)
+    rc = ccall((:hmcgpu_estimate_multi_loo, LIB), Cint,
+               (Ptr{Cint}, Cint, Ref{Problem}, Ref{Result}, Ref{Predictive}, Ref{Ranked}, Ref{Onestep}, Ref{Loo}),
+               devices, length(devices), prob, res, pred, rk, os, lo)
+    rc < 0 && throw(HmcGpuError(rc, unsafe_string(ccall((:hmcgpu_last_error, LIB), Cstring, (Ptr{Cvoid},), C_NULL))))
+    return rc
+end
+
+# The PSIS-LOO outputs of the last run of a plan (hmcgpu_plan_fetch_loo), computed from the kept draws.  `ctx` is the plan's
+# context.
+function plan_fetch_loo!(ctx::Context, plan::Ptr{Cvoid}, lo::Loo)
+    rc = ccall((:hmcgpu_plan_fetch_loo, LIB), Cint, (Ptr{Cvoid}, Ref{Loo}), plan, lo)
+    rc < 0 && throw(HmcGpuError(rc, lasterror(ctx)))
+    return lo
 end
 
 # The one-step-ahead scores of the last run of a plan (hmcgpu_plan_fetch_onestep).  `ctx` is the plan's context.

@@ -65,6 +65,9 @@ extern "C" {
 #define HMCGPU_FLAG_ONESTEP  1024u   /* fill hmcgpu_onestep: the one-step-ahead posterior predictive PIT and log density of every date
                                         of every window, and WAIC per window, computed on the device from every saved draw; K <= 8,
                                         no is_signal, n_chains * nrun >= 2 (see hmcgpu_onestep) */
+#define HMCGPU_FLAG_LOO  2048u       /* fill hmcgpu_loo: PSIS-LOO of every date of every window (leave-one-out predictive density,
+                                        Pareto k̂, LOO-PIT) and its per-window sums, computed at fetch from the mu / sigma2 / A draws
+                                        kept on the device; K <= 8, no is_signal, 2 <= n_chains * nrun <= 2^24 (see hmcgpu_loo) */
 
 typedef struct hmcgpu_ctx hmcgpu_ctx;
 typedef struct hmcgpu_plan hmcgpu_plan;
@@ -263,6 +266,53 @@ typedef struct hmcgpu_onestep {
     double* waic;         /* [n_windows][4]: lppd, p_waic, elpd_waic, se */
 } hmcgpu_onestep;
 
+/* Pareto-smoothed importance-sampling leave-one-out cross-validation of the in-sample dates (HMCGPU_FLAG_LOO; Vehtari, Gelman &
+ * Gabry 2017); caller-allocated, any pointer may be NULL.  For window w with N = N_w dates y_1..y_N (its own series, from
+ * win_start) and each saved draw d (mu_s, sigma2_s, A[r][s], fields 0 .. 2K + K^2 - 1 of the summary order), from the UNIFORM
+ * initial distribution as the one-step scores do, so that rho is integrated out:
+ *   forward   w_1,s = 1/K,  alpha_t proportional to w_t phi(y_t),  w_t+1 = alpha_t A          (the one-step filter)
+ *   backward  b_N,s = 1,    b_t,r = sum_s A[r][s] phi_s(y_t+1) b_t+1,s   (any positive rescaling per t; log domain)
+ *   ell_t,d = log sum_s w_t,s phi_s(y_t) b_t,s - log sum_s w_t,s b_t,s = log p(y_t | y_-t, theta_d)
+ *   F_t,d   = sum_s q_t,s Phi((y_t - mu_s) / sigma_s),  q_t,s = w_t,s b_t,s / sum_r w_t,r b_t,r
+ * This is the exact leave-one-out term of the HMM, not the one-step term (y_t also conditions every later date); at t = N,
+ * b = 1 and ell_N,d is the one-step term of hmcgpu_onestep.
+ * PSIS per date on the log ratios r_d = -ell_t,d over the R = n_chains*nrun draws (the algorithm of the R package loo 2.x,
+ * do_psis_i / psis_smooth_tail / gpdfit with wip = TRUE and min_grid_pts = 30, r_eff = 1):
+ *   1. M = ceil(min(0.2 R, 3 sqrt(R))), lw = r - max r;
+ *   2. lw sorted ascending, ties broken by the draw index d = chain*nrun + i;
+ *   3. if M >= 5 and the M largest values are not all equal (spread >= DBL_EPSILON/100): cutoff = the largest value below the
+ *      tail; a generalised Pareto distribution is fitted to x_j = exp(tail_j) - exp(cutoff) by Zhang & Stephens (grid of
+ *      30 + floor(sqrt(M)) points, prior 3, x* = x_(floor(M/4 + 1/2)), 1-based), k <- (M k + 5) / (M + 10), NaN k -> +inf; with
+ *      k finite, tail_j <- log(sigma expm1(-k log1p(-p_j)) / k + exp(cutoff)), p_j = (j - 1/2) / M;
+ *   4. otherwise k = +inf and the tail is left as it was;
+ *   5. lw <- min(lw, 0), W_d = exp(lw_d) / sum exp(lw).
+ * Per date (windows concatenated, window w at offset sum_{v<w} N_v, like pib_mean):
+ *   elpd[off_w + t]     = log sum_d W_d exp(ell_t,d)
+ *   lppd[off_w + t]     = log((1/R) sum_d exp(ell_t,d))
+ *   pareto_k[off_w + t] = k
+ *   pit[off_w + t]      = sum_d W_d F_t,d                                         (the LOO-PIT)
+ * Per window, t ascending: summary[w*6 + 0..5] = elpd_loo = sum_t elpd_t, se = sqrt(N var_t(elpd_t)) (denominator N - 1),
+ * p_loo = sum_t (lppd_t - elpd_t), lppd = sum_t lppd_t, max_t k_t, and the number of dates with k_t > min(1 - 1/log10(R), 0.7)
+ * (as a double; above it a date's estimate is unreliable).
+ * A window with a non-finite mu / sigma2 / A draw gets NaN in every output.  The filters run in the plan's precision (as the chain
+ * that produced the draw) and stay finite for an observation 50 sd from every state mean; everything after ell and F is fp64, and
+ * every sum runs in a fixed order with no atomics: a window's outputs are bit-identical however the windows are batched, chunked
+ * or sharded.  Needs K <= 8, no is_signal and 2 <= R <= 2^24 (the tail of up to 12 288 values and their draw indices sits in
+ * shared memory); pi_row_back is allowed.
+ * Memory: plan_run keeps mu, sigma2 and A of every saved draw, n_windows (2K + K^2) R values in the plan's precision (C2 fp32,
+ * K = 3: 500 x 15 x 256 000 x 4 B = 7.7 GB); with HMCGPU_FLAG_RANKED its retained draws serve and nothing more is kept.
+ * hmcgpu_plan_fetch_loo recomputes the terms in batches of dates whose scratch, R (16 + K * precision/8) bytes per date (ell and F
+ * in fp64, the backward vectors in the plan's precision), stays under 4 GiB (HMCGPU_LOO_SCRATCH_MB; at least one date).  Kept draws plus one batch are
+ * checked against the device's total memory at hmcgpu_plan_create (HMCGPU_ERR_ALLOC).  Not estimated: r_eff (the draws are
+ * treated as independent), the Monte Carlo error of elpd_loo, and moment matching or refits of the dates with a large k. */
+typedef struct hmcgpu_loo {
+    double* elpd;         /* [sum_w N_w] */
+    double* lppd;         /* [sum_w N_w] */
+    double* pareto_k;     /* [sum_w N_w] */
+    double* pit;          /* [sum_w N_w] */
+    double* summary;      /* [n_windows][6]: elpd_loo, se, p_loo, lppd, max k, dates with k above the threshold */
+} hmcgpu_loo;
+
 #define HMCGPU_KERNEL_THREAD 0  /* one thread per chain (gibbs_sweeps_kernel), wide batches, K <= 8 */
 #define HMCGPU_KERNEL_SCAN 1    /* one warp per chain, time-parallel scans (gibbs_scan_kernel), narrow batches */
 #define HMCGPU_KERNEL_LANE 2    /* one lane per state (gibbs_wide_kernel), K = 9..32 */
@@ -307,6 +357,12 @@ int hmcgpu_estimate_onestep(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_res
                             hmcgpu_onestep* os);
 int hmcgpu_estimate_multi_onestep(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
                                   hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os);
+/* The same filling the PSIS-LOO outputs too (hmcgpu_estimate_onestep and hmcgpu_estimate_multi_onestep are these with
+ * lo = NULL).  With HMCGPU_FLAG_LOO, lo must not be NULL (HMCGPU_ERR_ARG); without it lo is ignored. */
+int hmcgpu_estimate_loo(hmcgpu_ctx* ctx, const hmcgpu_problem* p, hmcgpu_result* r, hmcgpu_predictive* pr, hmcgpu_ranked* rk,
+                        hmcgpu_onestep* os, hmcgpu_loo* lo);
+int hmcgpu_estimate_multi_loo(const int* devices, int n_devices, const hmcgpu_problem* p, hmcgpu_result* r,
+                              hmcgpu_predictive* pr, hmcgpu_ranked* rk, hmcgpu_onestep* os, hmcgpu_loo* lo);
 
 /* Split form: create uploads inputs and allocates device state; run executes every sweep (inputs resident
  * in HBM, no host transfers); fetch copies the requested outputs back.  run may be repeated (it restarts
@@ -322,6 +378,9 @@ int hmcgpu_plan_fetch_predictive(hmcgpu_plan* plan, hmcgpu_predictive* pr);
 int hmcgpu_plan_fetch_ranked(hmcgpu_plan* plan, hmcgpu_ranked* rk);
 /* One-step-ahead scores of the last run; HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_ONESTEP or before a run. */
 int hmcgpu_plan_fetch_onestep(hmcgpu_plan* plan, hmcgpu_onestep* os);
+/* PSIS-LOO outputs of the last run, computed now from the kept draws; HMCGPU_ERR_ARG on a plan without HMCGPU_FLAG_LOO or
+ * before a run. */
+int hmcgpu_plan_fetch_loo(hmcgpu_plan* plan, hmcgpu_loo* lo);
 void hmcgpu_plan_destroy(hmcgpu_plan* plan);
 
 /* Forward filter for fixed parameters.  y: [T] shared by the batch (y_batch_stride = 0) or [B][T]
